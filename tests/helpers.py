@@ -56,7 +56,9 @@ KINK = 2e-5
 def gpu_relu_masks(model, out, r_rows, p_rows, hidden, depth, ddepth, ffn_depth=3):
     """The ReLU masks the GPU forward behind ``out`` used, in the order the oracle calls ``torch.relu`` (mpn_forward(r), mpn_forward(p),
     mpndiff_forward, ffn_forward), read from the activations saved in the autograd node's workspace.  Call BEFORE ``backward()`` (the
-    workspace is recycled afterwards); needs dropout 0 (a dropped entry would look like a masked one).
+    workspace is recycled afterwards); needs dropout 0 (a dropped entry would look like a masked one).  With dropout, use
+    tests/test_gpu_dropout.py::relu_masks_and_keeps, which pairs each mask with the host-regenerated keep mask of its site and passes
+    both to forced_relu_masks(masks, keeps=...).
     r_rows / p_rows = (n_atoms, n_bonds) of the two batches, padding rows included."""
     from reactranker_b200 import _lib
     hp = _lib.lib().rr_padded(hidden)
@@ -83,19 +85,26 @@ def gpu_relu_masks(model, out, r_rows, p_rows, hidden, depth, ddepth, ffn_depth=
 class forced_relu_masks:
     """Context manager: while active, the i-th ``torch.relu`` call (the oracle's) multiplies by ``masks[i]`` instead of [x > 0].
     Every entry where the forced mask differs from the oracle's own must lie within ``kink`` (relative to its row's largest
-    magnitude) of zero -- i.e. the GPU's forward error, not a wrong value, decided it.  ``flips`` counts them."""
+    magnitude) of zero -- i.e. the GPU's forward error, not a wrong value, decided it.  ``flips`` counts them.
+    ``keeps`` (optional, parallel to ``masks``; an entry may be None): where keeps[i] is False the entry was dropped by dropout, the GPU's
+    activation is 0 whatever its ReLU decided, and the oracle keeps its own decision there (it is multiplied by 0 afterwards)."""
 
-    def __init__(self, masks, kink=KINK):
+    def __init__(self, masks, kink=KINK, keeps=None):
         self.masks, self.kink, self.i, self.flips, self.worst = masks, kink, 0, 0, 0.0
+        self.keeps = keeps
 
     def __enter__(self):
         self._orig = torch.relu
 
         def relu(x):
             m = self.masks[self.i].to(x.device)
+            keep = self.keeps[self.i] if self.keeps is not None else None
             self.i += 1
             assert tuple(m.shape) == tuple(x.shape), (self.i - 1, tuple(m.shape), tuple(x.shape))
-            diff = m != (x.detach() > 0)
+            own = x.detach() > 0
+            if keep is not None:
+                m = torch.where(keep.to(x.device), m, own)
+            diff = m != own
             if bool(diff.any()):
                 rel = (x.detach().abs() / x.detach().abs().amax(dim=-1, keepdim=True).clamp_min(1e-300))[diff]
                 self.flips += int(diff.sum())
