@@ -15,9 +15,11 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 from oracle import ref_loader  # noqa: E402
 from reactranker_b200 import synthetic  # noqa: E402
+from helpers import add_features  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
 os.makedirs(OUT, exist_ok=True)
@@ -27,12 +29,13 @@ def np_sd(sd):
     return {k: v.detach().cpu().numpy().copy() for k, v in sd.items()}   # copy: Adam updates in place
 
 
-def build_ref_model(hidden, task_num, ffn_last_layer, task_type, seed, depth=3, diff_depth=3, dropout=0.0, dtype=torch.float32):
+def build_ref_model(hidden, task_num, ffn_last_layer, task_type, seed, depth=3, diff_depth=3, dropout=0.0, dtype=torch.float32,
+                    ffn_depth=3, use_bias=True, add_features_dim=1):
     bm = ref_loader.ref("models.base_model")
     torch.manual_seed(seed)
-    model = bm.build_model(hidden_size=hidden, mpnn_depth=depth, mpnn_diff_depth=diff_depth, ffn_depth=3,
-                           use_bias=True, dropout=dropout, task_num=task_num, ffn_last_layer=ffn_last_layer,
-                           task_type=task_type, add_features_dim=1)
+    model = bm.build_model(hidden_size=hidden, mpnn_depth=depth, mpnn_diff_depth=diff_depth, ffn_depth=ffn_depth,
+                           use_bias=use_bias, dropout=dropout, task_num=task_num, ffn_last_layer=ffn_last_layer,
+                           task_type=task_type, add_features_dim=add_features_dim)
     return model.to(dtype)
 
 
@@ -183,16 +186,19 @@ def golden_planner():
     print("planner.npz", len(out))
 
 
-def run_case(task, hidden, seed, sizes, star, dtype, depth=3, diff_depth=3):
+def run_case(task, hidden, seed, sizes, star, dtype, depth=3, diff_depth=3, ffn_depth=3, use_bias=True, add_features_dim=1):
+    """The reference's forward, loss and backward on a synthetic batch.  The add features are the temperature column and, beyond the
+    first, seeded normal columns (helpers.add_features); none for add_features_dim = 0."""
     ds, fz = dataset_case(seed, sizes, star)
     tn, last, tt = TASKS_ALL[task]
-    model = build_ref_model(hidden, tn, last, tt, seed=seed, depth=depth, diff_depth=diff_depth, dtype=dtype)
+    model = build_ref_model(hidden, tn, last, tt, seed=seed, depth=depth, diff_depth=diff_depth, dtype=dtype, ffn_depth=ffn_depth,
+                            use_bias=use_bias, add_features_dim=add_features_dim)
     model.train()
     reactions = np.stack([ds.rsmi, ds.psmi], axis=1)
     r_g, p_g = fz.parsing_reactions(reactions)
     for g in (r_g, p_g):                     # let the reference run in fp64 too
         g.f_atoms, g.f_bonds = g.f_atoms.to(dtype), g.f_bonds.to(dtype)
-    feats = ds.temp.reshape(-1, 1)
+    feats = add_features(ds, add_features_dim)
     if dtype == torch.float64:
         # mpn.py:183 casts add_features with FloatTensor (fp32); lift the result to fp64
         orig = torch.FloatTensor

@@ -21,6 +21,57 @@ def sd_from_golden(g, prefix, dtype=torch.float32):
     return {k[len(pre):]: torch.tensor(g[k]).to(dtype) for k in g.files if k.startswith(pre)}
 
 
+def add_features(ds, add):
+    """The ``add_features`` of a synthetic batch for a model built with ``add_features_dim = add``: none for 0, the temperature column
+    for 1 (the reference's setting), and seeded standard-normal columns after it for more."""
+    if add == 0:
+        return None
+    rng = np.random.default_rng(add)
+    return np.concatenate([ds.temp.reshape(-1, 1), rng.standard_normal((len(ds.temp), add - 1))], axis=1)
+
+
+# Model configurations outside the shape the other parity tests build (ffn_depth 3, biases, one add feature, equal depths), each taking
+# code that only it runs: the FFN as one Linear / with a third hidden layer; no W_i / W_h / FFN biases (W_o keeps its own); no encoder
+# W_h (depth 1) / no diff-encoder W_h (diff depth 1); unequal depths; no add features; add features beyond the padded hidden width
+# (hidden 302 + 3 -> vp 320); multi-column raw heads up to RR_OUT_LD; the narrowest padded width (hidden 8 -> 16); hidden > 1024, where the
+# message-passing row pipeline declines; molecules of one to three atoms (no bonds, in-degree 0, a batch whose only bond row is padding);
+# >= 256 reactions, where the FFN weight gradients go to the tensor cores.
+CONFIG_DEFAULTS = dict(hidden=40, depth=3, ddepth=3, ffn_depth=3, use_bias=True, add=1, task_num=1, sizes=(7, 5, 9, 4), atoms=(12, 28))
+CONFIGS = {
+    "ffn1_raw3": dict(ffn_depth=1, task_num=3),
+    "ffn4": dict(ffn_depth=4),
+    "nobias": dict(use_bias=False),
+    "depth1": dict(depth=1),
+    "diff_depth1": dict(ddepth=1),
+    "depth2_diff4": dict(depth=2, ddepth=4),
+    "add0": dict(add=0),
+    "raw16": dict(task_num=16),
+    "h8": dict(hidden=8),
+    "h1040": dict(hidden=1040, depth=2, ddepth=2, sizes=(3, 2, 4)),
+    "tiny_mols": dict(atoms=(1, 3), sizes=(5, 4, 6, 3, 5)),
+    "one_atom_mols": dict(atoms=(1, 1), sizes=(4, 3)),
+    "h302_add3_n320": dict(hidden=302, add=3, atoms=(3, 6), sizes=(40,) * 8),
+}
+
+
+def config(name):
+    """CONFIGS[name] with the defaults filled in."""
+    return dict(CONFIG_DEFAULTS, **CONFIGS[name])
+
+
+def config_model(c, dropout=0.0):
+    """build_model for a filled-in configuration (head: the raw output, ffn_last_layer 'with_softplus' with task_type None)."""
+    from reactranker_b200.models.base_model import build_model
+    return build_model(hidden_size=c["hidden"], mpnn_depth=c["depth"], mpnn_diff_depth=c["ddepth"], ffn_depth=c["ffn_depth"],
+                       use_bias=c["use_bias"], dropout=dropout, task_num=c["task_num"], ffn_last_layer="with_softplus",
+                       add_features_dim=c["add"])
+
+
+def config_dataset(c, seed=61):
+    ds = synthetic.make_dataset(seed, list(c["sizes"]), atoms_lo=c["atoms"][0], atoms_hi=c["atoms"][1])
+    return ds, add_features(ds, c["add"])
+
+
 def rel_err(a, b):
     a = np.asarray(a, np.float64)
     b = np.asarray(b, np.float64)

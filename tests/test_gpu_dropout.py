@@ -19,7 +19,7 @@ from reactranker_b200 import _lib, synthetic
 from reactranker_b200.features.featurization import BatchMolGraph, DeviceGraph
 from reactranker_b200.models.base_model import build_model
 from reactranker_b200.train import loss as RL
-from helpers import TOL, forced_relu_masks, grads_close, rel_err
+from helpers import KINK, TOL, add_features, forced_relu_masks, grads_close, rel_err
 
 GPU = 0
 DEV = "cuda:0"
@@ -312,7 +312,7 @@ def relu_masks_and_keeps(buf, keeps, lay, depth, ddepth, ffn_depth=3):
     return masks, kps
 
 
-def check_sites(buf, keeps, seed, p, lay, hidden, hp, vp, ids):
+def check_sites(buf, keeps, seed, p, lay, hidden, hp, vp, ids, add=1):
     """Nothing the host mask drops survives in the GPU's activations.  On a miss, name the stream ids in 1..64 whose mask the site's zero
     pattern does fit, so that a change of the launch schedule is told apart from a wrong counter."""
     for name, keep in keeps.items():
@@ -320,7 +320,7 @@ def check_sites(buf, keeps, seed, p, lay, hidden, hp, vp, ids):
         bad = (got != 0) & ~keep
         if not bool(bad.any()):
             continue
-        cols, ld = (hidden + 1, vp) if name == "vec" else (hidden, hp)
+        cols, ld = (hidden + add, vp) if name == "vec" else (hidden, hp)
         base = name.split(".")[-1]
         joint = name.startswith("enc")
         sid_key = f"enc.{base}" if joint else name
@@ -332,10 +332,11 @@ def check_sites(buf, keeps, seed, p, lay, hidden, hp, vp, ids):
                     f"stream ids in 1..64 whose mask fits: {fits}")
 
 
-def run_oracle(monkeypatch, sd, groups, drop_keeps, p, depth, ddepth, head, loss_fn, relu=None):
+def run_oracle(monkeypatch, sd, groups, drop_keeps, p, depth, ddepth, head, loss_fn, relu=None, ffn_depth=3, kink=KINK):
     """fp64 oracle forward (one per group) + loss + backward, ``_drop`` multiplying by the host keep masks / (1 - p) in call order; with
-    ``relu`` = (masks, keeps) the kept entries' ReLU decisions are the GPU's (helpers.forced_relu_masks asserts each differing one sits on
-    a kink).  Returns (scores, loss, {name: gradient}, [every _drop output in call order], flips)."""
+    ``relu`` = (masks, keeps) the kept entries' ReLU decisions are the GPU's (helpers.forced_relu_masks asserts each differing one sits
+    within ``kink`` of a kink).  Returns (scores, loss, {name: gradient}, [every _drop output in call order], flips, the largest relative
+    pre-activation of a differing decision)."""
     sd64 = {k: v.double().cpu() for k, v in sd.items()}
     params = {k: v.clone().requires_grad_(True) for k, v in sd64.items() if "cached_zero" not in k}
     full = dict(sd64)
@@ -351,34 +352,38 @@ def run_oracle(monkeypatch, sd, groups, drop_keeps, p, depth, ddepth, head, loss
     monkeypatch.setattr(O, "_drop", drop)
 
     def fwd():
-        return torch.cat([O.model_forward(full, r, q, f, mpnn_depth=depth, mpnn_diff_depth=ddepth, head=head, dropout=p, training=True)
-                          for r, q, f in groups])
-    flips = 0
+        return torch.cat([O.model_forward(full, r, q, f, mpnn_depth=depth, mpnn_diff_depth=ddepth, ffn_depth=ffn_depth, head=head, dropout=p,
+                                          training=True) for r, q, f in groups])
+    flips, worst = 0, 0.0
     if relu is None:
         scores = fwd()
     else:
-        with forced_relu_masks(relu[0], keeps=relu[1]) as fm:
+        with forced_relu_masks(relu[0], kink=kink, keeps=relu[1]) as fm:
             scores = fwd()
-        flips = fm.flips
+        flips, worst = fm.flips, fm.worst
     monkeypatch.undo()
     assert next(it, None) is None
     loss = loss_fn(scores)
     loss.backward(torch.ones_like(loss))
-    return scores.detach().numpy(), loss.detach().numpy(), {k: v.grad.numpy() for k, v in params.items()}, outs, flips
+    return scores.detach().numpy(), loss.detach().numpy(), {k: v.grad.numpy() for k, v in params.items()}, outs, flips, worst
 
 
 BENCH_TOL = {0: dict(max_rel=4e-3, l2=2e-3), 1: dict(max_rel=2.5e-2, l2=6e-3)}     # as test_gpu_model.py::BENCH_TOL
 
 
-def step_vs_oracle(monkeypatch, gemm_mode, *, task, hidden, depth, p, mols, feats, gpu_loss, oracle_loss, last="with_softplus", bench=False):
+def step_vs_oracle(monkeypatch, gemm_mode, *, task, hidden, depth, p, mols, feats, gpu_loss, oracle_loss, last="with_softplus", bench=False,
+                   ddepth=None, ffn_depth=3, use_bias=True, add=1, score_tol=None, kink=KINK):
     """One training step with dropout p on the GPU and the fp64 oracle under the same dropout masks (see the module docstring).
-    ``mols``: [(reactant molecules, product molecules)] per group; several groups run as the segments of one launch."""
+    ``mols``: [(reactant molecules, product molecules)] per group; several groups run as the segments of one launch.  ``ddepth``
+    defaults to ``depth``; ``feats`` must have ``add`` columns.  ``score_tol`` (default TOL[gemm_mode]['score']) bounds the scores and the
+    saved activations, ``kink`` the pre-activation of a ReLU decision the GPU takes differently.  Returns the measured figures."""
     tn, tt = {"mle": (1, None), "evidential_ranking": (2, "evidential_ranking")}[task]
+    ddepth = depth if ddepth is None else ddepth
     L = _lib.lib()
-    hp, vp = L.rr_padded(hidden), L.rr_padded(hidden + 1)
+    hp, vp = L.rr_padded(hidden), L.rr_padded(hidden + add)
     torch.manual_seed(3)
-    model = build_model(hidden_size=hidden, mpnn_depth=depth, mpnn_diff_depth=depth, ffn_depth=3, use_bias=True, dropout=p, task_num=tn,
-                        ffn_last_layer=last, task_type=tt, add_features_dim=1).cuda(GPU).train()
+    model = build_model(hidden_size=hidden, mpnn_depth=depth, mpnn_diff_depth=ddepth, ffn_depth=ffn_depth, use_bias=use_bias, dropout=p,
+                        task_num=tn, ffn_last_layer=last, task_type=tt, add_features_dim=add).cuda(GPU).train()
     sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
     r_batches, p_batches = [BatchMolGraph(r) for r, _ in mols], [BatchMolGraph(q) for _, q in mols]
     lay = Layout(r_batches, p_batches)
@@ -391,11 +396,11 @@ def step_vs_oracle(monkeypatch, gemm_mode, *, task, hidden, depth, p, mols, feat
     out = model(rg, pg, gpu=GPU, add_features=feats)
     seed = int(out.grad_fn.cfg.seed)
     assert seed != 0
-    ids = stream_ids(depth, depth)
-    keeps = site_keeps(seed, p, hidden, depth, depth, lay, hp, vp, ids)
-    buf = saved_buffers(model, out, lay, hidden, depth, depth)
-    check_sites(buf, keeps, seed, p, lay, hidden, hp, vp, ids)
-    relu = relu_masks_and_keeps(buf, keeps, lay, depth, depth)
+    ids = stream_ids(depth, ddepth, ffn_depth)
+    keeps = site_keeps(seed, p, hidden, depth, ddepth, lay, hp, vp, ids, add, ffn_depth)
+    buf = saved_buffers(model, out, lay, hidden, depth, ddepth, add, ffn_depth)
+    check_sites(buf, keeps, seed, p, lay, hidden, hp, vp, ids, add)
+    relu = relu_masks_and_keeps(buf, keeps, lay, depth, ddepth, ffn_depth)
     loss = gpu_loss(out)
     loss.backward()
     got = {k: q.grad.double().cpu().numpy() for k, q in model.named_parameters() if q.requires_grad}
@@ -403,14 +408,17 @@ def step_vs_oracle(monkeypatch, gemm_mode, *, task, hidden, depth, p, mols, feat
     head = O.resolve_task_type(tn, last, tt)
     groups, drops, names = [], [], []
     for grp, (r, q) in zip(lay.groups, mols):
-        groups.append((O.OracleBatch(r), O.OracleBatch(q), feats[grp["m"]]))
-        for name, rows in site_order(depth, depth):
+        groups.append((O.OracleBatch(r), O.OracleBatch(q), None if feats is None else feats[grp["m"]]))
+        for name, rows in site_order(depth, ddepth, ffn_depth):
             if name in keeps:
                 drops.append(keeps[name][grp[rows]])
                 names.append((name, rows, grp))
-    ws, wl, wg, outs, flips = run_oracle(monkeypatch, sd, groups, drops, p, depth, depth, head, oracle_loss, relu)
+    ws, wl, wg, outs, flips, kink_seen = run_oracle(monkeypatch, sd, groups, drops, p, depth, ddepth, head, oracle_loss, relu, ffn_depth, kink)
 
-    tol = TOL[gemm_mode]
+    tol = dict(TOL[gemm_mode])
+    if score_tol is not None:
+        tol["score"] = score_tol
+    measured = dict(flips=flips, worst_kink=kink_seen, act_rel={})
     # every saved activation a dropout acted on, padding rows included: same zero pattern (nothing the host drops survives: check_sites;
     # every kept ReLU decision on a kink: forced_relu_masks) and the same values
     per_site = {}
@@ -420,8 +428,10 @@ def step_vs_oracle(monkeypatch, gemm_mode, *, task, hidden, depth, p, mols, feat
         want = torch.cat([y for _, y in parts])
         gotb = torch.cat([buf[name][s] for s, _ in parts]).double()
         assert torch.equal(gotb != 0, want != 0), (name, int(((gotb != 0) != (want != 0)).sum()))
+        measured["act_rel"][name] = rel_err(gotb, want)
         assert rel_err(gotb, want) < tol["score"], (name, rel_err(gotb, want))
     e_s, e_l = rel_err(out.detach().cpu().numpy(), ws), rel_err(loss.detach().cpu().numpy(), wl)
+    measured.update(score_rel=e_s, loss_rel=e_l)
     assert e_s < tol["score"] and e_l < tol["loss"], (e_s, e_l)
     gscale = max(float(np.abs(v).max()) for v in wg.values())
     live = {k: wg[k] for k in got if float(np.abs(wg[k]).max()) >= 1e-6 * gscale}
@@ -432,19 +442,20 @@ def step_vs_oracle(monkeypatch, gemm_mode, *, task, hidden, depth, p, mols, feat
     if bench:
         # the unconditional bounds of test_gpu_model.py::test_gradients_at_bench_scale_vs_fp64_oracle, against the oracle's own ReLU
         # decisions under the same dropout masks
-        ws0, wl0, wg0, _, _ = run_oracle(monkeypatch, sd, groups, drops, p, depth, depth, head, oracle_loss)
+        ws0, wl0, wg0, _, _, _ = run_oracle(monkeypatch, sd, groups, drops, p, depth, ddepth, head, oracle_loss, ffn_depth=ffn_depth)
         e_s, e_l = rel_err(out.detach().cpu().numpy(), ws0), rel_err(loss.detach().cpu().numpy(), wl0)
         assert e_s < 1e-4 and e_l < 1e-4, (e_s, e_l)
         worst = max(float(np.abs(got[k] - wg0[k]).max() / np.abs(wg0[k]).max()) for k in live)
         worst_l2 = max(float(np.linalg.norm(got[k] - wg0[k]) / np.linalg.norm(wg0[k])) for k in live)
         assert worst <= BENCH_TOL[gemm_mode]["max_rel"] and worst_l2 <= BENCH_TOL[gemm_mode]["l2"], (worst, worst_l2)
+    return measured
 
 
-def _listwise_case(task, seed, sizes):
+def _listwise_case(task, seed, sizes, add=1):
     from reactranker_b200.train.train_listwise import batch_loss
     ds = synthetic.make_dataset(seed, sizes)
     targets = ds.lgk.astype(np.float32)
-    return dict(mols=[([ds.mols[t] for t in ds.rsmi], [ds.mols[t] for t in ds.psmi])], feats=ds.temp.reshape(-1, 1),
+    return dict(mols=[([ds.mols[t] for t in ds.rsmi], [ds.mols[t] for t in ds.psmi])], feats=add_features(ds, add),
                 gpu_loss=lambda out: batch_loss(task, out, sizes, torch.tensor(targets), GPU),
                 oracle_loss=lambda s: O.loss_for_task(task, s, sizes, torch.tensor(targets).double()))
 
@@ -491,6 +502,54 @@ def test_c5_batch_step_with_dropout_vs_fp64_oracle(monkeypatch):
     """A c5-shaped batch (24 groups x 50 candidates, ListMLE h300 d3, p = 0.1) on the product path, under the bench-scale bounds of the
     dropout-free test as well as the exact statement given the GPU's ReLU decisions."""
     step_vs_oracle(monkeypatch, 1, task="mle", hidden=300, depth=3, p=0.1, bench=True, **_listwise_case("mle", 4242, [50] * 24))
+
+
+# Models whose number of dense layers differs from the c5 model's, and with it the stream id of every later dropout site; one without the
+# W_i / W_h / FFN biases (the padding-row fix-up then adds no bias); one whose readout dropout runs over three add features that cross the
+# padded hidden width (hidden 46 + 3 -> vp 64).
+DROPOUT_CONFIGS = {"ffn1": dict(ffn_depth=1), "ffn4": dict(ffn_depth=4), "depth1_diff2": dict(depth=1, ddepth=2), "nobias": dict(use_bias=False),
+                   "add3": dict(hidden=46, add=3)}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name", list(DROPOUT_CONFIGS))
+def test_listmle_step_with_dropout_at_other_configurations_vs_fp64_oracle(monkeypatch, gemm_mode, name):
+    """p = 0.2 at FFN depth 1 and 4, encoder depth 1 with diff depth 2, no biases and three add features: the stream-id schedule, the
+    readout mask over every add-feature column and the training step against the oracle wherever the layer count changes."""
+    c = dict(dict(hidden=40, depth=3), **DROPOUT_CONFIGS[name])
+    step_vs_oracle(monkeypatch, gemm_mode, task="mle", p=0.2, **c, **_listwise_case("mle", 79, [7, 5, 9, 4], add=c.get("add", 1)))
+
+
+@pytest.fixture
+def precision_switches():
+    """The process-wide operand-split switches of rr_model_forward / rr_model_backward, put back as found after the test."""
+    L = _lib.lib()
+    prev = L.rr_get_forward_bf16(), L.rr_get_backward_bf16()
+    yield L
+    L.rr_set_forward_bf16(prev[0])
+    L.rr_set_backward_bf16(prev[1])
+
+
+# The forward GEMMs on the 3 x bf16 split (rr_set_forward_bf16(1)): the k_tc_gemm2 epilogue with bias, residual, ReLU and Philox dropout.
+# Its forward error is larger than the 3 x TF32 split's, so the scores / saved activations and the distance from zero at which a ReLU
+# decision may differ from the fp64 oracle's get bounds of their own.  Measured on this case and on three more batches of the same model
+# (seeds 78, 80, 81) on one B200 (1000 W power limit): scores within 1.25e-5 of the oracle (3 x TF32: 1.1e-5), saved activations within
+# 7.7e-6 of their maximum (3 x TF32: 6.7e-6), differing ReLU decisions at most 1.95e-6 (relative to the row) from zero, gradients given the
+# GPU's masks within 2.4e-5.  The bounds are 4x the measured score and activation error, as helpers.KINK is for the 3 x TF32 split:
+FWD_BF16_SCORE_TOL = 5e-5
+FWD_BF16_KINK = 3e-5
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("fwd_bf16,bwd_bf16", [(1, 1), (0, 0)], ids=["forward_bf16", "backward_tf32"])
+def test_listmle_step_with_dropout_under_the_precision_switches(monkeypatch, precision_switches, fwd_bf16, bwd_bf16):
+    """ListMLE h300 d3 at p = 0.1 on the tensor-core path with the forward GEMMs on the 3 x bf16 split, and with the backward GEMMs on the
+    3 x TF32 split: the dropout zero pattern of every site bit for bit, and every gradient, given the GPU's ReLU decisions, to 2e-4."""
+    L = precision_switches
+    L.rr_set_forward_bf16(fwd_bf16)
+    L.rr_set_backward_bf16(bwd_bf16)
+    kw = dict(score_tol=FWD_BF16_SCORE_TOL, kink=FWD_BF16_KINK) if fwd_bf16 else {}
+    step_vs_oracle(monkeypatch, 1, task="mle", hidden=300, depth=3, p=0.1, **kw, **_listwise_case("mle", 77, [7, 5, 9, 4]))
 
 
 @pytest.mark.gpu

@@ -15,8 +15,8 @@ from reactranker_b200 import _lib, synthetic
 from reactranker_b200.features.featurization import BatchMolGraph, DeviceGraph
 from reactranker_b200.models.base_model import build_model
 from reactranker_b200.train import loss as RL
-from helpers import (TOL, check_grads, dataset_from_golden, forced_relu_masks, gpu_relu_masks, grads_close, rel_err, sd_from_golden,
-                     star_dict)
+from helpers import (CONFIGS, TOL, add_features, check_grads, config, config_dataset, dataset_from_golden, forced_relu_masks, gpu_relu_masks,
+                     grads_close, rel_err, sd_from_golden, star_dict)
 
 pytestmark = pytest.mark.gpu
 GPU = 0
@@ -35,43 +35,46 @@ def product_loss(task, out, scope, targets, gpu=GPU):
     return batch_loss(task, out, scope, targets, gpu)
 
 
-def make_model(hidden, task, depth, ddepth, sd=None, dropout=0.0, last="with_softplus"):
+def make_model(hidden, task, depth, ddepth, sd=None, dropout=0.0, last="with_softplus", ffn_depth=3, use_bias=True, add=1, task_num=None):
+    """``task_num`` overrides the task's own (TASKS): with ffn_last_layer 'with_softplus' and no task_type that is a raw multi-column head."""
     tn, tt, *ll = TASKS[task]
     last = ll[0] if ll else last
-    m = build_model(hidden_size=hidden, mpnn_depth=depth, mpnn_diff_depth=ddepth, ffn_depth=3, use_bias=True, dropout=dropout,
-                    task_num=tn, ffn_last_layer=last, task_type=tt, add_features_dim=1)
+    m = build_model(hidden_size=hidden, mpnn_depth=depth, mpnn_diff_depth=ddepth, ffn_depth=ffn_depth, use_bias=use_bias, dropout=dropout,
+                    task_num=task_num or tn, ffn_last_layer=last, task_type=tt, add_features_dim=add)
     if sd is not None:
         m.load_state_dict(sd)
     return m.cuda(GPU)
 
 
-def oracle_run(sd, ds, sizes, task, depth, ddepth, masks=None, last="with_softplus", feats=None):
+def oracle_run(sd, ds, sizes, task, depth, ddepth, masks=None, last="with_softplus", feats=None, ffn_depth=3, add=1, task_num=None,
+               upstream=None):
     """fp64 oracle forward + loss + backward on the data set of a test; with ``masks`` the ReLU decisions are the GPU's
-    (helpers.forced_relu_masks).  Returns (scores, loss, {name: gradient}, mask flips)."""
+    (helpers.forced_relu_masks).  ``feats`` defaults to helpers.add_features(ds, add); with ``upstream`` the loss is (scores * upstream).sum()
+    instead of the task's.  Returns (scores, loss, {name: gradient}, mask flips)."""
     sd64 = {k: v.double().cpu() for k, v in sd.items()}
     params = {k: v.clone().requires_grad_(True) for k, v in sd64.items() if "cached_zero" not in k}
     full = dict(sd64)
     full.update(params)
     tn, tt, *ll = TASKS[task]
-    head = O.resolve_task_type(tn, ll[0] if ll else last, tt)
+    head = O.resolve_task_type(task_num or tn, ll[0] if ll else last, tt)
     r_o, p_o = O.OracleBatch([ds.mols[t] for t in ds.rsmi]), O.OracleBatch([ds.mols[t] for t in ds.psmi])
-    feats = ds.temp.reshape(-1, 1) if feats is None else feats
+    feats = add_features(ds, add) if feats is None else feats
     targets = torch.tensor(ds.lgk.astype(np.float32)).double()
     flips = 0
     if masks is None:
-        want = O.model_forward(full, r_o, p_o, feats, mpnn_depth=depth, mpnn_diff_depth=ddepth, head=head)
+        want = O.model_forward(full, r_o, p_o, feats, mpnn_depth=depth, mpnn_diff_depth=ddepth, ffn_depth=ffn_depth, head=head)
     else:
         with forced_relu_masks(masks) as fm:
-            want = O.model_forward(full, r_o, p_o, feats, mpnn_depth=depth, mpnn_diff_depth=ddepth, head=head)
+            want = O.model_forward(full, r_o, p_o, feats, mpnn_depth=depth, mpnn_diff_depth=ddepth, ffn_depth=ffn_depth, head=head)
         flips = fm.flips
-    wl = O.loss_for_task(task, want, sizes, targets)
+    wl = O.loss_for_task(task, want, sizes, targets) if upstream is None else (want * upstream.double()).sum()
     wl.backward(torch.ones_like(wl))
     return want.detach().numpy(), wl.detach().numpy(), {k: v.grad.numpy() for k, v in params.items()}, flips
 
 
 def masked_oracle_factory(model, out, r_g, p_g, sd, ds, sizes, task, hidden, depth, ddepth, **kw):
     """Reads the GPU's ReLU masks NOW (before backward recycles the workspace); the returned callable re-runs the oracle with them."""
-    masks = gpu_relu_masks(model, out, (r_g.n_atoms, r_g.n_bonds), (p_g.n_atoms, p_g.n_bonds), hidden, depth, ddepth)
+    masks = gpu_relu_masks(model, out, (r_g.n_atoms, r_g.n_bonds), (p_g.n_atoms, p_g.n_bonds), hidden, depth, ddepth, kw.get("ffn_depth", 3))
 
     def run():
         _, _, g, flips = oracle_run(sd, ds, sizes, task, depth, ddepth, masks=masks, **kw)
@@ -230,6 +233,59 @@ def test_vs_oracle_fresh_inputs(task, hidden, depth, gemm_mode):
     assert rel_err(loss.detach().cpu().numpy(), wl) < tol["loss"]
     got = {k: p.grad.cpu().numpy() for k, p in model.named_parameters() if p.requires_grad}
     check_grads(gemm_mode, got, {k: wg[k] for k in got}, redo)
+
+
+@pytest.mark.parametrize("name", list(CONFIGS))
+def test_configuration_vs_fp64_oracle(name, gemm_mode):
+    """Every model configuration of helpers.CONFIGS (FFN depth 1 and 4, no biases, encoder depth 1, diff depth 1, unequal depths, 0 or 3
+    add features, raw heads of 3 and 16 columns, hidden 8 and 1040, molecules of 1-3 atoms, 320 reactions) against the fp64 oracle at
+    dropout 0, in both GEMM modes.  The loss is a fixed random weighting of the outputs: a ranking loss is shift invariant, which would
+    leave the last bias without a gradient to compare.  Scores to TOL[mode], gradients by helpers.check_grads."""
+    c = config(name)
+    ds, feats = config_dataset(c)
+    sizes = list(c["sizes"])
+    kw = dict(ffn_depth=c["ffn_depth"], add=c["add"], task_num=c["task_num"])
+    torch.manual_seed(3)
+    model = make_model(c["hidden"], "mle", c["depth"], c["ddepth"], use_bias=c["use_bias"], **kw)
+    sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    n = sum(sizes)
+    w = torch.randn((n,) if c["task_num"] == 1 else (n, c["task_num"]), generator=torch.Generator().manual_seed(1))
+    ws, _, wg, _ = oracle_run(sd, ds, sizes, "mle", c["depth"], c["ddepth"], upstream=w, **kw)
+    r_g, p_g = BatchMolGraph([ds.mols[t] for t in ds.rsmi]), BatchMolGraph([ds.mols[t] for t in ds.psmi])
+    out = model(r_g, p_g, gpu=GPU, add_features=feats)
+    redo = masked_oracle_factory(model, out, r_g, p_g, sd, ds, sizes, "mle", c["hidden"], c["depth"], c["ddepth"], upstream=w, **kw) \
+        if gemm_mode == 1 else None
+    (out * w.to(out.device)).sum().backward()
+    assert tuple(out.shape) == tuple(ws.shape)
+    e_s = rel_err(out.detach().cpu().numpy(), ws)
+    assert e_s < TOL[gemm_mode]["score"], e_s
+    got = {k: p.grad.cpu().numpy() for k, p in model.named_parameters() if p.requires_grad}
+    assert set(got) == set(wg)
+    check_grads(gemm_mode, got, wg, redo)
+
+
+def test_ffn_backward_scratch_buffers_at_many_reactions():
+    """FFN depth 4 on 16384 one-atom reactions at hidden 300, on the exact-fp32 SIMT GEMMs.  The backward pass of the FFN's hidden layers
+    alternates two scratch buffers so that no dgrad writes the gradient it reads.  At a few dozen reactions an in-place dgrad would still
+    come out right, because every column tile of a row block reads its inputs before any of them writes.  Here the dgrad grid
+    (128 row blocks x 5 column tiles) is larger than the GPU holds at once, so the later column tiles of a row block start after the
+    earlier ones have written it.  Gradients against the fp64 oracle given the GPU's ReLU decisions, to 2e-4."""
+    sizes = [64] * 256
+    ds = synthetic.make_dataset(62, sizes, atoms_lo=1, atoms_hi=1)
+    _lib.check(_lib.lib().rr_set_gemm_mode(0))
+    torch.manual_seed(3)
+    model = make_model(300, "mle", 3, 3, ffn_depth=4)
+    sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    w = torch.randn(sum(sizes), generator=torch.Generator().manual_seed(1))
+    r_g, p_g = BatchMolGraph([ds.mols[t] for t in ds.rsmi]), BatchMolGraph([ds.mols[t] for t in ds.psmi])
+    out = model(r_g, p_g, gpu=GPU, add_features=ds.temp.reshape(-1, 1))
+    redo = masked_oracle_factory(model, out, r_g, p_g, sd, ds, sizes, "mle", 300, 3, 3, upstream=w, ffn_depth=4)
+    (out * w.to(out.device)).sum().backward()
+    got = {k: p.grad.double().cpu().numpy() for k, p in model.named_parameters() if p.requires_grad}
+    wg, _ = redo()
+    gscale = max(float(np.abs(v).max()) for v in wg.values())
+    live = {k: v for k, v in wg.items() if float(np.abs(v).max()) >= 1e-6 * gscale}     # one-atom molecules: encoder W_h sees zeros only
+    assert not grads_close(got, live, 2e-4)
 
 
 # Gradient tolerance on a FULL-SIZE batch.  A ReLU whose pre-activation lies within the forward pass's rounding error of zero may get the

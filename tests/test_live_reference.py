@@ -94,18 +94,31 @@ def _tasks():
 def test_oracle_equals_live_reference_on_fresh_inputs(task):
     """Every runnable task key (train_listwise.py:196-285): the oracle's scores, loss and all gradients against the reference's own modules
     in fp64, on a model / batch the goldens do not hold (hidden 32, depth 4 / 2, ragged groups with a single-candidate group and a star)."""
+    _oracle_vs_live_reference(task, 300 + len(task), 32, 4, 2)
+
+
+@pytest.mark.parametrize("ffn_depth,use_bias,add", [(1, True, 1), (4, True, 3), (3, False, 0)], ids=["ffn1", "ffn4_add3", "nobias_add0"])
+def test_oracle_equals_live_reference_at_other_configurations(ffn_depth, use_bias, add):
+    """The same at FFN depth 1 and 4, without the W_i / W_h / FFN biases, and with 0 or 3 add features: the model configurations the GPU
+    parity sweep (tests/test_gpu_model.py::test_configuration_vs_fp64_oracle) holds the kernels to the oracle at."""
+    _oracle_vs_live_reference("mle", 350 + ffn_depth, 32, 3, 2, ffn_depth=ffn_depth, use_bias=use_bias, add=add)
+
+
+def _oracle_vs_live_reference(task, seed, hidden, depth, ddepth, ffn_depth=3, use_bias=True, add=1):
     import make_golden as MG
+    from helpers import add_features
     tn, last, tt = MG.TASKS_ALL[task]
-    seed, sizes, star, hidden, depth, ddepth = 300 + len(task), [4, 1, 7, 3], {2: 6}, 32, 4, 2
+    sizes, star = [4, 1, 7, 3], {2: 6}
     with _quiet():
-        ds, model, scores, loss, grads = MG.run_case(task, hidden, seed, sizes, star, torch.float64, depth, ddepth)
+        ds, model, scores, loss, grads = MG.run_case(task, hidden, seed, sizes, star, torch.float64, depth, ddepth, ffn_depth, use_bias, add)
     sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
     params = {k: v.clone().requires_grad_(True) for k, v in sd.items() if "cached_zero" not in k}
     full = dict(sd)
     full.update(params)
     r_g = O.OracleBatch([ds.mols[t] for t in ds.rsmi])
     p_g = O.OracleBatch([ds.mols[t] for t in ds.psmi])
-    out = O.model_forward(full, r_g, p_g, ds.temp.reshape(-1, 1), mpnn_depth=depth, mpnn_diff_depth=ddepth, head=O.resolve_task_type(tn, last, tt))
+    out = O.model_forward(full, r_g, p_g, add_features(ds, add), mpnn_depth=depth, mpnn_diff_depth=ddepth, ffn_depth=ffn_depth,
+                          head=O.resolve_task_type(tn, last, tt))
     targets = torch.tensor(ds.lgk.astype(np.float32)).double()
     got_loss = O.loss_for_task(task, out, sizes, targets)
     got_loss.backward()
