@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define RR_ABI_VERSION 2
+#define RR_ABI_VERSION 3
 #define RR_ATOM_FDIM 61   /* features/featurization.py:63 */
 #define RR_BOND_FDIM 22   /* features/featurization.py:64 */
 #define RR_FBOND_TOTAL 83 /* models/base_model.py:129     */
@@ -295,13 +295,9 @@ int rr_model_backward(const rr_model_cfg* cfg, const rr_params* w, const rr_grap
 int rr_profile_begin(void);
 int rr_profile_end(double* h_ms_by_class, int64_t* h_launches_by_class, int n_classes);
 int rr_profile_classes(void);
-/* The RR_* environment switches (kernel experiments / diagnostics) are read once, at first use; this reads them again. */
+/* The RR_MP_V1 environment switch (first-generation gather kernels instead of the row pipeline) is read once, at first use; this reads it
+ * again. */
 void rr_reload_switches(void);
-/* Diagnostic: with RR_TC_DIAG & 16 the first CTA of every weight-gradient launch (k_tc_wgrad3, 32-row stages) and of every fp32-split
- * forward launch (k_tc_gemm2) stamps the SM clock at its pipeline hand-offs into one device buffer (96 stages or work items x 16 slots);
- * this synchronises the device and copies the first n stamps of the last such launch to host_out.  scripts/wgrad_trace.py and
- * scripts/gemm_trace.py print them; the slot meanings are listed there and next to the kernels. */
-int rr_debug_wgrad_trace(unsigned long long* host_out, int n);
 /* kernels launched on this thread since the last reset (for bench.py's gpu_launches) */
 int64_t rr_launch_count(void);
 void rr_launch_count_reset(void);

@@ -52,7 +52,7 @@ EXPORTS = [
     "rr_loss_fwdbwd", "rr_loss_fwdbwd_ex", "rr_loss_max_group", "rr_rank_metrics",
     "rr_model_workspace_bytes", "rr_model_buffer_offset", "rr_model_forward", "rr_model_backward", "rr_launch_count", "rr_launch_count_reset",
     "rr_profile_begin", "rr_profile_end", "rr_profile_classes", "rr_set_gemm_mode", "rr_get_gemm_mode", "rr_set_backward_bf16", "rr_get_backward_bf16",
-    "rr_set_forward_bf16", "rr_get_forward_bf16", "rr_reload_switches", "rr_debug_wgrad_trace",
+    "rr_set_forward_bf16", "rr_get_forward_bf16", "rr_reload_switches",
 ]
 KERNEL_CLASSES = ["gemm_fwd", "gemm_dgrad", "gemm_wgrad", "bond_fwd", "bond_bwd", "nbr_fwd", "nbr_bwd", "readout", "elementwise", "loss", "misc"]
 
@@ -122,7 +122,6 @@ def lib() -> ctypes.CDLL:
                 L.rr_reload_switches.restype = None
                 i32, i64, u64, f32, vp = ctypes.c_int, ctypes.c_int64, ctypes.c_uint64, ctypes.c_float, ctypes.c_void_p
                 L.rr_device_check.argtypes = [i32]
-                L.rr_debug_wgrad_trace.argtypes = [vp, i32]
                 L.rr_padded.argtypes = [i32]
                 L.rr_graph_assemble.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
                 L.rr_batch_build.argtypes = [i32, vp, i32, vp, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]

@@ -23,18 +23,7 @@ static int env_int(const char* name, int dflt) {
 void reload_switches() {
   std::lock_guard<std::mutex> lock(g_switches_mutex);
   Switches w;
-  const int ew = env_int("RR_TC_EW", 16);
-  w.tc_ew = (ew == 4 || ew == 8) ? ew : 16;
-  w.tc_diag = env_int("RR_TC_DIAG", 0);
-  w.tc_fake_presplit = getenv("RR_TC_FAKE_PRESPLIT") != nullptr;
-  w.wg_kt = env_int("RR_WG_KT", 0);
-  w.wg_tf32 = getenv("RR_WG_TF32") != nullptr;
-  w.wg_bkr = env_int("RR_WG_BKR", 0);
-  if (const char* c = getenv("RR_WG3_CFG")) sscanf(c, "%d,%d,%d", &w.wg3_bkr, &w.wg3_raw, &w.wg3_bf);
   w.mp_v1 = env_int("RR_MP_V1", 0);
-  if (const char* c = getenv("RR_MP_ACC_RED")) w.mp_acc_red = c[0] != '0';
-  w.mp_consumers = env_int("RR_MP_CONSUMERS", 0);
-  w.mp_kstage = env_int("RR_MP_KSTAGE", 0);
   g_switches = w;
   g_switches_loaded.store(true);
 }
@@ -212,7 +201,6 @@ int rr_profile_end(double* ms_by_class, int64_t* launches_by_class, int n_classe
 }
 int rr_profile_classes(void) { return rr::KC_COUNT; }
 void rr_reload_switches(void) { rr::reload_switches(); }
-int rr_debug_wgrad_trace(unsigned long long* host_out, int n) { return rr::tc_wgrad_trace(host_out, n); }
 int64_t rr_launch_count(void) { return rr::g_launches.load(); }
 void rr_launch_count_reset(void) { rr::g_launches.store(0); }
 

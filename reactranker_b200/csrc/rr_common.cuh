@@ -74,13 +74,10 @@ struct ProfScope {
 // 0 = fp32 SIMT GEMMs, 1 = tcgen05 3xTF32 GEMMs where the shape allows (forward + dgrad)
 extern std::atomic<int> g_gemm_mode;
 
-// Diagnostic / experiment switches from the environment (RR_TC_EW, RR_TC_DIAG, RR_TC_FAKE_PRESPLIT, RR_WG_KT, RR_WG_TF32, RR_WG_BKR, RR_WG3_CFG,
-// RR_MP_V1, RR_MP_ACC_RED, RR_MP_CONSUMERS): read ONCE, when the library is first used, not on every launch.  rr_reload_switches() reads
-// them again (tests and the micro-benchmarks flip them inside one process).
+// Switches from the environment (RR_MP_V1: the first-generation gather kernels instead of the row pipeline): read ONCE, when the library is
+// first used, not on every launch.  rr_reload_switches() reads them again (tests and the micro-benchmarks flip them inside one process).
 struct Switches {
-  int tc_ew = 16, tc_diag = 0, tc_fake_presplit = 0;
-  int wg_kt = 0, wg_tf32 = 0, wg_bkr = 0, wg3_bkr = 0, wg3_raw = 6, wg3_bf = 2;   // wg3_bkr 0: 64-row stages for narrow X tiles, 32 otherwise
-  int mp_v1 = 0, mp_acc_red = -1, mp_consumers = 0, mp_kstage = 0;
+  int mp_v1 = 0;
 };
 const Switches& switches();
 void reload_switches();
@@ -124,13 +121,12 @@ struct PerDeviceOnce {
 // The big kernels are persistent, one CTA per SM, with a prologue of a few microseconds (barrier init, TMEM allocation, descriptor prefetch).
 // Launched with cudaLaunchAttributeProgrammaticStreamSerialization, the CTAs of kernel N+1 start on every SM that kernel N has left and run
 // their prologue while N's tail still executes; pdl_wait() (griddepcontrol.wait) then holds every thread until kernel N has completed and
-// its writes are visible, BEFORE the first global access of N+1 (reads and writes alike).  RR_NO_PDL=1 falls back to plain launches.
+// its writes are visible, BEFORE the first global access of N+1 (reads and writes alike).
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
-  static const bool off = getenv("RR_NO_PDL") != nullptr;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid;
   cfg.blockDim = block;
@@ -140,7 +136,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = off ? 0 : 1;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
@@ -259,7 +255,6 @@ long long tc_dgrad_scratch_bytes(int n, int k);
 int tc_dgrad_standalone(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, void* scratch,
                         long long scratch_bytes, cudaStream_t s);
 bool tc_wgrad_supported(int M, int n, int k, int lddz, int ldx);
-int tc_wgrad_trace(unsigned long long* host_out, int n);
 int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s);
 
 }  // namespace rr

@@ -9,10 +9,9 @@
 // tensor cores (kind::tf32), accumulating in TMEM.
 //
 // Persistent warp-specialised CTAs (k_tc_gemm2): TMA producer, MMA issuer, four split warps that move the A operand through TENSOR
-// MEMORY, eight epilogue warps; see the comment above the kernel.  The backward GEMMs (dgrad: k_tc_gemm2<.., true>, wgrad:
+// MEMORY, sixteen epilogue warps; see the comment above the kernel.  The backward GEMMs (dgrad: k_tc_gemm2<.., true>, wgrad:
 // k_tc_wgrad3) use a 3 x bf16 split instead.  Two-source K (concat-free [x1 || x2] W^T) walks both sources through one accumulator.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "rr_common.cuh"
 
@@ -50,10 +49,7 @@ struct Args {
   float p, inv_keep;
   uint64_t seed, stream_id;
   int presplit;  // B arrives as two TF32-exact images (hi, lo) made once per step by the pack kernel: no B split in the main loop
-  int diag;      // RR_TC_DIAG bit mask (timing experiments only, results are wrong): 1 no A split, 2 no B split, 4 no MMA, 8 no epilogue traffic
-  unsigned long long* trace;   // RR_TC_DIAG & 16 (k_tc_gemm2<16, false, true>): clock64 stamps of CTA 0, 16 slots per work item
 };
-constexpr int G2_TRACE_ITEMS = 96, G2_TRACE_SLOTS = 16;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
 
@@ -184,12 +180,12 @@ __device__ __forceinline__ void split_tile(uint8_t* hi_p, uint8_t* lo_p, int byt
 // their row of the landed fp32 tile once and store (hi, lo) straight into TMEM with tcgen05.st; the MMAs take A from
 // TMEM and only B from shared memory.  The CTA is persistent (one per SM, static round-robin over tiles), a
 // separate epilogue warpgroup drains the accumulator while the producer and the split warps already work on the
-// next tile, and the epilogue moves 128-byte row segments (tcgen05.ld x32).
+// next tile, and the epilogue moves 64-byte row segments (tcgen05.ld x16).
 //   warp 0: TMA producer | warp 1: MMA issuer (+TMEM alloc) | warps 2-5: split (A -> TMEM, B -> smem hi/lo) |
-//   warps 6-21: epilogue (EW = 16; the 8- and 4-warp flavours remain behind RR_TC_EW)
+//   warps 6-21: epilogue (EW = 16)
 // TMEM columns: [0, 320) accumulator, [320 + 64 s, ...) A stage s = 32 columns hi + 32 columns lo.
 // ================================================================================================
-constexpr int THREADS2_BASE = 192;   // TMA warp + MMA warp + 4 split warps; the epilogue adds 4 or 8 warps
+constexpr int THREADS2_BASE = 192;   // TMA warp + MMA warp + 4 split warps; the epilogue adds 16 warps
 
 __device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -221,68 +217,15 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8])
                "r"(r[5]), "r"(r[6]), "r"(r[7])
                : "memory");
 }
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,"
-      "%30,%31}, [%32];\n\t"
-      "tcgen05.wait::ld.sync.aligned;"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]),
-        "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]),
-        "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// Epilogue of one [32 rows x 32 columns] block of the accumulator held one row per lane.
-// A lane owning a whole row would touch 32 different rows per global instruction (16 of every 32-byte sector wasted, no coalescing), and that
-// was half of the kernel's time.  The block is therefore transposed through a warp-private, XOR-swizzled 4 KB staging tile: afterwards 8
-// consecutive lanes cover one row's 128 contiguous bytes, so every global load / store instruction moves whole sectors of 4 rows.
-// The residual (or, for dgrad accumulation, the previous value of C) of a block is loaded one block AHEAD of its use (epi_issue), the first
-// block of a tile before the wait for its accumulator, so its latency hides behind the MMAs.
-__device__ __forceinline__ void epi_issue(const Args& g, float4 (&R)[8], int row0, int col0, int lane) {
-  const float* src = g.resid ? g.resid : (g.accumulate ? g.C : nullptr);
-  if (src == nullptr) return;
-  const int ld = g.resid ? g.ldr : g.ldc;
-  const int col = col0 + 4 * (lane & 7);
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int row = row0 + i * 4 + (lane >> 3);
-    if (row < g.M && col < g.N) R[i] = ld_f4_stream(src + static_cast<size_t>(row) * ld + col);
-  }
-}
-__device__ __forceinline__ void epilogue_block(const Args& g, const float (&v)[32], const float4 (&R)[8], uint32_t stage, int row0, int col0, int lane) {
-  const int j = lane & 7, rsub = lane >> 3;
-  const int col = col0 + 4 * j;
-  const bool col_ok = col < g.N;
-  const float4 bs = (g.bias && col_ok) ? ld_f4(g.bias + col) : f4_zero();
-#pragma unroll
-  for (int c = 0; c < 8; ++c)
-    sts_f4(stage + lane * 128 + ((c ^ (lane & 7)) << 4), make_float4(v[4 * c], v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]));
-  __syncwarp();
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int r = i * 4 + rsub, row = row0 + r;
-    float4 o = lds_f4(stage + r * 128 + ((j ^ (r & 7)) << 4));
-    if (row < g.M && col_ok) {
-      float* cp = g.C + static_cast<size_t>(row) * g.ldc + col;
-      if (g.bias) o = f4_add(o, bs);
-      if (g.resid) o = f4_add(o, R[i]);
-      if (g.relu) o = f4_relu(o);
-      if (g.p > 0.f) o = dropout4(o, g.p, g.inv_keep, g.seed, g.stream_id, (static_cast<uint64_t>(row) * g.ldc + col) >> 2);
-      if (g.accumulate) o = f4_add(o, g.resid ? *reinterpret_cast<const float4*>(cp) : R[i]);
-      st_f4(cp, o);
-    }
-  }
-  __syncwarp();
-}
-
-// 16-column flavour of the same epilogue for the 16-epilogue-warp kernel (EW = 16): a [32 rows x 16 columns] sub-block per step, a 2 KB
-// staging tile per warp (rows of 64 B; chunk c of row r sits at c ^ ((r >> 1) & 3), conflict-free for both the row-per-lane writes and the
-// 4-lanes-per-row reads), 8 rows x 64 contiguous bytes per global instruction.  Half the registers of the 32-column version, so twice the
-// warps fit: the epilogue is issue-bound (scripts/bench_gemm.py diag), not bandwidth-bound.
+// Epilogue of one [32 rows x 16 columns] sub-block of the accumulator, held one row per lane.
+// A lane owning a whole row would touch 32 different rows per global instruction (no coalescing, most of every 32-byte sector wasted), and that
+// was half of the kernel's time.  The sub-block is therefore transposed through a warp-private 2 KB staging tile (rows of 64 B; chunk c of
+// row r sits at c ^ ((r >> 1) & 3), conflict-free for both the row-per-lane writes and the 4-lanes-per-row reads): afterwards 4 consecutive
+// lanes cover one row's 64 contiguous bytes, 8 rows per global instruction.
+// The residual (or, for dgrad accumulation, the previous value of C) of a sub-block is loaded one sub-block AHEAD of its use (epi_issue_h),
+// the first of a tile before the wait for its accumulator, so its latency hides behind the MMAs.
+// Sub-blocks of 16 rather than 32 columns need half the registers, so 16 epilogue warps fit instead of 8: the epilogue is issue-bound, not
+// bandwidth-bound, and the 16-warp epilogue took 14 % off the forward GEMM (DESIGN.md §6b).
 __device__ __forceinline__ void epi_issue_h(const Args& g, float4 (&R)[4], int row0, int col0, int lane) {
   const float* src = g.resid ? g.resid : (g.accumulate ? g.C : nullptr);
   if (src == nullptr) return;
@@ -366,8 +309,9 @@ __device__ __forceinline__ void split_bf16_pair(float x0, float x1, uint32_t& hi
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(r1), "f"(r0));
 }
 
-template <int EW, bool BF, bool TR = false>
+template <int EW, bool BF>
 __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const __grid_constant__ Args g) {
+  static_assert(EW == 16, "the epilogue is written for 16 warps, four per TMEM lane quadrant");
   constexpr int S2 = BF ? S2_BF : tc::S2;
   constexpr int STAGE2 = BF ? STAGE2_BF : tc::STAGE2;
   constexpr int B2_BYTES = BF ? B2_BYTES_BF : tc::B2_BYTES;
@@ -382,12 +326,6 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // TR: slots per work item w of CTA 0 -- 0 producer starts the item, 1 its last stage issued; 2 MMA warp has the accumulator, 3 last MMA
-  // committed; 4 first stage split by warp 2, 5 last; epilogue warp 6: 8 residual of its first sub-block requested, 9 accumulator full,
-  // 10 + j after its j-th sub-block (j < 3); epilogue warp 21: 13 accumulator full, 14 done
-  auto stamp = [&](int w, int slot) {
-    if (TR && g.trace != nullptr && blockIdx.x == 0 && w < G2_TRACE_ITEMS) g.trace[w * G2_TRACE_SLOTS + slot] = clock64();
-  };
   const int m_tiles = (g.M + BM - 1) / BM, n_tiles = (g.N + NT2 - 1) / NT2;
   const int total_tiles = m_tiles * n_tiles;
   int nkb_total = 0;
@@ -425,10 +363,8 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
     if (lane == 0) {
       int it = 0;
       const uint32_t tx = static_cast<uint32_t>(A_BYTES + ((g.presplit || BF) ? 2 : 1) * B2_BYTES);
-      int pw = 0;
-      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++pw) {
+      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
         const int m0 = (tile / n_tiles) * BM, n0 = (tile % n_tiles) * NT2;
-        if (TR) stamp(pw, 0);
         for (int s = 0; s < g.nsrc; ++s) {
           const int nkb = (g.src[s].K + BK - 1) / BK;
           for (int kb = 0; kb < nkb; ++kb, ++it) {
@@ -442,7 +378,6 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
             if (g.presplit || BF) tma_load_2d(&g.src[s].tmBlo, full + st, base + A_BYTES + B2_BYTES, kb * BK, n0);
           }
         }
-        if (TR) stamp(pw, 1);
       }
     }
   } else if (warp == 1) {
@@ -457,7 +392,6 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
         const uint32_t d = tmem_base + buf * NT2;
         mbar_wait(acc_empty + buf, ((w >> 1) & 1) ^ 1);     // the epilogue has drained this accumulator
         tc_fence_after();
-        if (TR) stamp(w, 2);
         for (int kb = 0; kb < nkb_total; ++kb, ++it) {
           const int st = it % S2;
           const uint32_t ph = (it / S2) & 1;
@@ -466,29 +400,26 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
           const uint32_t base = smem_u32(smem + static_cast<size_t>(st) * STAGE2);
           const uint32_t b_hi = base + A_BYTES, b_lo = b_hi + B2_BYTES;
           const uint32_t a_hi = tmem_base + TM_A2 + st * A_COLS, a_lo = a_hi + A_COLS / 2;
-          if (!(g.diag & 4)) {
-            if constexpr (BF) {
+          if constexpr (BF) {
 #pragma unroll
-              for (int k = 0; k < BK / 16; ++k) {           // UMMA_K = 16 bf16 = 32 bytes of the 64-byte row = 8 TMEM columns of packed pairs
-                const uint32_t ko = k * 32;
-                umma_bf16_ts(d, a_lo + k * 8, umma_desc_sw64(b_hi + ko), idesc, (kb > 0 || k > 0) ? 1u : 0u);
-                umma_bf16_ts(d, a_hi + k * 8, umma_desc_sw64(b_lo + ko), idesc, 1u);
-                umma_bf16_ts(d, a_hi + k * 8, umma_desc_sw64(b_hi + ko), idesc, 1u);
-              }
-            } else {
+            for (int k = 0; k < BK / 16; ++k) {           // UMMA_K = 16 bf16 = 32 bytes of the 64-byte row = 8 TMEM columns of packed pairs
+              const uint32_t ko = k * 32;
+              umma_bf16_ts(d, a_lo + k * 8, umma_desc_sw64(b_hi + ko), idesc, (kb > 0 || k > 0) ? 1u : 0u);
+              umma_bf16_ts(d, a_hi + k * 8, umma_desc_sw64(b_lo + ko), idesc, 1u);
+              umma_bf16_ts(d, a_hi + k * 8, umma_desc_sw64(b_hi + ko), idesc, 1u);
+            }
+          } else {
 #pragma unroll
-              for (int k = 0; k < BK / UK; ++k) {
-                const uint32_t ko = k * UK * 4;
-                umma_tf32_ts(d, a_lo + k * UK, umma_desc(b_hi + ko), idesc, (kb > 0 || k > 0) ? 1u : 0u);
-                umma_tf32_ts(d, a_hi + k * UK, umma_desc(b_lo + ko), idesc, 1u);
-                umma_tf32_ts(d, a_hi + k * UK, umma_desc(b_hi + ko), idesc, 1u);
-              }
+            for (int k = 0; k < BK / UK; ++k) {
+              const uint32_t ko = k * UK * 4;
+              umma_tf32_ts(d, a_lo + k * UK, umma_desc(b_hi + ko), idesc, (kb > 0 || k > 0) ? 1u : 0u);
+              umma_tf32_ts(d, a_hi + k * UK, umma_desc(b_lo + ko), idesc, 1u);
+              umma_tf32_ts(d, a_hi + k * UK, umma_desc(b_hi + ko), idesc, 1u);
             }
           }
           umma_commit(empty + st);
         }
         umma_commit(acc_full + buf);
-        if (TR) stamp(w, 3);
       }
     }
   } else if (warp < 6) {
@@ -507,57 +438,26 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
         mbar_wait(full + st, ph);
         uint8_t* base = smem + static_cast<size_t>(st) * STAGE2;
         // A: this thread's row of 32 floats (128-byte swizzle: chunk c sits at c ^ (row & 7)) -> hi / lo -> TMEM
-        if (!(g.diag & 1)) {
-          const uint32_t rowp = smem_u32(base) + r * 128;
-          if constexpr (EW == 16) {
-            // 704 threads cap the kernel at 88 registers: two halves of 16 floats each instead of the whole row at once
+        // 704 threads cap the kernel at 88 registers: two halves of 16 floats each instead of the whole row at once
+        const uint32_t rowp = smem_u32(base) + r * 128;
 #pragma unroll
-            for (int hlf = 0; hlf < 2; ++hlf) {
-              float4 av[4];
+        for (int hlf = 0; hlf < 2; ++hlf) {
+          float4 av[4];
 #pragma unroll
-              for (int c = 0; c < 4; ++c) av[c] = lds_f4(rowp + (((4 * hlf + c) ^ (r & 7)) << 4));
-              if constexpr (BF) {
-                uint32_t hi[8], lo[8];
-#pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                  split_bf16_pair(av[c].x, av[c].y, hi[2 * c], lo[2 * c]);
-                  split_bf16_pair(av[c].z, av[c].w, hi[2 * c + 1], lo[2 * c + 1]);
-                }
-                tmem_st8(lane_addr + TM_A2 + st * A_COLS + 8 * hlf, hi);
-                tmem_st8(lane_addr + TM_A2 + st * A_COLS + 16 + 8 * hlf, lo);
-              } else {
-                uint32_t hi[16], lo[16];
-#pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                  const float e[4] = {av[c].x, av[c].y, av[c].z, av[c].w};
-#pragma unroll
-                  for (int j = 0; j < 4; ++j) {
-                    const uint32_t h = (__float_as_uint(e[j]) + 0x1000u) & 0xFFFFE000u;
-                    hi[4 * c + j] = h;
-                    lo[4 * c + j] = __float_as_uint(e[j] - __uint_as_float(h));
-                  }
-                }
-                tmem_st16(lane_addr + TM_A2 + st * A_COLS + 16 * hlf, hi);
-                tmem_st16(lane_addr + TM_A2 + st * A_COLS + 32 + 16 * hlf, lo);
-              }
-            }
-          } else {
-          float4 av[8];
-#pragma unroll
-          for (int c = 0; c < 8; ++c) av[c] = lds_f4(rowp + ((c ^ (r & 7)) << 4));
+          for (int c = 0; c < 4; ++c) av[c] = lds_f4(rowp + (((4 * hlf + c) ^ (r & 7)) << 4));
           if constexpr (BF) {
-            uint32_t hi[16], lo[16];
+            uint32_t hi[8], lo[8];
 #pragma unroll
-            for (int c = 0; c < 8; ++c) {
+            for (int c = 0; c < 4; ++c) {
               split_bf16_pair(av[c].x, av[c].y, hi[2 * c], lo[2 * c]);
               split_bf16_pair(av[c].z, av[c].w, hi[2 * c + 1], lo[2 * c + 1]);
             }
-            tmem_st16(lane_addr + TM_A2 + st * A_COLS, hi);
-            tmem_st16(lane_addr + TM_A2 + st * A_COLS + 16, lo);
+            tmem_st8(lane_addr + TM_A2 + st * A_COLS + 8 * hlf, hi);
+            tmem_st8(lane_addr + TM_A2 + st * A_COLS + 16 + 8 * hlf, lo);
           } else {
-            uint32_t hi[32], lo[32];
+            uint32_t hi[16], lo[16];
 #pragma unroll
-            for (int c = 0; c < 8; ++c) {
+            for (int c = 0; c < 4; ++c) {
               const float e[4] = {av[c].x, av[c].y, av[c].z, av[c].w};
 #pragma unroll
               for (int j = 0; j < 4; ++j) {
@@ -566,13 +466,12 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
                 lo[4 * c + j] = __float_as_uint(e[j] - __uint_as_float(h));
               }
             }
-            tmem_st32(lane_addr + TM_A2 + st * A_COLS, hi);
-            tmem_st32(lane_addr + TM_A2 + st * A_COLS + 32, lo);
-          }
+            tmem_st16(lane_addr + TM_A2 + st * A_COLS + 16 * hlf, hi);
+            tmem_st16(lane_addr + TM_A2 + st * A_COLS + 32 + 16 * hlf, lo);
           }
         }
         // B: elementwise split in shared memory (unless the weights arrived pre-split)
-        if (!BF && !g.presplit && !(g.diag & 2)) split_tile(base + A_BYTES, base + A_BYTES + B2_BYTES, b_used, wtid);
+        if (!BF && !g.presplit) split_tile(base + A_BYTES, base + A_BYTES + B2_BYTES, b_used, wtid);
         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
         if (!BF && !g.presplit) fence_proxy_async();
         tc_fence_before();
@@ -581,73 +480,21 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
       }
     }
   } else {
-    // ---------------- epilogue: EW / 4 warps per TMEM lane quadrant, taking the 32-column blocks of a tile in turn ----------------
+    // ---------------- epilogue: EW / 4 warps per TMEM lane quadrant, taking the 16-column sub-blocks of a tile in turn ----------------
     constexpr int EPQ = EW / 4;
     const int quad = warp & 3;
     const int eidx = (warp - 6) >> 2;
-    if constexpr (EW == 16) {
-      const uint32_t stage = smem_u32(reinterpret_cast<uint8_t*>(full) + 256) + (warp - 6) * 2048;   // warp-private 2 KB staging tile
-      int w = 0;
-      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++w) {
-        const int m0 = (tile / n_tiles) * BM, n0 = (tile % n_tiles) * NT2;
-        const int nblk = (min(NT2, g.N - n0) + 15) >> 4;            // 16-column sub-blocks (tile widths are multiples of 16)
-        const int row0 = m0 + quad * 32;
-        const int buf = w & 1;
-        const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + buf * NT2;
-        float4 R[4];
-        int c = (eidx + w) & (EPQ - 1);                              // rotate the start so the 10 sub-blocks of a tile spread evenly over tiles
-        if (c < nblk && !(g.diag & 8)) epi_issue_h(g, R, row0, n0 + 16 * c, lane);
-        const int tslot = (TR && lane == 0) ? (warp == 6 ? 8 : (warp == 21 ? 13 : -1)) : -1;
-        if (TR && tslot == 8) stamp(w, 8);
-        mbar_wait(acc_full + buf, (w >> 1) & 1);
-        tc_fence_after();
-        if (TR && tslot >= 0) stamp(w, tslot == 8 ? 9 : 13);
-        int tj = 0;
-        if (c >= nblk) {
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(acc_empty + buf);
-        }
-        for (; c < nblk; c += EPQ) {
-          float v[16];
-          tmem_ld16(taddr + 16 * c, v);
-          if (TR && tslot == 8 && tj == 0) stamp(w, 4);
-          const bool last = c + EPQ >= nblk;
-          if (last) {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(acc_empty + buf);
-          }
-          float4 Rn[4];
-          if (!last && !(g.diag & 8)) epi_issue_h(g, Rn, row0, n0 + 16 * (c + EPQ), lane);
-          if (TR && tslot == 8 && tj == 0) stamp(w, 5);
-          if (!(g.diag & 8)) epilogue_block_h(g, v, R, stage, row0, n0 + 16 * c, lane);
-          if (TR && tslot == 8 && tj == 0) stamp(w, 6);
-          if (!last) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) R[i] = Rn[i];
-          }
-          if (TR && tslot == 8 && tj == 0) {
-            if (__float_as_uint(R[0].x) == 0x7fc12345u) stamp(w, 15);      // consume the next block's residual: its latency ends here
-            stamp(w, 7);
-          }
-          if (TR && tslot == 8 && tj < 3) stamp(w, 10 + tj);
-          if (TR && tslot == 13 && last) stamp(w, 14);
-          ++tj;
-        }
-      }
-    } else {
-    const uint32_t stage = smem_u32(reinterpret_cast<uint8_t*>(full) + 256) + (warp - 6) * 4096;   // warp-private staging tile
+    const uint32_t stage = smem_u32(reinterpret_cast<uint8_t*>(full) + 256) + (warp - 6) * 2048;   // warp-private 2 KB staging tile
     int w = 0;
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++w) {
       const int m0 = (tile / n_tiles) * BM, n0 = (tile % n_tiles) * NT2;
-      const int nblk = (min(NT2, g.N - n0) + 31) >> 5;
+      const int nblk = (min(NT2, g.N - n0) + 15) >> 4;            // 16-column sub-blocks (tile widths are multiples of 16)
       const int row0 = m0 + quad * 32;
       const int buf = w & 1;
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + buf * NT2;
-      float4 R[8];
-      int c = eidx;
-      if (c < nblk && !(g.diag & 8)) epi_issue(g, R, row0, n0 + 32 * c, lane);
+      float4 R[4];
+      int c = (eidx + w) & (EPQ - 1);                              // rotate the start so the 10 sub-blocks of a tile spread evenly over tiles
+      if (c < nblk) epi_issue_h(g, R, row0, n0 + 16 * c, lane);
       mbar_wait(acc_full + buf, (w >> 1) & 1);
       tc_fence_after();
       if (c >= nblk) {                        // narrow tile: nothing for this warp, but the accumulator hand-back counts every epilogue warp
@@ -656,23 +503,22 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
         if (lane == 0) mbar_arrive(acc_empty + buf);
       }
       for (; c < nblk; c += EPQ) {
-        float v[32];
-        tmem_ld32(taddr + 32 * c, v);         // a 16-column tail reads 16 stale columns past the tile: never stored (col < N guard)
+        float v[16];
+        tmem_ld16(taddr + 16 * c, v);
         const bool last = c + EPQ >= nblk;
         if (last) {                           // last read of this accumulator: hand it back before the global traffic
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(acc_empty + buf);
         }
-        float4 Rn[8];
-        if (!last && !(g.diag & 8)) epi_issue(g, Rn, row0, n0 + 32 * (c + EPQ), lane);
-        if (!(g.diag & 8)) epilogue_block(g, v, R, stage, row0, n0 + 32 * c, lane);
+        float4 Rn[4];
+        if (!last) epi_issue_h(g, Rn, row0, n0 + 16 * (c + EPQ), lane);
+        epilogue_block_h(g, v, R, stage, row0, n0 + 16 * c, lane);
         if (!last) {
 #pragma unroll
-          for (int i = 0; i < 8; ++i) R[i] = Rn[i];
+          for (int i = 0; i < 4; ++i) R[i] = Rn[i];
         }
       }
-    }
     }
   }
   tc_fence_before();
@@ -708,10 +554,7 @@ struct WgArgs {
   float* dW;
   int lddw;
   float* dbias;
-  int diag;          // RR_TC_DIAG (timing experiments)
-  unsigned long long* trace;   // wgrad3, RR_TC_DIAG & 16: per-stage clock64 stamps of CTA (0,0,0) (rr_debug_wgrad_trace reads them back)
 };
-constexpr int WG_TRACE_STAGES = 96, WG_TRACE_SLOTS = 16;
 
 // MN-major tf32 operands have exactly one legal shared-memory layout: 128-byte swizzle with 32-byte atomicity
 // (cute::UMMA::LayoutType::SWIZZLE_128B_BASE32B = 1, TMA's CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B): atoms of 4 reduction rows x 128 B,
@@ -812,20 +655,18 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant_
         const uint32_t base = smem_u32(smem + static_cast<size_t>(st) * stage_bytes);
         const uint32_t b_hi = base + A_RAW, b_lo = b_hi + b_bytes;
         const uint32_t a_hi = tmem_base + g.tm_a + st * 2 * BKR, a_lo = a_hi + BKR;
-        if (!(g.diag & 4)) {
 #pragma unroll
-          for (int k = 0; k < BKR / UK; ++k) {
-            const uint32_t ko = k * 1024;                // next 8 rows of the reduction
-            const uint32_t first = (it > 0 || k > 0) ? 1u : 0u;
-            umma_tf32_ts(tmem_base, a_lo + k * UK, umma_desc_mn(b_hi + ko, BOX), idesc1, first);
-            umma_tf32_ts(tmem_base, a_hi + k * UK, umma_desc_mn(b_lo + ko, BOX), idesc1, 1u);
-            umma_tf32_ts(tmem_base, a_hi + k * UK, umma_desc_mn(b_hi + ko, BOX), idesc1, 1u);
-            if (n2) {
-              const uint32_t bo = static_cast<uint32_t>(n1 / 32) * BOX;
-              umma_tf32_ts(tmem_base + n1, a_lo + k * UK, umma_desc_mn(b_hi + bo + ko, BOX), idesc2, first);
-              umma_tf32_ts(tmem_base + n1, a_hi + k * UK, umma_desc_mn(b_lo + bo + ko, BOX), idesc2, 1u);
-              umma_tf32_ts(tmem_base + n1, a_hi + k * UK, umma_desc_mn(b_hi + bo + ko, BOX), idesc2, 1u);
-            }
+        for (int k = 0; k < BKR / UK; ++k) {
+          const uint32_t ko = k * 1024;                  // next 8 rows of the reduction
+          const uint32_t first = (it > 0 || k > 0) ? 1u : 0u;
+          umma_tf32_ts(tmem_base, a_lo + k * UK, umma_desc_mn(b_hi + ko, BOX), idesc1, first);
+          umma_tf32_ts(tmem_base, a_hi + k * UK, umma_desc_mn(b_lo + ko, BOX), idesc1, 1u);
+          umma_tf32_ts(tmem_base, a_hi + k * UK, umma_desc_mn(b_hi + ko, BOX), idesc1, 1u);
+          if (n2) {
+            const uint32_t bo = static_cast<uint32_t>(n1 / 32) * BOX;
+            umma_tf32_ts(tmem_base + n1, a_lo + k * UK, umma_desc_mn(b_hi + bo + ko, BOX), idesc2, first);
+            umma_tf32_ts(tmem_base + n1, a_hi + k * UK, umma_desc_mn(b_lo + bo + ko, BOX), idesc2, 1u);
+            umma_tf32_ts(tmem_base + n1, a_hi + k * UK, umma_desc_mn(b_hi + bo + ko, BOX), idesc2, 1u);
           }
         }
         umma_commit(empty + st);
@@ -843,29 +684,27 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant_
       const uint32_t ph = (it / S) & 1;
       mbar_wait(full + st, ph);
       uint8_t* base = smem + static_cast<size_t>(st) * stage_bytes;
-      if (!(g.diag & 1)) {
-        const uint32_t colp = smem_u32(base) + quad * BOX + lane * 4;
-        float a[BKR];
+      const uint32_t colp = smem_u32(base) + quad * BOX + lane * 4;
+      float a[BKR];
 #pragma unroll
-        for (int m = 0; m < BKR; ++m) asm volatile("ld.shared.f32 %0, [%1];" : "=f"(a[m]) : "r"(colp + m * 128));
-        uint32_t hi[BKR], lo[BKR];
+      for (int m = 0; m < BKR; ++m) asm volatile("ld.shared.f32 %0, [%1];" : "=f"(a[m]) : "r"(colp + m * 128));
+      uint32_t hi[BKR], lo[BKR];
 #pragma unroll
-        for (int m = 0; m < BKR; ++m) {
-          const uint32_t h = (__float_as_uint(a[m]) + 0x1000u) & 0xFFFFE000u;
-          hi[m] = h;
-          lo[m] = __float_as_uint(a[m] - __uint_as_float(h));
-          bsum += a[m];
-        }
-        const uint32_t ta = lane_addr + g.tm_a + st * 2 * BKR;
-        if constexpr (BKR == 32) {
-          tmem_st32(ta, hi);
-          tmem_st32(ta + BKR, lo);
-        } else {
-          tmem_st16(ta, hi);
-          tmem_st16(ta + BKR, lo);
-        }
+      for (int m = 0; m < BKR; ++m) {
+        const uint32_t h = (__float_as_uint(a[m]) + 0x1000u) & 0xFFFFE000u;
+        hi[m] = h;
+        lo[m] = __float_as_uint(a[m] - __uint_as_float(h));
+        bsum += a[m];
       }
-      if (!(g.diag & 2)) split_tile(base + A_RAW, base + A_RAW + b_bytes, b_bytes, wtid);
+      const uint32_t ta = lane_addr + g.tm_a + st * 2 * BKR;
+      if constexpr (BKR == 32) {
+        tmem_st32(ta, hi);
+        tmem_st32(ta + BKR, lo);
+      } else {
+        tmem_st16(ta, hi);
+        tmem_st16(ta + BKR, lo);
+      }
+      split_tile(base + A_RAW, base + A_RAW + b_bytes, b_bytes, wtid);
       asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
       fence_proxy_async();
       tc_fence_before();
@@ -880,7 +719,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant_
     for (int c = 0; c < width; c += 16) {
       float v[16];
       tmem_ld16(lane_addr + c, v);
-      if (row < g.n && !(g.diag & 8)) {
+      if (row < g.n) {
         float* cp = g.dW + static_cast<size_t>(row) * g.lddw + k0 + c;
 #pragma unroll
         for (int q = 0; q < 4; ++q)
@@ -905,13 +744,13 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant_
 //   MMA       : kind::f16, A from TMEM, B MN-major from the bf16 ring; the raw slot is free again as soon as the conversion is done
 // ================================================================================================
 // The raw ring (R slots: what TMA has in flight) and the bf16 ring (SB slots: what the tensor core reads) are sized separately, and the rows
-// of the reduction per stage are a template parameter, so that the pipeline shape can be measured (scripts/bench_wgrad_cfg.sh, RR_WG3_CFG).
+// of the reduction per stage (32 or 64) are a template parameter.
 // Measured on [321 778 x 304]^T [321 778 x 304] (profiles/r02_wgrad_cfg.md): 32 rows, 2 + 2 slots 266-273 us; 32 rows, 3 + 1 slots 330 us;
-// 16 rows with 4 + 2, 5 + 3, 6 + 2 or 5 + 2 slots 361 us each.  The clock64 trace of one CTA (RR_TC_DIAG & 16, profiles/r02_wgrad_trace.md)
-// says why: a raw slot's turn-around is TMA issue ~1200 clk (14 boxes at the TMA unit's ~85 clk per 32-float box) + arrival ~1000 + conversion
-// ~1650 (= the stage's 212 KB of shared-memory traffic at 128 B/clk) + hand-offs ~500, and two slots make that 2212 clk per stage; 16-row
-// stages double the per-row box cost, and a third 57 KB raw slot does not fit beside two 40 KB bf16 slots.  Narrow X tiles do fit more raw
-// slots (default: up to 6), worth 6-9 % there.
+// 16 rows with 4 + 2, 5 + 3, 6 + 2 or 5 + 2 slots 361 us each.  The timeline of one CTA's hand-offs (DESIGN.md §4.2) says why: a raw slot's
+// turn-around is TMA issue ~1200 clk (14 boxes at the TMA unit's ~85 clk per 32-float box) + arrival ~1000 + conversion ~1650 (= the stage's
+// 212 KB of shared-memory traffic at 128 B/clk) + hand-offs ~500, and two slots make that 2212 clk per stage; 16-row stages double the
+// per-row box cost, and a third 57 KB raw slot does not fit beside two 40 KB bf16 slots.  Narrow X tiles do fit more raw slots (up to 6),
+// worth 6-9 % there.
 constexpr int W3_A_COLS = 128;               // dZ columns per CTA == TMEM lanes
 
 template <int BKR>
@@ -928,8 +767,9 @@ __device__ __forceinline__ uint64_t umma_desc_mn_bf16(uint32_t smem_addr) {
 constexpr int W3_WORKERS = 256;   // 8 conversion warps (12 measured no faster): with 4 the fp32 -> bf16 conversion (not the MMAs) paced the kernel
 constexpr int W3_THREADS = 64 + W3_WORKERS;
 
-template <int BKR, bool TR = false>
+template <int BKR>
 __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_constant__ WgArgs g) {
+  static_assert(BKR == 32 || BKR == 64, "stages of 32 or 64 rows of the reduction");
   constexpr int BOX = BKR * 128;               // bytes of one raw TMA box [BKR x 32 floats] == one bf16 MN block [BKR x 64 bf16]
   constexpr int A_RAW = 4 * BOX;               // dZ: 128 columns
   extern __shared__ uint8_t smem_raw[];
@@ -953,10 +793,6 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
   const int m_end = min(g.M, m_beg + g.m_chunk);
   const int nst = (m_end - m_beg + BKR - 1) / BKR;
   const int width = min(g.kt, g.k_pad - k0);
-  const bool tracing = TR && g.trace != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0;
-  auto stamp = [&](int it, int slot) {      // TR is a separate instantiation: the stamps cost the default kernel nothing
-    if (TR && tracing && it < WG_TRACE_STAGES) g.trace[it * WG_TRACE_SLOTS + slot] = clock64();
-  };
 
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < R; ++s) {
@@ -990,14 +826,12 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
         const int st = it % R;
         const uint32_t ph = (it / R) & 1;
         mbar_wait(raw_empty + st, ph ^ 1);
-        stamp(it, 0);
         uint8_t* base = raw0 + static_cast<size_t>(st) * raw_bytes;
         const int m = m_beg + it * BKR;
         mbar_expect_tx(raw_full + st, tx);
         // ~85 clk per box: the TMA unit's rate for 32-float x 32-row boxes (one box per lane from 14 lanes takes exactly as long)
         for (int j = 0; j < 4; ++j) tma_load_2d(&g.tmA, raw_full + st, base + j * BOX, n0 + 32 * j, m);
         for (int j = 0; j < g.nb; ++j) tma_load_2d(&g.tmB, raw_full + st, base + A_RAW + j * BOX, k0 + 32 * j, m);
-        stamp(it, 1);
       }
     }
   } else if (warp == 1) {
@@ -1012,34 +846,29 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
         const uint32_t ph = (it / SB) & 1;
         mbar_wait(ready + st, ph);
         tc_fence_after();
-        stamp(it, 2);
         const uint32_t b_hi = smem_u32(bf0 + static_cast<size_t>(st) * bf_bytes), b_lo = b_hi + nblk * BOX;
         const uint32_t a_hi = tmem_base + g.tm_a + st * BKR, a_lo = a_hi + BKR / 2;
-        if (!(g.diag & 4)) {
 #pragma unroll
-          for (int k = 0; k < BKR / 16; ++k) {
-            const uint32_t ko = k * 2048;              // next 16 rows of the reduction = two 8-row atoms
-            const uint32_t first = (it > 0 || k > 0) ? 1u : 0u;
-            umma_bf16_ts(tmem_base, a_lo + k * 8, umma_desc_mn_bf16<BKR>(b_hi + ko), idesc1, first);
-            umma_bf16_ts(tmem_base, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_lo + ko), idesc1, 1u);
-            umma_bf16_ts(tmem_base, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_hi + ko), idesc1, 1u);
-            if (n2) {
-              const uint32_t bo = static_cast<uint32_t>(n1 / 64) * BOX;
-              umma_bf16_ts(tmem_base + n1, a_lo + k * 8, umma_desc_mn_bf16<BKR>(b_hi + bo + ko), idesc2, first);
-              umma_bf16_ts(tmem_base + n1, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_lo + bo + ko), idesc2, 1u);
-              umma_bf16_ts(tmem_base + n1, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_hi + bo + ko), idesc2, 1u);
-            }
+        for (int k = 0; k < BKR / 16; ++k) {
+          const uint32_t ko = k * 2048;                // next 16 rows of the reduction = two 8-row atoms
+          const uint32_t first = (it > 0 || k > 0) ? 1u : 0u;
+          umma_bf16_ts(tmem_base, a_lo + k * 8, umma_desc_mn_bf16<BKR>(b_hi + ko), idesc1, first);
+          umma_bf16_ts(tmem_base, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_lo + ko), idesc1, 1u);
+          umma_bf16_ts(tmem_base, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_hi + ko), idesc1, 1u);
+          if (n2) {
+            const uint32_t bo = static_cast<uint32_t>(n1 / 64) * BOX;
+            umma_bf16_ts(tmem_base + n1, a_lo + k * 8, umma_desc_mn_bf16<BKR>(b_hi + bo + ko), idesc2, first);
+            umma_bf16_ts(tmem_base + n1, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_lo + bo + ko), idesc2, 1u);
+            umma_bf16_ts(tmem_base + n1, a_hi + k * 8, umma_desc_mn_bf16<BKR>(b_hi + bo + ko), idesc2, 1u);
           }
         }
         umma_commit(mma_done + st);
-        stamp(it, 3);
       }
       umma_commit(acc_bar);
     }
   } else {
     const int wtid = threadIdx.x - 64;
     const int quad = warp & 3;
-    const int tw = (TR && lane == 0) ? (warp == 2 ? 4 : (warp == 9 ? 10 : -1)) : -1;   // traced: one dZ + X warp, one X-only warp
     const int r = quad * 32 + lane;                    // TMEM lane == column n0 + r of dZ
     const uint32_t lane_addr = tmem_base + (static_cast<uint32_t>(quad * 32) << 16);
     const int G = g.nb * 4;                            // 8-column groups per row of the X tile (whole boxes: the padding converts zeros)
@@ -1049,12 +878,10 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
     for (int it = 0; it < nst; ++it) {
       const int rs = it % R, bs = it % SB;
       mbar_wait(raw_full + rs, (it / R) & 1);
-      if (TR && tw >= 0) stamp(it, tw);
       mbar_wait(mma_done + bs, ((it / SB) & 1) ^ 1);  // the MMAs of the previous lap are done with this bf16 slot and TMEM slot
       tc_fence_after();
-      if (TR && tw >= 0) stamp(it, tw + 1);
       const uint32_t raw = smem_u32(raw0 + static_cast<size_t>(rs) * raw_bytes);
-      if (a_warp && !(g.diag & 1)) {
+      if (a_warp) {
         const uint32_t colp = raw + quad * BOX + lane * 4;
         float a[BKR];
 #pragma unroll
@@ -1069,43 +896,36 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
         if constexpr (BKR == 64) {
           tmem_st32(ta, hi);
           tmem_st32(ta + 32, lo);
-        } else if constexpr (BKR == 32) {
+        } else {
           tmem_st16(ta, hi);
           tmem_st16(ta + 16, lo);
-        } else {
-          tmem_st8(ta, hi);
-          tmem_st8(ta + 8, lo);
         }
       }
-      if (TR && tw >= 0) stamp(it, tw + 2);
-      if (!(g.diag & 2)) {
-        const uint32_t xraw = raw + A_RAW;
-        const uint32_t xhi = smem_u32(bf0 + static_cast<size_t>(bs) * bf_bytes), xlo = xhi + nblk * BOX;
-        int m = wtid / G, cg = wtid - m * G;
-        for (; m < BKR;) {
-          const int jb = cg >> 2, c2 = (cg & 3) << 1, sw = m & 7;
-          const uint32_t rp = xraw + jb * BOX + m * 128;
-          // two 16-byte chunks of 4 floats; boxes of odd index read theirs in the opposite order: 8 consecutive lanes hit 8 distinct bank groups
-          const int first = c2 + (jb & 1), second = c2 + 1 - (jb & 1);
-          const float4 f0 = lds_f4(rp + ((first ^ sw) << 4)), f1 = lds_f4(rp + ((second ^ sw) << 4));
-          const float4 lo4 = (jb & 1) ? f1 : f0, hi4 = (jb & 1) ? f0 : f1;     // columns 8cg..8cg+3 | 8cg+4..8cg+7
-          uint32_t h[4], l[4];
-          split_bf16_pair(lo4.x, lo4.y, h[0], l[0]);
-          split_bf16_pair(lo4.z, lo4.w, h[1], l[1]);
-          split_bf16_pair(hi4.x, hi4.y, h[2], l[2]);
-          split_bf16_pair(hi4.z, hi4.w, h[3], l[3]);
-          const uint32_t off = (cg >> 3) * BOX + m * 128 + (((cg & 7) ^ sw) << 4);
-          asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(xhi + off), "r"(h[0]), "r"(h[1]), "r"(h[2]), "r"(h[3]) : "memory");
-          asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(xlo + off), "r"(l[0]), "r"(l[1]), "r"(l[2]), "r"(l[3]) : "memory");
-          m += step_m;
-          cg += step_c;
-          if (cg >= G) {
-            cg -= G;
-            ++m;
-          }
+      const uint32_t xraw = raw + A_RAW;
+      const uint32_t xhi = smem_u32(bf0 + static_cast<size_t>(bs) * bf_bytes), xlo = xhi + nblk * BOX;
+      int m = wtid / G, cg = wtid - m * G;
+      for (; m < BKR;) {
+        const int jb = cg >> 2, c2 = (cg & 3) << 1, sw = m & 7;
+        const uint32_t rp = xraw + jb * BOX + m * 128;
+        // two 16-byte chunks of 4 floats; boxes of odd index read theirs in the opposite order: 8 consecutive lanes hit 8 distinct bank groups
+        const int first = c2 + (jb & 1), second = c2 + 1 - (jb & 1);
+        const float4 f0 = lds_f4(rp + ((first ^ sw) << 4)), f1 = lds_f4(rp + ((second ^ sw) << 4));
+        const float4 lo4 = (jb & 1) ? f1 : f0, hi4 = (jb & 1) ? f0 : f1;     // columns 8cg..8cg+3 | 8cg+4..8cg+7
+        uint32_t h[4], l[4];
+        split_bf16_pair(lo4.x, lo4.y, h[0], l[0]);
+        split_bf16_pair(lo4.z, lo4.w, h[1], l[1]);
+        split_bf16_pair(hi4.x, hi4.y, h[2], l[2]);
+        split_bf16_pair(hi4.z, hi4.w, h[3], l[3]);
+        const uint32_t off = (cg >> 3) * BOX + m * 128 + (((cg & 7) ^ sw) << 4);
+        asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(xhi + off), "r"(h[0]), "r"(h[1]), "r"(h[2]), "r"(h[3]) : "memory");
+        asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(xlo + off), "r"(l[0]), "r"(l[1]), "r"(l[2]), "r"(l[3]) : "memory");
+        m += step_m;
+        cg += step_c;
+        if (cg >= G) {
+          cg -= G;
+          ++m;
         }
       }
-      if (TR && tw >= 0) stamp(it, tw + 3);
       asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
       fence_proxy_async();
       tc_fence_before();
@@ -1114,7 +934,6 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
         mbar_arrive(ready + bs);
         mbar_arrive(raw_empty + rs);
       }
-      if (TR && tw >= 0) stamp(it, tw + 4);
     }
     if (a_warp && g.dbias != nullptr && blockIdx.y == 0 && n0 + r < g.n) atomicAdd(g.dbias + n0 + r, bsum);
     mbar_wait(acc_bar, 0);
@@ -1123,7 +942,7 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
     for (int c = 0; a_warp && c < width; c += 16) {
       float v[16];
       tmem_ld16(lane_addr + c, v);
-      if (row < g.n && !(g.diag & 8)) {
+      if (row < g.n) {
         float* cp = g.dW + static_cast<size_t>(row) * g.lddw + k0 + c;
 #pragma unroll
         for (int q = 0; q < 4; ++q)
@@ -1194,10 +1013,6 @@ static int make_map_bf16(CUtensorMap* map, const uint16_t* ptr, int rows, int co
 bool tc_linear_bf16_supported(int M, int n, int k, int ldx, int ldw) {
   return M > 0 && n >= 16 && !(n & 15) && k > 0 && !(k & 3) && !(ldx & 3) && !(ldw & 7);
 }
-// epilogue warps of k_tc_gemm2: 16 (16-column sub-blocks, 704 threads at 80 registers) by default; RR_TC_EW=8 / 4 select the earlier
-// 32-column-block flavours (8 warps: -13 % forward GEMM time per step, scripts/bench_gemm.py diag)
-static int epilogue_warps() { return switches().tc_ew; }
-
 // Full-featured bf16-split linear: Y = epi(X1 W1^T + X2 W2^T) with every weight given as bf16 (hi, lo) images.
 int tc_linear_bf16_full(int M, int n, const float* X1, int ldx1, const uint16_t* W1hi, const uint16_t* W1lo, int ldw1, int k1, const float* X2, int ldx2,
                         const uint16_t* W2hi, const uint16_t* W2lo, int ldw2, int k2, const float* bias, const float* resid, int ldr, float* Y, int ldy,
@@ -1218,7 +1033,6 @@ int tc_linear_bf16_full(int M, int n, const float* X1, int ldx1, const uint16_t*
     g.src[1].K = k2;
   }
   g.presplit = 1;
-  g.diag = switches().tc_diag;
   g.M = M;
   g.N = n;
   g.C = Y;
@@ -1234,15 +1048,13 @@ int tc_linear_bf16_full(int M, int n, const float* X1, int ldx1, const uint16_t*
   g.stream_id = stream_id;
   static PerDeviceOnce attr_set;
   if (attr_set.need()) {
-    RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     attr_set.mark();
   }
-  const size_t smem = static_cast<size_t>(S2_BF) * STAGE2_BF + 1024 + 256 + 8 * 4096;
+  const size_t smem = static_cast<size_t>(S2_BF) * STAGE2_BF + 1024 + 256 + 16 * 2048;
   const int total_tiles = ((M + BM - 1) / BM) * ((n + NT2 - 1) / NT2);
   const int ctas = total_tiles < num_sms() ? total_tiles : num_sms();
-  if (epilogue_warps() == 16) RR_CUDA(launch_pdl(k_tc_gemm2<16, true>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
-  else RR_CUDA(launch_pdl(k_tc_gemm2<8, true>, dim3(ctas), dim3(THREADS2_BASE + 256), smem, s, g));
+  RR_CUDA(launch_pdl(k_tc_gemm2<16, true>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
   RR_LAUNCH_CHECK("k_tc_gemm2<bf16>");
   return RR_OK;
 }
@@ -1307,25 +1119,6 @@ int tc_dgrad_standalone(int M, int n, int k, const float* dZ, int lddz, const fl
                    nullptr);
 }
 
-// RR_TC_DIAG & 16: CTA (0,0,0) of every k_tc_wgrad3 launch stamps clock64 at its pipeline hand-offs (a diagnostic; see scripts/wgrad_trace.py)
-static unsigned long long* wg_trace_buffer() {
-  static unsigned long long* buf[16] = {};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 16) return nullptr;
-  if (!buf[dev] && cudaMalloc(&buf[dev], sizeof(unsigned long long) * tc::WG_TRACE_STAGES * tc::WG_TRACE_SLOTS) != cudaSuccess) buf[dev] = nullptr;
-  return buf[dev];
-}
-
-int tc_wgrad_trace(unsigned long long* host_out, int n) {
-  unsigned long long* b = wg_trace_buffer();
-  const int cap = tc::WG_TRACE_STAGES * tc::WG_TRACE_SLOTS;
-  RR_REQUIRE(b != nullptr && host_out != nullptr && n > 0 && n <= cap, "wgrad trace: no buffer or n outside [1, %d]", cap);
-  RR_CUDA(cudaDeviceSynchronize());
-  RR_CUDA(cudaMemcpy(host_out, b, sizeof(unsigned long long) * n, cudaMemcpyDeviceToHost));
-  return RR_OK;
-}
-
 bool tc_wgrad_supported(int M, int n, int k, int lddz, int ldx) {
   return M > 0 && n >= 4 && k >= 4 && !(n & 3) && !(k & 3) && !(lddz & 3) && !(ldx & 3);
 }
@@ -1334,73 +1127,61 @@ int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int
   using namespace tc;
   ProfScope prof_scope(KC_GEMM_WGRAD, s);
   WgArgs g{};
-  const int kt_cap = switches().wg_kt == 160 ? 160 : MAX_NT;
   const int k_pad = (k + 15) / 16 * 16;                  // columns past k are zero-filled by TMA and never written back
-  const int ktiles = (k_pad + kt_cap - 1) / kt_cap;
-  g.kt = ktiles == 1 ? k_pad : kt_cap;
+  const int ktiles = (k_pad + MAX_NT - 1) / MAX_NT;
+  g.kt = ktiles == 1 ? k_pad : MAX_NT;
   g.nb = (g.kt + 31) / 32;
   g.tm_a = g.kt <= 160 ? 160 : 320;
-  // wide tiles: 16-row stages (4 x 48 KB in flight instead of 2 x 96 KB); narrow tiles fit 3+ stages of 32 rows
-  if (g_bwd_bf16.load() && !switches().wg_tf32) {
-    // 3 x bf16: raw ring (dZ + X boxes as TMA lands them) and bf16 ring (hi + lo images + the TMEM A slots), sized separately.
-    // RR_WG3_CFG="rows per stage,raw slots,bf16 slots" overrides the default (timing experiments).
-    // Narrow X tiles (<= 96 columns: the feature-matrix gradients W_i, W_o[:, :64], MPNDiff W_h[:, h:]) take 64 rows per stage: a stage's
-    // hand-offs and fixed conversion cost (~1400 clk, profiles/r02_wgrad_trace.md) are then paid half as often, and two 56 KB raw slots
-    // still fit.  RR_WG3_CFG's first field (16 / 32 / 64) overrides the choice.
-    int bkr = switches().wg3_bkr == 16 ? 16 : (switches().wg3_bkr == 64 ? 64 : 32), R = switches().wg3_raw, SB = switches().wg3_bf;
-    if (switches().wg3_bkr == 0) bkr = g.kt <= 96 ? 64 : 32;
-    if (bkr == 64 && g.kt > 96) bkr = 32;
+  if (g_bwd_bf16.load()) {
+    // 3 x bf16: raw ring (dZ + X boxes as TMA lands them, up to 6 slots) and bf16 ring (hi + lo images + the TMEM A slots, 2 slots),
+    // sized separately.  Narrow X tiles (<= 96 columns: the feature-matrix gradients W_i, W_o[:, :64], MPNDiff W_h[:, h:]) take 64 rows per
+    // stage: a stage's hand-offs and fixed conversion cost (~1400 clk, DESIGN.md §4.2) are then paid half as often, and two
+    // 56 KB raw slots still fit.
+    const int bkr = g.kt <= 96 ? 64 : 32;
     const int box = bkr * 128;
     const int nblk = (g.kt + 63) / 64;
     const int raw_bytes = 4 * box + g.nb * box, bf_bytes = 2 * nblk * box;
-    if (SB < 1) SB = 1;
-    if (SB > (512 - g.tm_a) / bkr) SB = (512 - g.tm_a) / bkr;
-    if (SB > 4) SB = 4;
+    int R = 6, SB = 2;
+    if (SB > (512 - g.tm_a) / bkr) SB = (512 - g.tm_a) / bkr;       // TMEM: accumulator + bkr columns of A per bf16 slot
     while (SB > 1 && 2 * raw_bytes + SB * bf_bytes > SMEM_LIMIT - 2048) --SB;
-    int Rmax = (SMEM_LIMIT - 2048 - SB * bf_bytes) / raw_bytes;
+    const int Rmax = (SMEM_LIMIT - 2048 - SB * bf_bytes) / raw_bytes;
     if (R > Rmax) R = Rmax;
-    if (R > 8) R = 8;
-    if (R >= 2 && SB >= 1) {
-      g.stages = R;
-      g.bf_stages = SB;
-      RR_TRY(make_map(&g.tmA, dZ, M, n, lddz, bkr, CU_TENSOR_MAP_SWIZZLE_NONE));
-      RR_TRY(make_map(&g.tmB, X, M, k, ldx, bkr, CU_TENSOR_MAP_SWIZZLE_128B));
-      g.M = M;
-      g.n = n;
-      g.k = k;
-      g.k_pad = k_pad;
-      g.dW = dW;
-      g.lddw = lddw;
-      g.dbias = dbias;
-      g.diag = switches().tc_diag;
-      g.trace = (g.diag & 16) ? wg_trace_buffer() : nullptr;
-      const int ntiles3 = (n + BM - 1) / BM;
-      int splits3 = num_sms() / (ntiles3 * ktiles);
-      const int max_splits3 = (M + 8 * 32 - 1) / (8 * 32);
-      if (splits3 > max_splits3) splits3 = max_splits3;
-      if (splits3 < 1) splits3 = 1;
-      int chunk3 = (M + splits3 - 1) / splits3;
-      chunk3 = (chunk3 + bkr - 1) / bkr * bkr;          // whole stages: a stage never reaches into the next split's rows
-      splits3 = (M + chunk3 - 1) / chunk3;
-      g.m_chunk = chunk3;
-      static PerDeviceOnce attr3_set;
-      if (attr3_set.need()) {
-        RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-        attr3_set.mark();
-      }
-      const size_t smem3 = static_cast<size_t>(R) * raw_bytes + static_cast<size_t>(SB) * bf_bytes + 1024 + 512;
-      if (bkr == 32 && g.trace) RR_CUDA(launch_pdl(k_tc_wgrad3<32, true>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
-      else if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad3<32>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
-      else if (bkr == 64) RR_CUDA(launch_pdl(k_tc_wgrad3<64>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
-      else RR_CUDA(launch_pdl(k_tc_wgrad3<16>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
-      RR_LAUNCH_CHECK("k_tc_wgrad3");
-      return RR_OK;
+    RR_REQUIRE(R >= 2, "tc_wgrad: %d columns do not fit two raw pipeline slots", g.kt);
+    g.stages = R;
+    g.bf_stages = SB;
+    RR_TRY(make_map(&g.tmA, dZ, M, n, lddz, bkr, CU_TENSOR_MAP_SWIZZLE_NONE));
+    RR_TRY(make_map(&g.tmB, X, M, k, ldx, bkr, CU_TENSOR_MAP_SWIZZLE_128B));
+    g.M = M;
+    g.n = n;
+    g.k = k;
+    g.k_pad = k_pad;
+    g.dW = dW;
+    g.lddw = lddw;
+    g.dbias = dbias;
+    const int ntiles3 = (n + BM - 1) / BM;
+    int splits3 = num_sms() / (ntiles3 * ktiles);
+    const int max_splits3 = (M + 8 * 32 - 1) / (8 * 32);
+    if (splits3 > max_splits3) splits3 = max_splits3;
+    if (splits3 < 1) splits3 = 1;
+    int chunk3 = (M + splits3 - 1) / splits3;
+    chunk3 = (chunk3 + bkr - 1) / bkr * bkr;          // whole stages: a stage never reaches into the next split's rows
+    splits3 = (M + chunk3 - 1) / chunk3;
+    g.m_chunk = chunk3;
+    static PerDeviceOnce attr3_set;
+    if (attr3_set.need()) {
+      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+      attr3_set.mark();
     }
+    const size_t smem3 = static_cast<size_t>(R) * raw_bytes + static_cast<size_t>(SB) * bf_bytes + 1024 + 512;
+    if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad3<32>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
+    else RR_CUDA(launch_pdl(k_tc_wgrad3<64>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
+    RR_LAUNCH_CHECK("k_tc_wgrad3");
+    return RR_OK;
   }
-  const int bkr = switches().wg_bkr ? (switches().wg_bkr == 16 ? 16 : 32) : (g.kt > 160 ? 16 : 32);
+  // 3 x TF32 (rr_set_backward_bf16(0)): wide tiles take 16-row stages (4 x 48 KB in flight instead of 2 x 96 KB); narrow tiles fit 3+ stages
+  // of 32 rows
+  const int bkr = g.kt > 160 ? 16 : 32;
   const int box = bkr * 128;
   const int stage_bytes = 4 * box + 2 * g.nb * box;
   int S = (SMEM_LIMIT - 2048) / stage_bytes;
@@ -1417,7 +1198,6 @@ int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int
   g.dW = dW;
   g.lddw = lddw;
   g.dbias = dbias;
-  g.diag = switches().tc_diag;
   // one CTA per SM (shared memory and TMEM are both taken whole): never more CTAs than SMs, or the stragglers run as a second wave
   const int ntiles = (n + BM - 1) / BM;
   int splits = num_sms() / (ntiles * ktiles);
@@ -1454,16 +1234,10 @@ int tc_linear(int M, int n, const float* X1, int ldx1, const float* W1, int ldw1
               int kclass, cudaStream_t s, const float* W1lo, const float* W2lo) {
   using namespace tc;
   ProfScope prof_scope(kclass, s);
-  if (switches().tc_fake_presplit && !W1lo) {  // timing experiments only (scripts/bench_gemm.py): wrong numerics, same traffic as pre-split weights
-    W1lo = W1;
-    W2lo = W2;
-  }
   Args g{};
   const bool two = X2 && k2 > 0;
   g.nsrc = two ? 2 : 1;
   g.presplit = (W1lo != nullptr && (!two || W2lo != nullptr)) ? 1 : 0;
-  g.diag = switches().tc_diag;
-  g.trace = (g.diag & 16) ? wg_trace_buffer() : nullptr;
   RR_TRY(make_map(&g.src[0].tmA, X1, M, k1, ldx1, BM));
   RR_TRY(make_map(&g.src[0].tmB, W1, n, k1, ldw1, NT2));
   if (g.presplit) RR_TRY(make_map(&g.src[0].tmBlo, W1lo, n, k1, ldw1, NT2));
@@ -1489,20 +1263,13 @@ int tc_linear(int M, int n, const float* X1, int ldx1, const float* W1, int ldw1
   g.stream_id = stream_id;
   static PerDeviceOnce attr_set;
   if (attr_set.need()) {
-    RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<16, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     attr_set.mark();
   }
-  const size_t smem = static_cast<size_t>(S2) * STAGE2 + 1024 + 256 + 8 * 4096;  // ring | barriers | epilogue staging
-  const int ew = epilogue_warps();
+  const size_t smem = static_cast<size_t>(S2) * STAGE2 + 1024 + 256 + 16 * 2048;  // ring | barriers | epilogue staging (16 warps x 2 KB)
   const int total_tiles = ((M + BM - 1) / BM) * ((n + NT2 - 1) / NT2);
   const int ctas = total_tiles < num_sms() ? total_tiles : num_sms();
-  if (ew == 16 && g.trace) RR_CUDA(launch_pdl(k_tc_gemm2<16, false, true>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
-  else if (ew == 16) RR_CUDA(launch_pdl(k_tc_gemm2<16, false>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
-  else if (ew == 8) RR_CUDA(launch_pdl(k_tc_gemm2<8, false>, dim3(ctas), dim3(THREADS2_BASE + 256), smem, s, g));
-  else RR_CUDA(launch_pdl(k_tc_gemm2<4, false>, dim3(ctas), dim3(THREADS2_BASE + 128), smem, s, g));
+  RR_CUDA(launch_pdl(k_tc_gemm2<16, false>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
   RR_LAUNCH_CHECK("k_tc_gemm2");
   return RR_OK;
 }

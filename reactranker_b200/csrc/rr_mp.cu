@@ -391,7 +391,7 @@ static void atom_launch_dims(int n_atoms, int ld, dim3* grid, dim3* block) {
   *block = dim3(threads);
 }
 
-// second-generation kernels (rr_mp_pipe.cu); RR_MP_V1=1 keeps the first generation for A/B measurements
+// second-generation kernels (rr_mp_pipe.cu); RR_MP_V1=1 selects the first generation, which the tests use as the pipeline's reference
 enum { PIPE_BOND_FWD = 0, PIPE_BOND_BWD = 1, PIPE_NBR_FWD = 2, PIPE_NBR_BWD_BOND = 3, PIPE_NBR_BWD_ATOM = 4 };
 static bool use_pipe() { return switches().mp_v1 != 1; }
 

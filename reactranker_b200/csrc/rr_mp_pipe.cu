@@ -26,7 +26,8 @@
 namespace rr {
 namespace pipe {
 
-constexpr int kFast = 4;          // neighbours staged per atom; larger in-degrees read the rest straight from global memory
+constexpr int kFast = 4;          // neighbours staged per atom; larger in-degrees read the rest straight from global memory (fewer
+                                  // staged rows and a deeper ring measured slower: profiles/r02_mp_kstage.md)
 constexpr int MAX_CONSUMERS = 512; // consumer threads: 16 warps when at least four such stages fit, else 8
 constexpr int PRODUCERS = 4;      // producer warps: one warp issuing every stage was the bottleneck (a single warp retires ~1 instruction per 4-5
                                   // cycles and a stage costs it several hundred); the warps take the rounds in turn
@@ -483,10 +484,10 @@ int rowpipe_launch(int op, const rr_graph* g, int which, const float* src, float
   if (cpr < 1 || cpr > 256 || (ld & 3)) return RR_ERR_UNSUPPORTED;
   A.row_bytes = ld * 4;
   const bool fused = y != nullptr;
-  A.kstage = (switches().mp_kstage >= 1 && switches().mp_kstage <= kFast) ? switches().mp_kstage : kFast;
+  A.kstage = kFast;   // a kernel argument, not a constant: compiled with a constant kFast the bond-row backward ran 2 % slower (B200, 1000 W)
   // measured (scripts/bench_mp.py): the bond-row backward gains 30 % (273 -> 190 us) from reducing into acc, the atom-row backward, whose
   // accumulator rows are one contiguous bulk copy per stage, loses 13 %: every acc element is added to exactly once, so both are deterministic
-  A.acc_red = switches().mp_acc_red >= 0 ? switches().mp_acc_red : (op == BOND_BWD);
+  A.acc_red = (op == BOND_BWD);
   const bool stage_acc = fused && A.acc_mode == 2 && !A.acc_red;
   switch (op) {
     case BOND_FWD: A.n_nbr = 1; A.n_own = 0; break;
@@ -495,7 +496,7 @@ int rowpipe_launch(int op, const rr_graph* g, int which, const float* src, float
     case NBR_BWD_BOND: A.n_nbr = fused ? (stage_acc ? 2 : 1) : 0; A.n_own = 1; break;
     default: A.n_nbr = 1; A.n_own = fused ? (stage_acc ? 3 : 2) : 1; break;
   }
-  for (int consumers = switches().mp_consumers ? switches().mp_consumers : MAX_CONSUMERS; consumers >= 256; consumers -= 256) {
+  for (int consumers = MAX_CONSUMERS; consumers >= 256; consumers -= 256) {
     A.consumer_warps = consumers / 32;
     A.apb = consumers / cpr;
     if (A.apb > 32) A.apb = 32;

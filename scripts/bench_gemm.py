@@ -1,5 +1,9 @@
-"""GPU micro-benchmark of the dense-layer kernels through the C ABI at the model's shapes (c5 batch: 160 889 bond rows, 82 001 atom rows).
-RR_TC_DIAG / RR_TC_FAKE_PRESPLIT switch off parts of the tcgen05 kernel (timing experiments, results are then wrong)."""
+"""GPU micro-benchmark of the dense-layer kernels through the C ABI at the model's shapes (c5 batch: 160 889 bond rows, 82 001 atom rows):
+the forward GEMM with its epilogues, the tensor-core dgrad (rr_linear_dgrad_tc), and the weight gradient in both backward operand splits
+(rr_set_backward_bf16 1 / 0).
+
+rr_linear_fwd is handed fp32 weights and splits them inside the kernel, while the model's own launches take weight images split once per
+step; the per-launch times of the model's GEMMs are in bench.py's roofline."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -40,6 +44,17 @@ def fwd_case(M, n, k1, k2=0, epi=True, p=0.1):
     return run, 2.0 * M * n * (k1 + k2), (M * (k1 + k2) + M * n * (2 if epi else 1)) * 4.0, (X1, W1, X2, W2, bias, R, Y)
 
 
+def dgrad_case(M, n, k, accumulate):
+    dZ = torch.randn(M, n, device=dev)
+    W = torch.randn(n, k, device=dev) * 0.05
+    dX = torch.zeros(M, k, device=dev)
+    scratch = torch.empty(int(L.rr_linear_dgrad_tc_scratch_bytes(n, k)), dtype=torch.uint8, device=dev)
+
+    def run():
+        _lib.check(L.rr_linear_dgrad_tc(M, n, k, dZ.data_ptr(), n, W.data_ptr(), k, dX.data_ptr(), k, accumulate, scratch.data_ptr(), scratch.numel(), st()))
+    return run, 2.0 * M * n * k, (M * n + M * k * (2 if accumulate else 1)) * 4.0, (dZ, W, dX, scratch)
+
+
 def wgrad_case(M, n, k):
     dZ = torch.randn(M, n, device=dev)
     X = torch.randn(M, k, device=dev)
@@ -51,78 +66,24 @@ def wgrad_case(M, n, k):
     return run, 2.0 * M * n * k, (M * (n + k)) * 4.0, (dZ, X, dW, db)
 
 
-def report(name, run, flops, bytes_):
-    L.rr_reload_switches()          # pick up whatever RR_* switch the caller just set or removed
+def report(name, case):
+    run, flops, bytes_, _ = case
     us = timeit(run)
     print(f"{name:58s} {us:8.1f} us  {flops / us * 1e-6:7.1f} TFLOP/s  {bytes_ / us * 1e-3:7.0f} GB/s (algorithmic)", flush=True)
 
 
 B, A = 160889, 82001
-which = sys.argv[1] if len(sys.argv) > 1 else "all"
-E = os.environ
-
-
-def setenv(**kw):
-    for k, v in kw.items():
-        E[k] = str(v)
-    L.rr_reload_switches()          # the library reads its RR_* switches once; re-read after every change
-
-
-if which in ("all", "fwd"):
-    cases = [("W_h fwd  [B,304]x[304,304] bias+resid+relu+dropout", fwd_case(B, 304, 304)),
-             ("W_h fwd  same, no dropout", fwd_case(B, 304, 304, p=0.0)),
-             ("dgrad-like [B,304]x[304,304] plain", fwd_case(B, 304, 304, epi=False)),
-             ("W_i fwd  [B,88]x[88,304] plain", fwd_case(B, 304, 88, epi=False)),
-             ("W_o fwd  [A,64|304]x[.,304] two-source + relu", fwd_case(A, 304, 64, 304)),
-             ("h600: [A,608]x[608,608] plain", fwd_case(A, 608, 608, epi=False))]
-    for promo in (128, 256):
-        for ew in (4, 8):
-            for fake in ("", "1"):
-                setenv(RR_TMA_PROMO=promo, RR_TC_EW=ew, RR_TC_DIAG=0)
-                if fake:
-                    E["RR_TC_FAKE_PRESPLIT"] = "1"
-                else:
-                    E.pop("RR_TC_FAKE_PRESPLIT", None)
-                for name, (run, fl, by, _) in cases:
-                    report(f"promo={promo} ew={ew} presplit={fake or 0} {name}", run, fl, by)
-        E["RR_TC_FAKE_PRESPLIT"] = "1"
-        for diag in (8, 15):
-            setenv(RR_TC_DIAG=diag)
-            for name, (run, fl, by, _) in cases[:1]:
-                report(f"promo={promo} ew=8 presplit=1 diag={diag} {name}", run, fl, by)
-    E.pop("RR_TC_FAKE_PRESPLIT", None)
-    setenv(RR_TC_DIAG=0, RR_TMA_PROMO=128, RR_TC_EW=8)
-if which in ("all", "wgrad"):
-    cases = [("wgrad [B,304]^T[B,304]", wgrad_case(B, 304, 304)), ("wgrad [B,304]^T[B,88]", wgrad_case(B, 304, 88)),
-             ("wgrad [A,304]^T[A,304]", wgrad_case(A, 304, 304)), ("wgrad h600 [A,608]^T[A,608]", wgrad_case(A, 608, 608))]
-    for tf32 in (1, 0):
-        if tf32:
-            E["RR_WG_TF32"] = "1"
-        else:
-            E.pop("RR_WG_TF32", None)
-        setenv(RR_TC_DIAG=0)
-        for name, c in cases:
-            report(f"{'3xtf32' if tf32 else '3xbf16'} {name}", c[0], c[1], c[2])
-        for diag in (4, 3, 7, 8):
-            setenv(RR_TC_DIAG=diag)
-            report(f"{'3xtf32' if tf32 else '3xbf16'} diag={diag} {cases[0][0]}", cases[0][1][0], cases[0][1][1], cases[0][1][2])
-    setenv(RR_TC_DIAG=0)
-if which == "diag":    # what bounds the forward kernel: switch its parts off one at a time (pre-split weights as in the model)
-    E["RR_TC_FAKE_PRESPLIT"] = "1"
-    cases = [("W_h fwd bias+resid+relu+dropout", fwd_case(B, 304, 304)), ("W_h fwd bias+resid+relu", fwd_case(B, 304, 304, p=0.0)),
-             ("plain [B,304]x[304,304]", fwd_case(B, 304, 304, epi=False))]
-    names = {0: "full", 1: "no A split", 4: "no MMA", 8: "no epilogue traffic", 5: "no A split, no MMA", 12: "no MMA, no epilogue", 9: "no A split, no epilogue",
-             13: "TMA ring only"}
-    for name, (run, fl, by, _) in cases:
-        for diag, what in names.items():
-            setenv(RR_TC_DIAG=diag)
-            report(f"{name}: {what}", run, fl, by)
-    setenv(RR_TC_DIAG=0)
-    E.pop("RR_TC_FAKE_PRESPLIT", None)
-if which == "one":     # one launch of each headline kernel, for ncu
-    run, *_ = fwd_case(B, 304, 304)
-    run2, *_ = wgrad_case(B, 304, 304)
-    for _ in range(2):
-        run()
-        run2()
-    torch.cuda.synchronize()
+report("W_h fwd  [B,304]x[304,304] bias+resid+relu+dropout", fwd_case(B, 304, 304))
+report("W_h fwd  same, no dropout", fwd_case(B, 304, 304, p=0.0))
+report("W_i fwd  [B,88]x[88,304] plain", fwd_case(B, 304, 88, epi=False))
+report("W_o fwd  [A,64|304]x[.,304] two-source + relu", fwd_case(A, 304, 64, 304))
+report("plain [B,304]x[304,304]", fwd_case(B, 304, 304, epi=False))
+report("h600 resid [A,608]x[608,608]", fwd_case(A, 608, 608))
+report("dgrad 3xbf16 accumulate [2B,304]x[304,304]", dgrad_case(2 * B, 304, 304, 1))
+report("dgrad 3xbf16 plain [2B,304]x[304,304]", dgrad_case(2 * B, 304, 304, 0))
+wcases = [("[B,304]^T[B,304]", (B, 304, 304)), ("[B,304]^T[B,88]", (B, 304, 88)), ("[A,304]^T[A,304]", (A, 304, 304)),
+          ("h600 [A,608]^T[A,608]", (A, 608, 608))]
+for bf16 in (1, 0):
+    _lib.check(L.rr_set_backward_bf16(bf16))
+    for name, shape in wcases:
+        report(f"wgrad {'3xbf16' if bf16 else '3xtf32'} {name}", wgrad_case(*shape))

@@ -100,20 +100,15 @@ def test_host_philox_keep_rate_and_high_words():
 
 
 # ------------------------------------------------------------------------------------------------
-# kernel level: dense layer epilogue (SIMT and both tcgen05 epilogues) and the readout
+# kernel level: dense layer epilogue (SIMT and tcgen05) and the readout
 # ------------------------------------------------------------------------------------------------
 def S():
     return torch.cuda.current_stream().cuda_stream
 
 
-def _set_path(monkeypatch, path):
+def _set_path(path):
     L = _lib.lib()
-    if path == "simt":
-        _lib.check(L.rr_set_gemm_mode(0))
-    else:
-        monkeypatch.setenv("RR_TC_EW", path[2:])
-        L.rr_reload_switches()
-        _lib.check(L.rr_set_gemm_mode(1))
+    _lib.check(L.rr_set_gemm_mode(0 if path == "simt" else 1))
     return L
 
 
@@ -128,12 +123,12 @@ def _assert_zero_pattern(got, want, z, what):
 @pytest.mark.gpu
 @pytest.mark.parametrize("M,n,k1,k2,ldy", [(5, 16, 304, 0, 16), (130, 48, 64, 48, 48), (130, 48, 64, 48, 64), (777, 304, 304, 88, 304),
                                            (777, 304, 304, 88, 320), (4100, 608, 608, 608, 608)])
-@pytest.mark.parametrize("path", ["simt", "tc16", "tc8"])
-def test_linear_dropout_mask_is_bit_exact(monkeypatch, path, M, n, k1, k2, ldy):
-    """rr_linear_fwd with flags 3 (ReLU + dropout) and 2 (dropout only) on the SIMT kernel and on both tcgen05 epilogues (RR_TC_EW=16 / 8):
+@pytest.mark.parametrize("path", ["simt", "tc16"])
+def test_linear_dropout_mask_is_bit_exact(path, M, n, k1, k2, ldy):
+    """rr_linear_fwd with flags 3 (ReLU + dropout) and 2 (dropout only) on the SIMT kernel and on the tcgen05 kernel (16 epilogue warps):
     relu(z) * keep / (1 - p) with the host's keep mask, p in {0.1, 0.2, 0.5}, seed and stream id above 2^32.  With ldy > n the
     counter runs over the output stride: the columns [n, ldy) are never written."""
-    L = _set_path(monkeypatch, path)
+    L = _set_path(path)
     g = torch.Generator().manual_seed(M + n + ldy)
     X1, W1 = torch.randn(M, k1, generator=g), torch.randn(n, k1, generator=g) / k1 ** 0.5
     X2 = torch.randn(M, k2, generator=g) if k2 else None

@@ -377,13 +377,10 @@ def test_argument_errors_are_reported_not_crashed():
 
 @pytest.mark.parametrize("M,n,k1,k2", [(128, 48, 64, 0), (1000, 304, 88, 0), (777, 304, 304, 88), (130, 48, 64, 48), (5, 16, 304, 0),
                                        (4100, 608, 608, 608), (40000, 304, 304, 0), (300, 304, 16, 0)])
-@pytest.mark.parametrize("ew", [16, 8])
-def test_tcgen05_linear_matches_fp64(tc_mode, monkeypatch, ew, M, n, k1, k2):
+def test_tcgen05_linear_matches_fp64(tc_mode, M, n, k1, k2):
     """tcgen05 3xTF32 forward GEMM (bias + residual + ReLU epilogue, two-source K) against an fp64 matmul:
-    fp32-class accuracy, 5e-6 of the largest output.  Both epilogue flavours: 16 warps on 16-column sub-blocks (default), 8 on 32."""
-    monkeypatch.setenv("RR_TC_EW", str(ew))
+    fp32-class accuracy, 5e-6 of the largest output."""
     L = _lib.lib()
-    L.rr_reload_switches()                           # the RR_* switches are read once; re-read them after changing the environment
     g = torch.Generator().manual_seed(M + n)
     X1, W1 = torch.randn(M, k1, generator=g), torch.randn(n, k1, generator=g) / k1 ** 0.5
     X2 = torch.randn(M, k2, generator=g) if k2 else None
@@ -404,11 +401,8 @@ def test_tcgen05_linear_matches_fp64(tc_mode, monkeypatch, ew, M, n, k1, k2):
     close(Y, X1.double() @ W1.double().T, 1e-5 if k1 > 500 else 5e-6)
 
 
-@pytest.mark.parametrize("ew", [16, 8])
-def test_tcgen05_and_simt_draw_the_same_dropout_mask(tc_mode, monkeypatch, ew):
-    monkeypatch.setenv("RR_TC_EW", str(ew))
+def test_tcgen05_and_simt_draw_the_same_dropout_mask(tc_mode):
     L = _lib.lib()
-    L.rr_reload_switches()
     M, n, k, p = 1024, 304, 64, 0.3
     X, W = torch.randn(M, k, device=DEV), torch.randn(n, k, device=DEV)
     Yt, Ys = torch.empty(M, n, device=DEV), torch.empty(M, n, device=DEV)

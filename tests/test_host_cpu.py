@@ -99,7 +99,7 @@ def test_c_abi_exports_every_declared_symbol():
     L = ctypes.CDLL(_lib.SO_PATH)
     for name in declared:
         assert hasattr(L, name), name
-    assert L.rr_version() == 2
+    assert L.rr_version() == 3
     assert L.rr_padded(300) == 304 and L.rr_padded(600) == 608 and L.rr_padded(40) == 48
     L.rr_loss_max_group.restype = ctypes.c_int
     assert L.rr_loss_max_group() >= 500           # config 5 sweeps groups of 50..500 candidates
