@@ -212,6 +212,17 @@ int rr_get_backward_bf16(void);
  * the environment selects 1 at load. */
 int rr_set_forward_bf16(int on);
 int rr_get_forward_bf16(void);
+/* Deterministic mode (torch.use_deterministic_algorithms of the Python package): 1 = every kernel rr_model_backward and
+ * rr_loss_fwdbwd(_ex) launch produces the same bits on every run for identical inputs, in every GEMM mode, backward split and gather
+ * generation.  The sums the default path forms with atomics (weight-gradient row slabs, segment padding rows, loss parts) are written as
+ * partials with plain stores and added in a fixed order instead.  The guarantee holds on one GPU model with one build of this library:
+ * the weight gradient's slab count follows the SM count, so a part with a different SM count may round differently.
+ * Scratch: rr_model_workspace_bytes includes it when the switch is on (rr_model_backward fails with RR_ERR_WORKSPACE, writing nothing,
+ * if the workspace was sized without it); entry points without a workspace take it from the stream-ordered allocator (cudaMallocAsync /
+ * cudaFreeAsync on `stream`) in this mode only.  rr_model_backward with rr_model_cfg.r_atom_map returns RR_ERR_UNSUPPORTED in this mode.
+ * on must be 0 (default) or 1, else RR_ERR_INVALID.  Process-wide. */
+int rr_set_deterministic(int on);
+int rr_get_deterministic(void);
 /* dX[M,k] (+)= dZ[M,n] W[n,k]   (accumulate != 0 adds) */
 int rr_linear_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw,
                     float* dX, int lddx, int accumulate, void* stream);

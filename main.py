@@ -66,11 +66,15 @@ def parse():
     ap.add_argument("--hidden_size", type=int, default=300)
     ap.add_argument("--depth", type=int, default=3)
     ap.add_argument("--dropout", type=float, default=0.1)
+    ap.add_argument("--deterministic", action="store_true",
+                    help="torch.use_deterministic_algorithms(True): bit-identical losses, gradients and weights from the same seed")
     return ap.parse_args()
 
 
 def main():
     a = parse()
+    if a.deterministic:
+        torch.use_deterministic_algorithms(True)
     from reactranker_b200 import parallel
     rank, world, local_rank = parallel.world_from_env()
     if world > 1:

@@ -35,11 +35,15 @@ def parse():
     ap.add_argument("--save_metric", default="all")
     ap.add_argument("--train_strategy", default="sum_session", choices=["sum_session", "accelerate_grad"])
     ap.add_argument("--resume", action="store_true", help="write <path>/<fold>.state.pt after every epoch and continue from it if present")
+    ap.add_argument("--deterministic", action="store_true",
+                    help="torch.use_deterministic_algorithms(True): bit-identical losses, gradients and weights from the same seed")
     return ap.parse_args()
 
 
 def main():
     a = parse()
+    if a.deterministic:
+        torch.use_deterministic_algorithms(True)
     from reactranker_b200 import parallel
     rank, world, local_rank = parallel.world_from_env()        # under torchrun: one process per GPU, windows sharded by group
     if world > 1:

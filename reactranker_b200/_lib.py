@@ -52,7 +52,7 @@ EXPORTS = [
     "rr_loss_fwdbwd", "rr_loss_fwdbwd_ex", "rr_loss_max_group", "rr_rank_metrics",
     "rr_model_workspace_bytes", "rr_model_buffer_offset", "rr_model_forward", "rr_model_backward", "rr_launch_count", "rr_launch_count_reset",
     "rr_profile_begin", "rr_profile_end", "rr_profile_classes", "rr_set_gemm_mode", "rr_get_gemm_mode", "rr_set_backward_bf16", "rr_get_backward_bf16",
-    "rr_set_forward_bf16", "rr_get_forward_bf16", "rr_reload_switches",
+    "rr_set_forward_bf16", "rr_get_forward_bf16", "rr_reload_switches", "rr_set_deterministic", "rr_get_deterministic",
 ]
 KERNEL_CLASSES = ["gemm_fwd", "gemm_dgrad", "gemm_wgrad", "bond_fwd", "bond_bwd", "nbr_fwd", "nbr_bwd", "readout", "elementwise", "loss", "misc"]
 
@@ -157,6 +157,8 @@ def lib() -> ctypes.CDLL:
                 L.rr_set_backward_bf16(int(os.environ.get("RR_BWD_BF16", "1")))
                 L.rr_set_forward_bf16.argtypes = [i32]
                 L.rr_set_forward_bf16(int(os.environ.get("RR_FWD_BF16", "0")))
+                L.rr_set_deterministic.argtypes = [i32]
+                L.rr_get_deterministic.argtypes = []
                 _lib = L
     return _lib
 
@@ -183,6 +185,17 @@ def require_device(device) -> int:
         check(lib().rr_device_check(int(idx)))
         _checked_devices.add(idx)
     return int(idx)
+
+
+def deterministic_requested() -> bool:
+    """torch.use_deterministic_algorithms(True) (also with warn_only=True) asks for bit-identical results."""
+    import torch
+    return bool(torch.are_deterministic_algorithms_enabled())
+
+
+def set_deterministic(on: bool) -> None:
+    """The library's process-wide deterministic switch (rr_set_deterministic)."""
+    check(lib().rr_set_deterministic(1 if on else 0))
 
 
 def ptr(t) -> Optional[int]:

@@ -10,6 +10,7 @@ std::atomic<int64_t> g_launches{0};
 std::atomic<int> g_gemm_mode{0};
 std::atomic<int> g_bwd_bf16{1};
 std::atomic<int> g_fwd_bf16{0};
+std::atomic<int> g_deterministic{0};
 ProfState g_prof;
 std::mutex g_prof_mutex;
 
@@ -31,6 +32,19 @@ const Switches& switches() {
   if (!g_switches_loaded.load()) reload_switches();
   return g_switches;
 }
+int det_scratch(DetScratch* d, void* given, long long given_bytes, long long need, cudaStream_t s) {
+  if (given) {
+    if (given_bytes < need) return fail(RR_ERR_WORKSPACE, "deterministic mode: workspace has %lld bytes of scratch, needs %lld", given_bytes, need);
+    d->p = given;
+    return RR_OK;
+  }
+  if (need <= 0) return RR_OK;
+  RR_CUDA(cudaMallocAsync(&d->p, static_cast<size_t>(need), s));
+  d->s = s;
+  d->owned = true;
+  return RR_OK;
+}
+
 void prof_push(int cls, cudaEvent_t a, cudaEvent_t b) {
   std::lock_guard<std::mutex> lock(g_prof_mutex);
   ProfState& p = g_prof;
@@ -171,6 +185,12 @@ int rr_set_forward_bf16(int on) {
   return RR_OK;
 }
 int rr_get_forward_bf16(void) { return rr::g_fwd_bf16.load(); }
+int rr_set_deterministic(int on) {
+  RR_REQUIRE(on == 0 || on == 1, "rr_set_deterministic: on must be 0 or 1 (got %d)", on);
+  rr::g_deterministic.store(on);
+  return RR_OK;
+}
+int rr_get_deterministic(void) { return rr::g_deterministic.load(); }
 int rr_profile_begin(void) {
   std::lock_guard<std::mutex> lock(rr::g_prof_mutex);
   rr::g_prof.enabled = true;

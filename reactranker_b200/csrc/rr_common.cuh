@@ -74,6 +74,25 @@ struct ProfScope {
 // 0 = fp32 SIMT GEMMs, 1 = tcgen05 3xTF32 GEMMs where the shape allows (forward + dgrad)
 extern std::atomic<int> g_gemm_mode;
 
+// Deterministic mode (rr_set_deterministic): every sum the backward pass and the losses would form with atomics is instead written as
+// partials to scratch with plain stores and summed in a fixed order.  Process-wide.
+extern std::atomic<int> g_deterministic;
+inline bool deterministic() { return g_deterministic.load() != 0; }
+
+// Scratch of a deterministic launch: the caller's (the model's workspace) when given, else transient stream-ordered memory that is freed on
+// the same stream once the launches that use it are enqueued, so the library still holds nothing between calls.
+struct DetScratch {
+  void* p = nullptr;
+  cudaStream_t s = nullptr;
+  bool owned = false;
+  DetScratch() = default;
+  DetScratch(const DetScratch&) = delete;
+  DetScratch& operator=(const DetScratch&) = delete;
+  ~DetScratch() {
+    if (owned) cudaFreeAsync(p, s);
+  }
+};
+
 // Switches from the environment (RR_MP_V1: the first-generation gather kernels instead of the row pipeline): read ONCE, when the library is
 // first used, not on every launch.  rr_reload_switches() reads them again (tests and the micro-benchmarks flip them inside one process).
 struct Switches {
@@ -166,6 +185,31 @@ __device__ __forceinline__ void red_add_f4(float* p, float4 v) {
   atomicAdd(p + 3, v.w);
 }
 
+// ---- deterministic padding-row partials ------------------------------------------------------
+// A gather backward adds every atom's share of its segment's padding row into that row.  In deterministic mode each "unit" (one atom slot of
+// a CTA, which walks its atoms in increasing order and so meets the segments in increasing order) stores the partial of every padding row it
+// meets, entry unit * jcap + j for the j-th row it meets, and tags the entry with the row; pad_rows_sum() then adds the entries of each row
+// in entry order: CTA 0, 1, 2, ..., and inside a CTA slot 0, 1, 2, ...
+struct PadParts {
+  float* parts;     // [entries, ld]
+  int* tags;        // [entries] padding row of the entry, -1 = unused
+  int jcap;         // entries per unit
+  long long entries;
+};
+// pad_parts_setup sizes jcap so that a unit never meets more rows than it has entries; should that bound ever fail, the unit's last entry is
+// poisoned with NaN, so that its padding row's gradient shows the error instead of silently missing a partial.
+__device__ __forceinline__ void pad_part_store(const PadParts& pp, long long unit, int& j, int pad_row, int ld, int c4, float4 v) {
+  if (j < pp.jcap) {
+    const long long e = unit * pp.jcap + j;
+    st_f4(pp.parts + e * ld + c4, v);
+    if (c4 == 0) pp.tags[e] = pad_row;
+  } else {
+    const float nan = __int_as_float(0x7fc00000);
+    st_f4(pp.parts + (unit * pp.jcap + pp.jcap - 1) * ld + c4, make_float4(nan, nan, nan, nan));
+  }
+  ++j;
+}
+
 // ---- Philox4x32-7: counter-based dropout masks, regenerable from (seed, stream, index) -----
 // Seven rounds is the smallest Philox4x32 variant that passes BigCrush (Salmon et al., SC'11, table 2; ten is the default safety margin).
 // The masks are drawn in the GEMM epilogue, whose ALU work competes with the warps that feed the tensor core, so rounds are not free.
@@ -204,14 +248,24 @@ int bond_message_bwd(const rr_graph*, const float*, float*, int, cudaStream_t);
 int neighbor_sum_fwd(const rr_graph*, int, const float*, float*, int, int, cudaStream_t);
 int neighbor_sum_bwd(const rr_graph*, int, const float*, float*, int, cudaStream_t);
 // gather backward + the ReLU / dropout backward that follows it (y: activation the mask comes from; acc_mode 0 none, 1 acc = dz, 2 acc += dz)
+// det / det_bytes: scratch of deterministic mode (NULL: transient, see DetScratch)
 int bond_message_bwd_act(const rr_graph*, const float* dpre, float* dm, int hp, const float* y, float scale, int preact, float* acc, int acc_mode,
-                         int skip_out, cudaStream_t);
+                         int skip_out, cudaStream_t, void* det = nullptr, long long det_bytes = 0);
 int neighbor_sum_bwd_act(const rr_graph*, int which, const float* dout, float* dsrc, int ld, const float* y, float scale, int preact, float* acc,
-                         int acc_mode, int skip_out, cudaStream_t);
+                         int acc_mode, int skip_out, cudaStream_t, void* det = nullptr, long long det_bytes = 0);
+// det != NULL: the deterministic variant of a backward op, its padding-row partials carved from det (see PadParts)
 int rowpipe_launch(int op, const rr_graph* g, int which, const float* src, float* out, int ld, int relu_src, const float* y, float scale, int preact,
-                   float* acc, int acc_mode, int skip_out, cudaStream_t s);
+                   float* acc, int acc_mode, int skip_out, cudaStream_t s, void* det = nullptr, long long det_bytes = 0, PadParts* pp = nullptr);
 int pad_rows_act(float* out, const int* rows, int n_rows, int ld, const float* y, float scale, int preact, float* acc, int acc_mode, int skip_out,
                  cudaStream_t s);
+// deterministic padding rows: bytes of scratch a gather backward over n_atoms rows of n_segments segments may need (either generation)
+long long pad_parts_bytes(int n_atoms, int n_segments, int ld);
+// carve the entries of `units` units of at most atoms_per_unit atoms out of scratch (RR_ERR_WORKSPACE when it is too small) and mark them unused
+int pad_parts_setup(void* scratch, long long bytes, long long units, long long atoms_per_unit, int n_segments, int ld, PadParts* pp, cudaStream_t s);
+// out[rows[r]] = sum of the entries tagged rows[r], in entry order
+int pad_rows_sum(float* out, const int* rows, int n_rows, int ld, const PadParts& pp, cudaStream_t s);
+// scratch for a deterministic launch: `given` when not NULL (RR_ERR_WORKSPACE if smaller than need), else cudaMallocAsync on s
+int det_scratch(DetScratch* d, void* given, long long given_bytes, long long need, cudaStream_t s);
 int readout_fwd(const rr_graph*, const float*, int, int, const float*, int, float*, int, float, uint64_t, uint64_t, cudaStream_t);
 int readout_bwd(const rr_graph*, const float*, int, const float*, const float*, float*, int, float, cudaStream_t);
 int relu_bwd(long long, int, const float*, const float*, float, int, float*, float*, int, cudaStream_t);
@@ -225,7 +279,9 @@ int linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1,
                cudaStream_t s, ptrdiff_t hi_off = 0, ptrdiff_t lo_off = 0, const float* packed = nullptr, const uint16_t* bhi = nullptr,
                const uint16_t* blo = nullptr);
 int linear_dgrad(int, int, int, const float*, int, const float*, int, float*, int, int, cudaStream_t);
-int linear_wgrad(int, int, int, const float*, int, const float*, int, float*, int, float*, cudaStream_t);
+int linear_wgrad(int, int, int, const float*, int, const float*, int, float*, int, float*, cudaStream_t, void* det = nullptr, long long det_bytes = 0);
+// deterministic mode: bytes of scratch linear_wgrad(M, n, k, ...) needs (row-slab partials of dW and of the bias gradient), any GEMM mode
+long long wgrad_det_bytes(int M, int n, int k);
 int loss_fwdbwd(int, int, int, const float*, const float*, const int*, float, float, float*, float*, cudaStream_t, int max_group = 0);
 int loss_max_group();
 int rank_metrics(int, int, const float*, int, const double*, const int*, int, double, double*, cudaStream_t);
@@ -255,6 +311,10 @@ long long tc_dgrad_scratch_bytes(int n, int k);
 int tc_dgrad_standalone(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, void* scratch,
                         long long scratch_bytes, cudaStream_t s);
 bool tc_wgrad_supported(int M, int n, int k, int lddz, int ldx);
-int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s);
+// slab != NULL (deterministic mode): slab z of the reduction stores its dW tile to slab + z * n * k (row stride k) and, when dbias != NULL,
+// its bias partial to slab + splits * n * k + z * n, instead of adding into dW / dbias; *splits receives the slab count
+int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s,
+             float* slab = nullptr, int* splits = nullptr);
+int tc_wgrad_max_splits(int M, int n, int k);
 
 }  // namespace rr

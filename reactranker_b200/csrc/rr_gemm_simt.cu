@@ -14,7 +14,8 @@ namespace rr {
 constexpr int BM = 128, BN = 64, BK = 16, NT = 256;
 constexpr int APAD = BM + 4, BPAD = BN + 4;
 
-enum { EPI_FWD = 0, EPI_STORE = 1, EPI_ACCUM = 2, EPI_ATOMIC = 3 };
+// EPI_SLAB: EPI_ATOMIC of deterministic mode, slab z STORES its tile to C + z * slab_stride and its bias partial to dbias + z * M
+enum { EPI_FWD = 0, EPI_STORE = 1, EPI_ACCUM = 2, EPI_ATOMIC = 3, EPI_SLAB = 4 };
 
 struct GemmSrc {
   const float* A;
@@ -38,6 +39,7 @@ struct GemmArgs {
   // EPI_ATOMIC (wgrad)
   float* dbias;
   int k_chunk;  // reduction rows per blockIdx.z
+  long long slab_stride;  // EPI_SLAB
 };
 
 template <bool A_KC>
@@ -106,12 +108,12 @@ __global__ void __launch_bounds__(NT, 2) k_gemm(GemmArgs g) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
   float bias_acc = 0.f;
-  const bool do_bias = (EPI == EPI_ATOMIC) && g.dbias != nullptr && blockIdx.y == 0;
+  const bool do_bias = (EPI == EPI_ATOMIC || EPI == EPI_SLAB) && g.dbias != nullptr && blockIdx.y == 0;
 
   for (int s = 0; s < g.nsrc; ++s) {
     const GemmSrc src = g.src[s];
     int kbeg = 0, kend = src.K;
-    if (EPI == EPI_ATOMIC) {
+    if (EPI == EPI_ATOMIC || EPI == EPI_SLAB) {
       kbeg = blockIdx.z * g.k_chunk;
       kend = min(src.K, kbeg + g.k_chunk);
     }
@@ -148,7 +150,11 @@ __global__ void __launch_bounds__(NT, 2) k_gemm(GemmArgs g) {
   }
 
   const int n = n0 + tx * 4;
-  if (do_bias && t < BM && m0 + t < g.M) atomicAdd(g.dbias + m0 + t, bias_acc);
+  if constexpr (EPI == EPI_SLAB) {
+    if (do_bias && t < BM && m0 + t < g.M) g.dbias[static_cast<size_t>(blockIdx.z) * g.M + m0 + t] = bias_acc;
+  } else {
+    if (do_bias && t < BM && m0 + t < g.M) atomicAdd(g.dbias + m0 + t, bias_acc);
+  }
   if (n >= g.N) return;
   float4 bv = f4_zero();
   if (EPI == EPI_FWD && g.bias) bv = ld_f4(g.bias + n);
@@ -158,7 +164,9 @@ __global__ void __launch_bounds__(NT, 2) k_gemm(GemmArgs g) {
     if (m >= g.M) break;
     float4 v = make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]);
     float* cp = g.C + static_cast<size_t>(m) * g.ldc + n;
-    if (EPI == EPI_FWD) {
+    if constexpr (EPI == EPI_SLAB) {
+      st_f4(cp + blockIdx.z * g.slab_stride, v);
+    } else if (EPI == EPI_FWD) {
       v = f4_add(v, bv);
       if (g.resid) v = f4_add(v, ld_f4(g.resid + static_cast<size_t>(m) * g.ldr + n));
       if (g.relu) v = f4_relu(v);
@@ -258,9 +266,95 @@ int linear_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W,
   return RR_OK;
 }
 
-int linear_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s) {
-  if (g_gemm_mode.load() == 1 && M >= 256 && tc_wgrad_supported(M, n, k, lddz, ldx) && aligned16(dZ) && aligned16(X) && aligned16(dW) && (lddw & 3) == 0)
-    return tc_wgrad(M, n, k, dZ, lddz, X, ldx, dW, lddw, dbias, s);
+// slab count of the SIMT split below
+static int simt_wgrad_splits(int M, int n, int k, int* chunk_out) {
+  const int tiles = ((n + BM - 1) / BM) * ((k + BN - 1) / BN);
+  int splits = (num_sms() * 2 + tiles - 1) / tiles;
+  const int max_splits = (M + BK * 8 - 1) / (BK * 8);
+  if (splits > max_splits) splits = max_splits;
+  if (splits < 1) splits = 1;
+  int chunk = (M + splits - 1) / splits;
+  chunk = (chunk + BK - 1) / BK * BK;
+  if (chunk_out) *chunk_out = chunk;
+  return (M + chunk - 1) / chunk;
+}
+
+long long wgrad_det_bytes(int M, int n, int k) {
+  if (M <= 0 || n <= 0 || k <= 0) return 0;
+  const int tcs = tc_wgrad_max_splits(M, n, k), simt = simt_wgrad_splits(M, n, k, nullptr);
+  const long long splits = tcs > simt ? tcs : simt;
+  return splits * (static_cast<long long>(n) * k + n) * static_cast<long long>(sizeof(float));
+}
+
+// dW[i, j] += sum over z = 0, 1, 2, ... of slab[z][i, j];  dbias[i] += the same over the bias partials
+__global__ void k_wgrad_slab_sum(int n, int k, int splits, const float* __restrict__ slab, const float* __restrict__ slab_bias, float* __restrict__ dW,
+                                 int lddw, float* __restrict__ dbias) {
+  const int k4 = k >> 2;
+  const long long plane = static_cast<long long>(n) * k;
+  const long long total = static_cast<long long>(n) * k4;
+  for (long long t = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; t < total + n; t += static_cast<long long>(gridDim.x) * blockDim.x) {
+    if (t < total) {
+      const int i = static_cast<int>(t / k4), j = static_cast<int>(t - static_cast<long long>(i) * k4) << 2;
+      const float* p = slab + static_cast<long long>(i) * k + j;
+      float4 acc = ld_f4(p);
+#pragma unroll 8
+      for (int z = 1; z < splits; ++z) acc = f4_add(acc, ld_f4(p + z * plane));
+      float* d = dW + static_cast<size_t>(i) * lddw + j;
+      st_f4(d, f4_add(*reinterpret_cast<const float4*>(d), acc));
+    } else if (dbias) {
+      const int i = static_cast<int>(t - total);
+      float acc = slab_bias[i];
+      for (int z = 1; z < splits; ++z) acc += slab_bias[static_cast<long long>(z) * n + i];
+      dbias[i] += acc;
+    }
+  }
+}
+
+int linear_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s, void* det,
+                 long long det_bytes) {
+  const bool use_tc = g_gemm_mode.load() == 1 && M >= 256 && tc_wgrad_supported(M, n, k, lddz, ldx) && aligned16(dZ) && aligned16(X) && aligned16(dW) &&
+                      (lddw & 3) == 0;
+  if (!deterministic()) {
+    if (use_tc) return tc_wgrad(M, n, k, dZ, lddz, X, ldx, dW, lddw, dbias, s);
+  } else {
+    // Deterministic: every row slab stores its partial dW tile (and bias partial) to scratch, then k_wgrad_slab_sum adds them in slab order.
+    RR_REQUIRE(M >= 0 && n > 0 && k > 0 && (n & 3) == 0 && (k & 3) == 0, "linear_wgrad: M %d n %d k %d", M, n, k);
+    RR_TRY(check_mat("dW", dW, lddw));
+    if (M == 0) return RR_OK;
+    DetScratch ds;
+    RR_TRY(det_scratch(&ds, det, det_bytes, wgrad_det_bytes(M, n, k), s));
+    float* slab = static_cast<float*>(ds.p);
+    int splits = 0;
+    if (use_tc) {
+      RR_TRY(tc_wgrad(M, n, k, dZ, lddz, X, ldx, dW, lddw, dbias, s, slab, &splits));
+    } else {
+      ProfScope prof_scope(KC_GEMM_WGRAD, s);
+      RR_TRY(check_mat("dZ", dZ, lddz));
+      RR_TRY(check_mat("X", X, ldx));
+      GemmArgs g{};
+      g.src[0] = {dZ, X, lddz, ldx, M};
+      g.nsrc = 1;
+      g.M = n;
+      g.N = k;
+      g.C = slab;
+      g.ldc = k;
+      g.slab_stride = static_cast<long long>(n) * k;
+      int chunk = 0;
+      splits = simt_wgrad_splits(M, n, k, &chunk);
+      g.k_chunk = chunk;
+      g.dbias = dbias ? slab + splits * g.slab_stride : nullptr;
+      dim3 grid((n + BM - 1) / BM, (k + BN - 1) / BN, splits);
+      k_gemm<false, false, EPI_SLAB><<<grid, NT, 0, s>>>(g);
+      RR_LAUNCH_CHECK("k_gemm<wgrad slab>");
+    }
+    ProfScope prof_scope(KC_GEMM_WGRAD, s);
+    const long long work = static_cast<long long>(n) * (k >> 2) + n;
+    long long blocks = (work + 255) / 256;
+    if (blocks > num_sms() * 8) blocks = num_sms() * 8;
+    k_wgrad_slab_sum<<<static_cast<int>(blocks), 256, 0, s>>>(n, k, splits, slab, slab + splits * static_cast<long long>(n) * k, dW, lddw, dbias);
+    RR_LAUNCH_CHECK("k_wgrad_slab_sum");
+    return RR_OK;
+  }
   ProfScope prof_scope(KC_GEMM_WGRAD, s);
   RR_REQUIRE(M >= 0 && n > 0 && k > 0 && (n & 3) == 0 && (k & 3) == 0, "linear_wgrad: M %d n %d k %d", M, n, k);
   RR_TRY(check_mat("dZ", dZ, lddz));
@@ -275,14 +369,8 @@ int linear_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X,
   g.C = dW;
   g.ldc = lddw;
   g.dbias = dbias;
-  const int tiles = ((n + BM - 1) / BM) * ((k + BN - 1) / BN);
-  int splits = (num_sms() * 2 + tiles - 1) / tiles;
-  const int max_splits = (M + BK * 8 - 1) / (BK * 8);
-  if (splits > max_splits) splits = max_splits;
-  if (splits < 1) splits = 1;
-  int chunk = (M + splits - 1) / splits;
-  chunk = (chunk + BK - 1) / BK * BK;
-  splits = (M + chunk - 1) / chunk;
+  int chunk = 0;
+  const int splits = simt_wgrad_splits(M, n, k, &chunk);
   g.k_chunk = chunk;
   dim3 grid((n + BM - 1) / BM, (k + BN - 1) / BN, splits);
   k_gemm<false, false, EPI_ATOMIC><<<grid, NT, 0, s>>>(g);

@@ -554,6 +554,7 @@ struct WgArgs {
   float* dW;
   int lddw;
   float* dbias;
+  long long slab_stride;   // SLAB kernels (deterministic mode): slab z stores to dW + z * slab_stride and dbias + z * n
 };
 
 // MN-major tf32 operands have exactly one legal shared-memory layout: 128-byte swizzle with 32-byte atomicity
@@ -582,7 +583,8 @@ __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, 
 // TMEM: accumulator from column 0 | stage s: BKR columns hi + BKR columns lo from column tm_a + 2 BKR s.
 // ================================================================================================
 
-template <int BKR>
+// SLAB = true (deterministic mode): the slab's tile is STORED to its own slice of scratch, never added (see tc_wgrad).
+template <int BKR, bool SLAB>
 __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant__ WgArgs g) {
   constexpr int BOX = BKR * 128;          // bytes of one [BKR x 32 floats] TMA box
   constexpr int A_RAW = 4 * BOX;          // 128 n-columns
@@ -711,7 +713,11 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant_
       __syncwarp();
       if (lane == 0) mbar_arrive(ready + st);
     }
-    if (g.dbias != nullptr && blockIdx.y == 0 && n0 + r < g.n) atomicAdd(g.dbias + n0 + r, bsum);
+    if constexpr (SLAB) {
+      if (g.dbias != nullptr && blockIdx.y == 0 && n0 + r < g.n) g.dbias[static_cast<size_t>(blockIdx.z) * g.n + n0 + r] = bsum;
+    } else {
+      if (g.dbias != nullptr && blockIdx.y == 0 && n0 + r < g.n) atomicAdd(g.dbias + n0 + r, bsum);
+    }
     mbar_wait(acc_bar, 0);
     tc_fence_after();
     const int row = n0 + r;
@@ -720,10 +726,17 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant_
       float v[16];
       tmem_ld16(lane_addr + c, v);
       if (row < g.n) {
-        float* cp = g.dW + static_cast<size_t>(row) * g.lddw + k0 + c;
+        if constexpr (SLAB) {
+          float* cp = g.dW + blockIdx.z * g.slab_stride + static_cast<size_t>(row) * g.lddw + k0 + c;
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
-          if (k0 + c + 4 * q < g.k) red_add_v4(cp + 4 * q, v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+          for (int q = 0; q < 4; ++q)
+            if (k0 + c + 4 * q < g.k) st_f4(cp + 4 * q, make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]));
+        } else {
+          float* cp = g.dW + static_cast<size_t>(row) * g.lddw + k0 + c;
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            if (k0 + c + 4 * q < g.k) red_add_v4(cp + 4 * q, v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+        }
       }
     }
   }
@@ -767,7 +780,7 @@ __device__ __forceinline__ uint64_t umma_desc_mn_bf16(uint32_t smem_addr) {
 constexpr int W3_WORKERS = 256;   // 8 conversion warps (12 measured no faster): with 4 the fp32 -> bf16 conversion (not the MMAs) paced the kernel
 constexpr int W3_THREADS = 64 + W3_WORKERS;
 
-template <int BKR>
+template <int BKR, bool SLAB>
 __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_constant__ WgArgs g) {
   static_assert(BKR == 32 || BKR == 64, "stages of 32 or 64 rows of the reduction");
   constexpr int BOX = BKR * 128;               // bytes of one raw TMA box [BKR x 32 floats] == one bf16 MN block [BKR x 64 bf16]
@@ -935,7 +948,11 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
         mbar_arrive(raw_empty + rs);
       }
     }
-    if (a_warp && g.dbias != nullptr && blockIdx.y == 0 && n0 + r < g.n) atomicAdd(g.dbias + n0 + r, bsum);
+    if constexpr (SLAB) {
+      if (a_warp && g.dbias != nullptr && blockIdx.y == 0 && n0 + r < g.n) g.dbias[static_cast<size_t>(blockIdx.z) * g.n + n0 + r] = bsum;
+    } else {
+      if (a_warp && g.dbias != nullptr && blockIdx.y == 0 && n0 + r < g.n) atomicAdd(g.dbias + n0 + r, bsum);
+    }
     mbar_wait(acc_bar, 0);
     tc_fence_after();
     const int row = n0 + r;
@@ -943,10 +960,17 @@ __global__ void __launch_bounds__(W3_THREADS, 1) k_tc_wgrad3(const __grid_consta
       float v[16];
       tmem_ld16(lane_addr + c, v);
       if (row < g.n) {
-        float* cp = g.dW + static_cast<size_t>(row) * g.lddw + k0 + c;
+        if constexpr (SLAB) {
+          float* cp = g.dW + blockIdx.z * g.slab_stride + static_cast<size_t>(row) * g.lddw + k0 + c;
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
-          if (k0 + c + 4 * q < g.k) red_add_v4(cp + 4 * q, v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+          for (int q = 0; q < 4; ++q)
+            if (k0 + c + 4 * q < g.k) st_f4(cp + 4 * q, make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]));
+        } else {
+          float* cp = g.dW + static_cast<size_t>(row) * g.lddw + k0 + c;
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            if (k0 + c + 4 * q < g.k) red_add_v4(cp + 4 * q, v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+        }
       }
     }
   }
@@ -1123,10 +1147,28 @@ bool tc_wgrad_supported(int M, int n, int k, int lddz, int ldx) {
   return M > 0 && n >= 4 && k >= 4 && !(n & 3) && !(k & 3) && !(lddz & 3) && !(ldx & 3);
 }
 
-int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s) {
+// Upper bound of the slab count of either split below (rounding the slab height up to whole stages only lowers it).
+int tc_wgrad_max_splits(int M, int n, int k) {
+  using namespace tc;
+  const int k_pad = (k + 15) / 16 * 16;
+  const int tiles = ((n + BM - 1) / BM) * ((k_pad + MAX_NT - 1) / MAX_NT);
+  int splits = num_sms() / tiles;
+  const int max_splits = (M + 8 * 32 - 1) / (8 * 32);
+  if (splits > max_splits) splits = max_splits;
+  return splits < 1 ? 1 : splits;
+}
+
+int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s, float* slab,
+             int* n_splits) {
   using namespace tc;
   ProfScope prof_scope(KC_GEMM_WGRAD, s);
+  const bool det = slab != nullptr;
+  if (det) {
+    dW = slab;
+    lddw = k;
+  }
   WgArgs g{};
+  g.slab_stride = static_cast<long long>(n) * k;
   const int k_pad = (k + 15) / 16 * 16;                  // columns past k are zero-filled by TMA and never written back
   const int ktiles = (k_pad + MAX_NT - 1) / MAX_NT;
   g.kt = ktiles == 1 ? k_pad : MAX_NT;
@@ -1167,15 +1209,25 @@ int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int
     chunk3 = (chunk3 + bkr - 1) / bkr * bkr;          // whole stages: a stage never reaches into the next split's rows
     splits3 = (M + chunk3 - 1) / chunk3;
     g.m_chunk = chunk3;
+    if (det && dbias) g.dbias = slab + splits3 * g.slab_stride;   // bias partials follow the slab tiles
     static PerDeviceOnce attr3_set;
     if (attr3_set.need()) {
-      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<64, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
       attr3_set.mark();
     }
     const size_t smem3 = static_cast<size_t>(R) * raw_bytes + static_cast<size_t>(SB) * bf_bytes + 1024 + 512;
-    if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad3<32>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
-    else RR_CUDA(launch_pdl(k_tc_wgrad3<64>, dim3(ntiles3, ktiles, splits3), dim3(W3_THREADS), smem3, s, g));
+    const dim3 grid3(ntiles3, ktiles, splits3);
+    if (det) {
+      if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad3<32, true>, grid3, dim3(W3_THREADS), smem3, s, g));
+      else RR_CUDA(launch_pdl(k_tc_wgrad3<64, true>, grid3, dim3(W3_THREADS), smem3, s, g));
+      *n_splits = splits3;
+    } else {
+      if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad3<32, false>, grid3, dim3(W3_THREADS), smem3, s, g));
+      else RR_CUDA(launch_pdl(k_tc_wgrad3<64, false>, grid3, dim3(W3_THREADS), smem3, s, g));
+    }
     RR_LAUNCH_CHECK("k_tc_wgrad3");
     return RR_OK;
   }
@@ -1208,16 +1260,25 @@ int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int
   chunk = (chunk + WG_BK - 1) / WG_BK * WG_BK;
   splits = (M + chunk - 1) / chunk;
   g.m_chunk = chunk;
+  if (det && dbias) g.dbias = slab + splits * g.slab_stride;
   dim3 grid(ntiles, ktiles, splits);
   const size_t smem = static_cast<size_t>(S) * stage_bytes + 1024 + 256;
   static PerDeviceOnce attr_set;
   if (attr_set.need()) {
-    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     attr_set.mark();
   }
-  if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad2<32>, grid, dim3(THREADS), smem, s, g));
-  else RR_CUDA(launch_pdl(k_tc_wgrad2<16>, grid, dim3(THREADS), smem, s, g));
+  if (det) {
+    if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad2<32, true>, grid, dim3(THREADS), smem, s, g));
+    else RR_CUDA(launch_pdl(k_tc_wgrad2<16, true>, grid, dim3(THREADS), smem, s, g));
+    *n_splits = splits;
+  } else {
+    if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad2<32, false>, grid, dim3(THREADS), smem, s, g));
+    else RR_CUDA(launch_pdl(k_tc_wgrad2<16, false>, grid, dim3(THREADS), smem, s, g));
+  }
   RR_LAUNCH_CHECK("k_tc_wgrad2");
   return RR_OK;
 }

@@ -68,12 +68,20 @@ __device__ void block_scan(float* buf, float* tmp, int n) {
   __syncthreads();
 }
 
+// A block's share of the loss: added into loss[0] with an atomic, or (DET, deterministic mode) stored to loss[block], the partials that
+// k_sum_parts then adds in block order.  (A macro, not a function: the default kernels then compile exactly as they did before DET existed.)
+#define RR_PUT_LOSS(loss, v)                                          \
+  do {                                                                \
+    if constexpr (DET) (loss)[blockIdx.y * gridDim.x + blockIdx.x] = (v); \
+    else atomicAdd((loss), (v));                                      \
+  } while (0)
+
 // ---------------------------------------------------------------------------------------
 // ListMLE  (MLEloss loss.py:64-99, LogCumsumExp loss.py:9-61)
 // ---------------------------------------------------------------------------------------
 // DIS = true: MLEDisLoss (loss.py:102-141) on scores [N,2] = (mean, variance).  Its n x n lower-triangular form reduces to ListMLE of
 // z = mean + variance / 2 plus the group mean of the variance:  mean_j( lcse_j(z) - z_j + v_j ).
-template <bool DIS>
+template <bool DIS, bool DET>
 __global__ void __launch_bounds__(kLossThreads) k_listmle(const float* __restrict__ scores, const float* __restrict__ targets,
                                                           const int* __restrict__ seg, float inv_norm, float* __restrict__ loss,
                                                           float* __restrict__ dscore, int cap) {
@@ -87,7 +95,7 @@ __global__ void __launch_bounds__(kLossThreads) k_listmle(const float* __restric
   if (n <= 0) return;
   if (n > cap) {   // the shared arrays hold `cap` candidates: a larger group poisons the result instead of overrunning them
     for (int i = threadIdx.x; i < n * (DIS ? 2 : 1); i += blockDim.x) dscore[static_cast<size_t>(o) * (DIS ? 2 : 1) + i] = CUDART_NAN_F;
-    if (threadIdx.x == 0) atomicAdd(loss, CUDART_NAN_F);
+    if (threadIdx.x == 0) RR_PUT_LOSS(loss, CUDART_NAN_F);
     return;
   }
   int P = 1;
@@ -158,7 +166,7 @@ __global__ void __launch_bounds__(kLossThreads) k_listmle(const float* __restric
       dscore[o + id[i]] = gz;
     }
   }
-  if (threadIdx.x == 0) atomicAdd(loss, (total + (DIS ? vsum : 0.f)) * gscale);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, (total + (DIS ? vsum : 0.f)) * gscale);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -166,7 +174,7 @@ __global__ void __launch_bounds__(kLossThreads) k_listmle(const float* __restric
 // ---------------------------------------------------------------------------------------
 // DIS = true: Listnet_For_Gauss (loss.py:233-272) on scores [N,2] = (mean, variance): with u = mean + variance / 2 its n x n form is
 // -p_i log pred_i = p_i (lse(u) - u_i + v_i), averaged over the items of the GROUP and then over groups (inv_norm = 1 / G here).
-template <bool DIS>
+template <bool DIS, bool DET>
 __global__ void __launch_bounds__(kLossThreads) k_listnet(const float* __restrict__ scores, const float* __restrict__ targets,
                                                           const int* __restrict__ seg, float inv_norm, float* __restrict__ loss,
                                                           float* __restrict__ dscore) {
@@ -206,12 +214,13 @@ __global__ void __launch_bounds__(kLossThreads) k_listnet(const float* __restric
     }
   }
   part = block_sum(part, red);
-  if (threadIdx.x == 0) atomicAdd(loss, part * c);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, part * c);
 }
 
 // ---------------------------------------------------------------------------------------
 // UC-Listwise  (evidential_ranking loss.py:526-554): scores [N,2] = (mean, variance)
 // ---------------------------------------------------------------------------------------
+template <bool DET>
 __global__ void __launch_bounds__(kLossThreads) k_evidential(const float* __restrict__ scores, const float* __restrict__ targets,
                                                              const int* __restrict__ seg, float inv_norm, float* __restrict__ loss,
                                                              float* __restrict__ dscore) {
@@ -252,7 +261,7 @@ __global__ void __launch_bounds__(kLossThreads) k_evidential(const float* __rest
     dscore[2 * (o + i)] = (expf(logq) * dsum - d / v + sgn) * gscale;
     dscore[2 * (o + i) + 1] = (-0.5f * d * d / (v * v) + 0.5f / v) * gscale;
   }
-  if (threadIdx.x == 0) atomicAdd(loss, part * gscale);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, part * gscale);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -260,6 +269,7 @@ __global__ void __launch_bounds__(kLossThreads) k_evidential(const float* __rest
 //   group loss = (1/n) sum_i p_i c_i  +  coef * mean_i |c_i (s_i - 1)|        (KLDivLoss 'batchmean' of a 1-D input divides by n)
 // coef = max_coeff * (epoch / (epochs - 1))^3 is computed by the caller.  Mean over groups.
 // ---------------------------------------------------------------------------------------
+template <bool DET>
 __global__ void __launch_bounds__(kLossThreads) k_listnet_uq(const float* __restrict__ scores, const float* __restrict__ targets,
                                                              const int* __restrict__ seg, float inv_norm, float coef, float* __restrict__ loss,
                                                              float* __restrict__ dscore) {
@@ -299,13 +309,14 @@ __global__ void __launch_bounds__(kLossThreads) k_listnet_uq(const float* __rest
     const float dpen = sg / ssum + sgn * (c - (s - 1.f) / s);               // d/ds_k of sum_i |c_i (s_i - 1)|
     dscore[o + i] = (dkl + coef * dpen) * gscale;
   }
-  if (threadIdx.x == 0) atomicAdd(loss, (kl + coef * pen) * gscale);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, (kl + coef * pen) * gscale);
 }
 
 // ---------------------------------------------------------------------------------------
 // Dirichlet_uq (loss.py:440-474) on 1-D positive concentrations a: pred = a / S, p = softmax(t),
 //   group loss = mean_i( (pred_i - p_i)^2 + pred_i (1 - pred_i) / (S + 1) + coef |log(p_i / pred_i) (a_i - 1)| ),  mean over groups.
 // ---------------------------------------------------------------------------------------
+template <bool DET>
 __global__ void __launch_bounds__(kLossThreads) k_dirichlet_uq(const float* __restrict__ scores, const float* __restrict__ targets,
                                                                const int* __restrict__ seg, float inv_norm, float coef,
                                                                float* __restrict__ loss, float* __restrict__ dscore) {
@@ -351,7 +362,7 @@ __global__ void __launch_bounds__(kLossThreads) k_dirichlet_uq(const float* __re
     const float dpen = sg / S + sgn * (c - (a - 1.f) / a);
     dscore[o + i] = (derr + dvar + coef * dpen) * gscale;
   }
-  if (threadIdx.x == 0) atomicAdd(loss, part * gscale);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, part * gscale);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -371,6 +382,7 @@ __device__ double digamma_d(double x) {      // x > 0: recurrence up to x >= 6, 
 }
 constexpr int kNigRows = 128;
 constexpr int kNigCols = 512;
+template <bool DET>
 __global__ void __launch_bounds__(kNigRows) k_nig_allpairs(int N, const float* __restrict__ scores, const float* __restrict__ targets,
                                                            float inv_norm, float lam, float* __restrict__ loss, float* __restrict__ dscore) {
   __shared__ float ts[kNigCols];
@@ -403,14 +415,18 @@ __global__ void __launch_bounds__(kNigRows) k_nig_allpairs(int N, const float* _
     const float g_v = fj * (-0.5f / v - al * 2.f * be / om) + ah * (s_d2inv + 2.f * be * s_inv) + 2.f * lam * s_abs;
     const float g_al = fj * (-logf(om) + dpsi) + s_log + lam * s_abs;
     const float g_be = -fj * al / be + ah * 2.f * (1.f + v) * s_inv;
-    float* dr = dscore + 4 * static_cast<size_t>(i);
-    atomicAdd(dr + 0, g_mu * inv_norm);
-    atomicAdd(dr + 1, g_v * inv_norm);
-    atomicAdd(dr + 2, g_al * inv_norm);
-    atomicAdd(dr + 3, g_be * inv_norm);
+    if constexpr (DET) {   // this column block's partial row gradient; k_nig_dscore_sum adds the blocks in order
+      st_f4(dscore + 4 * (static_cast<size_t>(blockIdx.y) * N + i), make_float4(g_mu * inv_norm, g_v * inv_norm, g_al * inv_norm, g_be * inv_norm));
+    } else {
+      float* dr = dscore + 4 * static_cast<size_t>(i);
+      atomicAdd(dr + 0, g_mu * inv_norm);
+      atomicAdd(dr + 1, g_v * inv_norm);
+      atomicAdd(dr + 2, g_al * inv_norm);
+      atomicAdd(dr + 3, g_be * inv_norm);
+    }
   }
   part = block_sum(part, red);
-  if (threadIdx.x == 0) atomicAdd(loss, part * inv_norm);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, part * inv_norm);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -419,6 +435,7 @@ __global__ void __launch_bounds__(kNigRows) k_nig_allpairs(int N, const float* _
 __device__ __forceinline__ float softplus_f(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
 __device__ __forceinline__ float sigmoid_f(float x) { return 1.f / (1.f + expf(-x)); }
 
+template <bool DET>
 __global__ void __launch_bounds__(kLossThreads) k_ranknet(const float* __restrict__ scores, const float* __restrict__ targets,
                                                           const int* __restrict__ seg, float inv_norm, float sigma, float gfac,
                                                           float* __restrict__ loss, float* __restrict__ dscore, int cap) {
@@ -430,7 +447,7 @@ __global__ void __launch_bounds__(kLossThreads) k_ranknet(const float* __restric
   if (n <= 0) return;
   if (n > cap) {   // as in k_listmle: NaN, never a shared-memory overrun (direct C-ABI callers bypass the Python-side check)
     for (int i = threadIdx.x; i < n; i += blockDim.x) dscore[o + i] = CUDART_NAN_F;
-    if (threadIdx.x == 0) atomicAdd(loss, CUDART_NAN_F);
+    if (threadIdx.x == 0) RR_PUT_LOSS(loss, CUDART_NAN_F);
     return;
   }
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -456,12 +473,13 @@ __global__ void __launch_bounds__(kLossThreads) k_ranknet(const float* __restric
     dscore[o + i] = gfac * sigma * g * inv_norm;
   }
   part = block_sum(part, red);
-  if (threadIdx.x == 0) atomicAdd(loss, part * inv_norm);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, part * inv_norm);
 }
 
 // ---------------------------------------------------------------------------------------
 // pointwise: GaussDisLoss (loss.py:144-162), nn.MSELoss (train_listwise.py:166-167), the 'regression_exploss' key (276-281)
 // ---------------------------------------------------------------------------------------
+template <bool DET>
 __global__ void __launch_bounds__(kLossThreads) k_pointwise(int kind, int N, const float* __restrict__ scores, const float* __restrict__ targets,
                                                             float inv_norm, float* __restrict__ loss, float* __restrict__ dscore) {
   __shared__ float red[32];
@@ -492,11 +510,31 @@ __global__ void __launch_bounds__(kLossThreads) k_pointwise(int kind, int N, con
     }
   }
   part = block_sum(part, red);
-  if (threadIdx.x == 0) atomicAdd(loss, part * inv_norm);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, part * inv_norm);
 }
 
-int loss_fwdbwd(int kind, int N, int G, const float* scores, const float* targets, const int* seg_off, float norm, float sigma,
-                float* loss, float* dscore, cudaStream_t s, int max_group) {
+// deterministic mode: loss[0] = sum of the n block partials (each thread a strided run in order, then the fixed block_sum tree)
+__global__ void __launch_bounds__(kLossThreads) k_sum_parts(int n, const float* __restrict__ parts, float* __restrict__ loss) {
+  __shared__ float red[32];
+  float v = 0.f;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) v += parts[i];
+  v = block_sum(v, red);
+  if (threadIdx.x == 0) loss[0] = v;
+}
+// deterministic mode: dscore[i] = sum over column blocks y = 0, 1, ... of the NIG partials
+__global__ void k_nig_dscore_sum(int N, int ny, const float* __restrict__ parts, float* __restrict__ dscore) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
+    float4 acc = ld_f4(parts + 4 * static_cast<size_t>(i));
+    for (int y = 1; y < ny; ++y) acc = f4_add(acc, ld_f4(parts + 4 * (static_cast<size_t>(y) * N + i)));
+    st_f4(dscore + 4 * static_cast<size_t>(i), acc);
+  }
+}
+
+// DET (deterministic mode): every block stores its loss part to scratch (zeroed first: an empty group stores nothing), NIG its per-column-block
+// gradient rows too, and k_sum_parts / k_nig_dscore_sum add them in block order.  The scratch is transient (cudaMallocAsync on s).
+template <bool DET>
+static int loss_launch(int kind, int N, int G, const float* scores, const float* targets, const int* seg_off, float norm, float sigma,
+                       float* loss, float* dscore, cudaStream_t s, int max_group) {
   ProfScope prof_scope(KC_LOSS, s);
   RR_REQUIRE(N > 0 && scores && targets && loss && dscore, "loss: NULL argument or N <= 0");
   RR_REQUIRE(norm > 0.f, "loss: norm must be positive (got %g)", norm);
@@ -508,8 +546,29 @@ int loss_fwdbwd(int kind, int N, int G, const float* scores, const float* target
     cap = 64;
     while (cap < max_group) cap <<= 1;
   }
-  RR_CUDA(cudaMemsetAsync(loss, 0, sizeof(float), s));
   const float inv = 1.f / norm;
+  const dim3 nig_grid((N + kNigRows - 1) / kNigRows, (N + kNigCols - 1) / kNigCols);
+  int pw_blocks = (N + kLossThreads - 1) / kLossThreads;
+  if (pw_blocks > num_sms() * 4) pw_blocks = num_sms() * 4;
+  long long n_parts = 0;
+  switch (kind) {
+    case RR_LOSS_NIG: n_parts = static_cast<long long>(nig_grid.x) * nig_grid.y; break;
+    case RR_LOSS_GAUSS: case RR_LOSS_MSE: case RR_LOSS_LOGNORM: case RR_LOSS_EXPMSE: n_parts = pw_blocks; break;
+    default: n_parts = G > 0 ? G : 0; break;
+  }
+  DetScratch ds;
+  float* out = loss;        // where the kernels put their parts
+  float* dparts = dscore;   // NIG: where the kernel puts its gradient rows
+  if (DET) {
+    const long long nig_floats = kind == RR_LOSS_NIG ? 4LL * N * nig_grid.y : 0;
+    const long long parts_floats = (n_parts + 3) / 4 * 4;
+    RR_TRY(det_scratch(&ds, nullptr, 0, (parts_floats + nig_floats) * static_cast<long long>(sizeof(float)), s));
+    out = static_cast<float*>(ds.p);
+    dparts = out + parts_floats;
+    if (n_parts > 0) RR_CUDA(cudaMemsetAsync(out, 0, n_parts * sizeof(float), s));
+  } else {
+    RR_CUDA(cudaMemsetAsync(loss, 0, sizeof(float), s));
+  }
   switch (kind) {
     case RR_LOSS_LISTMLE:
     case RR_LOSS_LISTNET:
@@ -524,42 +583,55 @@ int loss_fwdbwd(int kind, int N, int G, const float* scores, const float* target
       {
         static PerDeviceOnce attr_set;           // up to 128 KB of dynamic shared memory for groups of up to kMaxGroup candidates
         if (attr_set.need()) {
-          RR_CUDA(cudaFuncSetAttribute(k_listmle<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
-          RR_CUDA(cudaFuncSetAttribute(k_listmle<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
-          RR_CUDA(cudaFuncSetAttribute(k_ranknet, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * kMaxGroup * static_cast<int>(sizeof(float))));
+          RR_CUDA(cudaFuncSetAttribute(k_listmle<false, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
+          RR_CUDA(cudaFuncSetAttribute(k_listmle<true, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
+          RR_CUDA(cudaFuncSetAttribute(k_ranknet<DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * kMaxGroup * static_cast<int>(sizeof(float))));
           attr_set.mark();
         }
       }
-      if (kind == RR_LOSS_LISTMLE) k_listmle<false><<<G, kLossThreads, 4 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, loss, dscore, cap);
-      else if (kind == RR_LOSS_LISTMLE_DIS) k_listmle<true><<<G, kLossThreads, 4 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, loss, dscore, cap);
-      else if (kind == RR_LOSS_LISTNET) k_listnet<false><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, loss, dscore);
-      else if (kind == RR_LOSS_LISTNET_DIS) k_listnet<true><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, loss, dscore);
-      else if (kind == RR_LOSS_EVIDENTIAL) k_evidential<<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, loss, dscore);
-      else if (kind == RR_LOSS_DIRICHLET_UQ) k_dirichlet_uq<<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, sigma, loss, dscore);
-      else if (kind == RR_LOSS_LISTNET_UQ) k_listnet_uq<<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, sigma, loss, dscore);
-      else k_ranknet<<<G, kLossThreads, 2 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, sigma, kind == RR_LOSS_RANKNET_ACC ? 1.f : 2.f, loss, dscore, cap);
+      if (kind == RR_LOSS_LISTMLE) k_listmle<false, DET><<<G, kLossThreads, 4 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, out, dscore, cap);
+      else if (kind == RR_LOSS_LISTMLE_DIS) k_listmle<true, DET><<<G, kLossThreads, 4 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, out, dscore, cap);
+      else if (kind == RR_LOSS_LISTNET) k_listnet<false, DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, out, dscore);
+      else if (kind == RR_LOSS_LISTNET_DIS) k_listnet<true, DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, out, dscore);
+      else if (kind == RR_LOSS_EVIDENTIAL) k_evidential<DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, out, dscore);
+      else if (kind == RR_LOSS_DIRICHLET_UQ) k_dirichlet_uq<DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, sigma, out, dscore);
+      else if (kind == RR_LOSS_LISTNET_UQ) k_listnet_uq<DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, sigma, out, dscore);
+      else k_ranknet<DET><<<G, kLossThreads, 2 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, sigma, kind == RR_LOSS_RANKNET_ACC ? 1.f : 2.f, out, dscore, cap);
       break;
     case RR_LOSS_NIG: {            // norm = N * N (the reference's mean over the broadcast matrix); `sigma` carries lam
       RR_REQUIRE((reinterpret_cast<uintptr_t>(scores) & 15) == 0, "loss: NIG scores must be 16-byte aligned");
-      RR_CUDA(cudaMemsetAsync(dscore, 0, sizeof(float) * 4 * static_cast<size_t>(N), s));
-      dim3 grid((N + kNigRows - 1) / kNigRows, (N + kNigCols - 1) / kNigCols);
-      k_nig_allpairs<<<grid, kNigRows, 0, s>>>(N, scores, targets, inv, sigma, loss, dscore);
+      if (!DET) RR_CUDA(cudaMemsetAsync(dscore, 0, sizeof(float) * 4 * static_cast<size_t>(N), s));
+      k_nig_allpairs<DET><<<nig_grid, kNigRows, 0, s>>>(N, scores, targets, inv, sigma, out, dparts);
       break;
     }
     case RR_LOSS_GAUSS:
     case RR_LOSS_MSE:
     case RR_LOSS_LOGNORM:
     case RR_LOSS_EXPMSE: {
-      int blocks = (N + kLossThreads - 1) / kLossThreads;
-      if (blocks > num_sms() * 4) blocks = num_sms() * 4;
-      k_pointwise<<<blocks, kLossThreads, 0, s>>>(kind, N, scores, targets, inv, loss, dscore);
+      k_pointwise<DET><<<pw_blocks, kLossThreads, 0, s>>>(kind, N, scores, targets, inv, out, dscore);
       break;
     }
     default:
       return fail(RR_ERR_INVALID, "unknown loss kind %d", kind);
   }
   RR_LAUNCH_CHECK("loss kernel");
+  if (DET) {
+    k_sum_parts<<<1, kLossThreads, 0, s>>>(static_cast<int>(n_parts), out, loss);
+    RR_LAUNCH_CHECK("k_sum_parts");
+    if (kind == RR_LOSS_NIG) {
+      int blocks = (N + 255) / 256;
+      if (blocks > num_sms() * 4) blocks = num_sms() * 4;
+      k_nig_dscore_sum<<<blocks, 256, 0, s>>>(N, static_cast<int>(nig_grid.y), dparts, dscore);
+      RR_LAUNCH_CHECK("k_nig_dscore_sum");
+    }
+  }
   return RR_OK;
+}
+
+int loss_fwdbwd(int kind, int N, int G, const float* scores, const float* targets, const int* seg_off, float norm, float sigma,
+                float* loss, float* dscore, cudaStream_t s, int max_group) {
+  if (deterministic()) return loss_launch<true>(kind, N, G, scores, targets, seg_off, norm, sigma, loss, dscore, s, max_group);
+  return loss_launch<false>(kind, N, G, scores, targets, seg_off, norm, sigma, loss, dscore, s, max_group);
 }
 
 int loss_max_group() { return kMaxGroup; }

@@ -340,6 +340,10 @@ struct Workspace {
   float* x[RR_MAX_FFN];
   // backward scratch
   float *gB1, *gB2, *dinp, *gA1, *gA2, *gA3, *dD, *dI2, *dvec, *gN1, *gN2, *dzout;
+  // deterministic mode only (last, so that every other offset is the same in both modes): the weight-gradient slabs and the padding-row
+  // partials of the backward pass, one launch at a time
+  float* det;
+  long long det_bytes;
   size_t bytes;
 };
 
@@ -430,6 +434,24 @@ static int carve(const rr_model_cfg& c, const rr_graph& r, const rr_graph& p, vo
   W->gN1 = take(N * hp);
   W->gN2 = take(N * hp);
   W->dzout = take(N * RR_OUT_LD);
+  W->det = nullptr;
+  W->det_bytes = 0;
+  if (deterministic()) {
+    const int A_J_ = static_cast<int>(A_J), B_J_ = static_cast<int>(B_J), A_ = static_cast<int>(A), N_ = static_cast<int>(N), hp_ = static_cast<int>(hp);
+    long long need = 0;
+    auto at_least = [&](long long b) { need = b > need ? b : need; };
+    at_least(wgrad_det_bytes(B_J_, hp_, hp_));            // encoder W_h
+    at_least(wgrad_det_bytes(B_J_, hp_, RR_FB_LD));       // encoder W_i
+    at_least(wgrad_det_bytes(A_J_, hp_, hp_));            // encoder W_o (message part)
+    at_least(wgrad_det_bytes(A_J_, hp_, RR_FA_LD));       // encoder W_o (atom features)
+    at_least(wgrad_det_bytes(A_, hp_, hp_));              // diff encoder W_i, W_h, W_o
+    at_least(wgrad_det_bytes(A_, hp_, RR_FB_LD));         // diff encoder W_h (bond features)
+    for (int l = 0; l < c.ffn_depth; ++l) at_least(wgrad_det_bytes(N_, W->L.ffn_out[l], W->L.ffn_in[l]));
+    at_least(pad_parts_bytes(A_J_, r.n_segments + p.n_segments, hp_));   // gathers over the joint graph
+    at_least(pad_parts_bytes(A_, p.n_segments, hp_));                    // and over the product graph
+    W->det = take(static_cast<size_t>((need + 3) / 4));
+    W->det_bytes = (need + 3) / 4 * 4;
+  }
   W->bytes = used;
   return RR_OK;
 }
@@ -631,6 +653,8 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
   Workspace W;
   RR_TRY(check_model_args(c, w, r, p, ws, ws_bytes, &W));
   RR_REQUIRE(dscores && grads, "backward: NULL argument");
+  if (deterministic() && c->r_atom_map)
+    return fail(RR_ERR_UNSUPPORTED, "deterministic mode: the backward pass of de-duplicated reactants (r_atom_map) sums rows with atomics");
   const PackedLayout& L = W.L;
   const int hp = L.hp, vp = L.vp;
   const int T = c->depth - 1, Td = c->diff_depth - 1;
@@ -653,7 +677,7 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
     float* scratch[2] = {W.gN1, W.gN2};
     for (int l = c->ffn_depth - 1; l >= 0; --l) {
       const float* x = (l == 0) ? W.vec : W.x[l - 1];
-      RR_TRY(linear_wgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, x, L.ffn_in[l], G + L.ffn_W[l], L.ffn_in[l], G + L.ffn_b[l], s));
+      RR_TRY(linear_wgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, x, L.ffn_in[l], G + L.ffn_W[l], L.ffn_in[l], G + L.ffn_b[l], s, W.det, W.det_bytes));
       if (l > 0) {
         float* dx = scratch[l & 1];
         RR_TRY(dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], dx, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
@@ -667,25 +691,25 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
   }
   // readout + W_o of the diff encoder
   RR_TRY(readout_bwd(p, W.dvec, vp, W.vec, W.hid2, W.gA1, hp, pdrop, s));
-  RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.d, hp, G + L.dif_Wo_d, hp, G + L.dif_bo, s));
-  RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.am2, hp, G + L.dif_Wo_m, hp, nullptr, s));
+  RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.d, hp, G + L.dif_Wo_d, hp, G + L.dif_bo, s, W.det, W.det_bytes));
+  RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.am2, hp, G + L.dif_Wo_m, hp, nullptr, s, W.det, W.det_bytes));
   RR_TRY(dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_d, hp, P + L.dif_Wo_d_T, hp, W.dD, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
   RR_TRY(dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_m, hp, P + L.dif_Wo_m_T, hp, W.gA2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
   // Every gather backward is followed by exactly one ReLU (+ dropout) backward: the mask of the message it produced the gradient of.
   // Both run as one kernel (rr_mp_pipe.cu): t_next >= 1 -> mask of m2^{t_next}, result kept (gA1) and summed into dI2;
   // t_next == 0 -> mask [inp2 > 0] of m2^0 = relu(inp2), only the sum into dI2 is wanted.
   auto diff_nbr_bwd = [&](int t_next) {
-    if (t_next >= 1) return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA1, hp, W.m2[t_next], keep, 0, W.dI2, t_next == Td ? 1 : 2, 0, s);
-    return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA3, hp, W.inp2, 1.f, 1, W.dI2, Td == 0 ? 1 : 2, 1, s);
+    if (t_next >= 1) return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA1, hp, W.m2[t_next], keep, 0, W.dI2, t_next == Td ? 1 : 2, 0, s, W.det, W.det_bytes);
+    return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA3, hp, W.inp2, 1.f, 1, W.dI2, Td == 0 ? 1 : 2, 1, s, W.det, W.det_bytes);
   };
   RR_TRY(diff_nbr_bwd(Td));
   for (int t = Td; t >= 1; --t) {
-    RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.nm[t - 1], hp, G + L.dif_Wh_m, hp, G + L.dif_bh, s));
-    RR_TRY(linear_wgrad(A, hp, RR_FB_LD, W.gA1, hp, W.nf, RR_FB_LD, G + L.dif_Wh_f, RR_FB_LD, nullptr, s));
+    RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.nm[t - 1], hp, G + L.dif_Wh_m, hp, G + L.dif_bh, s, W.det, W.det_bytes));
+    RR_TRY(linear_wgrad(A, hp, RR_FB_LD, W.gA1, hp, W.nf, RR_FB_LD, G + L.dif_Wh_f, RR_FB_LD, nullptr, s, W.det, W.det_bytes));
     RR_TRY(dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wh_m, hp, P + L.dif_Wh_m_T, hp, W.gA2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
     RR_TRY(diff_nbr_bwd(t - 1));
   }
-  RR_TRY(linear_wgrad(A, hp, hp, W.dI2, hp, W.d, hp, G + L.dif_Wi, hp, G + L.dif_bi, s));
+  RR_TRY(linear_wgrad(A, hp, hp, W.dI2, hp, W.d, hp, G + L.dif_Wi, hp, G + L.dif_bi, s, W.det, W.det_bytes));
   RR_TRY(dgrad(A, hp, hp, W.dI2, hp, P + L.dif_Wi, hp, P + L.dif_Wi_T, hp, W.dD, hp, 1, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
 
   // shared encoder, once over [reactant rows | product rows]: d(hid_p) = +dD, d(hid_r) = -dD (base_model.py:168), each through the
@@ -704,18 +728,18 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
     } else {
       RR_TRY(relu_bwd(A_r, hp, W.dD, W.enc[0].hid, -keep, 0, W.gA1, nullptr, 0, s));
     }
-    RR_TRY(linear_wgrad(A_J, hp, RR_FA_LD, W.gA1, hp, g->f_atoms, RR_FA_LD, G + L.enc_Wo_a, RR_FA_LD, G + L.enc_bo, s));
-    RR_TRY(linear_wgrad(A_J, hp, hp, W.gA1, hp, e.am, hp, G + L.enc_Wo_m, hp, nullptr, s));
+    RR_TRY(linear_wgrad(A_J, hp, RR_FA_LD, W.gA1, hp, g->f_atoms, RR_FA_LD, G + L.enc_Wo_a, RR_FA_LD, G + L.enc_bo, s, W.det, W.det_bytes));
+    RR_TRY(linear_wgrad(A_J, hp, hp, W.gA1, hp, e.am, hp, G + L.enc_Wo_m, hp, nullptr, s, W.det, W.det_bytes));
     RR_TRY(dgrad(A_J, hp, hp, W.gA1, hp, P + L.enc_Wo_m, hp, P + L.enc_Wo_m_T, hp, W.gA2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
-    if (T >= 1) RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.m[T], keep, 0, W.dinp, 1, 0, s));
-    else RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 1, 1, s));
+    if (T >= 1) RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.m[T], keep, 0, W.dinp, 1, 0, s, W.det, W.det_bytes));
+    else RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 1, 1, s, W.det, W.det_bytes));
     for (int t = T; t >= 1; --t) {
-      RR_TRY(linear_wgrad(B_J, hp, hp, W.gB1, hp, e.pre[t - 1], hp, G + L.enc_Wh, hp, G + L.enc_bh, s));
+      RR_TRY(linear_wgrad(B_J, hp, hp, W.gB1, hp, e.pre[t - 1], hp, G + L.enc_Wh, hp, G + L.enc_bh, s, W.det, W.det_bytes));
       RR_TRY(dgrad(B_J, hp, hp, W.gB1, hp, P + L.enc_Wh, hp, P + L.enc_Wh_T, hp, W.gB2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
-      if (t - 1 >= 1) RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.m[t - 1], keep, 0, W.dinp, 2, 0, s));
-      else RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 2, 1, s));
+      if (t - 1 >= 1) RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.m[t - 1], keep, 0, W.dinp, 2, 0, s, W.det, W.det_bytes));
+      else RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 2, 1, s, W.det, W.det_bytes));
     }
-    RR_TRY(linear_wgrad(B_J, hp, RR_FB_LD, W.dinp, hp, g->f_bonds, RR_FB_LD, G + L.enc_Wi, RR_FB_LD, G + L.enc_bi, s));
+    RR_TRY(linear_wgrad(B_J, hp, RR_FB_LD, W.dinp, hp, g->f_bonds, RR_FB_LD, G + L.enc_Wi, RR_FB_LD, G + L.enc_bi, s, W.det, W.det_bytes));
   }
 
   PackTable Tb = make_table(*c, L, *grads, false);

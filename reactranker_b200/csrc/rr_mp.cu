@@ -107,18 +107,26 @@ __global__ void __launch_bounds__(512, 2) k_bond_fwd(rr_graph g, const float* __
 // ---------------------------------------------------------------------------------------
 // backward: dm from dpre.  dm[b_k] = S_a - dpre[rev(b_k)],  S_a = sum_k dpre[rev(b_k)]
 // padding row: dm[pad] += sum_a pad_count_a * S_a - dpre[pad]   (row pre-zeroed by k_zero_rows)
+// DET = true (deterministic mode): the padding-row partials go to pp, and pad_rows_sum() adds them (rr_common.cuh: PadParts)
 // ---------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(512, 2) k_bond_bwd(rr_graph g, const float* __restrict__ dpre, float* __restrict__ dm, int ld) {
+template <bool DET>
+__global__ void __launch_bounds__(512, 2) k_bond_bwd(rr_graph g, const float* __restrict__ dpre, float* __restrict__ dm, int ld, PadParts pp) {
   RR_ATOM_SETUP();
   float4 pad_acc = f4_zero();
   int pad_row = -1;
+  int pad_j = 0;
+  const long long unit = static_cast<long long>(blockIdx.x) * apb + slot;
   Task nx;
   load_task<true>(nx, g, g.a2b, a);
   for (; a < g.n_atoms; a += stride) {
     const Task t = nx;
     if (a + stride < g.n_atoms) load_task<true>(nx, g, g.a2b, a + stride);
     if (t.pad_bond != pad_row) {
-      if (pad_row >= 0) red_add_f4(dm + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+      if constexpr (DET) {
+        if (pad_row >= 0) pad_part_store(pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+      } else {
+        if (pad_row >= 0) red_add_f4(dm + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+      }
       pad_acc = f4_zero();
       pad_row = t.pad_bond;
     }
@@ -146,7 +154,11 @@ __global__ void __launch_bounds__(512, 2) k_bond_bwd(rr_graph g, const float* __
     pad_acc = f4_fma(static_cast<float>(t.pad_count), S, pad_acc);
     pad_acc = f4_sub(pad_acc, self);
   }
-  if (pad_row >= 0) red_add_f4(dm + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+  if constexpr (DET) {
+    if (pad_row >= 0) pad_part_store(pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+  } else {
+    if (pad_row >= 0) red_add_f4(dm + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+  }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -176,10 +188,13 @@ __global__ void __launch_bounds__(512, 2) k_nbr_sum_fwd(rr_graph g, int which, c
 }
 
 // backward over bond rows (which = 0): dsrc[b_k] = dout[a]; dsrc[pad] += pad_count * dout[a]
-__global__ void __launch_bounds__(512, 2) k_nbr_sum_bwd_bond(rr_graph g, const float* __restrict__ dout, float* __restrict__ dsrc, int ld) {
+template <bool DET>
+__global__ void __launch_bounds__(512, 2) k_nbr_sum_bwd_bond(rr_graph g, const float* __restrict__ dout, float* __restrict__ dsrc, int ld, PadParts pp) {
   RR_ATOM_SETUP();
   float4 pad_acc = f4_zero();
   int pad_row = -1;
+  int pad_j = 0;
+  const long long unit = static_cast<long long>(blockIdx.x) * apb + slot;
   Task nx;
   load_task<false>(nx, g, g.a2b, a);
   float4 vn = ld_row(dout, a, ld, c4, false);
@@ -191,7 +206,11 @@ __global__ void __launch_bounds__(512, 2) k_nbr_sum_bwd_bond(rr_graph g, const f
       vn = ld_row(dout, a + stride, ld, c4, false);
     }
     if (t.pad_bond != pad_row) {
-      if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+      if constexpr (DET) {
+        if (pad_row >= 0) pad_part_store(pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+      } else {
+        if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+      }
       pad_acc = f4_zero();
       pad_row = t.pad_bond;
     }
@@ -202,22 +221,33 @@ __global__ void __launch_bounds__(512, 2) k_nbr_sum_bwd_bond(rr_graph g, const f
     for (int k = kFast; k < t.deg; ++k) st_f4(dsrc + static_cast<size_t>(__ldg(ib + k)) * ld + c4, v);
     pad_acc = f4_fma(static_cast<float>(t.pad_count), v, pad_acc);
   }
-  if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+  if constexpr (DET) {
+    if (pad_row >= 0) pad_part_store(pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+  } else {
+    if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+  }
 }
 
 // backward over atom rows (which = 1): the neighbour relation is symmetric, so
 // dsrc[a] = sum_k dout[a2a[a,k]] (real neighbours only); dsrc[pad_atom] += pad_count_a * dout[a]
-__global__ void __launch_bounds__(512, 2) k_nbr_sum_bwd_atom(rr_graph g, const float* __restrict__ dout, float* __restrict__ dsrc, int ld) {
+template <bool DET>
+__global__ void __launch_bounds__(512, 2) k_nbr_sum_bwd_atom(rr_graph g, const float* __restrict__ dout, float* __restrict__ dsrc, int ld, PadParts pp) {
   RR_ATOM_SETUP();
   float4 pad_acc = f4_zero();
   int pad_row = -1;
+  int pad_j = 0;
+  const long long unit = static_cast<long long>(blockIdx.x) * apb + slot;
   Task nx;
   load_task<false>(nx, g, g.a2a, a);
   for (; a < g.n_atoms; a += stride) {
     const Task t = nx;
     if (a + stride < g.n_atoms) load_task<false>(nx, g, g.a2a, a + stride);
     if (t.pad_atom != pad_row) {
-      if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+      if constexpr (DET) {
+        if (pad_row >= 0) pad_part_store(pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+      } else {
+        if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+      }
       pad_acc = f4_zero();
       pad_row = t.pad_atom;
     }
@@ -236,7 +266,11 @@ __global__ void __launch_bounds__(512, 2) k_nbr_sum_bwd_atom(rr_graph g, const f
     if (!t.is_pad) st_f4(dsrc + static_cast<size_t>(a) * ld + c4, acc);
     pad_acc = f4_fma(static_cast<float>(t.pad_count), self, pad_acc);
   }
-  if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+  if constexpr (DET) {
+    if (pad_row >= 0) pad_part_store(pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+  } else {
+    if (pad_row >= 0) red_add_f4(dsrc + static_cast<size_t>(pad_row) * ld + c4, pad_acc);
+  }
 }
 
 __global__ void k_zero_rows(float* __restrict__ base, const int* __restrict__ rows, int n_rows, int ld) {
@@ -426,23 +460,52 @@ static int check_act(const float* y, float* acc, int acc_mode, int skip_out) {
 
 // dm = bond_message_bwd(dpre), then (y != NULL) the ReLU / dropout backward that follows it in the model:
 // dz = dm * mask(y) * scale written to dm (unless skip_out) and stored / added into acc
+// Deterministic mode: scratch for the padding-row partials (the caller's `det` when given, else transient)
+static int det_pad_scratch(DetScratch* ds, const rr_graph* g, int ld, void* det, long long det_bytes, long long* bytes, cudaStream_t s) {
+  const long long need = pad_parts_bytes(g->n_atoms, g->n_segments, ld);
+  RR_TRY(det_scratch(ds, det, det_bytes, need, s));
+  *bytes = det ? det_bytes : need;
+  return RR_OK;
+}
+// first generation, deterministic: the partials of the launch's units (blocks x atoms per block, see atom_launch_dims)
+static int v1_pad_parts(const DetScratch& ds, long long bytes, const rr_graph* g, int ld, dim3 grid, PadParts* pp, cudaStream_t s) {
+  const int apb = 256 / (ld >> 2) > 0 ? 256 / (ld >> 2) : 1;
+  const long long units = static_cast<long long>(grid.x) * apb;
+  return pad_parts_setup(ds.p, bytes, units, (g->n_atoms + units - 1) / units, g->n_segments, ld, pp, s);
+}
+
 int bond_message_bwd_act(const rr_graph* g, const float* dpre, float* dm, int hp, const float* y, float scale, int preact, float* acc, int acc_mode,
-                         int skip_out, cudaStream_t s) {
+                         int skip_out, cudaStream_t s, void* det, long long det_bytes) {
   RR_TRY(check_graph(g, hp));
   RR_REQUIRE(dpre && dm && aligned16(dpre) && aligned16(dm), "dpre/dm must be non-NULL and 16-byte aligned");
   RR_REQUIRE(g->pad_bonds && g->n_segments > 0, "graph needs pad_bonds/n_segments");
   if (y) RR_TRY(check_act(y, acc, acc_mode, skip_out));
   {
     ProfScope prof_scope(KC_BOND_BWD, s);
+    DetScratch ds;
+    long long ds_bytes = 0;
+    PadParts pp{};
+    const bool in_det = deterministic();
+    if (in_det) RR_TRY(det_pad_scratch(&ds, g, hp, det, det_bytes, &ds_bytes, s));
     RR_TRY(zero_rows(dm, g->pad_bonds, g->n_segments, hp, s));
     int st = RR_ERR_UNSUPPORTED;
-    if (use_pipe()) st = rowpipe_launch(PIPE_BOND_BWD, g, 0, dpre, dm, hp, 0, y, scale, preact, acc, acc_mode, skip_out, s);
-    if (st == RR_OK) return y ? pad_rows_act(dm, g->pad_bonds, g->n_segments, hp, y, scale, preact, acc, acc_mode, skip_out, s) : RR_OK;
+    if (use_pipe()) st = rowpipe_launch(PIPE_BOND_BWD, g, 0, dpre, dm, hp, 0, y, scale, preact, acc, acc_mode, skip_out, s, ds.p, ds_bytes, &pp);
+    if (st == RR_OK) {
+      if (in_det) RR_TRY(pad_rows_sum(dm, g->pad_bonds, g->n_segments, hp, pp, s));
+      return y ? pad_rows_act(dm, g->pad_bonds, g->n_segments, hp, y, scale, preact, acc, acc_mode, skip_out, s) : RR_OK;
+    }
     if (st != RR_ERR_UNSUPPORTED) return st;
     dim3 grid, block;
     atom_launch_dims(g->n_atoms, hp, &grid, &block);
-    k_bond_bwd<<<grid, block, 0, s>>>(*g, dpre, dm, hp);
-    RR_LAUNCH_CHECK("k_bond_bwd");
+    if (in_det) {
+      RR_TRY(v1_pad_parts(ds, ds_bytes, g, hp, grid, &pp, s));
+      k_bond_bwd<true><<<grid, block, 0, s>>>(*g, dpre, dm, hp, pp);
+      RR_LAUNCH_CHECK("k_bond_bwd");
+      RR_TRY(pad_rows_sum(dm, g->pad_bonds, g->n_segments, hp, pp, s));
+    } else {
+      k_bond_bwd<false><<<grid, block, 0, s>>>(*g, dpre, dm, hp, pp);
+      RR_LAUNCH_CHECK("k_bond_bwd");
+    }
   }
   return y ? relu_bwd(g->n_bonds, hp, dm, y, scale, preact, skip_out ? nullptr : dm, acc, acc_mode, s) : RR_OK;
 }
@@ -467,7 +530,7 @@ int neighbor_sum_fwd(const rr_graph* g, int which, const float* src, float* out,
 }
 
 int neighbor_sum_bwd_act(const rr_graph* g, int which, const float* dout, float* dsrc, int ld, const float* y, float scale, int preact, float* acc,
-                         int acc_mode, int skip_out, cudaStream_t s) {
+                         int acc_mode, int skip_out, cudaStream_t s, void* det, long long det_bytes) {
   RR_TRY(check_graph(g, ld));
   RR_REQUIRE(dout && dsrc && aligned16(dout) && aligned16(dsrc), "dout/dsrc must be non-NULL and 16-byte aligned");
   RR_REQUIRE(g->pad_bonds && g->pad_atoms && g->n_segments > 0, "graph needs pad rows/n_segments");
@@ -475,20 +538,34 @@ int neighbor_sum_bwd_act(const rr_graph* g, int which, const float* dout, float*
   const int* pads = which == 0 ? g->pad_bonds : g->pad_atoms;
   {
     ProfScope prof_scope(KC_NBR_BWD, s);
+    DetScratch ds;
+    long long ds_bytes = 0;
+    PadParts pp{};
+    const bool in_det = deterministic();
+    if (in_det) RR_TRY(det_pad_scratch(&ds, g, ld, det, det_bytes, &ds_bytes, s));
     RR_TRY(zero_rows(dsrc, pads, g->n_segments, ld, s));
     int st = RR_ERR_UNSUPPORTED;
-    if (use_pipe()) st = rowpipe_launch(which == 0 ? PIPE_NBR_BWD_BOND : PIPE_NBR_BWD_ATOM, g, which, dout, dsrc, ld, 0, y, scale, preact, acc, acc_mode, skip_out, s);
-    if (st == RR_OK) return y ? pad_rows_act(dsrc, pads, g->n_segments, ld, y, scale, preact, acc, acc_mode, skip_out, s) : RR_OK;
+    if (use_pipe())
+      st = rowpipe_launch(which == 0 ? PIPE_NBR_BWD_BOND : PIPE_NBR_BWD_ATOM, g, which, dout, dsrc, ld, 0, y, scale, preact, acc, acc_mode, skip_out, s, ds.p,
+                          ds_bytes, &pp);
+    if (st == RR_OK) {
+      if (in_det) RR_TRY(pad_rows_sum(dsrc, pads, g->n_segments, ld, pp, s));
+      return y ? pad_rows_act(dsrc, pads, g->n_segments, ld, y, scale, preact, acc, acc_mode, skip_out, s) : RR_OK;
+    }
     if (st != RR_ERR_UNSUPPORTED) return st;
     dim3 grid, block;
     atom_launch_dims(g->n_atoms, ld, &grid, &block);
+    if (in_det) RR_TRY(v1_pad_parts(ds, ds_bytes, g, ld, grid, &pp, s));
     if (which == 0) {
-      k_nbr_sum_bwd_bond<<<grid, block, 0, s>>>(*g, dout, dsrc, ld);
+      if (in_det) k_nbr_sum_bwd_bond<true><<<grid, block, 0, s>>>(*g, dout, dsrc, ld, pp);
+      else k_nbr_sum_bwd_bond<false><<<grid, block, 0, s>>>(*g, dout, dsrc, ld, pp);
       RR_LAUNCH_CHECK("k_nbr_sum_bwd_bond");
     } else {
-      k_nbr_sum_bwd_atom<<<grid, block, 0, s>>>(*g, dout, dsrc, ld);
+      if (in_det) k_nbr_sum_bwd_atom<true><<<grid, block, 0, s>>>(*g, dout, dsrc, ld, pp);
+      else k_nbr_sum_bwd_atom<false><<<grid, block, 0, s>>>(*g, dout, dsrc, ld, pp);
       RR_LAUNCH_CHECK("k_nbr_sum_bwd_atom");
     }
+    if (in_det) RR_TRY(pad_rows_sum(dsrc, pads, g->n_segments, ld, pp, s));
   }
   return y ? relu_bwd(which == 0 ? g->n_bonds : g->n_atoms, ld, dsrc, y, scale, preact, skip_out ? nullptr : dsrc, acc, acc_mode, s) : RR_OK;
 }

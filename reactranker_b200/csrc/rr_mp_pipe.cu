@@ -18,7 +18,8 @@
 //   NBR_BWD_ATOM  dsrc[a] = sum_k dout[a2a[a,k]]                                               (symmetric relation)
 // The backward ops optionally carry the ReLU / inverted-dropout backward that always follows them in the model
 // (rr_relu_bwd: dz = d * [y != 0] * scale, acc (+)= dz) so that the raw gradient never makes a round trip through HBM;
-// the segment padding rows, which are reduced with atomics, get that epilogue from a tiny follow-up kernel.
+// the segment padding rows, which are reduced with atomics, get that epilogue from a tiny follow-up kernel.  In deterministic mode the
+// backward ops store the padding-row partials instead (k_rowpipe<.., DET = true>) and k_pad_rows_sum adds them in a fixed order first.
 #include <stdlib.h>
 
 #include "rr_common.cuh"
@@ -67,6 +68,7 @@ struct Args {
   int producers, round_stages, consumer_warps;   // active producer warps, stages per producer round
   int n_nbr, n_own; // row sources per neighbour / per atom
   int stage_bytes, row_bytes;
+  PadParts pp;      // DET kernels: padding-row partials, unit = blockIdx.x * apb + slot
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
@@ -132,7 +134,8 @@ __device__ __forceinline__ const float* own_source(const Args& a, int j) {
   return j == 0 ? a.src : (j == 1 ? a.y : a.acc);             // NBR_BWD_ATOM: dout[a], y[a], acc[a]
 }
 
-template <int OP, bool FUSED>
+// DET = true (deterministic mode, backward ops): a padding-row partial is stored to A.pp instead of added into the row with atomics.
+template <int OP, bool FUSED, bool DET>
 __global__ void __launch_bounds__(MAX_CONSUMERS + 32 * PRODUCERS, 1) k_rowpipe(const __grid_constant__ Args A) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 127) & ~static_cast<uintptr_t>(127));
@@ -262,6 +265,8 @@ __global__ void __launch_bounds__(MAX_CONSUMERS + 32 * PRODUCERS, 1) k_rowpipe(c
     constexpr bool REDUCES = (OP == BOND_BWD || OP == NBR_BWD_BOND || OP == NBR_BWD_ATOM);
     float4 pad_acc = f4_zero();
     int pad_row = -1;
+    int pad_j = 0;                    // DET: padding rows this unit has met
+    const long long unit = static_cast<long long>(blockIdx.x) * apb + slot;
     float4 padv_c = f4_zero();        // this thread's chunk of the segment's padding row of src: constant while the segment lasts
     int padv_row = -1;
     const float* src_c = A.src + c4;
@@ -309,7 +314,11 @@ __global__ void __launch_bounds__(MAX_CONSUMERS + 32 * PRODUCERS, 1) k_rowpipe(c
           asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(q1.x), "=r"(q1.y), "=r"(q1.z), "=r"(q1.w) : "r"(base + task_off + 16));
         const int wrow[kFast] = {q1.x, q1.y, q1.z, q1.w};
         if (REDUCES && prow != pad_row) {
-          if (pad_row >= 0) red_add_f4(out_c + static_cast<size_t>(pad_row) * ld, pad_acc);
+          if constexpr (DET) {
+            if (pad_row >= 0) pad_part_store(A.pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+          } else {
+            if (pad_row >= 0) red_add_f4(out_c + static_cast<size_t>(pad_row) * ld, pad_acc);
+          }
           pad_acc = f4_zero();
           pad_row = prow;
         }
@@ -442,7 +451,11 @@ __global__ void __launch_bounds__(MAX_CONSUMERS + 32 * PRODUCERS, 1) k_rowpipe(c
         ph ^= 1;
       }
     }
-    if (REDUCES && active && pad_row >= 0) red_add_f4(out_c + static_cast<size_t>(pad_row) * ld, pad_acc);
+    if constexpr (DET) {
+      if (REDUCES && active && pad_row >= 0) pad_part_store(A.pp, unit, pad_j, pad_row, ld, c4, pad_acc);
+    } else {
+      if (REDUCES && active && pad_row >= 0) red_add_f4(out_c + static_cast<size_t>(pad_row) * ld, pad_acc);
+    }
   }
 }
 
@@ -460,11 +473,76 @@ __global__ void k_pad_rows_act(float* __restrict__ out, const int* __restrict__ 
   }
 }
 
+// Deterministic mode: out[rows[r]] = the entries tagged rows[r].  One block per row: threadIdx.x walks the row's 16-byte chunks, and each
+// of the blockDim.y slices adds a fixed contiguous run of entries in entry order (four loads in flight; an entry of another row adds an
+// exact 0); the slices' sums are then added in slice order.  The partition depends only on the entry count and the row width.
+__global__ void k_pad_rows_sum(float* __restrict__ out, const int* __restrict__ rows, int ld, const float* __restrict__ parts,
+                               const int* __restrict__ tags, long long entries) {
+  extern __shared__ float4 slice_sum[];
+  const int row = __ldg(rows + blockIdx.x);
+  const int c = threadIdx.x * 4;
+  const long long per = (entries + blockDim.y - 1) / blockDim.y;
+  const long long e_beg = per * threadIdx.y, e_end = min(entries, e_beg + per);
+  float4 acc = f4_zero();
+  if (c < ld) {
+    long long e = e_beg;
+    for (; e + 4 <= e_end; e += 4) {
+      float4 v[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) v[q] = __ldg(tags + e + q) == row ? ld_f4(parts + (e + q) * ld + c) : f4_zero();
+#pragma unroll
+      for (int q = 0; q < 4; ++q) acc = f4_add(acc, v[q]);
+    }
+    for (; e < e_end; ++e)
+      if (__ldg(tags + e) == row) acc = f4_add(acc, ld_f4(parts + e * ld + c));
+  }
+  slice_sum[threadIdx.y * blockDim.x + threadIdx.x] = acc;
+  __syncthreads();
+  if (threadIdx.y == 0 && c < ld) {
+    for (int y = 1; y < static_cast<int>(blockDim.y); ++y) acc = f4_add(acc, slice_sum[y * blockDim.x + threadIdx.x]);
+    st_f4(out + static_cast<size_t>(row) * ld + c, acc);
+  }
+}
+
 }  // namespace pipe
+
+long long pad_parts_bytes(int n_atoms, int n_segments, int ld) {
+  const long long cpr = ld >> 2;
+  const long long v1_units = static_cast<long long>(num_sms()) * 4 * (cpr < 256 ? 256 / cpr : 1);
+  const long long pipe_units = static_cast<long long>(num_sms()) * 32;
+  const long long U = v1_units > pipe_units ? v1_units : pipe_units;
+  long long entries = U * n_segments;
+  if (entries > n_atoms + 2 * U) entries = n_atoms + 2 * U;   // a unit meets at most as many padding rows as it has atoms
+  return entries * (static_cast<long long>(ld) * 4 + 4) + 64;
+}
+
+int pad_parts_setup(void* scratch, long long bytes, long long units, long long atoms_per_unit, int n_segments, int ld, PadParts* pp, cudaStream_t s) {
+  // Segments are concatenated (rr_graph), so a unit walking its atoms upwards meets each padding row in one run: at most
+  // min(n_segments, its atoms) of them.
+  long long jcap = atoms_per_unit < n_segments ? atoms_per_unit : n_segments;
+  if (jcap < 1) jcap = 1;
+  const long long entries = units * jcap;
+  const long long need = entries * (static_cast<long long>(ld) * 4 + 4);
+  if (scratch == nullptr || need > bytes) return fail(RR_ERR_WORKSPACE, "deterministic padding rows: scratch of %lld bytes < %lld", bytes, need);
+  pp->parts = static_cast<float*>(scratch);
+  pp->tags = reinterpret_cast<int*>(static_cast<char*>(scratch) + entries * ld * 4);
+  pp->jcap = static_cast<int>(jcap);
+  pp->entries = entries;
+  RR_CUDA(cudaMemsetAsync(pp->tags, 0xFF, static_cast<size_t>(entries) * sizeof(int), s));
+  return RR_OK;
+}
+
+int pad_rows_sum(float* out, const int* rows, int n_rows, int ld, const PadParts& pp, cudaStream_t s) {
+  if (n_rows <= 0) return RR_OK;
+  const int tx = ((ld >> 2) + 31) / 32 * 32, ty = 1024 / tx;
+  pipe::k_pad_rows_sum<<<n_rows, dim3(tx, ty), static_cast<size_t>(tx) * ty * sizeof(float4), s>>>(out, rows, ld, pp.parts, pp.tags, pp.entries);
+  RR_LAUNCH_CHECK("k_pad_rows_sum");
+  return RR_OK;
+}
 
 // Host side: returns RR_ERR_UNSUPPORTED (without launching) when the shape does not suit the pipeline, so callers can use the first-generation kernel.
 int rowpipe_launch(int op, const rr_graph* g, int which, const float* src, float* out, int ld, int relu_src, const float* y, float scale, int preact,
-                   float* acc, int acc_mode, int skip_out, cudaStream_t s) {
+                   float* acc, int acc_mode, int skip_out, cudaStream_t s, void* det, long long det_bytes, PadParts* pp) {
   using namespace pipe;
   Args A{};
   A.g = *g;
@@ -515,24 +593,35 @@ int rowpipe_launch(int op, const rr_graph* g, int which, const float* src, float
   int grid = num_sms();
   if (grid > A.n_stage_total) grid = A.n_stage_total;
   const size_t smem = 128 + 256 + static_cast<size_t>(A.stages) * A.stage_bytes;
-#define RR_PIPE_LAUNCH(OPV, F)                                                                                              \
+  const bool det_op = det != nullptr && (op == BOND_BWD || op == NBR_BWD_BOND || op == NBR_BWD_ATOM);
+  if (det_op) {
+    RR_TRY(pad_parts_setup(det, det_bytes, static_cast<long long>(grid) * A.apb, (A.n_stage_total + grid - 1) / grid, g->n_segments, ld, &A.pp, s));
+    *pp = A.pp;
+  }
+#define RR_PIPE_LAUNCH1(OPV, F, D)                                                                                          \
   do {                                                                                                                      \
     static PerDeviceOnce attr_set;                                                                                           \
     if (attr_set.need()) {                                                                                                        \
-      RR_CUDA(cudaFuncSetAttribute(k_rowpipe<OPV, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BUDGET + 1024));   \
+      RR_CUDA(cudaFuncSetAttribute(k_rowpipe<OPV, F, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BUDGET + 1024));   \
       attr_set.mark();                                                                                                      \
     }                                                                                                                       \
-    RR_CUDA(launch_pdl(k_rowpipe<OPV, F>, dim3(grid), dim3(A.consumer_warps * 32 + 32 * PRODUCERS), smem, s, A));                                                                    \
+    RR_CUDA(launch_pdl(k_rowpipe<OPV, F, D>, dim3(grid), dim3(A.consumer_warps * 32 + 32 * PRODUCERS), smem, s, A));                                                                    \
+  } while (0)
+#define RR_PIPE_LAUNCH(OPV, F)                      \
+  do {                                              \
+    if (det_op) RR_PIPE_LAUNCH1(OPV, F, true);      \
+    else RR_PIPE_LAUNCH1(OPV, F, false);            \
   } while (0)
   switch (op) {
-    case BOND_FWD: RR_PIPE_LAUNCH(BOND_FWD, false); break;
+    case BOND_FWD: RR_PIPE_LAUNCH1(BOND_FWD, false, false); break;
     case BOND_BWD: if (fused) RR_PIPE_LAUNCH(BOND_BWD, true); else RR_PIPE_LAUNCH(BOND_BWD, false); break;
-    case NBR_FWD: RR_PIPE_LAUNCH(NBR_FWD, false); break;
+    case NBR_FWD: RR_PIPE_LAUNCH1(NBR_FWD, false, false); break;
     case NBR_BWD_BOND: if (fused) RR_PIPE_LAUNCH(NBR_BWD_BOND, true); else RR_PIPE_LAUNCH(NBR_BWD_BOND, false); break;
     case NBR_BWD_ATOM: if (fused) RR_PIPE_LAUNCH(NBR_BWD_ATOM, true); else RR_PIPE_LAUNCH(NBR_BWD_ATOM, false); break;
     default: return fail(RR_ERR_INVALID, "rowpipe: unknown op %d", op);
   }
 #undef RR_PIPE_LAUNCH
+#undef RR_PIPE_LAUNCH1
   RR_LAUNCH_CHECK("k_rowpipe");
   return RR_OK;
 }

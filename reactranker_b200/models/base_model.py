@@ -58,6 +58,18 @@ class FFN(nn.Module):
         raise NotImplementedError("FFN runs fused inside ReactionModel.forward (reactranker_b200/csrc/rr_model.cu)")
 
 
+def reactant_dedup_exact(model) -> bool:
+    """Whether ``model`` may encode each distinct reactant once (rr_model_cfg.r_atom_map) instead of once per candidate.  The scores are the
+    same in eval mode and at dropout 0 (with dropout the reference draws a mask per copy).  Under torch.use_deterministic_algorithms it is
+    used only where no backward pass can follow (eval mode with grad disabled): the gradient of a shared row is a sum over its copies
+    that rr_model_backward forms with atomics, so the deterministic backward refuses it."""
+    if not getattr(model, "dedup_reactants", False):
+        return False
+    if model.training and getattr(model, "_dropout", 0) > 0:
+        return False
+    return not _lib.deterministic_requested() or (not model.training and not torch.is_grad_enabled())
+
+
 class _WorkspacePool:
     """Saved-for-backward workspaces (3-7 GB per step) recycled between steps.  Batch composition changes every step, so
     the exact size does too: asking the caching allocator for a fresh block per step ends in cudaMalloc / cudaFree
@@ -90,6 +102,10 @@ class _ReactionFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model, rg: DeviceGraph, pg: DeviceGraph, addf, *params):
         L = _lib.lib()
+        # torch.use_deterministic_algorithms(True) selects the library's deterministic mode for this step: set before the workspace is
+        # sized (it then includes the backward's scratch) and recorded, so that the backward runs in the same mode
+        det = _lib.deterministic_requested()
+        _lib.set_deterministic(det)
         cfg = model._cfg(training=model.training)
         amap = getattr(rg, "atom_map", None)
         if amap is not None:
@@ -109,7 +125,7 @@ class _ReactionFn(torch.autograd.Function):
         if not any(ctx.needs_input_grad):        # inference: nothing will come back for the activations
             model._ws_pool.give(ws)
             ws = None
-        ctx.model, ctx.rg, ctx.pg, ctx.cfg, ctx.ws, ctx.addf = model, rg, pg, cfg, ws, addf
+        ctx.model, ctx.rg, ctx.pg, ctx.cfg, ctx.ws, ctx.addf, ctx.det = model, rg, pg, cfg, ws, addf, det
         ctx.save_for_backward(*params)
         return scores
 
@@ -132,6 +148,7 @@ class _ReactionFn(torch.autograd.Function):
         grads = [flat[o:o + p.numel()].view(p.shape) for o, p in zip(offs, params)]
         gw = model._param_struct(grads)
         dscores = dscores.contiguous().float()
+        _lib.set_deterministic(ctx.det)
         _lib.check(L.rr_model_backward(ctypes.byref(ctx.cfg), ctypes.byref(w), ctypes.byref(ctx.rg.c), ctypes.byref(ctx.pg.c),
                                        dscores.data_ptr(), ctypes.byref(gw), ctx.ws.data_ptr(), ctx.ws.numel(), _lib.stream_ptr()))
         model._ws_pool.give(ctx.ws)
@@ -217,7 +234,7 @@ class ReactionModel(nn.Module):
         params = [p for _, p in self._named_slots()]
         if params[0].device != dev:
             raise _lib.RRError(f"model parameters live on {params[0].device}, expected {dev}: call model.cuda({dev_idx}) first")
-        if (self.dedup_reactants and not (self.training and self._dropout > 0) and isinstance(r_inputs, BatchMolGraph)
+        if (reactant_dedup_exact(self) and isinstance(r_inputs, BatchMolGraph)
                 and isinstance(p_inputs, BatchMolGraph) and r_inputs._ids is not None and p_inputs._ids is not None):
             # every candidate of a group repeats the reactant graph (load_reactions.py:574-576): without dropout the copies are identical,
             # so each distinct reactant is encoded once (rr_model_cfg.r_atom_map); with dropout the reference draws a mask per copy
@@ -240,6 +257,10 @@ class ReactionModel(nn.Module):
                 addf = host.pin_memory().to(dev, non_blocking=True)
                 h2d += host.numel() * 4
         self.last_h2d_bytes = h2d
+        if getattr(rg, "atom_map", None) is not None and torch.is_grad_enabled() and _lib.deterministic_requested():
+            raise _lib.RRError("deterministic mode (torch.use_deterministic_algorithms) has no backward pass for de-duplicated reactants: "
+                               "build the graphs with one reactant row per candidate (DeviceGraph.from_batches / pair_from_batches), "
+                               "or run the forward under torch.no_grad()")
         with torch.cuda.device(dev):
             return _ReactionFn.apply(self, rg, pg, addf, *params)
 

@@ -11,6 +11,7 @@ import torch
 
 from .. import _lib
 from ..features.featurization import DeviceGraph
+from ..models.base_model import reactant_dedup_exact
 from .loss import segment_offsets
 
 GROUPS_PER_LAUNCH = 256
@@ -21,7 +22,7 @@ def _forward_chunks(model, gpu, chunks, smiles2graph_dic):
     ``max_num_bonds``, exactly as if it had been the reference's whole BatchMolGraph).  Yields ``(lo, hi, preds)`` with the scores of
     chunks[lo:hi] on the device, rows in chunk order."""
     dev = torch.device("cuda", gpu) if isinstance(gpu, int) else torch.device(gpu)
-    dedup = bool(getattr(model, "dedup_reactants", False)) and not (model.training and getattr(model, "_dropout", 0) > 0)
+    dedup = reactant_dedup_exact(model)
     fast = hasattr(smiles2graph_dic, "parsing_ids")
     for lo in range(0, len(chunks), GROUPS_PER_LAUNCH):
         part = chunks[lo:lo + GROUPS_PER_LAUNCH]

@@ -66,6 +66,7 @@ class _LossFn(torch.autograd.Function):
         scores_c = scores.contiguous()
         loss = torch.empty(1, dtype=torch.float32, device=scores.device)
         dscore = torch.empty_like(scores_c)
+        _lib.set_deterministic(_lib.deterministic_requested())
         with torch.cuda.device(scores.device):
             _lib.check(L.rr_loss_fwdbwd_ex(kind, n_items, n_groups, scores_c.data_ptr(), targets.data_ptr(), _lib.ptr(seg_off), int(max_group),
                                            float(norm), float(sigma), loss.data_ptr(), dscore.data_ptr(), _lib.stream_ptr()))
@@ -253,6 +254,7 @@ class _GaussFn(torch.autograd.Function):
         n = both.shape[0]
         loss = torch.empty(1, dtype=torch.float32, device=both.device)
         d = torch.empty_like(both)
+        _lib.set_deterministic(_lib.deterministic_requested())
         with torch.cuda.device(both.device):
             _lib.check(L.rr_loss_fwdbwd(_lib.LOSS_GAUSS, n, 0, both.data_ptr(), targets.data_ptr(), None, _items_norm(n), 1.0,
                                         loss.data_ptr(), d.data_ptr(), _lib.stream_ptr()))

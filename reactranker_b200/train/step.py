@@ -22,6 +22,7 @@ import numpy as np
 import torch
 
 from .. import _lib, parallel
+from ..models.base_model import reactant_dedup_exact
 from .loss import dp_normalisers
 
 
@@ -85,7 +86,7 @@ class TrainStep:
         if device_graphs or self.world > 1:
             model = self.model
             store_backed = isinstance(r_inputs, BatchMolGraph) and r_inputs._ids is not None and p_inputs._ids is not None
-            if (store_backed and getattr(model, "dedup_reactants", False) and not (model.training and getattr(model, "_dropout", 0) > 0)):
+            if store_backed and reactant_dedup_exact(model):
                 r_inputs, p_inputs = DeviceGraph.from_batches_dedup([r_inputs], [p_inputs], self.dev)     # exact without dropout only
             else:
                 r_inputs, p_inputs = DeviceGraph.pair_from_batches([r_inputs], [p_inputs], self.dev)
@@ -136,7 +137,7 @@ class TrainStep:
         if r1 == r0:
             return PreparedBatch(None, None, targets_t, [], feats, G, N, 0)
         model = self.model
-        dedup = bool(getattr(model, "dedup_reactants", False)) and not (model.training and getattr(model, "_dropout", 0) > 0)
+        dedup = reactant_dedup_exact(model)
         rg, pg = DeviceGraph.from_id_groups(store, r_all[r0:r1], p_all[r0:r1], [r1 - r0], self.dev, dedup, w_r, w_p)
         h2d = rg.h2d_bytes + pg.h2d_bytes
         if pinned:
