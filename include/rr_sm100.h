@@ -198,18 +198,25 @@ int rr_linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int 
                   const float* X2, int ldx2, const float* W2, int k2, const float* bias,
                   const float* residual, int ldr, float* Y, int ldy, int flags, float dropout,
                   uint64_t seed, uint64_t stream_id, void* stream);
-/* Which GEMM implementation the dense layers use: 0 = exact fp32 SIMT kernels, 1 = tcgen05 tensor cores with
- * an on-chip 3xTF32 split (fp32-class accuracy, ~1e-6 relative), TMA-fed, accumulating in TMEM.  Process-wide. */
+/* Which GEMM implementation the dense layers use.  TC = the tcgen05 tensor cores (TMA-fed, accumulating in TMEM) where the shape suits
+ * them, the exact-fp32 SIMT kernels otherwise:
+ *   mode | forward | dgrad of rr_model_backward | wgrad           | padding rows of rr_model_forward
+ *    0   | SIMT    | SIMT                       | SIMT            | as computed
+ *    1   | TC      | TC                         | TC for M >= 256 | recomputed in exact arithmetic, also where a shape fell back to SIMT
+ *    2   | TC      | SIMT                       | SIMT            | recomputed, as in mode 1
+ *    3   | SIMT    | TC                         | SIMT            | as computed
+ * rr_linear_dgrad is SIMT in every mode, rr_linear_dgrad_tc TC in every mode.  A TC GEMM splits its fp32 operands into 3 x TF32 products
+ * (fp32-class accuracy, ~1e-6 relative) or 3 x bf16 products, as the two switches below select.  Process-wide. */
 int rr_set_gemm_mode(int mode);
 int rr_get_gemm_mode(void);
-/* Operand split of the BACKWARD tensor-core GEMMs (dgrad; gradients never decide a ReLU mask): 1 (default) = 3 x bf16 products
+/* Operand split of the BACKWARD tensor-core GEMMs (dgrad and wgrad; gradients never decide a ReLU mask): 1 (default) = 3 x bf16 products
  * (x = bf16(x) + bf16(x - bf16(x)): 16 significand bits per operand, fp32 accumulation, ~5e-6 relative, half the tensor-pipe time),
- * 0 = the forward's 3 x tf32 split.  Process-wide; RR_BWD_BF16=0 in the environment selects 0 at load. */
+ * 0 = the forward's 3 x tf32 split.  Process-wide; the Python package sets it from RR_BWD_BF16 when it loads the library. */
 int rr_set_backward_bf16(int on);
 int rr_get_backward_bf16(void);
 /* Operand split of the FORWARD tensor-core GEMMs of rr_model_forward: 0 (default) = 3 x tf32, 1 = the backward's 3 x bf16 split (same
- * kernel, half the tensor-pipe time and operand bytes; 16 instead of 21 significand bits per operand).  Process-wide; RR_FWD_BF16=1 in
- * the environment selects 1 at load. */
+ * kernel, half the tensor-pipe time and operand bytes; 16 instead of 21 significand bits per operand).  rr_linear_fwd always takes 3 x tf32.
+ * Process-wide; the Python package sets it from RR_FWD_BF16 when it loads the library. */
 int rr_set_forward_bf16(int on);
 int rr_get_forward_bf16(void);
 /* Deterministic mode (torch.use_deterministic_algorithms of the Python package): 1 = every kernel rr_model_backward and

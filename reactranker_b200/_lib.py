@@ -15,7 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_HERE)
 CSRC = os.path.join(_HERE, "csrc")
 SO_PATH = os.path.join(_HERE, "librr_sm100.so")
-SOURCES = ["rr_api.cu", "rr_host.cu", "rr_mp.cu", "rr_mp_pipe.cu", "rr_gemm_simt.cu", "rr_gemm_tc.cu", "rr_assemble.cu", "rr_loss.cu", "rr_model.cu"]
+SOURCES = ["rr_api.cu", "rr_host.cu", "rr_mp.cu", "rr_mp_pipe.cu", "rr_gemm_simt.cu", "rr_gemm_tc.cu", "rr_linear.cu", "rr_assemble.cu", "rr_loss.cu", "rr_model.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

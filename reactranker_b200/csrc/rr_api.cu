@@ -118,12 +118,12 @@ int rr_linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int 
   return rr::linear_fwd(M, n, X1, ldx1, W1, k1, X2, ldx2, W2, k2, bias, residual, ldr, Y, ldy, flags, dropout, seed, stream_id, S(stream));
 }
 int rr_linear_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, void* stream) {
-  return rr::linear_dgrad(M, n, k, dZ, lddz, W, ldw, dX, lddx, accumulate, S(stream));
+  return rr::simt_dgrad(M, n, k, dZ, lddz, W, ldw, dX, lddx, accumulate, S(stream));
 }
 int64_t rr_linear_dgrad_tc_scratch_bytes(int n, int k) { return rr::tc_dgrad_scratch_bytes(n, k); }
 int rr_linear_dgrad_tc(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, void* scratch,
                        int64_t scratch_bytes, void* stream) {
-  return rr::tc_dgrad_standalone(M, n, k, dZ, lddz, W, ldw, dX, lddx, accumulate, scratch, scratch_bytes, S(stream));
+  return rr::linear_dgrad_tc(M, n, k, dZ, lddz, W, ldw, dX, lddx, accumulate, scratch, scratch_bytes, S(stream));
 }
 int rr_linear_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, void* stream) {
   return rr::linear_wgrad(M, n, k, dZ, lddz, X, ldx, dW, lddw, dbias, S(stream));

@@ -71,8 +71,11 @@ struct ProfScope {
   }
 };
 
-// 0 = fp32 SIMT GEMMs, 1 = tcgen05 3xTF32 GEMMs where the shape allows (forward + dgrad)
+// Precision switches of the dense layers (rr_set_gemm_mode / _backward_bf16 / _forward_bf16), read only by rr_linear.cu, whose header
+// comment gives the policy they select
 extern std::atomic<int> g_gemm_mode;
+extern std::atomic<int> g_fwd_bf16;
+extern std::atomic<int> g_bwd_bf16;
 
 // Deterministic mode (rr_set_deterministic): every sum the backward pass and the losses would form with atomics is instead written as
 // partials to scratch with plain stores and summed in a fixed order.  Process-wide.
@@ -113,6 +116,11 @@ void reload_switches();
   } while (0)
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+inline int check_mat(const char* what, const void* p, int ld) {
+  RR_REQUIRE(p != nullptr, "%s is NULL", what);
+  RR_REQUIRE(aligned16(p) && (ld & 3) == 0, "%s must be 16-byte aligned with a row stride multiple of 4 (ld %d)", what, ld);
+  return RR_OK;
+}
 constexpr int kMaxDevices = 64;
 inline int current_device() {
   int dev = 0;
@@ -272,16 +280,6 @@ int relu_bwd(long long, int, const float*, const float*, float, int, float*, flo
 int sub(long long, const float*, const float*, float*, cudaStream_t);
 int sub_gather(long long rows, int ld, const float* a, const float* b, const int* map, float* out, cudaStream_t);
 int scatter_add_rows(long long rows, int ld, const float* src, const int* map, float* dst, cudaStream_t);
-// hi_off / lo_off: float offsets from W1 / W2 to their pre-split TF32 images (0 = split on chip)
-// packed / bhi / blo: base of the packed weights and of their bf16 (hi, lo) images (image of W = bhi + (W - packed)); used when g_fwd_bf16
-int linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2, int k2,
-               const float* bias, const float* resid, int ldr, float* Y, int ldy, int flags, float p, uint64_t seed, uint64_t stream_id,
-               cudaStream_t s, ptrdiff_t hi_off = 0, ptrdiff_t lo_off = 0, const float* packed = nullptr, const uint16_t* bhi = nullptr,
-               const uint16_t* blo = nullptr);
-int linear_dgrad(int, int, int, const float*, int, const float*, int, float*, int, int, cudaStream_t);
-int linear_wgrad(int, int, int, const float*, int, const float*, int, float*, int, float*, cudaStream_t, void* det = nullptr, long long det_bytes = 0);
-// deterministic mode: bytes of scratch linear_wgrad(M, n, k, ...) needs (row-slab partials of dW and of the bias gradient), any GEMM mode
-long long wgrad_det_bytes(int M, int n, int k);
 int loss_fwdbwd(int, int, int, const float*, const float*, const int*, float, float, float*, float*, cudaStream_t, int max_group = 0);
 int loss_max_group();
 int rank_metrics(int, int, const float*, int, const double*, const int*, int, double, double*, cudaStream_t);
@@ -292,29 +290,69 @@ long long model_buffer_offset(const rr_model_cfg*, const rr_graph*, const rr_gra
 int model_forward(const rr_model_cfg*, const rr_params*, const rr_graph*, const rr_graph*, const float*, float*, void*, long long, cudaStream_t);
 int model_backward(const rr_model_cfg*, const rr_params*, const rr_graph*, const rr_graph*, const float*, rr_params*, void*, long long, cudaStream_t);
 
-// ---- tcgen05 GEMM entry points (rr_gemm_tc.cu) ---------------------------------------------
-bool tc_supported(int M, int n, int k1, int k2, int ldx1, int ldx2);
-int tc_linear(int M, int n, const float* X1, int ldx1, const float* W1, int ldw1, int k1, const float* X2, int ldx2, const float* W2, int ldw2, int k2,
-              const float* bias, const float* resid, int ldr, float* Y, int ldy, int relu, int accumulate, float p, uint64_t seed, uint64_t stream_id,
-              int kclass, cudaStream_t s, const float* W1lo = nullptr, const float* W2lo = nullptr);
-bool tc_linear_bf16_supported(int M, int n, int k, int ldx, int ldw);
-int tc_linear_bf16(int M, int n, const float* X, int ldx, const uint16_t* Whi, const uint16_t* Wlo, int ldw, int k, float* Y, int ldy, int accumulate,
-                   int kclass, cudaStream_t s);
-int tc_linear_bf16_full(int M, int n, const float* X1, int ldx1, const uint16_t* W1hi, const uint16_t* W1lo, int ldw1, int k1, const float* X2, int ldx2,
-                        const uint16_t* W2hi, const uint16_t* W2lo, int ldw2, int k2, const float* bias, const float* resid, int ldr, float* Y, int ldy,
-                        int relu, int accumulate, float p, uint64_t seed, uint64_t stream_id, int kclass, cudaStream_t s);
-// forward GEMMs: 0 = 3 x tf32 split (default), 1 = 3 x bf16 split (RR_FWD_BF16=1 or rr_set_forward_bf16(1))
-extern std::atomic<int> g_fwd_bf16;
-// backward GEMMs: 1 = 3 x bf16 split (default; RR_BWD_BF16=0 or rr_set_backward_bf16(0) keeps 3 x tf32)
-extern std::atomic<int> g_bwd_bf16;
-long long tc_dgrad_scratch_bytes(int n, int k);
-int tc_dgrad_standalone(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, void* scratch,
-                        long long scratch_bytes, cudaStream_t s);
-bool tc_wgrad_supported(int M, int n, int k, int lddz, int ldx);
+// ---- dense layers (nn.Linear) ---------------------------------------------------------------------
+// Pre-split images of fp32 weights for the tensor-core GEMMs: the images of the weight at base[i] are element i of each array.  The model
+// makes them for its packed weights once per step (k_pack); rr_linear_dgrad_tc makes them for one transposed weight in caller scratch.
+struct WeightImages {
+  const float* base;
+  float *tf32_hi, *tf32_lo;     // hi = w rounded to the nearest TF32 value, lo = w - hi
+  uint16_t *bf16_hi, *bf16_lo;  // hi = bf16(w), lo = bf16(w - hi)
+};
+
+// Dispatch (rr_linear.cu): which kernel and operand split runs, from the precision switches and the shape.
+// img: pre-split images of W1 / W2 (NULL: the tensor cores split the fp32 weights on chip).  pad_rows: the n_pad segment padding rows of Y,
+// recomputed in exact arithmetic after a tensor-core forward (NULL: none).
+int linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2, int k2,
+               const float* bias, const float* resid, int ldr, float* Y, int ldy, int flags, float p, uint64_t seed, uint64_t stream_id,
+               cudaStream_t s, const WeightImages* img = nullptr, const int* pad_rows = nullptr, int n_pad = 0);
+// dX[M, k] (+)= dZ[M, n] W[n, k]; the tensor cores read the images of the transposed copy Wt[k, ldwt], the SIMT kernel reads W
+int linear_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, const float* Wt, int ldwt, float* dX, int lddx,
+                 int accumulate, const WeightImages& img, cudaStream_t s);
+int linear_dgrad_tc(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, void* scratch,
+                    long long scratch_bytes, cudaStream_t s);
+int linear_wgrad(int, int, int, const float*, int, const float*, int, float*, int, float*, cudaStream_t, void* det = nullptr, long long det_bytes = 0);
+// deterministic mode: bytes of scratch linear_wgrad(M, n, k, ...) needs (row-slab partials of dW and of the bias gradient), any GEMM mode
+long long wgrad_det_bytes(int M, int n, int k);
+
+// fp32 SIMT launchers (rr_gemm_simt.cu)
+int simt_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2, int k2, const float* bias,
+             const float* resid, int ldr, float* Y, int ldy, int flags, float p, uint64_t seed, uint64_t stream_id, cudaStream_t s);
+int simt_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, cudaStream_t s);
+// Weight gradient, split over row slabs of the M reduction rows (its arguments checked by the caller).
 // slab != NULL (deterministic mode): slab z of the reduction stores its dW tile to slab + z * n * k (row stride k) and, when dbias != NULL,
-// its bias partial to slab + splits * n * k + z * n, instead of adding into dW / dbias; *splits receives the slab count
-int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s,
+// its bias partial to slab + splits * n * k + z * n, instead of adding into dW / dbias; *splits receives the slab count.  The same holds
+// for tc_wgrad.
+int simt_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s,
+               float* slab = nullptr, int* splits = nullptr);
+int simt_wgrad_splits(int M, int n, int k, int* chunk);
+
+// tcgen05 launchers (rr_gemm_tc.cu).  The B operand of the forward / dgrad GEMM (the weights W[n, K], row stride ldw elements) arrives as
+enum TcSplit {
+  TC_FP32,       // the fp32 weights (hi), split into TF32 (hi, lo) on chip
+  TC_TF32_PAIR,  // TF32 images: hi and lo are float
+  TC_BF16_PAIR,  // bf16 images: hi and lo are uint16_t, 3 x bf16 products
+};
+struct TcSrc {    // one source of the K reduction: X[M, K] (row stride ldx floats) times W^T
+  const float* X;
+  int ldx;
+  const void *hi, *lo;
+  int ldw, K;
+};
+bool tc_supported(int M, int n, int k1, int k2, int ldx1, int ldx2);
+bool tc_linear_bf16_supported(int M, int n, int k, int ldx, int ldw);
+// Y[M, n] = epi(sum over the nsrc sources of X W^T) on k_tc_gemm2
+int tc_linear(TcSplit split, int M, int n, const TcSrc* src, int nsrc, const float* bias, const float* resid, int ldr, float* Y, int ldy, int relu,
+              int accumulate, float p, uint64_t seed, uint64_t stream_id, int kclass, cudaStream_t s);
+// rr_linear_dgrad_tc: layout of the images of Wt = W[n, k]^T (row stride *ldt) in caller scratch, and the kernel that fills it
+long long tc_dgrad_scratch_bytes(int n, int k);
+WeightImages tc_dgrad_images(int n, int k, void* scratch, int* ldt);
+int tc_transpose_split(const float* W, int n, int k, int ldw, const WeightImages& img, int ldt, cudaStream_t s);
+bool tc_wgrad_supported(int M, int n, int k, int lddz, int ldx);
+// bf16: 3 x bf16 products (k_tc_wgrad3), else 3 x TF32 (k_tc_wgrad2)
+int tc_wgrad(bool bf16, int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s,
              float* slab = nullptr, int* splits = nullptr);
-int tc_wgrad_max_splits(int M, int n, int k);
+// slab count of tc_wgrad with slabs of whole stages of stage_rows rows (*chunk rows each); stage_rows = 0: the upper bound over every stage
+// height, which sizes the deterministic scratch
+int tc_wgrad_splits(int M, int n, int k, int stage_rows = 0, int* chunk = nullptr);
 
 }  // namespace rr

@@ -183,30 +183,8 @@ __global__ void __launch_bounds__(NT, 2) k_gemm(GemmArgs g) {
 }
 
 
-static int check_mat(const char* what, const void* p, int ld) {
-  RR_REQUIRE(p != nullptr, "%s is NULL", what);
-  RR_REQUIRE(aligned16(p) && (ld & 3) == 0, "%s must be 16-byte aligned with a row stride multiple of 4 (ld %d)", what, ld);
-  return RR_OK;
-}
-
-int linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2, int k2,
-               const float* bias, const float* resid, int ldr, float* Y, int ldy, int flags, float p, uint64_t seed, uint64_t stream_id,
-               cudaStream_t s, ptrdiff_t hi_off, ptrdiff_t lo_off, const float* packed, const uint16_t* bhi, const uint16_t* blo) {
-  // hi_off / lo_off != 0: TF32-exact (hi, remainder) images of W1 / W2 live at W + hi_off / W + lo_off (the model's packed weights)
-  const bool pre = hi_off != 0 && lo_off != 0;
-  const bool two = X2 && k2 > 0;
-  if (g_fwd_bf16.load() && packed && bhi && blo && (g_gemm_mode.load() == 1 || g_gemm_mode.load() == 2) && tc_linear_bf16_supported(M, n, k1, ldx1, k1) &&
-      (!two || tc_linear_bf16_supported(M, n, k2, ldx2, k2)) && aligned16(X1) && aligned16(Y) && (!two || aligned16(X2)) &&
-      (!resid || (aligned16(resid) && (ldr & 3) == 0)) && (!bias || aligned16(bias)) && (ldy & 3) == 0 && p >= 0.f && p < 1.f)
-    return tc_linear_bf16_full(M, n, X1, ldx1, bhi + (W1 - packed), blo + (W1 - packed), k1, k1, two ? X2 : nullptr, ldx2,
-                               two ? bhi + (W2 - packed) : nullptr, two ? blo + (W2 - packed) : nullptr, k2, two ? k2 : 0, bias, resid, ldr, Y, ldy,
-                               flags & 1, 0, (flags & 2) ? p : 0.f, seed, stream_id, KC_GEMM_FWD, s);
-  if ((g_gemm_mode.load() == 1 || g_gemm_mode.load() == 2) && tc_supported(M, n, k1, X2 ? k2 : 0, ldx1, X2 ? ldx2 : 0) && aligned16(X1) && aligned16(W1) && aligned16(Y) &&
-      (!X2 || (aligned16(X2) && aligned16(W2))) && (!resid || (aligned16(resid) && (ldr & 3) == 0)) && (!bias || aligned16(bias)) && (ldy & 3) == 0 &&
-      p >= 0.f && p < 1.f)
-    return tc_linear(M, n, X1, ldx1, pre ? W1 + hi_off : W1, k1, k1, X2, ldx2, (pre && W2) ? W2 + hi_off : W2, k2, X2 ? k2 : 0, bias, resid, ldr, Y, ldy,
-                     flags & 1, 0, (flags & 2) ? p : 0.f, seed, stream_id, KC_GEMM_FWD, s, pre ? W1 + lo_off : nullptr,
-                     (pre && W2) ? W2 + lo_off : nullptr);
+int simt_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2, int k2, const float* bias,
+             const float* resid, int ldr, float* Y, int ldy, int flags, float p, uint64_t seed, uint64_t stream_id, cudaStream_t s) {
   ProfScope prof_scope(KC_GEMM_FWD, s);
   RR_REQUIRE(M >= 0 && n > 0 && (n & 3) == 0 && k1 > 0 && (k1 & 3) == 0 && (k2 & 3) == 0, "linear_fwd: M %d n %d k1 %d k2 %d (n, k multiples of 4)", M, n, k1, k2);
   RR_TRY(check_mat("X1", X1, ldx1));
@@ -245,7 +223,7 @@ int linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1,
   return RR_OK;
 }
 
-int linear_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, cudaStream_t s) {
+int simt_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, cudaStream_t s) {
   ProfScope prof_scope(KC_GEMM_DGRAD, s);
   RR_REQUIRE(M >= 0 && n > 0 && k > 0 && (n & 3) == 0 && (k & 3) == 0, "linear_dgrad: M %d n %d k %d", M, n, k);
   RR_TRY(check_mat("dZ", dZ, lddz));
@@ -266,8 +244,7 @@ int linear_dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W,
   return RR_OK;
 }
 
-// slab count of the SIMT split below
-static int simt_wgrad_splits(int M, int n, int k, int* chunk_out) {
+int simt_wgrad_splits(int M, int n, int k, int* chunk_out) {
   const int tiles = ((n + BM - 1) / BM) * ((k + BN - 1) / BN);
   int splits = (num_sms() * 2 + tiles - 1) / tiles;
   const int max_splits = (M + BK * 8 - 1) / (BK * 8);
@@ -279,88 +256,9 @@ static int simt_wgrad_splits(int M, int n, int k, int* chunk_out) {
   return (M + chunk - 1) / chunk;
 }
 
-long long wgrad_det_bytes(int M, int n, int k) {
-  if (M <= 0 || n <= 0 || k <= 0) return 0;
-  const int tcs = tc_wgrad_max_splits(M, n, k), simt = simt_wgrad_splits(M, n, k, nullptr);
-  const long long splits = tcs > simt ? tcs : simt;
-  return splits * (static_cast<long long>(n) * k + n) * static_cast<long long>(sizeof(float));
-}
-
-// dW[i, j] += sum over z = 0, 1, 2, ... of slab[z][i, j];  dbias[i] += the same over the bias partials
-__global__ void k_wgrad_slab_sum(int n, int k, int splits, const float* __restrict__ slab, const float* __restrict__ slab_bias, float* __restrict__ dW,
-                                 int lddw, float* __restrict__ dbias) {
-  const int k4 = k >> 2;
-  const long long plane = static_cast<long long>(n) * k;
-  const long long total = static_cast<long long>(n) * k4;
-  for (long long t = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; t < total + n; t += static_cast<long long>(gridDim.x) * blockDim.x) {
-    if (t < total) {
-      const int i = static_cast<int>(t / k4), j = static_cast<int>(t - static_cast<long long>(i) * k4) << 2;
-      const float* p = slab + static_cast<long long>(i) * k + j;
-      float4 acc = ld_f4(p);
-#pragma unroll 8
-      for (int z = 1; z < splits; ++z) acc = f4_add(acc, ld_f4(p + z * plane));
-      float* d = dW + static_cast<size_t>(i) * lddw + j;
-      st_f4(d, f4_add(*reinterpret_cast<const float4*>(d), acc));
-    } else if (dbias) {
-      const int i = static_cast<int>(t - total);
-      float acc = slab_bias[i];
-      for (int z = 1; z < splits; ++z) acc += slab_bias[static_cast<long long>(z) * n + i];
-      dbias[i] += acc;
-    }
-  }
-}
-
-int linear_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s, void* det,
-                 long long det_bytes) {
-  const bool use_tc = g_gemm_mode.load() == 1 && M >= 256 && tc_wgrad_supported(M, n, k, lddz, ldx) && aligned16(dZ) && aligned16(X) && aligned16(dW) &&
-                      (lddw & 3) == 0;
-  if (!deterministic()) {
-    if (use_tc) return tc_wgrad(M, n, k, dZ, lddz, X, ldx, dW, lddw, dbias, s);
-  } else {
-    // Deterministic: every row slab stores its partial dW tile (and bias partial) to scratch, then k_wgrad_slab_sum adds them in slab order.
-    RR_REQUIRE(M >= 0 && n > 0 && k > 0 && (n & 3) == 0 && (k & 3) == 0, "linear_wgrad: M %d n %d k %d", M, n, k);
-    RR_TRY(check_mat("dW", dW, lddw));
-    if (M == 0) return RR_OK;
-    DetScratch ds;
-    RR_TRY(det_scratch(&ds, det, det_bytes, wgrad_det_bytes(M, n, k), s));
-    float* slab = static_cast<float*>(ds.p);
-    int splits = 0;
-    if (use_tc) {
-      RR_TRY(tc_wgrad(M, n, k, dZ, lddz, X, ldx, dW, lddw, dbias, s, slab, &splits));
-    } else {
-      ProfScope prof_scope(KC_GEMM_WGRAD, s);
-      RR_TRY(check_mat("dZ", dZ, lddz));
-      RR_TRY(check_mat("X", X, ldx));
-      GemmArgs g{};
-      g.src[0] = {dZ, X, lddz, ldx, M};
-      g.nsrc = 1;
-      g.M = n;
-      g.N = k;
-      g.C = slab;
-      g.ldc = k;
-      g.slab_stride = static_cast<long long>(n) * k;
-      int chunk = 0;
-      splits = simt_wgrad_splits(M, n, k, &chunk);
-      g.k_chunk = chunk;
-      g.dbias = dbias ? slab + splits * g.slab_stride : nullptr;
-      dim3 grid((n + BM - 1) / BM, (k + BN - 1) / BN, splits);
-      k_gemm<false, false, EPI_SLAB><<<grid, NT, 0, s>>>(g);
-      RR_LAUNCH_CHECK("k_gemm<wgrad slab>");
-    }
-    ProfScope prof_scope(KC_GEMM_WGRAD, s);
-    const long long work = static_cast<long long>(n) * (k >> 2) + n;
-    long long blocks = (work + 255) / 256;
-    if (blocks > num_sms() * 8) blocks = num_sms() * 8;
-    k_wgrad_slab_sum<<<static_cast<int>(blocks), 256, 0, s>>>(n, k, splits, slab, slab + splits * static_cast<long long>(n) * k, dW, lddw, dbias);
-    RR_LAUNCH_CHECK("k_wgrad_slab_sum");
-    return RR_OK;
-  }
+int simt_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s, float* slab,
+               int* n_splits) {
   ProfScope prof_scope(KC_GEMM_WGRAD, s);
-  RR_REQUIRE(M >= 0 && n > 0 && k > 0 && (n & 3) == 0 && (k & 3) == 0, "linear_wgrad: M %d n %d k %d", M, n, k);
-  RR_TRY(check_mat("dZ", dZ, lddz));
-  RR_TRY(check_mat("X", X, ldx));
-  RR_TRY(check_mat("dW", dW, lddw));
-  if (M == 0) return RR_OK;
   GemmArgs g{};
   g.src[0] = {dZ, X, lddz, ldx, M};  // reduction runs over the M rows
   g.nsrc = 1;
@@ -373,7 +271,16 @@ int linear_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X,
   const int splits = simt_wgrad_splits(M, n, k, &chunk);
   g.k_chunk = chunk;
   dim3 grid((n + BM - 1) / BM, (k + BN - 1) / BN, splits);
-  k_gemm<false, false, EPI_ATOMIC><<<grid, NT, 0, s>>>(g);
+  if (slab) {
+    g.C = slab;
+    g.ldc = k;
+    g.slab_stride = static_cast<long long>(n) * k;
+    g.dbias = dbias ? slab + splits * g.slab_stride : nullptr;
+    *n_splits = splits;
+    k_gemm<false, false, EPI_SLAB><<<grid, NT, 0, s>>>(g);
+  } else {
+    k_gemm<false, false, EPI_ATOMIC><<<grid, NT, 0, s>>>(g);
+  }
   RR_LAUNCH_CHECK("k_gemm<wgrad>");
   return RR_OK;
 }

@@ -537,8 +537,6 @@ __global__ void __launch_bounds__(THREADS2_BASE + 32 * EW, 1) k_tc_gemm2(const _
 // added to dW with vector reductions (split over m like the SIMT kernel).
 // ================================================================================================
 constexpr int WG_BK = 32;                 // rows of the reduction per stage
-constexpr int WG_BOX = WG_BK * 128;       // bytes of one TMA box (32 rows x 128 B)
-constexpr int WG_A_BYTES = 4 * WG_BOX;    // 128 n-columns
 
 struct WgArgs {
   CUtensorMap tmA;   // dZ [M, n]
@@ -764,7 +762,6 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_wgrad2(const __grid_constant_
 // 212 KB of shared-memory traffic at 128 B/clk) + hand-offs ~500, and two slots make that 2212 clk per stage; 16-row stages double the
 // per-row box cost, and a third 57 KB raw slot does not fit beside two 40 KB bf16 slots.  Narrow X tiles do fit more raw slots (up to 6),
 // worth 6-9 % there.
-constexpr int W3_A_COLS = 128;               // dZ columns per CTA == TMEM lanes
 
 template <int BKR>
 __device__ __forceinline__ uint64_t umma_desc_mn_bf16(uint32_t smem_addr) {
@@ -1032,31 +1029,36 @@ static int make_map_bf16(CUtensorMap* map, const uint16_t* ptr, int rows, int co
 
 }  // namespace tc
 
-// dX[M, n] (+)= dZ[M, k] W^T with the weight given as bf16 (hi, lo) images of Wt[n, k] (row stride ldw elements): the backward flavour of
-// k_tc_gemm2 (3 x bf16 products, five pipeline stages).  Needs n % 16 == 0, k % 8 == 0 (16-byte bf16 rows).
+// Can this problem run on k_tc_gemm2?  (everything the model produces can; odd C-ABI calls fall back to SIMT)
+bool tc_supported(int M, int n, int k1, int k2, int ldx1, int ldx2) {
+  return M > 0 && n >= 16 && !(n & 15) && k1 > 0 && !(k1 & 3) && !(k2 & 3) && !(ldx1 & 3) && !(ldx2 & 3);
+}
+// The same for one source with bf16 images of W (row stride ldw elements): 16-byte bf16 rows need ldw % 8 == 0.
 bool tc_linear_bf16_supported(int M, int n, int k, int ldx, int ldw) {
   return M > 0 && n >= 16 && !(n & 15) && k > 0 && !(k & 3) && !(ldx & 3) && !(ldw & 7);
 }
-// Full-featured bf16-split linear: Y = epi(X1 W1^T + X2 W2^T) with every weight given as bf16 (hi, lo) images.
-int tc_linear_bf16_full(int M, int n, const float* X1, int ldx1, const uint16_t* W1hi, const uint16_t* W1lo, int ldw1, int k1, const float* X2, int ldx2,
-                        const uint16_t* W2hi, const uint16_t* W2lo, int ldw2, int k2, const float* bias, const float* resid, int ldr, float* Y, int ldy,
-                        int relu, int accumulate, float p, uint64_t seed, uint64_t stream_id, int kclass, cudaStream_t s) {
+
+// TC_BF16_PAIR runs the backward flavour k_tc_gemm2<16, true> (3 x bf16 products, five pipeline stages), the others k_tc_gemm2<16, false>.
+int tc_linear(TcSplit split, int M, int n, const TcSrc* src, int nsrc, const float* bias, const float* resid, int ldr, float* Y, int ldy, int relu,
+              int accumulate, float p, uint64_t seed, uint64_t stream_id, int kclass, cudaStream_t s) {
   using namespace tc;
   ProfScope prof_scope(kclass, s);
+  const bool bf = split == TC_BF16_PAIR;
   Args g{};
-  const bool two = X2 && k2 > 0;
-  g.nsrc = two ? 2 : 1;
-  RR_TRY(make_map(&g.src[0].tmA, X1, M, k1, ldx1, BM));
-  RR_TRY(make_map_bf16(&g.src[0].tmB, W1hi, n, k1, ldw1, NT2));
-  RR_TRY(make_map_bf16(&g.src[0].tmBlo, W1lo, n, k1, ldw1, NT2));
-  g.src[0].K = k1;
-  if (two) {
-    RR_TRY(make_map(&g.src[1].tmA, X2, M, k2, ldx2, BM));
-    RR_TRY(make_map_bf16(&g.src[1].tmB, W2hi, n, k2, ldw2, NT2));
-    RR_TRY(make_map_bf16(&g.src[1].tmBlo, W2lo, n, k2, ldw2, NT2));
-    g.src[1].K = k2;
+  g.nsrc = nsrc;
+  g.presplit = split != TC_FP32;
+  for (int i = 0; i < nsrc; ++i) {
+    const TcSrc& q = src[i];
+    RR_TRY(make_map(&g.src[i].tmA, q.X, M, q.K, q.ldx, BM));
+    if (bf) {
+      RR_TRY(make_map_bf16(&g.src[i].tmB, static_cast<const uint16_t*>(q.hi), n, q.K, q.ldw, NT2));
+      RR_TRY(make_map_bf16(&g.src[i].tmBlo, static_cast<const uint16_t*>(q.lo), n, q.K, q.ldw, NT2));
+    } else {
+      RR_TRY(make_map(&g.src[i].tmB, static_cast<const float*>(q.hi), n, q.K, q.ldw, NT2));
+      if (g.presplit) RR_TRY(make_map(&g.src[i].tmBlo, static_cast<const float*>(q.lo), n, q.K, q.ldw, NT2));
+    }
+    g.src[i].K = q.K;
   }
-  g.presplit = 1;
   g.M = M;
   g.N = n;
   g.C = Y;
@@ -1072,24 +1074,20 @@ int tc_linear_bf16_full(int M, int n, const float* X1, int ldx1, const uint16_t*
   g.stream_id = stream_id;
   static PerDeviceOnce attr_set;
   if (attr_set.need()) {
+    RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     attr_set.mark();
   }
-  const size_t smem = static_cast<size_t>(S2_BF) * STAGE2_BF + 1024 + 256 + 16 * 2048;
+  // ring | barriers | epilogue staging (16 warps x 2 KB)
+  const size_t smem = static_cast<size_t>(bf ? S2_BF * STAGE2_BF : S2 * STAGE2) + 1024 + 256 + 16 * 2048;
   const int total_tiles = ((M + BM - 1) / BM) * ((n + NT2 - 1) / NT2);
   const int ctas = total_tiles < num_sms() ? total_tiles : num_sms();
-  RR_CUDA(launch_pdl(k_tc_gemm2<16, true>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
-  RR_LAUNCH_CHECK("k_tc_gemm2<bf16>");
+  RR_CUDA(launch_pdl(bf ? k_tc_gemm2<16, true> : k_tc_gemm2<16, false>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
+  RR_LAUNCH_CHECK(bf ? "k_tc_gemm2<bf16>" : "k_tc_gemm2");
   return RR_OK;
 }
-int tc_linear_bf16(int M, int n, const float* X, int ldx, const uint16_t* Whi, const uint16_t* Wlo, int ldw, int k, float* Y, int ldy, int accumulate,
-                   int kclass, cudaStream_t s) {
-  return tc_linear_bf16_full(M, n, X, ldx, Whi, Wlo, ldw, k, nullptr, 0, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, Y, ldy, 0, accumulate, 0.f, 0, 0,
-                             kclass, s);
-}
 
-
-// ---- stand-alone tensor-core dgrad (C ABI: rr_linear_dgrad_tc) ---------------------------------------------------------------------
+// ---- images for the stand-alone tensor-core dgrad (C ABI: rr_linear_dgrad_tc) ---------------------------------------------------------
 // The model keeps the transposed, pre-split operand images of every weight in its packed workspace (k_pack).  A direct caller of the C ABI
 // hands over W[n, k] only, so the images are made here, into caller-provided scratch: Wt[k, ldt] as TF32 (hi, lo) floats and bf16 (hi, lo).
 __global__ void k_transpose_split(const float* __restrict__ W, int n, int k, int ldw, float* __restrict__ thi, float* __restrict__ tlo,
@@ -1109,77 +1107,82 @@ __global__ void k_transpose_split(const float* __restrict__ W, int n, int k, int
     blo[o] = b2;
   }
 }
-static inline int dgrad_ldt(int n) { return (n + 7) / 8 * 8; }
-long long tc_dgrad_scratch_bytes(int n, int k) {
-  const size_t e = static_cast<size_t>(k) * dgrad_ldt(n);
-  return static_cast<long long>((e * 4 + 255) / 256 * 256 * 2 + (e * 2 + 255) / 256 * 256 * 2);
+// bytes of one TF32 image and of one bf16 image of Wt[k, ldt], each rounded up to 256
+static void dgrad_image_bytes(int n, int k, int* ldt, size_t* fb, size_t* hb) {
+  *ldt = (n + 7) / 8 * 8;
+  const size_t e = static_cast<size_t>(k) * *ldt;
+  *fb = (e * 4 + 255) / 256 * 256;
+  *hb = (e * 2 + 255) / 256 * 256;
 }
-int tc_dgrad_standalone(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, float* dX, int lddx, int accumulate, void* scratch,
-                        long long scratch_bytes, cudaStream_t s) {
-  RR_REQUIRE(M > 0 && n > 0 && k > 0 && dZ && W && dX && scratch, "linear_dgrad_tc: bad argument");
-  RR_REQUIRE(aligned16(dZ) && aligned16(dX) && aligned16(scratch) && !(lddz & 3) && !(lddx & 3), "linear_dgrad_tc: operands must be 16-byte aligned rows");
-  RR_REQUIRE(scratch_bytes >= tc_dgrad_scratch_bytes(n, k), "linear_dgrad_tc: scratch %lld bytes < required %lld", scratch_bytes, tc_dgrad_scratch_bytes(n, k));
-  const int ldt = dgrad_ldt(n);
-  const size_t e = static_cast<size_t>(k) * ldt;
-  const size_t fb = (e * 4 + 255) / 256 * 256, hb = (e * 2 + 255) / 256 * 256;
+long long tc_dgrad_scratch_bytes(int n, int k) {
+  int ldt;
+  size_t fb, hb;
+  dgrad_image_bytes(n, k, &ldt, &fb, &hb);
+  return static_cast<long long>(2 * fb + 2 * hb);
+}
+WeightImages tc_dgrad_images(int n, int k, void* scratch, int* ldt) {
+  size_t fb, hb;
+  dgrad_image_bytes(n, k, ldt, &fb, &hb);
   char* base = static_cast<char*>(scratch);
-  float* thi = reinterpret_cast<float*>(base);
-  float* tlo = reinterpret_cast<float*>(base + fb);
-  uint16_t* bhi = reinterpret_cast<uint16_t*>(base + 2 * fb);
-  uint16_t* blo = reinterpret_cast<uint16_t*>(base + 2 * fb + hb);
-  const bool bf = g_bwd_bf16.load() != 0;
-  if (bf ? !tc_linear_bf16_supported(M, k, n, lddz, ldt) : !tc_supported(M, k, n, 0, lddz, 0))
-    return fail(RR_ERR_UNSUPPORTED, "linear_dgrad_tc: shape M %d n %d k %d does not suit the tensor-core kernel (k %% 16, n %% 4)", M, n, k);
-  RR_CUDA(cudaMemsetAsync(scratch, 0, 2 * fb + 2 * hb, s));
-  {
-    const long long total = static_cast<long long>(n) * k;
-    int blocks = static_cast<int>((total + 255) / 256);
-    if (blocks > num_sms() * 8) blocks = num_sms() * 8;
-    k_transpose_split<<<blocks, 256, 0, s>>>(W, n, k, ldw, thi, tlo, bhi, blo, ldt);
-    RR_LAUNCH_CHECK("k_transpose_split");
-  }
-  if (bf) return tc_linear_bf16(M, k, dZ, lddz, bhi, blo, ldt, n, dX, lddx, accumulate, KC_GEMM_DGRAD, s);
-  return tc_linear(M, k, dZ, lddz, thi, ldt, n, nullptr, 0, nullptr, 0, 0, nullptr, nullptr, 0, dX, lddx, 0, accumulate, 0.f, 0, 0, KC_GEMM_DGRAD, s, tlo,
-                   nullptr);
+  WeightImages img;
+  img.tf32_hi = reinterpret_cast<float*>(base);
+  img.tf32_lo = reinterpret_cast<float*>(base + fb);
+  img.bf16_hi = reinterpret_cast<uint16_t*>(base + 2 * fb);
+  img.bf16_lo = reinterpret_cast<uint16_t*>(base + 2 * fb + hb);
+  img.base = img.tf32_hi;   // no fp32 copy of Wt is kept: the images are indexed like the hi image
+  return img;
+}
+int tc_transpose_split(const float* W, int n, int k, int ldw, const WeightImages& img, int ldt, cudaStream_t s) {
+  RR_CUDA(cudaMemsetAsync(img.tf32_hi, 0, tc_dgrad_scratch_bytes(n, k), s));   // the padding columns of every image are zero
+  const long long total = static_cast<long long>(n) * k;
+  int blocks = static_cast<int>((total + 255) / 256);
+  if (blocks > num_sms() * 8) blocks = num_sms() * 8;
+  k_transpose_split<<<blocks, 256, 0, s>>>(W, n, k, ldw, img.tf32_hi, img.tf32_lo, img.bf16_hi, img.bf16_lo, ldt);
+  RR_LAUNCH_CHECK("k_transpose_split");
+  return RR_OK;
 }
 
+// ---- weight gradient ----------------------------------------------------------------------------------------------------------------
 bool tc_wgrad_supported(int M, int n, int k, int lddz, int ldx) {
   return M > 0 && n >= 4 && k >= 4 && !(n & 3) && !(k & 3) && !(lddz & 3) && !(ldx & 3);
 }
 
-// Upper bound of the slab count of either split below (rounding the slab height up to whole stages only lowers it).
-int tc_wgrad_max_splits(int M, int n, int k) {
+// One CTA per SM (shared memory and TMEM are both taken whole): never more CTAs than SMs, or the stragglers run as a second wave.  Rounding
+// the slab height up to whole stages only lowers the count, so the count before rounding bounds that of every stage height.
+int tc_wgrad_splits(int M, int n, int k, int stage_rows, int* chunk) {
   using namespace tc;
   const int k_pad = (k + 15) / 16 * 16;
   const int tiles = ((n + BM - 1) / BM) * ((k_pad + MAX_NT - 1) / MAX_NT);
   int splits = num_sms() / tiles;
-  const int max_splits = (M + 8 * 32 - 1) / (8 * 32);
+  const int max_splits = (M + 8 * WG_BK - 1) / (8 * WG_BK);
   if (splits > max_splits) splits = max_splits;
-  return splits < 1 ? 1 : splits;
+  if (splits < 1) splits = 1;
+  if (stage_rows <= 0) return splits;
+  *chunk = ((M + splits - 1) / splits + stage_rows - 1) / stage_rows * stage_rows;   // a stage never reaches into the next slab's rows
+  return (M + *chunk - 1) / *chunk;
 }
 
-int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s, float* slab,
-             int* n_splits) {
+int tc_wgrad(bool bf16, int M, int n, int k, const float* dZ, int lddz, const float* X, int ldx, float* dW, int lddw, float* dbias, cudaStream_t s,
+             float* slab, int* n_splits) {
   using namespace tc;
   ProfScope prof_scope(KC_GEMM_WGRAD, s);
-  const bool det = slab != nullptr;
-  if (det) {
-    dW = slab;
-    lddw = k;
-  }
   WgArgs g{};
-  g.slab_stride = static_cast<long long>(n) * k;
   const int k_pad = (k + 15) / 16 * 16;                  // columns past k are zero-filled by TMA and never written back
   const int ktiles = (k_pad + MAX_NT - 1) / MAX_NT;
   g.kt = ktiles == 1 ? k_pad : MAX_NT;
   g.nb = (g.kt + 31) / 32;
   g.tm_a = g.kt <= 160 ? 160 : 320;
-  if (g_bwd_bf16.load()) {
+  // the ring: rows of the reduction per stage (bkr), slots and shared memory, and the instantiation
+  int bkr, stage_rows, threads;
+  size_t smem;
+  CUtensorMapSwizzle x_swizzle;
+  void (*kernel)(WgArgs);
+  if (bf16) {
     // 3 x bf16: raw ring (dZ + X boxes as TMA lands them, up to 6 slots) and bf16 ring (hi + lo images + the TMEM A slots, 2 slots),
     // sized separately.  Narrow X tiles (<= 96 columns: the feature-matrix gradients W_i, W_o[:, :64], MPNDiff W_h[:, h:]) take 64 rows per
     // stage: a stage's hand-offs and fixed conversion cost (~1400 clk, DESIGN.md §4.2) are then paid half as often, and two
     // 56 KB raw slots still fit.
-    const int bkr = g.kt <= 96 ? 64 : 32;
+    bkr = g.kt <= 96 ? 64 : 32;
     const int box = bkr * 128;
     const int nblk = (g.kt + 63) / 64;
     const int raw_bytes = 4 * box + g.nb * box, bf_bytes = 2 * nblk * box;
@@ -1191,58 +1194,32 @@ int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int
     RR_REQUIRE(R >= 2, "tc_wgrad: %d columns do not fit two raw pipeline slots", g.kt);
     g.stages = R;
     g.bf_stages = SB;
-    RR_TRY(make_map(&g.tmA, dZ, M, n, lddz, bkr, CU_TENSOR_MAP_SWIZZLE_NONE));
-    RR_TRY(make_map(&g.tmB, X, M, k, ldx, bkr, CU_TENSOR_MAP_SWIZZLE_128B));
-    g.M = M;
-    g.n = n;
-    g.k = k;
-    g.k_pad = k_pad;
-    g.dW = dW;
-    g.lddw = lddw;
-    g.dbias = dbias;
-    const int ntiles3 = (n + BM - 1) / BM;
-    int splits3 = num_sms() / (ntiles3 * ktiles);
-    const int max_splits3 = (M + 8 * 32 - 1) / (8 * 32);
-    if (splits3 > max_splits3) splits3 = max_splits3;
-    if (splits3 < 1) splits3 = 1;
-    int chunk3 = (M + splits3 - 1) / splits3;
-    chunk3 = (chunk3 + bkr - 1) / bkr * bkr;          // whole stages: a stage never reaches into the next split's rows
-    splits3 = (M + chunk3 - 1) / chunk3;
-    g.m_chunk = chunk3;
-    if (det && dbias) g.dbias = slab + splits3 * g.slab_stride;   // bias partials follow the slab tiles
-    static PerDeviceOnce attr3_set;
-    if (attr3_set.need()) {
-      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<64, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-      RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad3<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-      attr3_set.mark();
-    }
-    const size_t smem3 = static_cast<size_t>(R) * raw_bytes + static_cast<size_t>(SB) * bf_bytes + 1024 + 512;
-    const dim3 grid3(ntiles3, ktiles, splits3);
-    if (det) {
-      if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad3<32, true>, grid3, dim3(W3_THREADS), smem3, s, g));
-      else RR_CUDA(launch_pdl(k_tc_wgrad3<64, true>, grid3, dim3(W3_THREADS), smem3, s, g));
-      *n_splits = splits3;
-    } else {
-      if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad3<32, false>, grid3, dim3(W3_THREADS), smem3, s, g));
-      else RR_CUDA(launch_pdl(k_tc_wgrad3<64, false>, grid3, dim3(W3_THREADS), smem3, s, g));
-    }
-    RR_LAUNCH_CHECK("k_tc_wgrad3");
-    return RR_OK;
+    smem = static_cast<size_t>(R) * raw_bytes + static_cast<size_t>(SB) * bf_bytes + 1024 + 512;
+    stage_rows = bkr;
+    threads = W3_THREADS;
+    x_swizzle = CU_TENSOR_MAP_SWIZZLE_128B;
+    if (bkr == 32) kernel = slab ? k_tc_wgrad3<32, true> : k_tc_wgrad3<32, false>;
+    else kernel = slab ? k_tc_wgrad3<64, true> : k_tc_wgrad3<64, false>;
+  } else {
+    // 3 x TF32 (rr_set_backward_bf16(0)): wide tiles take 16-row stages (4 x 48 KB in flight instead of 2 x 96 KB); narrow tiles fit 3+
+    // stages of 32 rows
+    bkr = g.kt > 160 ? 16 : 32;
+    const int box = bkr * 128;
+    const int stage_bytes = 4 * box + 2 * g.nb * box;
+    int S = (SMEM_LIMIT - 2048) / stage_bytes;
+    if (S > (512 - g.tm_a) / (2 * bkr)) S = (512 - g.tm_a) / (2 * bkr);   // TMEM: accumulator + 2 * bkr columns of A per stage
+    if (S > 6) S = 6;
+    RR_REQUIRE(S >= 2, "tc_wgrad: %d columns do not fit two pipeline stages", g.kt);
+    g.stages = S;
+    smem = static_cast<size_t>(S) * stage_bytes + 1024 + 256;
+    stage_rows = WG_BK;
+    threads = THREADS;
+    x_swizzle = CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B;
+    if (bkr == 32) kernel = slab ? k_tc_wgrad2<32, true> : k_tc_wgrad2<32, false>;
+    else kernel = slab ? k_tc_wgrad2<16, true> : k_tc_wgrad2<16, false>;
   }
-  // 3 x TF32 (rr_set_backward_bf16(0)): wide tiles take 16-row stages (4 x 48 KB in flight instead of 2 x 96 KB); narrow tiles fit 3+ stages
-  // of 32 rows
-  const int bkr = g.kt > 160 ? 16 : 32;
-  const int box = bkr * 128;
-  const int stage_bytes = 4 * box + 2 * g.nb * box;
-  int S = (SMEM_LIMIT - 2048) / stage_bytes;
-  if (S > (512 - g.tm_a) / (2 * bkr)) S = (512 - g.tm_a) / (2 * bkr);   // TMEM: accumulator + 2 * bkr columns of A per stage
-  if (S > 6) S = 6;
-  RR_REQUIRE(S >= 2, "tc_wgrad: %d columns do not fit two pipeline stages", g.kt);
-  g.stages = S;
   RR_TRY(make_map(&g.tmA, dZ, M, n, lddz, bkr, CU_TENSOR_MAP_SWIZZLE_NONE));
-  RR_TRY(make_map(&g.tmB, X, M, k, ldx, bkr, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B));
+  RR_TRY(make_map(&g.tmB, X, M, k, ldx, bkr, x_swizzle));
   g.M = M;
   g.n = n;
   g.k = k;
@@ -1250,88 +1227,25 @@ int tc_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X, int
   g.dW = dW;
   g.lddw = lddw;
   g.dbias = dbias;
-  // one CTA per SM (shared memory and TMEM are both taken whole): never more CTAs than SMs, or the stragglers run as a second wave
-  const int ntiles = (n + BM - 1) / BM;
-  int splits = num_sms() / (ntiles * ktiles);
-  const int max_splits = (M + 8 * WG_BK - 1) / (8 * WG_BK);
-  if (splits > max_splits) splits = max_splits;
-  if (splits < 1) splits = 1;
-  int chunk = (M + splits - 1) / splits;
-  chunk = (chunk + WG_BK - 1) / WG_BK * WG_BK;
-  splits = (M + chunk - 1) / chunk;
+  g.slab_stride = static_cast<long long>(n) * k;
+  int chunk = 0;
+  const int splits = tc_wgrad_splits(M, n, k, stage_rows, &chunk);
   g.m_chunk = chunk;
-  if (det && dbias) g.dbias = slab + splits * g.slab_stride;
-  dim3 grid(ntiles, ktiles, splits);
-  const size_t smem = static_cast<size_t>(S) * stage_bytes + 1024 + 256;
-  static PerDeviceOnce attr_set;
-  if (attr_set.need()) {
-    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    RR_CUDA(cudaFuncSetAttribute(k_tc_wgrad2<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
-    attr_set.mark();
-  }
-  if (det) {
-    if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad2<32, true>, grid, dim3(THREADS), smem, s, g));
-    else RR_CUDA(launch_pdl(k_tc_wgrad2<16, true>, grid, dim3(THREADS), smem, s, g));
+  if (slab) {
+    g.dW = slab;
+    g.lddw = k;
+    if (dbias) g.dbias = slab + splits * g.slab_stride;   // bias partials follow the slab tiles
     *n_splits = splits;
-  } else {
-    if (bkr == 32) RR_CUDA(launch_pdl(k_tc_wgrad2<32, false>, grid, dim3(THREADS), smem, s, g));
-    else RR_CUDA(launch_pdl(k_tc_wgrad2<16, false>, grid, dim3(THREADS), smem, s, g));
   }
-  RR_LAUNCH_CHECK("k_tc_wgrad2");
-  return RR_OK;
-}
-
-// Can this problem run on the tcgen05 kernel?  (everything the model produces can; odd C-ABI calls fall back to SIMT)
-bool tc_supported(int M, int n, int k1, int k2, int ldx1, int ldx2) {
-  return M > 0 && n >= 16 && !(n & 15) && k1 > 0 && !(k1 & 3) && !(k2 & 3) && !(ldx1 & 3) && !(ldx2 & 3);
-}
-
-// Y = epi(X1 W1^T + X2 W2^T): W* row-major [n, k*] (K-major B operand)
-// W1lo / W2lo != NULL: W1 / W2 are the TF32-exact hi images of the weights and W*lo the remainders (same shape and stride)
-int tc_linear(int M, int n, const float* X1, int ldx1, const float* W1, int ldw1, int k1, const float* X2, int ldx2, const float* W2, int ldw2, int k2,
-              const float* bias, const float* resid, int ldr, float* Y, int ldy, int relu, int accumulate, float p, uint64_t seed, uint64_t stream_id,
-              int kclass, cudaStream_t s, const float* W1lo, const float* W2lo) {
-  using namespace tc;
-  ProfScope prof_scope(kclass, s);
-  Args g{};
-  const bool two = X2 && k2 > 0;
-  g.nsrc = two ? 2 : 1;
-  g.presplit = (W1lo != nullptr && (!two || W2lo != nullptr)) ? 1 : 0;
-  RR_TRY(make_map(&g.src[0].tmA, X1, M, k1, ldx1, BM));
-  RR_TRY(make_map(&g.src[0].tmB, W1, n, k1, ldw1, NT2));
-  if (g.presplit) RR_TRY(make_map(&g.src[0].tmBlo, W1lo, n, k1, ldw1, NT2));
-  g.src[0].K = k1;
-  if (two) {
-    RR_TRY(make_map(&g.src[1].tmA, X2, M, k2, ldx2, BM));
-    RR_TRY(make_map(&g.src[1].tmB, W2, n, k2, ldw2, NT2));
-    if (g.presplit) RR_TRY(make_map(&g.src[1].tmBlo, W2lo, n, k2, ldw2, NT2));
-    g.src[1].K = k2;
-  }
-  g.M = M;
-  g.N = n;
-  g.C = Y;
-  g.ldc = ldy;
-  g.bias = bias;
-  g.resid = resid;
-  g.ldr = ldr;
-  g.relu = relu;
-  g.accumulate = accumulate;
-  g.p = p;
-  g.inv_keep = p > 0.f ? 1.f / (1.f - p) : 1.f;
-  g.seed = seed;
-  g.stream_id = stream_id;
   static PerDeviceOnce attr_set;
   if (attr_set.need()) {
-    RR_CUDA(cudaFuncSetAttribute(k_tc_gemm2<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
+    void (*const all[])(WgArgs) = {k_tc_wgrad2<16, false>, k_tc_wgrad2<32, false>, k_tc_wgrad2<16, true>, k_tc_wgrad2<32, true>,
+                                   k_tc_wgrad3<32, false>, k_tc_wgrad3<64, false>, k_tc_wgrad3<32, true>, k_tc_wgrad3<64, true>};
+    for (auto* f : all) RR_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
     attr_set.mark();
   }
-  const size_t smem = static_cast<size_t>(S2) * STAGE2 + 1024 + 256 + 16 * 2048;  // ring | barriers | epilogue staging (16 warps x 2 KB)
-  const int total_tiles = ((M + BM - 1) / BM) * ((n + NT2 - 1) / NT2);
-  const int ctas = total_tiles < num_sms() ? total_tiles : num_sms();
-  RR_CUDA(launch_pdl(k_tc_gemm2<16, false>, dim3(ctas), dim3(THREADS2_BASE + 512), smem, s, g));
-  RR_LAUNCH_CHECK("k_tc_gemm2");
+  RR_CUDA(launch_pdl(kernel, dim3((n + BM - 1) / BM, ktiles, splits), dim3(threads), smem, s, g));
+  RR_LAUNCH_CHECK(bf16 ? "k_tc_wgrad3" : "k_tc_wgrad2");
   return RR_OK;
 }
 

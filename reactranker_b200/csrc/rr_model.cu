@@ -197,87 +197,6 @@ __global__ void k_head_bwd(int N, int task, int head, const float* __restrict__ 
   }
 }
 
-// ---- padding rows in exact arithmetic -------------------------------------------------------
-// A segment's padding bond / padding atom row is gathered by EVERY padded neighbour slot of the segment (featurization.py:281-286), so in
-// the backward pass it collects the gradient of all of them: at the c5 batch one such row weighs as much as ~10^5 ordinary rows.  Its ReLU
-// masks must therefore be decided as the reference's fp32 run decides them.  The tensor-core forward (3 x TF32, RZ accumulation) leaves
-// 2-5e-6 of relative error on a pre-activation, which flips the mask of an entry that lies that close to zero; on an ordinary row such a
-// flip moves the gradient by one row's share, on a padding row by a macroscopic amount.  After every tensor-core forward GEMM whose output
-// feeds a ReLU, the n_segments padding rows are therefore recomputed here from the unsplit fp32 weights with fp64 accumulation (one
-// rounding, tighter than any fp32 GEMM) and overwritten, epilogue (bias, residual, ReLU, the same Philox dropout mask) included.
-struct PadFix {
-  const int* rows;
-  int n_rows, n;
-  const float *X1, *W1, *X2, *W2, *bias, *resid;
-  int ldx1, k1, ldx2, k2, ldr;
-  float* Y;
-  int ldy, relu;
-  float p, inv_keep;
-  uint64_t seed, stream_id;
-};
-// One warp per output column (grid = rows x ceil(n / 8), 8 warps per block): the k loop is unrolled into independent loads and four
-// fp64 partial sums, so a launch is a couple of microseconds (the first version, one warp per ~5 columns with a serial chain, took 20).
-__device__ __forceinline__ double pad_dot(const float* __restrict__ x, const float* __restrict__ w, int k, int lane) {
-  double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0;
-  int i = lane;
-  for (; i + 96 < k; i += 128) {
-    const float x0 = x[i], x1 = x[i + 32], x2 = x[i + 64], x3 = x[i + 96];
-    const float w0 = __ldg(w + i), w1 = __ldg(w + i + 32), w2 = __ldg(w + i + 64), w3 = __ldg(w + i + 96);
-    a0 = fma(static_cast<double>(x0), static_cast<double>(w0), a0);
-    a1 = fma(static_cast<double>(x1), static_cast<double>(w1), a1);
-    a2 = fma(static_cast<double>(x2), static_cast<double>(w2), a2);
-    a3 = fma(static_cast<double>(x3), static_cast<double>(w3), a3);
-  }
-  for (; i < k; i += 32) a0 = fma(static_cast<double>(x[i]), static_cast<double>(__ldg(w + i)), a0);
-  return (a0 + a1) + (a2 + a3);
-}
-__global__ void __launch_bounds__(256) k_pad_rows_linear(PadFix a) {
-  const size_t row = static_cast<size_t>(__ldg(a.rows + blockIdx.x));
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int c = blockIdx.y * 8 + warp;
-  if (c >= a.n) return;
-  double acc = pad_dot(a.X1 + row * a.ldx1, a.W1 + static_cast<size_t>(c) * a.k1, a.k1, lane);
-  if (a.X2) acc += pad_dot(a.X2 + row * a.ldx2, a.W2 + static_cast<size_t>(c) * a.k2, a.k2, lane);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-  if (lane == 0) {
-    if (a.bias) acc += static_cast<double>(a.bias[c]);
-    if (a.resid) acc += static_cast<double>(a.resid[row * a.ldr + c]);
-    float o = static_cast<float>(acc);
-    if (a.relu) o = fmaxf(o, 0.f);
-    if (a.p > 0.f) {   // element (c & 3) of the 4-wide Philox draw the GEMM epilogue makes for this chunk (dropout4)
-      const uint4 r = philox4x32(a.seed, a.stream_id, (row * a.ldy + c) >> 2);
-      const uint32_t thr = static_cast<uint32_t>(fminf(a.p, 1.f) * 4294967295.f);
-      const uint32_t rv = (c & 3) == 0 ? r.x : ((c & 3) == 1 ? r.y : ((c & 3) == 2 ? r.z : r.w));
-      o = rv >= thr ? o * a.inv_keep : 0.f;
-    }
-    a.Y[row * a.ldy + c] = o;
-  }
-}
-// same argument order as linear_fwd; W1 / W2 are the raw (unsplit) packed weights
-static int pad_rows_linear(const int* rows, int n_rows, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2,
-                           int k2, const float* bias, const float* resid, int ldr, float* Y, int ldy, int flags, float p, uint64_t seed,
-                           uint64_t stream_id, cudaStream_t s) {
-  if (n_rows <= 0 || rows == nullptr) return RR_OK;
-  ProfScope prof_scope(KC_MISC, s);
-  PadFix a{};
-  a.rows = rows;
-  a.n_rows = n_rows;
-  a.n = n;
-  a.X1 = X1; a.ldx1 = ldx1; a.W1 = W1; a.k1 = k1;
-  a.X2 = (X2 && k2 > 0) ? X2 : nullptr; a.ldx2 = ldx2; a.W2 = W2; a.k2 = k2;
-  a.bias = bias; a.resid = resid; a.ldr = ldr;
-  a.Y = Y; a.ldy = ldy;
-  a.relu = flags & 1;
-  a.p = (flags & 2) ? p : 0.f;
-  a.inv_keep = a.p > 0.f ? 1.f / (1.f - a.p) : 1.f;
-  a.seed = seed;
-  a.stream_id = stream_id;
-  k_pad_rows_linear<<<dim3(n_rows, (n + 7) / 8), 256, 0, s>>>(a);
-  RR_LAUNCH_CHECK("k_pad_rows_linear");
-  return RR_OK;
-}
-
 // ---- joint graph ------------------------------------------------------------------------------
 // Index tables of the concatenation [reactant batch | product batch] in joint row space: the reactant part is copied, the product part
 // is shifted by the reactant batch's row counts (valid slots only: an unused slot stays 0 and is never read, its multiplicity lives in
@@ -323,9 +242,8 @@ struct EncBufs {
 };
 struct Workspace {
   PackedLayout L;
-  float* packed;      // raw | TF32 hi image | TF32 lo image, L.total floats each
-  ptrdiff_t hi_off, lo_off;
-  uint16_t *bhi, *blo; // bf16 (hi, lo) images, L.total elements each
+  float* packed;       // L.total floats, followed by its TF32 hi and lo images (img.tf32_hi, img.tf32_lo)
+  WeightImages img;    // of packed; the bf16 images are L.total elements each
   float* dpacked;
   // The shared-weight encoder runs ONCE over the reactant and product batches together (mpn.py:61-108 is row-wise apart from the gathers,
   // and those stay inside a segment): every encoder buffer holds the reactant rows followed by the product rows.
@@ -369,11 +287,12 @@ static int carve(const rr_model_cfg& c, const rr_graph& r, const rr_graph& p, vo
     used += (floats * sizeof(float) + 255) / 256 * 256;
     return ptr;
   };
-  W->packed = take(3 * W->L.total);
-  W->hi_off = static_cast<ptrdiff_t>(W->L.total);
-  W->lo_off = static_cast<ptrdiff_t>(2 * W->L.total);
-  W->bhi = reinterpret_cast<uint16_t*>(take((W->L.total + 1) / 2));
-  W->blo = reinterpret_cast<uint16_t*>(take((W->L.total + 1) / 2));
+  W->packed = take(W->L.total);   // L.total is a multiple of 64 floats: the two TF32 images follow it without a gap
+  W->img.base = W->packed;
+  W->img.tf32_hi = take(W->L.total);
+  W->img.tf32_lo = take(W->L.total);
+  W->img.bf16_hi = reinterpret_cast<uint16_t*>(take((W->L.total + 1) / 2));
+  W->img.bf16_lo = reinterpret_cast<uint16_t*>(take((W->L.total + 1) / 2));
   W->dpacked = take(W->L.grad_total);
   const size_t A_r = r.n_atoms, B_r = r.n_bonds, A_J = A_r + p.n_atoms, B_J = B_r + p.n_bonds;
   {
@@ -456,18 +375,6 @@ static int carve(const rr_model_cfg& c, const rr_graph& r, const rr_graph& p, vo
   return RR_OK;
 }
 
-// dX[M, k] (+)= dZ[M, n] W[n, k]: tensor cores read the transposed copy Wt[k, n] as a K-major operand, the SIMT path reads W
-static int dgrad(int M, int n, int k, const float* dZ, int lddz, const float* W, int ldw, const float* Wt, int ldwt, float* dX, int lddx,
-                 int accumulate, cudaStream_t s, ptrdiff_t hi_off, ptrdiff_t lo_off, const float* packed, const uint16_t* bhi, const uint16_t* blo) {
-  const bool tc = g_gemm_mode.load() == 1 || g_gemm_mode.load() == 3;
-  if (tc && g_bwd_bf16.load() && tc_linear_bf16_supported(M, k, n, lddz, ldwt))
-    return tc_linear_bf16(M, k, dZ, lddz, bhi + (Wt - packed), blo + (Wt - packed), ldwt, n, dX, lddx, accumulate, KC_GEMM_DGRAD, s);
-  if (tc && tc_supported(M, k, n, 0, lddz, 0))
-    return tc_linear(M, k, dZ, lddz, Wt + hi_off, ldwt, n, nullptr, 0, nullptr, 0, 0, nullptr, nullptr, 0, dX, lddx, 0, accumulate, 0.f, 0, 0, KC_GEMM_DGRAD, s,
-                     Wt + lo_off, nullptr);
-  return linear_dgrad(M, n, k, dZ, lddz, W, ldw, dX, lddx, accumulate, s);
-}
-
 // byte offset of a named forward buffer inside the workspace (tests compare per-layer activations with the oracle)
 long long model_buffer_offset(const rr_model_cfg* c, const rr_graph* r, const rr_graph* p, const char* name) {
   Workspace W;
@@ -535,11 +442,11 @@ static int check_model_args(const rr_model_cfg* c, const rr_params* w, const rr_
 }
 
 static int pack_params(const rr_model_cfg& c, const Workspace& W, const rr_params& w, cudaStream_t s) {
-  RR_CUDA(cudaMemsetAsync(W.packed, 0, 3 * W.L.total * sizeof(float), s));
-  RR_CUDA(cudaMemsetAsync(W.bhi, 0, W.L.total * sizeof(uint16_t), s));
-  RR_CUDA(cudaMemsetAsync(W.blo, 0, W.L.total * sizeof(uint16_t), s));
+  RR_CUDA(cudaMemsetAsync(W.packed, 0, 3 * W.L.total * sizeof(float), s));   // the weights and their TF32 images
+  RR_CUDA(cudaMemsetAsync(W.img.bf16_hi, 0, W.L.total * sizeof(uint16_t), s));
+  RR_CUDA(cudaMemsetAsync(W.img.bf16_lo, 0, W.L.total * sizeof(uint16_t), s));
   PackTable T = make_table(c, W.L, w, true);
-  k_pack<<<dim3(32, T.n), 256, 0, s>>>(T, W.packed, 0, W.hi_off, W.lo_off, W.bhi, W.blo);
+  k_pack<<<dim3(32, T.n), 256, 0, s>>>(T, W.packed, 0, W.img.tf32_hi - W.packed, W.img.tf32_lo - W.packed, W.img.bf16_hi, W.img.bf16_lo);
   RR_LAUNCH_CHECK("k_pack");
   return RR_OK;
 }
@@ -578,18 +485,11 @@ int model_forward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r, 
   uint64_t sid = 1;
   RR_TRY(pack_params(*c, W, *w, s));
 
-  // Y = act(X1 W1^T + X2 W2^T + bias + resid), then the segment padding rows once more in exact arithmetic when the GEMM ran on tensor cores
-  const int gmode = g_gemm_mode.load();
-  const bool fix_pads = (gmode == 1 || gmode == 2);
+  // Y = act(X1 W1^T + X2 W2^T + bias + resid); pad_rows: the segment padding rows of Y (see linear_fwd)
   auto lin = [&](const int* pad_rows, int n_pad, int M, int n, const float* X1, int ldx1, size_t W1, int k1, const float* X2, int ldx2, size_t W2, int k2,
                  size_t bias, const float* resid, float* Y, int ldy, int flags) -> int {
-    const uint64_t id = sid++;
-    RR_TRY(linear_fwd(M, n, X1, ldx1, P + W1, k1, X2, ldx2, X2 ? P + W2 : nullptr, k2, P + bias, resid, hp, Y, ldy, flags, pdrop, c->seed, id, s, W.hi_off,
-                      W.lo_off, W.packed, W.bhi, W.blo));
-    if (fix_pads && pad_rows)
-      RR_TRY(pad_rows_linear(pad_rows, n_pad, n, X1, ldx1, P + W1, k1, X2, ldx2, X2 ? P + W2 : nullptr, k2, P + bias, resid, hp, Y, ldy, flags, pdrop, c->seed,
-                             id, s));
-    return RR_OK;
+    return linear_fwd(M, n, X1, ldx1, P + W1, k1, X2, ldx2, X2 ? P + W2 : nullptr, k2, P + bias, resid, hp, Y, ldy, flags, pdrop, c->seed, sid++, s,
+                      &W.img, pad_rows, n_pad);
   };
   RR_TRY(build_joint(W, *r, *p, s));
   {  // mpn.py:61-108, once over [reactant rows | product rows]: the weights are shared (base_model.py:155-156)
@@ -680,12 +580,12 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
       RR_TRY(linear_wgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, x, L.ffn_in[l], G + L.ffn_W[l], L.ffn_in[l], G + L.ffn_b[l], s, W.det, W.det_bytes));
       if (l > 0) {
         float* dx = scratch[l & 1];
-        RR_TRY(dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], dx, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
+        RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], dx, hp, 0, W.img, s));
         RR_TRY(relu_bwd(N, hp, dx, W.x[l - 1], keep, 0, dx, nullptr, 0, s));
         g = dx;
         ldg = hp;
       } else {
-        RR_TRY(dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], W.dvec, vp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
+        RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], W.dvec, vp, 0, W.img, s));
       }
     }
   }
@@ -693,8 +593,8 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
   RR_TRY(readout_bwd(p, W.dvec, vp, W.vec, W.hid2, W.gA1, hp, pdrop, s));
   RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.d, hp, G + L.dif_Wo_d, hp, G + L.dif_bo, s, W.det, W.det_bytes));
   RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.am2, hp, G + L.dif_Wo_m, hp, nullptr, s, W.det, W.det_bytes));
-  RR_TRY(dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_d, hp, P + L.dif_Wo_d_T, hp, W.dD, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
-  RR_TRY(dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_m, hp, P + L.dif_Wo_m_T, hp, W.gA2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
+  RR_TRY(linear_dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_d, hp, P + L.dif_Wo_d_T, hp, W.dD, hp, 0, W.img, s));
+  RR_TRY(linear_dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_m, hp, P + L.dif_Wo_m_T, hp, W.gA2, hp, 0, W.img, s));
   // Every gather backward is followed by exactly one ReLU (+ dropout) backward: the mask of the message it produced the gradient of.
   // Both run as one kernel (rr_mp_pipe.cu): t_next >= 1 -> mask of m2^{t_next}, result kept (gA1) and summed into dI2;
   // t_next == 0 -> mask [inp2 > 0] of m2^0 = relu(inp2), only the sum into dI2 is wanted.
@@ -706,11 +606,11 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
   for (int t = Td; t >= 1; --t) {
     RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.nm[t - 1], hp, G + L.dif_Wh_m, hp, G + L.dif_bh, s, W.det, W.det_bytes));
     RR_TRY(linear_wgrad(A, hp, RR_FB_LD, W.gA1, hp, W.nf, RR_FB_LD, G + L.dif_Wh_f, RR_FB_LD, nullptr, s, W.det, W.det_bytes));
-    RR_TRY(dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wh_m, hp, P + L.dif_Wh_m_T, hp, W.gA2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
+    RR_TRY(linear_dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wh_m, hp, P + L.dif_Wh_m_T, hp, W.gA2, hp, 0, W.img, s));
     RR_TRY(diff_nbr_bwd(t - 1));
   }
   RR_TRY(linear_wgrad(A, hp, hp, W.dI2, hp, W.d, hp, G + L.dif_Wi, hp, G + L.dif_bi, s, W.det, W.det_bytes));
-  RR_TRY(dgrad(A, hp, hp, W.dI2, hp, P + L.dif_Wi, hp, P + L.dif_Wi_T, hp, W.dD, hp, 1, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
+  RR_TRY(linear_dgrad(A, hp, hp, W.dI2, hp, P + L.dif_Wi, hp, P + L.dif_Wi_T, hp, W.dD, hp, 1, W.img, s));
 
   // shared encoder, once over [reactant rows | product rows]: d(hid_p) = +dD, d(hid_r) = -dD (base_model.py:168), each through the
   // ReLU / dropout mask of its own rows; the weight gradients of both halves come out of one launch per layer (base_model.py:155-156)
@@ -730,12 +630,12 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
     }
     RR_TRY(linear_wgrad(A_J, hp, RR_FA_LD, W.gA1, hp, g->f_atoms, RR_FA_LD, G + L.enc_Wo_a, RR_FA_LD, G + L.enc_bo, s, W.det, W.det_bytes));
     RR_TRY(linear_wgrad(A_J, hp, hp, W.gA1, hp, e.am, hp, G + L.enc_Wo_m, hp, nullptr, s, W.det, W.det_bytes));
-    RR_TRY(dgrad(A_J, hp, hp, W.gA1, hp, P + L.enc_Wo_m, hp, P + L.enc_Wo_m_T, hp, W.gA2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
+    RR_TRY(linear_dgrad(A_J, hp, hp, W.gA1, hp, P + L.enc_Wo_m, hp, P + L.enc_Wo_m_T, hp, W.gA2, hp, 0, W.img, s));
     if (T >= 1) RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.m[T], keep, 0, W.dinp, 1, 0, s, W.det, W.det_bytes));
     else RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 1, 1, s, W.det, W.det_bytes));
     for (int t = T; t >= 1; --t) {
       RR_TRY(linear_wgrad(B_J, hp, hp, W.gB1, hp, e.pre[t - 1], hp, G + L.enc_Wh, hp, G + L.enc_bh, s, W.det, W.det_bytes));
-      RR_TRY(dgrad(B_J, hp, hp, W.gB1, hp, P + L.enc_Wh, hp, P + L.enc_Wh_T, hp, W.gB2, hp, 0, s, W.hi_off, W.lo_off, W.packed, W.bhi, W.blo));
+      RR_TRY(linear_dgrad(B_J, hp, hp, W.gB1, hp, P + L.enc_Wh, hp, P + L.enc_Wh_T, hp, W.gB2, hp, 0, W.img, s));
       if (t - 1 >= 1) RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.m[t - 1], keep, 0, W.dinp, 2, 0, s, W.det, W.det_bytes));
       else RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 2, 1, s, W.det, W.det_bytes));
     }

@@ -406,8 +406,8 @@ def test_full_batch_properties_at_config2_size():
 
 @pytest.mark.parametrize("task,hidden,depth", [("mle", 300, 3), ("evidential_ranking", 600, 5)])
 def test_tcgen05_backward_with_exact_forward(tc_mode, task, hidden, depth):
-    """gemm mode 3 = exact-fp32 forward (the oracle's masks up to fp32 rounding) + tensor-core dgrad / wgrad (3 x bf16): isolates the
-    backward GEMMs' accuracy from the forward's mask decisions.  Held to the SIMT path's 2e-4."""
+    """gemm mode 3 = exact-fp32 forward (the oracle's masks up to fp32 rounding) + tensor-core dgrad (3 x bf16) + SIMT wgrad: isolates
+    the tensor-core dgrad's accuracy from the forward's mask decisions.  Held to the SIMT path's 2e-4."""
     sizes = [7, 5, 9, 4]
     ds = synthetic.make_dataset(77, sizes)
     torch.manual_seed(3)
@@ -425,7 +425,7 @@ def test_tcgen05_backward_with_exact_forward(tc_mode, task, hidden, depth):
 
 def test_padding_rows_are_exact_on_the_tensor_core_path(tc_mode):
     """After every tensor-core forward GEMM the segment padding rows are recomputed from the unsplit fp32 weights with fp64 accumulation
-    (rr_model.cu: k_pad_rows_linear): one such row collects the gradient of every padded neighbour slot of its segment, so its ReLU masks
+    (rr_linear.cu: k_pad_rows_linear): one such row collects the gradient of every padded neighbour slot of its segment, so its ReLU masks
     must be the reference's.  Check: padding rows of every saved activation agree with the fp64 oracle to fp32 rounding (5e-7 of the row's
     maximum; the tensor-core rows carry 2-5e-6), also with several segments in one launch."""
     sizes = [6, 4, 5]
