@@ -102,11 +102,12 @@ typedef enum {
   RR_HEAD_NIG = 6                 /* base_model.py:61-70   (mu, sp + 1e-6, sp + 1 + 1e-6, sp + 1e-6), task_num % 4 == 0 */
 } rr_head;
 
-/* build_model(...) (models/base_model.py:235-297) */
+/* build_model(...) (models/base_model.py:235-297): one hidden size and one dropout for every sub-module.  rr_model_cfg_ex below gives
+ * the diff encoder and the FFN their own. */
 typedef struct {
-  int32_t hidden;       /* hidden_size                                    */
-  int32_t depth;        /* mpnn_depth       (>= 1)                        */
-  int32_t diff_depth;   /* mpnn_diff_depth  (>= 1)                        */
+  int32_t hidden;       /* hidden_size (1..4096)                          */
+  int32_t depth;        /* mpnn_depth       (1..16)                       */
+  int32_t diff_depth;   /* mpnn_diff_depth  (0..16; 0: no message passing, mpn.py:220-221) */
   int32_t ffn_depth;    /* ffn_depth        (1..RR_MAX_FFN)               */
   int32_t task_num;     /* width of the last layer (<= RR_OUT_LD)         */
   int32_t add_features; /* add_features_dim                               */
@@ -123,17 +124,32 @@ typedef struct {
   const int32_t* r_atom_map;
 } rr_model_cfg;
 
-/* Parameters in the reference's state_dict layout (row-major [out, in], SURVEY.md §5).
- * NULL bias = use_bias False.  The same struct with writable pointers receives the
+/* ReactionModel(mpnn_hidden_size, mpnn_diff_hidden_size, ffn_hidden_size, mpnn_dropout, mpnn_diff_dropout, ffn_dropout, ...)
+ * (models/base_model.py:111-148): per-sub-module widths and dropouts.  base.hidden and base.dropout are the encoder's (MPN).  Every field is
+ * required: widths in 1..4096, dropouts in [0, 1).  The diff encoder reads the encoder's width (W_i [diff_hidden, hidden]) and the FFN's
+ * first layer diff_hidden + add_features.  Dropout sites: the encoder's messages and atom hiddens take base.dropout, the diff encoder's
+ * diff_dropout, the readout vector and the FFN's hidden layers ffn_dropout.  r_atom_map is refused while training if any of the three
+ * is > 0. */
+typedef struct {
+  rr_model_cfg base;
+  int32_t diff_hidden;  /* mpnn_diff_hidden_size */
+  int32_t ffn_hidden;   /* ffn_hidden_size       */
+  float diff_dropout;   /* mpnn_diff_dropout     */
+  float ffn_dropout;    /* ffn_dropout           */
+} rr_model_cfg_ex;
+
+/* Parameters in the reference's state_dict layout (row-major [out, in], SURVEY.md §5); he / hd / hf: the encoder's, diff encoder's
+ * and FFN's hidden size (all = hidden with rr_model_cfg).  NULL bias = use_bias False.  encoder.W_h is needed for depth > 1,
+ * diff_encoder.W_h for diff_depth > 1, diff_encoder.W_o for diff_depth > 0.  The same struct with writable pointers receives the
  * gradients (overwritten, not accumulated). */
 typedef struct {
-  float* enc_Wi; float* enc_bi;   /* encoder.W_i   [h, 83]        mpn.py:50  */
-  float* enc_Wh; float* enc_bh;   /* encoder.W_h   [h, h]         mpn.py:57  */
-  float* enc_Wo; float* enc_bo;   /* encoder.W_o   [h, 61+h]      mpn.py:59  */
-  float* dif_Wi; float* dif_bi;   /* diff_encoder.W_i [h, h]      mpn.py:161 */
-  float* dif_Wh; float* dif_bh;   /* diff_encoder.W_h [h, h+83]   mpn.py:165 */
-  float* dif_Wo; float* dif_bo;   /* diff_encoder.W_o [h, 2h]     mpn.py:168 */
-  float* ffn_W[RR_MAX_FFN];       /* ffn.ffn.{1,4,7,..}           base_model.py:40-56 */
+  float* enc_Wi; float* enc_bi;   /* encoder.W_i   [he, 83]        mpn.py:50  */
+  float* enc_Wh; float* enc_bh;   /* encoder.W_h   [he, he]        mpn.py:57  */
+  float* enc_Wo; float* enc_bo;   /* encoder.W_o   [he, 61+he]     mpn.py:59  */
+  float* dif_Wi; float* dif_bi;   /* diff_encoder.W_i [hd, he]     mpn.py:161 */
+  float* dif_Wh; float* dif_bh;   /* diff_encoder.W_h [hd, hd+83]  mpn.py:165 */
+  float* dif_Wo; float* dif_bo;   /* diff_encoder.W_o [hd, he+hd]  mpn.py:168 */
+  float* ffn_W[RR_MAX_FFN];       /* ffn.ffn.{1,4,7,..}: (hd+add) -> hf -> ... -> task_num  base_model.py:40-56 */
   float* ffn_b[RR_MAX_FFN];
 } rr_params;
 
@@ -187,7 +203,7 @@ int rr_neighbor_sum_bwd_act(const rr_graph* g, int which, const float* dout, flo
  * then the FFN's first dropout (base_model.py:40).  hid is [n_atoms, hp], vec is [n_mols, vp]. */
 int rr_readout_fwd(const rr_graph* g, const float* hid, int hp, int hidden, const float* add_features, int n_add,
                    float* vec, int vp, float dropout, uint64_t seed, uint64_t stream_id, void* stream);
-/* backward, fused with the relu/dropout mask of hid: dz[a] = dvec[mol(a)]/size * [hid!=0]*scale */
+/* backward, fused with the relu/dropout mask of hid: dz[a] = dvec[mol(a)]/size * [hid!=0]*scale (the same dropout p on vec and hid) */
 int rr_readout_bwd(const rr_graph* g, const float* dvec, int vp, const float* vec, const float* hid, float* dz,
                    int hp, float dropout, void* stream);
 
@@ -298,7 +314,7 @@ int rr_rank_metrics(int N, int G, const float* scores, int score_ld, const doubl
 int64_t rr_model_workspace_bytes(const rr_model_cfg* cfg, const rr_graph* r, const rr_graph* p);
 /* Byte offset, inside the workspace, of a forward activation saved for backward -- for per-layer parity tests.
  * Names: enc{0,1}.inp, enc{0,1}.pre<t>, enc{0,1}.m<t+1>, enc{0,1}.am, enc{0,1}.hid (0 = reactants, 1 = products),
- * d, inp2, nf, nm<t>, m2_<t+1>, am2, hid2, vec, zout.  -1 on error. */
+ * d, inp2, nf, nm<t>, m2_<t+1>, am2, hid2, vec, x<l>, zout.  -1 on error, and for inp2 / nf / am2 at diff_depth 0, where they do not exist. */
 int64_t rr_model_buffer_offset(const rr_model_cfg* cfg, const rr_graph* r, const rr_graph* p, const char* name);
 /* scores: [n_mols] if task_num==1 else [n_mols, task_num].  ws must stay untouched until the
  * matching rr_model_backward has run. */
@@ -307,6 +323,14 @@ int rr_model_forward(const rr_model_cfg* cfg, const rr_params* w, const rr_graph
 /* dscores has the shape of scores; grads receives d/d(parameter) in state_dict layout */
 int rr_model_backward(const rr_model_cfg* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p,
                       const float* dscores, rr_params* grads, void* ws, int64_t ws_bytes, void* stream);
+/* The same four with per-sub-module widths and dropouts.  The entry points above are these with diff_hidden = ffn_hidden = hidden and
+ * diff_dropout = ffn_dropout = dropout; a workspace sized by one must be used with a configuration of the same widths. */
+int64_t rr_model_workspace_bytes_ex(const rr_model_cfg_ex* cfg, const rr_graph* r, const rr_graph* p);
+int64_t rr_model_buffer_offset_ex(const rr_model_cfg_ex* cfg, const rr_graph* r, const rr_graph* p, const char* name);
+int rr_model_forward_ex(const rr_model_cfg_ex* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p,
+                        const float* add_features, float* scores, void* ws, int64_t ws_bytes, void* stream);
+int rr_model_backward_ex(const rr_model_cfg_ex* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p,
+                         const float* dscores, rr_params* grads, void* ws, int64_t ws_bytes, void* stream);
 /* Per-kernel-class device timing for bench.py's roofline: between begin and end every launch is bracketed by
  * CUDA events on its own stream; end() waits for them and returns summed milliseconds / launch counts per class
  * (0 gemm_fwd 1 gemm_dgrad 2 gemm_wgrad 3 bond_fwd 4 bond_bwd 5 nbr_fwd 6 nbr_bwd 7 readout 8 elementwise 9 loss 10 misc). */

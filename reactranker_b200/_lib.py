@@ -35,6 +35,13 @@ class RRModelCfg(ctypes.Structure):
                 ("seed", ctypes.c_uint64), ("r_atom_map", ctypes.c_void_p)]
 
 
+class RRModelCfgEx(ctypes.Structure):
+    """rr_model_cfg_ex: ``base`` is anonymous, so ``cfg.seed`` etc. read through, and ``byref(cfg)`` is also a valid ``rr_model_cfg*``."""
+    _anonymous_ = ("base",)
+    _fields_ = [("base", RRModelCfg), ("diff_hidden", ctypes.c_int32), ("ffn_hidden", ctypes.c_int32),
+                ("diff_dropout", ctypes.c_float), ("ffn_dropout", ctypes.c_float)]
+
+
 class RRMolStore(ctypes.Structure):
     _fields_ = [(k, ctypes.c_void_p) for k in ("f_atoms", "f_bonds", "n_atoms", "n_bonds", "atom_off", "bond_off", "deg", "a2b_start", "a2b_flat", "b2a")]
 
@@ -50,7 +57,8 @@ EXPORTS = [
     "rr_graph_assemble", "rr_batch_build", "rr_bond_message_fwd", "rr_bond_message_bwd", "rr_neighbor_sum_fwd", "rr_neighbor_sum_bwd",
     "rr_bond_message_bwd_act", "rr_neighbor_sum_bwd_act", "rr_readout_fwd", "rr_readout_bwd", "rr_linear_fwd", "rr_linear_dgrad", "rr_linear_dgrad_tc", "rr_linear_dgrad_tc_scratch_bytes", "rr_linear_wgrad", "rr_relu_bwd", "rr_sub",
     "rr_loss_fwdbwd", "rr_loss_fwdbwd_ex", "rr_loss_max_group", "rr_rank_metrics",
-    "rr_model_workspace_bytes", "rr_model_buffer_offset", "rr_model_forward", "rr_model_backward", "rr_launch_count", "rr_launch_count_reset",
+    "rr_model_workspace_bytes", "rr_model_buffer_offset", "rr_model_forward", "rr_model_backward", "rr_model_workspace_bytes_ex",
+    "rr_model_buffer_offset_ex", "rr_model_forward_ex", "rr_model_backward_ex", "rr_launch_count", "rr_launch_count_reset",
     "rr_profile_begin", "rr_profile_end", "rr_profile_classes", "rr_set_gemm_mode", "rr_get_gemm_mode", "rr_set_backward_bf16", "rr_get_backward_bf16",
     "rr_set_forward_bf16", "rr_get_forward_bf16", "rr_reload_switches", "rr_set_deterministic", "rr_get_deterministic",
 ]
@@ -149,6 +157,12 @@ def lib() -> ctypes.CDLL:
                 L.rr_model_buffer_offset.restype = ctypes.c_int64
                 L.rr_model_forward.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, vp]
                 L.rr_model_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, vp]
+                L.rr_model_workspace_bytes_ex.argtypes = [vp, vp, vp]
+                L.rr_model_workspace_bytes_ex.restype = ctypes.c_int64
+                L.rr_model_buffer_offset_ex.argtypes = [vp, vp, vp, ctypes.c_char_p]
+                L.rr_model_buffer_offset_ex.restype = ctypes.c_int64
+                L.rr_model_forward_ex.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, vp]
+                L.rr_model_backward_ex.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, vp]
                 L.rr_profile_end.argtypes = [vp, vp, i32]
                 L.rr_set_gemm_mode.argtypes = [i32]
                 # dense layers: tcgen05 tensor cores (3xTF32 split) unless RR_GEMM_MODE=0 asks for the exact-fp32 SIMT kernels

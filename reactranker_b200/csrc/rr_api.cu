@@ -110,7 +110,7 @@ int rr_readout_fwd(const rr_graph* g, const float* hid, int hp, int hidden, cons
   return rr::readout_fwd(g, hid, hp, hidden, add_features, n_add, vec, vp, dropout, seed, stream_id, S(stream));
 }
 int rr_readout_bwd(const rr_graph* g, const float* dvec, int vp, const float* vec, const float* hid, float* dz, int hp, float dropout, void* stream) {
-  return rr::readout_bwd(g, dvec, vp, vec, hid, dz, hp, dropout, S(stream));
+  return rr::readout_bwd(g, dvec, vp, vec, hid, dz, hp, dropout, dropout, S(stream));
 }
 int rr_linear_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2, int k2,
                   const float* bias, const float* residual, int ldr, float* Y, int ldy, int flags, float dropout, uint64_t seed,
@@ -147,27 +147,51 @@ int rr_rank_metrics(int N, int G, const float* scores, int score_ld, const doubl
   return rr::rank_metrics(N, G, scores, score_ld, targets, seg_off, max_group, ratio, out, S(stream));
 }
 
-int64_t rr_model_workspace_bytes(const rr_model_cfg* cfg, const rr_graph* r, const rr_graph* p) {
+int64_t rr_model_workspace_bytes_ex(const rr_model_cfg_ex* cfg, const rr_graph* r, const rr_graph* p) {
   if (!cfg || !r || !p) {
     rr::fail(RR_ERR_INVALID, "rr_model_workspace_bytes: NULL argument");
     return -1;
   }
   return rr::model_workspace_bytes(cfg, r, p);
 }
-int64_t rr_model_buffer_offset(const rr_model_cfg* cfg, const rr_graph* r, const rr_graph* p, const char* name) {
+int64_t rr_model_buffer_offset_ex(const rr_model_cfg_ex* cfg, const rr_graph* r, const rr_graph* p, const char* name) {
   if (!cfg || !r || !p || !name) {
     rr::fail(RR_ERR_INVALID, "rr_model_buffer_offset: NULL argument");
     return -1;
   }
   return rr::model_buffer_offset(cfg, r, p, name);
 }
+int rr_model_forward_ex(const rr_model_cfg_ex* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* add_features,
+                        float* scores, void* ws, int64_t ws_bytes, void* stream) {
+  return rr::model_forward(cfg, w, r, p, add_features, scores, ws, ws_bytes, S(stream));
+}
+int rr_model_backward_ex(const rr_model_cfg_ex* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* dscores,
+                         rr_params* grads, void* ws, int64_t ws_bytes, void* stream) {
+  return rr::model_backward(cfg, w, r, p, dscores, grads, ws, ws_bytes, S(stream));
+}
+// ABI 3: every sub-module has cfg->hidden and cfg->dropout (a NULL cfg stays NULL for the _ex entry point to report)
+static const rr_model_cfg_ex* tied(const rr_model_cfg* cfg, rr_model_cfg_ex* ex) {
+  if (!cfg) return nullptr;
+  *ex = rr_model_cfg_ex{*cfg, cfg->hidden, cfg->hidden, cfg->dropout, cfg->dropout};
+  return ex;
+}
+int64_t rr_model_workspace_bytes(const rr_model_cfg* cfg, const rr_graph* r, const rr_graph* p) {
+  rr_model_cfg_ex ex;
+  return rr_model_workspace_bytes_ex(tied(cfg, &ex), r, p);
+}
+int64_t rr_model_buffer_offset(const rr_model_cfg* cfg, const rr_graph* r, const rr_graph* p, const char* name) {
+  rr_model_cfg_ex ex;
+  return rr_model_buffer_offset_ex(tied(cfg, &ex), r, p, name);
+}
 int rr_model_forward(const rr_model_cfg* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* add_features,
                      float* scores, void* ws, int64_t ws_bytes, void* stream) {
-  return rr::model_forward(cfg, w, r, p, add_features, scores, ws, ws_bytes, S(stream));
+  rr_model_cfg_ex ex;
+  return rr_model_forward_ex(tied(cfg, &ex), w, r, p, add_features, scores, ws, ws_bytes, stream);
 }
 int rr_model_backward(const rr_model_cfg* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* dscores,
                       rr_params* grads, void* ws, int64_t ws_bytes, void* stream) {
-  return rr::model_backward(cfg, w, r, p, dscores, grads, ws, ws_bytes, S(stream));
+  rr_model_cfg_ex ex;
+  return rr_model_backward_ex(tied(cfg, &ex), w, r, p, dscores, grads, ws, ws_bytes, stream);
 }
 int rr_set_gemm_mode(int mode) {
   RR_REQUIRE(mode >= 0 && mode <= 3, "gemm mode must be 0 (fp32 SIMT), 1 (tcgen05 3xTF32) or the debug masks 2 (forward only) / 3 (dgrad only)");

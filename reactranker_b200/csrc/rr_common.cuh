@@ -275,7 +275,9 @@ int pad_rows_sum(float* out, const int* rows, int n_rows, int ld, const PadParts
 // scratch for a deterministic launch: `given` when not NULL (RR_ERR_WORKSPACE if smaller than need), else cudaMallocAsync on s
 int det_scratch(DetScratch* d, void* given, long long given_bytes, long long need, cudaStream_t s);
 int readout_fwd(const rr_graph*, const float*, int, int, const float*, int, float*, int, float, uint64_t, uint64_t, cudaStream_t);
-int readout_bwd(const rr_graph*, const float*, int, const float*, const float*, float*, int, float, cudaStream_t);
+// p_vec: the FFN's dropout on vec, p_hid: the diff encoder's on hid
+int readout_bwd(const rr_graph*, const float* dvec, int vp, const float* vec, const float* hid, float* dz, int hp, float p_vec, float p_hid,
+                cudaStream_t);
 int relu_bwd(long long, int, const float*, const float*, float, int, float*, float*, int, cudaStream_t);
 int sub(long long, const float*, const float*, float*, cudaStream_t);
 int sub_gather(long long rows, int ld, const float* a, const float* b, const int* map, float* out, cudaStream_t);
@@ -285,10 +287,11 @@ int loss_max_group();
 int rank_metrics(int, int, const float*, int, const double*, const int*, int, double, double*, cudaStream_t);
 int graph_assemble(const rr_mol_store*, int, const int*, const int*, const int*, const int*, const int*, const int*, int, const int*, const int*,
                    const int*, const rr_graph*, cudaStream_t);
-long long model_workspace_bytes(const rr_model_cfg*, const rr_graph*, const rr_graph*);
-long long model_buffer_offset(const rr_model_cfg*, const rr_graph*, const rr_graph*, const char*);
-int model_forward(const rr_model_cfg*, const rr_params*, const rr_graph*, const rr_graph*, const float*, float*, void*, long long, cudaStream_t);
-int model_backward(const rr_model_cfg*, const rr_params*, const rr_graph*, const rr_graph*, const float*, rr_params*, void*, long long, cudaStream_t);
+long long model_workspace_bytes(const rr_model_cfg_ex*, const rr_graph*, const rr_graph*);
+long long model_buffer_offset(const rr_model_cfg_ex*, const rr_graph*, const rr_graph*, const char*);
+int model_forward(const rr_model_cfg_ex*, const rr_params*, const rr_graph*, const rr_graph*, const float*, float*, void*, long long, cudaStream_t);
+int model_backward(const rr_model_cfg_ex*, const rr_params*, const rr_graph*, const rr_graph*, const float*, rr_params*, void*, long long,
+                   cudaStream_t);
 
 // ---- dense layers (nn.Linear) ---------------------------------------------------------------------
 // Pre-split images of fp32 weights for the tensor-core GEMMs: the images of the weight at base[i] are element i of each array.  The model

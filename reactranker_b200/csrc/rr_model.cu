@@ -18,8 +18,10 @@ int padded(int w) { return pad16(w); }
 constexpr int kMaxDepth = 16;
 
 // ---- packed parameter layout (float offsets) ---------------------------------------------
+// Every sub-module has its own padded width: hpe (encoder, and the difference d = p - r it produces), hpd (diff encoder), hpf (FFN hidden
+// layers); the readout vector [mean(hid2) || add_features] is vp = pad16(hd + add_features) wide.
 struct PackedLayout {
-  int h, hp, vp, F;
+  int hpe, hpd, hpf, vp, F;
   size_t enc_Wi, enc_bi, enc_Wh, enc_bh, enc_Wo_a, enc_Wo_m, enc_bo;
   size_t dif_Wi, dif_bi, dif_Wh_m, dif_Wh_f, dif_bh, dif_Wo_d, dif_Wo_m, dif_bo;
   size_t ffn_W[RR_MAX_FFN], ffn_b[RR_MAX_FFN];
@@ -30,38 +32,39 @@ struct PackedLayout {
   size_t grad_total;  // floats of the gradient image (no transposed copies)
 };
 
-static PackedLayout make_packed(const rr_model_cfg& c) {
+static PackedLayout make_packed(const rr_model_cfg_ex& c) {
   PackedLayout L{};
-  L.h = c.hidden;
-  L.hp = pad16(c.hidden);
-  L.vp = pad16(c.hidden + c.add_features);
-  L.F = c.ffn_depth;
+  L.hpe = pad16(c.base.hidden);
+  L.hpd = pad16(c.diff_hidden);
+  L.hpf = pad16(c.ffn_hidden);
+  L.vp = pad16(c.diff_hidden + c.base.add_features);
+  L.F = c.base.ffn_depth;
   size_t o = 0;
   auto take = [&](size_t n) {
     size_t r = o;
     o += (n + 63) / 64 * 64;
     return r;
   };
-  const size_t hp = L.hp;
-  L.enc_Wi = take(hp * RR_FB_LD); L.enc_bi = take(hp);
-  L.enc_Wh = take(hp * hp);       L.enc_bh = take(hp);
-  L.enc_Wo_a = take(hp * RR_FA_LD); L.enc_Wo_m = take(hp * hp); L.enc_bo = take(hp);
-  L.dif_Wi = take(hp * hp);       L.dif_bi = take(hp);
-  L.dif_Wh_m = take(hp * hp);     L.dif_Wh_f = take(hp * RR_FB_LD); L.dif_bh = take(hp);
-  L.dif_Wo_d = take(hp * hp);     L.dif_Wo_m = take(hp * hp);       L.dif_bo = take(hp);
+  const size_t he = L.hpe, hd = L.hpd;
+  L.enc_Wi = take(he * RR_FB_LD); L.enc_bi = take(he);
+  L.enc_Wh = take(he * he);       L.enc_bh = take(he);
+  L.enc_Wo_a = take(he * RR_FA_LD); L.enc_Wo_m = take(he * he); L.enc_bo = take(he);
+  L.dif_Wi = take(hd * he);       L.dif_bi = take(hd);
+  L.dif_Wh_m = take(hd * hd);     L.dif_Wh_f = take(hd * RR_FB_LD); L.dif_bh = take(hd);
+  L.dif_Wo_d = take(hd * he);     L.dif_Wo_m = take(hd * hd);       L.dif_bo = take(hd);
   for (int l = 0; l < L.F; ++l) {
-    L.ffn_in[l] = (l == 0) ? L.vp : L.hp;
-    L.ffn_out[l] = (l == L.F - 1) ? RR_OUT_LD : L.hp;
+    L.ffn_in[l] = (l == 0) ? L.vp : L.hpf;
+    L.ffn_out[l] = (l == L.F - 1) ? RR_OUT_LD : L.hpf;
     L.ffn_W[l] = take(static_cast<size_t>(L.ffn_in[l]) * L.ffn_out[l]);
     L.ffn_b[l] = take(L.ffn_out[l]);
   }
   L.grad_total = o;
-  L.enc_Wh_T = take(hp * hp);
-  L.enc_Wo_m_T = take(hp * hp);
-  L.dif_Wi_T = take(hp * hp);
-  L.dif_Wh_m_T = take(hp * hp);
-  L.dif_Wo_d_T = take(hp * hp);
-  L.dif_Wo_m_T = take(hp * hp);
+  L.enc_Wh_T = take(he * he);
+  L.enc_Wo_m_T = take(he * he);
+  L.dif_Wi_T = take(he * hd);
+  L.dif_Wh_m_T = take(hd * hd);
+  L.dif_Wo_d_T = take(he * hd);
+  L.dif_Wo_m_T = take(hd * hd);
   for (int l = 0; l < L.F; ++l) L.ffn_W_T[l] = take(static_cast<size_t>(L.ffn_in[l]) * L.ffn_out[l]);
   L.total = o;
   return L;
@@ -79,9 +82,9 @@ struct PackTable {
   int n;
 };
 
-static PackTable make_table(const rr_model_cfg& c, const PackedLayout& L, const rr_params& w, bool with_transposes) {
+static PackTable make_table(const rr_model_cfg_ex& c, const PackedLayout& L, const rr_params& w, bool with_transposes) {
   PackTable T{};
-  const int h = c.hidden, hp = L.hp;
+  const int he = c.base.hidden, hd = c.diff_hidden, hf = c.ffn_hidden, hpe = L.hpe, hpd = L.hpd;
   auto add = [&](float* ref, size_t off, int rows, int cols, int ref_ld, int col0, int pld) {
     if (ref == nullptr) return;
     T.e[T.n++] = PackEntry{ref, static_cast<long long>(off), rows, cols, ref_ld, col0, pld, 0};
@@ -90,34 +93,34 @@ static PackTable make_table(const rr_model_cfg& c, const PackedLayout& L, const 
     if (ref == nullptr || !with_transposes) return;
     T.e[T.n++] = PackEntry{ref, static_cast<long long>(off), rows, cols, ref_ld, col0, pld, 1};
   };
-  add(w.enc_Wi, L.enc_Wi, h, RR_FBOND_TOTAL, RR_FBOND_TOTAL, 0, RR_FB_LD);
-  add(w.enc_bi, L.enc_bi, 1, h, h, 0, hp);
-  add(w.enc_Wh, L.enc_Wh, h, h, h, 0, hp);
-  add(w.enc_bh, L.enc_bh, 1, h, h, 0, hp);
-  add(w.enc_Wo, L.enc_Wo_a, h, RR_ATOM_FDIM, RR_ATOM_FDIM + h, 0, RR_FA_LD);
-  add(w.enc_Wo, L.enc_Wo_m, h, h, RR_ATOM_FDIM + h, RR_ATOM_FDIM, hp);
-  add(w.enc_bo, L.enc_bo, 1, h, h, 0, hp);
-  add(w.dif_Wi, L.dif_Wi, h, h, h, 0, hp);
-  add(w.dif_bi, L.dif_bi, 1, h, h, 0, hp);
-  add(w.dif_Wh, L.dif_Wh_m, h, h, h + RR_FBOND_TOTAL, 0, hp);
-  add(w.dif_Wh, L.dif_Wh_f, h, RR_FBOND_TOTAL, h + RR_FBOND_TOTAL, h, RR_FB_LD);
-  add(w.dif_bh, L.dif_bh, 1, h, h, 0, hp);
-  add(w.dif_Wo, L.dif_Wo_d, h, h, 2 * h, 0, hp);
-  add(w.dif_Wo, L.dif_Wo_m, h, h, 2 * h, h, hp);
-  add(w.dif_bo, L.dif_bo, 1, h, h, 0, hp);
+  add(w.enc_Wi, L.enc_Wi, he, RR_FBOND_TOTAL, RR_FBOND_TOTAL, 0, RR_FB_LD);
+  add(w.enc_bi, L.enc_bi, 1, he, he, 0, hpe);
+  add(w.enc_Wh, L.enc_Wh, he, he, he, 0, hpe);
+  add(w.enc_bh, L.enc_bh, 1, he, he, 0, hpe);
+  add(w.enc_Wo, L.enc_Wo_a, he, RR_ATOM_FDIM, RR_ATOM_FDIM + he, 0, RR_FA_LD);
+  add(w.enc_Wo, L.enc_Wo_m, he, he, RR_ATOM_FDIM + he, RR_ATOM_FDIM, hpe);
+  add(w.enc_bo, L.enc_bo, 1, he, he, 0, hpe);
+  add(w.dif_Wi, L.dif_Wi, hd, he, he, 0, hpe);
+  add(w.dif_bi, L.dif_bi, 1, hd, hd, 0, hpd);
+  add(w.dif_Wh, L.dif_Wh_m, hd, hd, hd + RR_FBOND_TOTAL, 0, hpd);
+  add(w.dif_Wh, L.dif_Wh_f, hd, RR_FBOND_TOTAL, hd + RR_FBOND_TOTAL, hd, RR_FB_LD);
+  add(w.dif_bh, L.dif_bh, 1, hd, hd, 0, hpd);
+  add(w.dif_Wo, L.dif_Wo_d, hd, he, he + hd, 0, hpe);
+  add(w.dif_Wo, L.dif_Wo_m, hd, hd, he + hd, he, hpd);
+  add(w.dif_bo, L.dif_bo, 1, hd, hd, 0, hpd);
   for (int l = 0; l < L.F; ++l) {
-    const int in = (l == 0) ? h + c.add_features : h;
-    const int out = (l == L.F - 1) ? c.task_num : h;
+    const int in = (l == 0) ? hd + c.base.add_features : hf;
+    const int out = (l == L.F - 1) ? c.base.task_num : hf;
     add(w.ffn_W[l], L.ffn_W[l], out, in, in, 0, L.ffn_in[l]);
     add(w.ffn_b[l], L.ffn_b[l], 1, out, out, 0, L.ffn_out[l]);
     add_t(w.ffn_W[l], L.ffn_W_T[l], out, in, in, 0, L.ffn_out[l]);
   }
-  add_t(w.enc_Wh, L.enc_Wh_T, h, h, h, 0, hp);
-  add_t(w.enc_Wo, L.enc_Wo_m_T, h, h, RR_ATOM_FDIM + h, RR_ATOM_FDIM, hp);
-  add_t(w.dif_Wi, L.dif_Wi_T, h, h, h, 0, hp);
-  add_t(w.dif_Wh, L.dif_Wh_m_T, h, h, h + RR_FBOND_TOTAL, 0, hp);
-  add_t(w.dif_Wo, L.dif_Wo_d_T, h, h, 2 * h, 0, hp);
-  add_t(w.dif_Wo, L.dif_Wo_m_T, h, h, 2 * h, h, hp);
+  add_t(w.enc_Wh, L.enc_Wh_T, he, he, he, 0, hpe);
+  add_t(w.enc_Wo, L.enc_Wo_m_T, he, he, RR_ATOM_FDIM + he, RR_ATOM_FDIM, hpe);
+  add_t(w.dif_Wi, L.dif_Wi_T, hd, he, he, 0, hpd);
+  add_t(w.dif_Wh, L.dif_Wh_m_T, hd, hd, hd + RR_FBOND_TOTAL, 0, hpd);
+  add_t(w.dif_Wo, L.dif_Wo_d_T, hd, he, he + hd, 0, hpd);
+  add_t(w.dif_Wo, L.dif_Wo_m_T, hd, hd, he + hd, he, hpd);
   return T;
 }
 
@@ -265,21 +268,24 @@ struct Workspace {
   size_t bytes;
 };
 
-static int carve(const rr_model_cfg& c, const rr_graph& r, const rr_graph& p, void* base, Workspace* W) {
+static int carve(const rr_model_cfg_ex& cx, const rr_graph& r, const rr_graph& p, void* base, Workspace* W) {
+  const rr_model_cfg& c = cx.base;
   RR_REQUIRE(c.hidden > 0 && c.hidden <= 4096, "hidden %d out of range", c.hidden);
+  RR_REQUIRE(cx.diff_hidden > 0 && cx.diff_hidden <= 4096, "diff_hidden %d out of range", cx.diff_hidden);
+  RR_REQUIRE(cx.ffn_hidden > 0 && cx.ffn_hidden <= 4096, "ffn_hidden %d out of range", cx.ffn_hidden);
   RR_REQUIRE(c.depth >= 1 && c.depth <= kMaxDepth && c.diff_depth >= 0 && c.diff_depth <= kMaxDepth, "depth %d / diff_depth %d out of range", c.depth, c.diff_depth);
-  if (c.diff_depth < 1) return fail(RR_ERR_UNSUPPORTED, "mpnn_diff_depth = 0 (mpn.py:220-221) is not built");
   RR_REQUIRE(c.ffn_depth >= 1 && c.ffn_depth <= RR_MAX_FFN, "ffn_depth %d out of range", c.ffn_depth);
   RR_REQUIRE(c.task_num >= 1 && c.task_num <= RR_OUT_LD, "task_num %d out of range", c.task_num);
   RR_REQUIRE(c.add_features >= 0, "add_features < 0");
   RR_REQUIRE(c.r_atom_map != nullptr || (r.n_atoms == p.n_atoms && r.n_mols == p.n_mols),
              "reactant and product batches must have identical atom rows (p - r is atom-wise, base_model.py:168): %d vs %d", r.n_atoms, p.n_atoms);
-  RR_REQUIRE(c.r_atom_map == nullptr || !(c.training && c.dropout > 0.f),
+  RR_REQUIRE(c.r_atom_map == nullptr || !(c.training && (c.dropout > 0.f || cx.diff_dropout > 0.f || cx.ffn_dropout > 0.f)),
              "r_atom_map (de-duplicated reactants) is exact only without dropout: pass NULL when training with dropout > 0");
-  W->L = make_packed(c);
-  const size_t hp = W->L.hp, vp = W->L.vp;
+  W->L = make_packed(cx);
+  const size_t hpe = W->L.hpe, hpd = W->L.hpd, hpf = W->L.hpf, vp = W->L.vp;
   const size_t A = p.n_atoms, N = p.n_mols;
   const int T = c.depth - 1, Td = c.diff_depth - 1;
+  const bool msg2 = c.diff_depth > 0;   // the diff encoder passes messages (mpn.py:199-216); at depth 0 it is W_i alone (mpn.py:220-221)
   char* cur = static_cast<char*>(base);
   size_t used = 0;
   auto take = [&](size_t floats) {
@@ -297,12 +303,12 @@ static int carve(const rr_model_cfg& c, const rr_graph& r, const rr_graph& p, vo
   const size_t A_r = r.n_atoms, B_r = r.n_bonds, A_J = A_r + p.n_atoms, B_J = B_r + p.n_bonds;
   {
     EncBufs& e = W->j;
-    e.inp = take(B_J * hp);
-    for (int t = 0; t < T; ++t) e.pre[t] = take(B_J * hp);
-    for (int t = 1; t <= T; ++t) e.m[t] = take(B_J * hp);
-    e.am = take(A_J * hp);
-    e.hid = take(A_J * hp);
-    auto part = [&](float* q, size_t rows) { return q ? q + rows * hp : nullptr; };
+    e.inp = take(B_J * hpe);
+    for (int t = 0; t < T; ++t) e.pre[t] = take(B_J * hpe);
+    for (int t = 1; t <= T; ++t) e.m[t] = take(B_J * hpe);
+    e.am = take(A_J * hpe);
+    e.hid = take(A_J * hpe);
+    auto part = [&](float* q, size_t rows) { return q ? q + rows * hpe : nullptr; };
     W->enc[0] = e;
     EncBufs& q = W->enc[1];
     q.inp = part(e.inp, B_r);
@@ -331,43 +337,47 @@ static int carve(const rr_model_cfg& c, const rr_graph& r, const rr_graph& p, vo
     J.f_atoms = W->copy_feats ? W->j_fa : r.f_atoms;
     J.f_bonds = W->copy_feats ? W->j_fb : r.f_bonds;
   }
-  W->d = take(A * hp);
-  W->inp2 = take(A * hp);
-  W->nf = take(A * RR_FB_LD);
-  for (int t = 0; t < Td; ++t) W->nm[t] = take(A * hp);
-  for (int t = 1; t <= Td; ++t) W->m2[t] = take(A * hp);
-  W->am2 = take(A * hp);
-  W->hid2 = take(A * hp);
+  W->d = take(A * hpe);
+  W->inp2 = msg2 ? take(A * hpd) : nullptr;
+  W->nf = msg2 ? take(A * RR_FB_LD) : nullptr;
+  for (int t = 0; t < Td; ++t) W->nm[t] = take(A * hpd);
+  for (int t = 1; t <= Td; ++t) W->m2[t] = take(A * hpd);
+  W->am2 = msg2 ? take(A * hpd) : nullptr;
+  W->hid2 = take(A * hpd);
   W->vec = take(N * vp);
-  for (int l = 0; l + 1 < c.ffn_depth; ++l) W->x[l] = take(N * hp);
+  for (int l = 0; l + 1 < c.ffn_depth; ++l) W->x[l] = take(N * hpf);
   W->zout = take(N * RR_OUT_LD);
-  W->gB1 = take(B_J * hp);
-  W->gB2 = take(B_J * hp);
-  W->dinp = take(B_J * hp);
-  W->gA1 = take(A_J * hp);
-  W->gA2 = take(A_J * hp);
-  W->gA3 = take(A * hp);
-  W->dD = take(A * hp);
-  W->dI2 = take(A * hp);
+  W->gB1 = take(B_J * hpe);
+  W->gB2 = take(B_J * hpe);
+  W->dinp = take(B_J * hpe);
+  // gA1 / gA2: encoder atom gradients over the joint rows, and before that the diff encoder's over the product rows
+  const size_t gA = A_J * hpe > A * hpd ? A_J * hpe : A * hpd;
+  W->gA1 = take(gA);
+  W->gA2 = take(gA);
+  W->gA3 = msg2 ? take(A * hpd) : nullptr;
+  W->dD = take(A * hpe);
+  W->dI2 = msg2 ? take(A * hpd) : nullptr;
   W->dvec = take(N * vp);
-  W->gN1 = take(N * hp);
-  W->gN2 = take(N * hp);
+  W->gN1 = take(N * hpf);
+  W->gN2 = take(N * hpf);
   W->dzout = take(N * RR_OUT_LD);
   W->det = nullptr;
   W->det_bytes = 0;
   if (deterministic()) {
-    const int A_J_ = static_cast<int>(A_J), B_J_ = static_cast<int>(B_J), A_ = static_cast<int>(A), N_ = static_cast<int>(N), hp_ = static_cast<int>(hp);
+    const int A_J_ = static_cast<int>(A_J), B_J_ = static_cast<int>(B_J), A_ = static_cast<int>(A), N_ = static_cast<int>(N);
+    const int he = static_cast<int>(hpe), hd = static_cast<int>(hpd);
     long long need = 0;
     auto at_least = [&](long long b) { need = b > need ? b : need; };
-    at_least(wgrad_det_bytes(B_J_, hp_, hp_));            // encoder W_h
-    at_least(wgrad_det_bytes(B_J_, hp_, RR_FB_LD));       // encoder W_i
-    at_least(wgrad_det_bytes(A_J_, hp_, hp_));            // encoder W_o (message part)
-    at_least(wgrad_det_bytes(A_J_, hp_, RR_FA_LD));       // encoder W_o (atom features)
-    at_least(wgrad_det_bytes(A_, hp_, hp_));              // diff encoder W_i, W_h, W_o
-    at_least(wgrad_det_bytes(A_, hp_, RR_FB_LD));         // diff encoder W_h (bond features)
+    at_least(wgrad_det_bytes(B_J_, he, he));              // encoder W_h
+    at_least(wgrad_det_bytes(B_J_, he, RR_FB_LD));        // encoder W_i
+    at_least(wgrad_det_bytes(A_J_, he, he));              // encoder W_o (message part)
+    at_least(wgrad_det_bytes(A_J_, he, RR_FA_LD));        // encoder W_o (atom features)
+    at_least(wgrad_det_bytes(A_, hd, he));                // diff encoder W_i, W_o (d part)
+    at_least(wgrad_det_bytes(A_, hd, hd));                // diff encoder W_h, W_o (message parts)
+    at_least(wgrad_det_bytes(A_, hd, RR_FB_LD));          // diff encoder W_h (bond features)
     for (int l = 0; l < c.ffn_depth; ++l) at_least(wgrad_det_bytes(N_, W->L.ffn_out[l], W->L.ffn_in[l]));
-    at_least(pad_parts_bytes(A_J_, r.n_segments + p.n_segments, hp_));   // gathers over the joint graph
-    at_least(pad_parts_bytes(A_, p.n_segments, hp_));                    // and over the product graph
+    at_least(pad_parts_bytes(A_J_, r.n_segments + p.n_segments, he));   // gathers over the joint graph
+    at_least(pad_parts_bytes(A_, p.n_segments, hd));                    // and over the product graph
     W->det = take(static_cast<size_t>((need + 3) / 4));
     W->det_bytes = (need + 3) / 4 * 4;
   }
@@ -376,11 +386,18 @@ static int carve(const rr_model_cfg& c, const rr_graph& r, const rr_graph& p, vo
 }
 
 // byte offset of a named forward buffer inside the workspace (tests compare per-layer activations with the oracle)
-long long model_buffer_offset(const rr_model_cfg* c, const rr_graph* r, const rr_graph* p, const char* name) {
+long long model_buffer_offset(const rr_model_cfg_ex* cx, const rr_graph* r, const rr_graph* p, const char* name) {
+  const rr_model_cfg* c = &cx->base;
   Workspace W;
   char* base = reinterpret_cast<char*>(static_cast<uintptr_t>(4096));
-  if (carve(*c, *r, *p, base, &W) != RR_OK) return -1;
-  auto off = [&](const float* ptr) { return static_cast<long long>(reinterpret_cast<const char*>(ptr) - base); };
+  if (carve(*cx, *r, *p, base, &W) != RR_OK) return -1;
+  auto off = [&](const float* ptr) -> long long {
+    if (ptr == nullptr) {
+      fail(RR_ERR_INVALID, "buffer %s does not exist at diff_depth %d", name, c->diff_depth);
+      return -1;
+    }
+    return static_cast<long long>(reinterpret_cast<const char*>(ptr) - base);
+  };
   char buf[64];
   for (int k = 0; k < 2; ++k) {
     snprintf(buf, sizeof(buf), "enc%d.inp", k);
@@ -417,22 +434,27 @@ long long model_buffer_offset(const rr_model_cfg* c, const rr_graph* r, const rr
   return -1;
 }
 
-long long model_workspace_bytes(const rr_model_cfg* c, const rr_graph* r, const rr_graph* p) {
+long long model_workspace_bytes(const rr_model_cfg_ex* c, const rr_graph* r, const rr_graph* p) {
   Workspace W;
   if (carve(*c, *r, *p, nullptr, &W) != RR_OK) return -1;
   return static_cast<long long>(W.bytes);
 }
 
-static int check_model_args(const rr_model_cfg* c, const rr_params* w, const rr_graph* r, const rr_graph* p, void* ws, long long ws_bytes, Workspace* W) {
-  RR_REQUIRE(c && w && r && p && ws, "model: NULL argument");
+static int check_model_args(const rr_model_cfg_ex* cx, const rr_params* w, const rr_graph* r, const rr_graph* p, void* ws, long long ws_bytes,
+                            Workspace* W) {
+  RR_REQUIRE(cx && w && r && p && ws, "model: NULL argument");
+  const rr_model_cfg* c = &cx->base;
   RR_REQUIRE(aligned16(ws), "workspace must be 16-byte aligned");
-  RR_TRY(carve(*c, *r, *p, ws, W));
+  RR_TRY(carve(*cx, *r, *p, ws, W));
   if (static_cast<long long>(W->bytes) > ws_bytes) return fail(RR_ERR_WORKSPACE, "workspace %lld bytes < required %zu", ws_bytes, W->bytes);
-  RR_REQUIRE(w->enc_Wi && w->enc_Wo && w->enc_bo && w->dif_Wi && w->dif_Wo && w->dif_bo, "model: missing parameter pointer");
+  RR_REQUIRE(w->enc_Wi && w->enc_Wo && w->enc_bo && w->dif_Wi, "model: missing parameter pointer");
   RR_REQUIRE(c->depth == 1 || w->enc_Wh, "model: encoder.W_h missing for depth > 1");
-  RR_REQUIRE(c->diff_depth == 1 || w->dif_Wh, "model: diff_encoder.W_h missing for diff_depth > 1");
+  RR_REQUIRE(c->diff_depth <= 1 || w->dif_Wh, "model: diff_encoder.W_h missing for diff_depth > 1");
+  RR_REQUIRE(c->diff_depth == 0 || (w->dif_Wo && w->dif_bo), "model: diff_encoder.W_o missing for diff_depth > 0");
   for (int l = 0; l < c->ffn_depth; ++l) RR_REQUIRE(w->ffn_W[l], "model: ffn weight %d missing", l);
   RR_REQUIRE(c->dropout >= 0.f && c->dropout < 1.f, "dropout must be in [0,1)");
+  RR_REQUIRE(cx->diff_dropout >= 0.f && cx->diff_dropout < 1.f, "diff_dropout must be in [0,1)");
+  RR_REQUIRE(cx->ffn_dropout >= 0.f && cx->ffn_dropout < 1.f, "ffn_dropout must be in [0,1)");
   RR_REQUIRE(r->f_bonds && r->f_atoms && p->f_bonds && p->f_atoms, "model: graph features missing");
   RR_REQUIRE(c->head >= RR_HEAD_RAW && c->head <= RR_HEAD_NIG, "unknown head %d", c->head);
   if (c->head == RR_HEAD_NIG) RR_REQUIRE((c->task_num & 3) == 0, "the NIG head needs task_num %% 4 == 0");
@@ -441,7 +463,7 @@ static int check_model_args(const rr_model_cfg* c, const rr_params* w, const rr_
   return RR_OK;
 }
 
-static int pack_params(const rr_model_cfg& c, const Workspace& W, const rr_params& w, cudaStream_t s) {
+static int pack_params(const rr_model_cfg_ex& c, const Workspace& W, const rr_params& w, cudaStream_t s) {
   RR_CUDA(cudaMemsetAsync(W.packed, 0, 3 * W.L.total * sizeof(float), s));   // the weights and their TF32 images
   RR_CUDA(cudaMemsetAsync(W.img.bf16_hi, 0, W.L.total * sizeof(uint16_t), s));
   RR_CUDA(cudaMemsetAsync(W.img.bf16_lo, 0, W.L.total * sizeof(uint16_t), s));
@@ -470,25 +492,30 @@ static int build_joint(const Workspace& W, const rr_graph& r, const rr_graph& p,
   return RR_OK;
 }
 
-int model_forward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* addf, float* scores,
+// Dropout: each sub-module's sites use its own p (encoder: m^t, hid; diff encoder: m2^t, hid2; FFN: vec, x[l]).  Philox stream ids, which
+// tests regenerate the masks from: sid starts at 1 and every lin() call takes the next one, with or without dropout, in launch order --
+// encoder W_i, W_h x (depth - 1), W_o; diff encoder W_i, W_h x (diff_depth - 1), W_o; then the readout (vec); then the FFN layers.  At
+// diff_depth 0 the diff encoder is W_i alone, and its id is the one that carries hid2's ReLU and dropout.
+int model_forward(const rr_model_cfg_ex* cx, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* addf, float* scores,
                   void* ws, long long ws_bytes, cudaStream_t s) {
   Workspace W;
-  RR_TRY(check_model_args(c, w, r, p, ws, ws_bytes, &W));
+  RR_TRY(check_model_args(cx, w, r, p, ws, ws_bytes, &W));
+  const rr_model_cfg* c = &cx->base;
   RR_REQUIRE(scores != nullptr, "scores is NULL");
   RR_REQUIRE(c->add_features == 0 || addf != nullptr, "add_features is NULL but add_features_dim = %d", c->add_features);
   const PackedLayout& L = W.L;
-  const int hp = L.hp, vp = L.vp;
+  const int hpe = L.hpe, hpd = L.hpd, vp = L.vp;
   const int T = c->depth - 1, Td = c->diff_depth - 1;
-  const float pdrop = c->training ? c->dropout : 0.f;
-  const int act = 1 | (pdrop > 0.f ? 2 : 0);
+  const float pe = c->training ? c->dropout : 0.f, pd = c->training ? cx->diff_dropout : 0.f, pf = c->training ? cx->ffn_dropout : 0.f;
+  const int act_e = 1 | (pe > 0.f ? 2 : 0), act_d = 1 | (pd > 0.f ? 2 : 0), act_f = 1 | (pf > 0.f ? 2 : 0);
   const float* P = W.packed;
   uint64_t sid = 1;
-  RR_TRY(pack_params(*c, W, *w, s));
+  RR_TRY(pack_params(*cx, W, *w, s));
 
-  // Y = act(X1 W1^T + X2 W2^T + bias + resid); pad_rows: the segment padding rows of Y (see linear_fwd)
+  // Y = act(X1 W1^T + X2 W2^T + bias + resid) with dropout p; resid has Y's row stride; pad_rows: the segment padding rows of Y (see linear_fwd)
   auto lin = [&](const int* pad_rows, int n_pad, int M, int n, const float* X1, int ldx1, size_t W1, int k1, const float* X2, int ldx2, size_t W2, int k2,
-                 size_t bias, const float* resid, float* Y, int ldy, int flags) -> int {
-    return linear_fwd(M, n, X1, ldx1, P + W1, k1, X2, ldx2, X2 ? P + W2 : nullptr, k2, P + bias, resid, hp, Y, ldy, flags, pdrop, c->seed, sid++, s,
+                 size_t bias, const float* resid, float* Y, int ldy, int flags, float pdrop) -> int {
+    return linear_fwd(M, n, X1, ldx1, P + W1, k1, X2, ldx2, X2 ? P + W2 : nullptr, k2, P + bias, resid, ldy, Y, ldy, flags, pdrop, c->seed, sid++, s,
                       &W.img, pad_rows, n_pad);
   };
   RR_TRY(build_joint(W, *r, *p, s));
@@ -496,38 +523,42 @@ int model_forward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r, 
     const rr_graph* g = &W.J;
     EncBufs& e = W.j;
     // f_bonds[pad] = 0: the padding rows of W_i's output are the bias exactly, on any GEMM path
-    RR_TRY(lin(nullptr, 0, g->n_bonds, hp, g->f_bonds, RR_FB_LD, L.enc_Wi, RR_FB_LD, nullptr, 0, 0, 0, L.enc_bi, nullptr, e.inp, hp, 0));
+    RR_TRY(lin(nullptr, 0, g->n_bonds, hpe, g->f_bonds, RR_FB_LD, L.enc_Wi, RR_FB_LD, nullptr, 0, 0, 0, L.enc_bi, nullptr, e.inp, hpe, 0, pe));
     const float* src = e.inp;
     int relu_src = 1;
     for (int t = 0; t < T; ++t) {
-      RR_TRY(bond_message_fwd(g, src, e.pre[t], hp, relu_src, s));
-      RR_TRY(lin(g->pad_bonds, g->n_segments, g->n_bonds, hp, e.pre[t], hp, L.enc_Wh, hp, nullptr, 0, 0, 0, L.enc_bh, e.inp, e.m[t + 1], hp, act));
+      RR_TRY(bond_message_fwd(g, src, e.pre[t], hpe, relu_src, s));
+      RR_TRY(lin(g->pad_bonds, g->n_segments, g->n_bonds, hpe, e.pre[t], hpe, L.enc_Wh, hpe, nullptr, 0, 0, 0, L.enc_bh, e.inp, e.m[t + 1], hpe, act_e, pe));
       src = e.m[t + 1];
       relu_src = 0;
     }
-    RR_TRY(neighbor_sum_fwd(g, 0, src, e.am, hp, relu_src, s));
-    RR_TRY(lin(g->pad_atoms, g->n_segments, g->n_atoms, hp, g->f_atoms, RR_FA_LD, L.enc_Wo_a, RR_FA_LD, e.am, hp, L.enc_Wo_m, hp, L.enc_bo, nullptr, e.hid, hp, act));
+    RR_TRY(neighbor_sum_fwd(g, 0, src, e.am, hpe, relu_src, s));
+    RR_TRY(lin(g->pad_atoms, g->n_segments, g->n_atoms, hpe, g->f_atoms, RR_FA_LD, L.enc_Wo_a, RR_FA_LD, e.am, hpe, L.enc_Wo_m, hpe, L.enc_bo, nullptr, e.hid,
+               hpe, act_e, pe));
   }
   const int A = p->n_atoms;
-  if (c->r_atom_map) RR_TRY(sub_gather(A, hp, W.enc[1].hid, W.enc[0].hid, c->r_atom_map, W.d, s));
-  else RR_TRY(sub(static_cast<long long>(A) * hp, W.enc[1].hid, W.enc[0].hid, W.d, s));  // base_model.py:168
+  if (c->r_atom_map) RR_TRY(sub_gather(A, hpe, W.enc[1].hid, W.enc[0].hid, c->r_atom_map, W.d, s));
+  else RR_TRY(sub(static_cast<long long>(A) * hpe, W.enc[1].hid, W.enc[0].hid, W.d, s));  // base_model.py:168
 
   // mpn.py:170-240 over the product graph
-  RR_TRY(lin(p->pad_atoms, p->n_segments, A, hp, W.d, hp, L.dif_Wi, hp, nullptr, 0, 0, 0, L.dif_bi, nullptr, W.inp2, hp, 0));
-  if (Td > 0) RR_TRY(neighbor_sum_fwd(p, 0, p->f_bonds, W.nf, RR_FB_LD, 0, s));
-  {
+  if (c->diff_depth == 0) {  // mpn.py:220-221: atom_hiddens = dropout(relu(W_i(diff)))
+    RR_TRY(lin(p->pad_atoms, p->n_segments, A, hpd, W.d, hpe, L.dif_Wi, hpe, nullptr, 0, 0, 0, L.dif_bi, nullptr, W.hid2, hpd, act_d, pd));
+  } else {
+    RR_TRY(lin(p->pad_atoms, p->n_segments, A, hpd, W.d, hpe, L.dif_Wi, hpe, nullptr, 0, 0, 0, L.dif_bi, nullptr, W.inp2, hpd, 0, pd));
+    if (Td > 0) RR_TRY(neighbor_sum_fwd(p, 0, p->f_bonds, W.nf, RR_FB_LD, 0, s));
     const float* src = W.inp2;
     int relu_src = 1;
     for (int t = 0; t < Td; ++t) {
-      RR_TRY(neighbor_sum_fwd(p, 1, src, W.nm[t], hp, relu_src, s));
-      RR_TRY(lin(p->pad_atoms, p->n_segments, A, hp, W.nm[t], hp, L.dif_Wh_m, hp, W.nf, RR_FB_LD, L.dif_Wh_f, RR_FB_LD, L.dif_bh, W.inp2, W.m2[t + 1], hp, act));
+      RR_TRY(neighbor_sum_fwd(p, 1, src, W.nm[t], hpd, relu_src, s));
+      RR_TRY(lin(p->pad_atoms, p->n_segments, A, hpd, W.nm[t], hpd, L.dif_Wh_m, hpd, W.nf, RR_FB_LD, L.dif_Wh_f, RR_FB_LD, L.dif_bh, W.inp2, W.m2[t + 1],
+                 hpd, act_d, pd));
       src = W.m2[t + 1];
       relu_src = 0;
     }
-    RR_TRY(neighbor_sum_fwd(p, 1, src, W.am2, hp, relu_src, s));
+    RR_TRY(neighbor_sum_fwd(p, 1, src, W.am2, hpd, relu_src, s));
+    RR_TRY(lin(p->pad_atoms, p->n_segments, A, hpd, W.d, hpe, L.dif_Wo_d, hpe, W.am2, hpd, L.dif_Wo_m, hpd, L.dif_bo, nullptr, W.hid2, hpd, act_d, pd));
   }
-  RR_TRY(lin(p->pad_atoms, p->n_segments, A, hp, W.d, hp, L.dif_Wo_d, hp, W.am2, hp, L.dif_Wo_m, hp, L.dif_bo, nullptr, W.hid2, hp, act));
-  RR_TRY(readout_fwd(p, W.hid2, hp, c->hidden, addf, c->add_features, W.vec, vp, pdrop, c->seed, sid++, s));
+  RR_TRY(readout_fwd(p, W.hid2, hpd, cx->diff_hidden, addf, c->add_features, W.vec, vp, pf, c->seed, sid++, s));
 
   // base_model.py:40-60
   const int N = p->n_mols;
@@ -536,7 +567,7 @@ int model_forward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r, 
   for (int l = 0; l < c->ffn_depth; ++l) {
     const bool last = (l == c->ffn_depth - 1);
     float* y = last ? W.zout : W.x[l];
-    RR_TRY(lin(nullptr, 0, N, L.ffn_out[l], x, ldx, L.ffn_W[l], L.ffn_in[l], nullptr, 0, 0, 0, L.ffn_b[l], nullptr, y, L.ffn_out[l], last ? 0 : act));
+    RR_TRY(lin(nullptr, 0, N, L.ffn_out[l], x, ldx, L.ffn_W[l], L.ffn_in[l], nullptr, 0, 0, 0, L.ffn_b[l], nullptr, y, L.ffn_out[l], last ? 0 : act_f, pf));
     x = y;
     ldx = L.ffn_out[l];
   }
@@ -548,18 +579,19 @@ int model_forward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r, 
   return RR_OK;
 }
 
-int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* dscores, rr_params* grads,
+int model_backward(const rr_model_cfg_ex* cx, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* dscores, rr_params* grads,
                    void* ws, long long ws_bytes, cudaStream_t s) {
   Workspace W;
-  RR_TRY(check_model_args(c, w, r, p, ws, ws_bytes, &W));
+  RR_TRY(check_model_args(cx, w, r, p, ws, ws_bytes, &W));
+  const rr_model_cfg* c = &cx->base;
   RR_REQUIRE(dscores && grads, "backward: NULL argument");
   if (deterministic() && c->r_atom_map)
     return fail(RR_ERR_UNSUPPORTED, "deterministic mode: the backward pass of de-duplicated reactants (r_atom_map) sums rows with atomics");
   const PackedLayout& L = W.L;
-  const int hp = L.hp, vp = L.vp;
+  const int hpe = L.hpe, hpd = L.hpd, hpf = L.hpf, vp = L.vp;
   const int T = c->depth - 1, Td = c->diff_depth - 1;
-  const float pdrop = c->training ? c->dropout : 0.f;
-  const float keep = pdrop > 0.f ? 1.f / (1.f - pdrop) : 1.f;
+  const float pe = c->training ? c->dropout : 0.f, pd = c->training ? cx->diff_dropout : 0.f, pf = c->training ? cx->ffn_dropout : 0.f;
+  const float keep_e = pe > 0.f ? 1.f / (1.f - pe) : 1.f, keep_d = pd > 0.f ? 1.f / (1.f - pd) : 1.f, keep_f = pf > 0.f ? 1.f / (1.f - pf) : 1.f;
   const float* P = W.packed;  // still holds this step's packed weights
   float* G = W.dpacked;
   RR_CUDA(cudaMemsetAsync(G, 0, L.grad_total * sizeof(float), s));
@@ -580,37 +612,43 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
       RR_TRY(linear_wgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, x, L.ffn_in[l], G + L.ffn_W[l], L.ffn_in[l], G + L.ffn_b[l], s, W.det, W.det_bytes));
       if (l > 0) {
         float* dx = scratch[l & 1];
-        RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], dx, hp, 0, W.img, s));
-        RR_TRY(relu_bwd(N, hp, dx, W.x[l - 1], keep, 0, dx, nullptr, 0, s));
+        RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], dx, hpf, 0, W.img, s));
+        RR_TRY(relu_bwd(N, hpf, dx, W.x[l - 1], keep_f, 0, dx, nullptr, 0, s));
         g = dx;
-        ldg = hp;
+        ldg = hpf;
       } else {
         RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], W.dvec, vp, 0, W.img, s));
       }
     }
   }
-  // readout + W_o of the diff encoder
-  RR_TRY(readout_bwd(p, W.dvec, vp, W.vec, W.hid2, W.gA1, hp, pdrop, s));
-  RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.d, hp, G + L.dif_Wo_d, hp, G + L.dif_bo, s, W.det, W.det_bytes));
-  RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.am2, hp, G + L.dif_Wo_m, hp, nullptr, s, W.det, W.det_bytes));
-  RR_TRY(linear_dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_d, hp, P + L.dif_Wo_d_T, hp, W.dD, hp, 0, W.img, s));
-  RR_TRY(linear_dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wo_m, hp, P + L.dif_Wo_m_T, hp, W.gA2, hp, 0, W.img, s));
-  // Every gather backward is followed by exactly one ReLU (+ dropout) backward: the mask of the message it produced the gradient of.
-  // Both run as one kernel (rr_mp_pipe.cu): t_next >= 1 -> mask of m2^{t_next}, result kept (gA1) and summed into dI2;
-  // t_next == 0 -> mask [inp2 > 0] of m2^0 = relu(inp2), only the sum into dI2 is wanted.
-  auto diff_nbr_bwd = [&](int t_next) {
-    if (t_next >= 1) return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA1, hp, W.m2[t_next], keep, 0, W.dI2, t_next == Td ? 1 : 2, 0, s, W.det, W.det_bytes);
-    return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA3, hp, W.inp2, 1.f, 1, W.dI2, Td == 0 ? 1 : 2, 1, s, W.det, W.det_bytes);
-  };
-  RR_TRY(diff_nbr_bwd(Td));
-  for (int t = Td; t >= 1; --t) {
-    RR_TRY(linear_wgrad(A, hp, hp, W.gA1, hp, W.nm[t - 1], hp, G + L.dif_Wh_m, hp, G + L.dif_bh, s, W.det, W.det_bytes));
-    RR_TRY(linear_wgrad(A, hp, RR_FB_LD, W.gA1, hp, W.nf, RR_FB_LD, G + L.dif_Wh_f, RR_FB_LD, nullptr, s, W.det, W.det_bytes));
-    RR_TRY(linear_dgrad(A, hp, hp, W.gA1, hp, P + L.dif_Wh_m, hp, P + L.dif_Wh_m_T, hp, W.gA2, hp, 0, W.img, s));
-    RR_TRY(diff_nbr_bwd(t - 1));
+  // readout: the gradient of the diff encoder's last layer (W_o, or W_i at diff_depth 0) through hid2's ReLU / dropout mask
+  RR_TRY(readout_bwd(p, W.dvec, vp, W.vec, W.hid2, W.gA1, hpd, pf, pd, s));
+  const float* dWi = W.gA1;   // gradient of W_i's output
+  if (c->diff_depth > 0) {
+    RR_TRY(linear_wgrad(A, hpd, hpe, W.gA1, hpd, W.d, hpe, G + L.dif_Wo_d, hpe, G + L.dif_bo, s, W.det, W.det_bytes));
+    RR_TRY(linear_wgrad(A, hpd, hpd, W.gA1, hpd, W.am2, hpd, G + L.dif_Wo_m, hpd, nullptr, s, W.det, W.det_bytes));
+    RR_TRY(linear_dgrad(A, hpd, hpe, W.gA1, hpd, P + L.dif_Wo_d, hpe, P + L.dif_Wo_d_T, hpd, W.dD, hpe, 0, W.img, s));
+    RR_TRY(linear_dgrad(A, hpd, hpd, W.gA1, hpd, P + L.dif_Wo_m, hpd, P + L.dif_Wo_m_T, hpd, W.gA2, hpd, 0, W.img, s));
+    // Every gather backward is followed by exactly one ReLU (+ dropout) backward: the mask of the message it produced the gradient of.
+    // Both run as one kernel (rr_mp_pipe.cu): t_next >= 1 -> mask of m2^{t_next}, result kept (gA1) and summed into dI2;
+    // t_next == 0 -> mask [inp2 > 0] of m2^0 = relu(inp2), only the sum into dI2 is wanted.
+    auto diff_nbr_bwd = [&](int t_next) {
+      if (t_next >= 1)
+        return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA1, hpd, W.m2[t_next], keep_d, 0, W.dI2, t_next == Td ? 1 : 2, 0, s, W.det, W.det_bytes);
+      return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA3, hpd, W.inp2, 1.f, 1, W.dI2, Td == 0 ? 1 : 2, 1, s, W.det, W.det_bytes);
+    };
+    RR_TRY(diff_nbr_bwd(Td));
+    for (int t = Td; t >= 1; --t) {
+      RR_TRY(linear_wgrad(A, hpd, hpd, W.gA1, hpd, W.nm[t - 1], hpd, G + L.dif_Wh_m, hpd, G + L.dif_bh, s, W.det, W.det_bytes));
+      RR_TRY(linear_wgrad(A, hpd, RR_FB_LD, W.gA1, hpd, W.nf, RR_FB_LD, G + L.dif_Wh_f, RR_FB_LD, nullptr, s, W.det, W.det_bytes));
+      RR_TRY(linear_dgrad(A, hpd, hpd, W.gA1, hpd, P + L.dif_Wh_m, hpd, P + L.dif_Wh_m_T, hpd, W.gA2, hpd, 0, W.img, s));
+      RR_TRY(diff_nbr_bwd(t - 1));
+    }
+    dWi = W.dI2;
   }
-  RR_TRY(linear_wgrad(A, hp, hp, W.dI2, hp, W.d, hp, G + L.dif_Wi, hp, G + L.dif_bi, s, W.det, W.det_bytes));
-  RR_TRY(linear_dgrad(A, hp, hp, W.dI2, hp, P + L.dif_Wi, hp, P + L.dif_Wi_T, hp, W.dD, hp, 1, W.img, s));
+  RR_TRY(linear_wgrad(A, hpd, hpe, dWi, hpd, W.d, hpe, G + L.dif_Wi, hpe, G + L.dif_bi, s, W.det, W.det_bytes));
+  // accumulates onto W_o's share of dD; at diff_depth 0 it is the only share
+  RR_TRY(linear_dgrad(A, hpd, hpe, dWi, hpd, P + L.dif_Wi, hpe, P + L.dif_Wi_T, hpd, W.dD, hpe, c->diff_depth > 0 ? 1 : 0, W.img, s));
 
   // shared encoder, once over [reactant rows | product rows]: d(hid_p) = +dD, d(hid_r) = -dD (base_model.py:168), each through the
   // ReLU / dropout mask of its own rows; the weight gradients of both halves come out of one launch per layer (base_model.py:155-156)
@@ -619,30 +657,30 @@ int model_backward(const rr_model_cfg* c, const rr_params* w, const rr_graph* r,
     const rr_graph* g = &W.J;
     EncBufs& e = W.j;
     const int A_r = r->n_atoms, A_J = g->n_atoms, B_J = g->n_bonds;
-    float* gA1_p = W.gA1 + static_cast<size_t>(A_r) * hp;
-    RR_TRY(relu_bwd(A, hp, W.dD, W.enc[1].hid, keep, 0, gA1_p, nullptr, 0, s));
+    float* gA1_p = W.gA1 + static_cast<size_t>(A_r) * hpe;
+    RR_TRY(relu_bwd(A, hpe, W.dD, W.enc[1].hid, keep_e, 0, gA1_p, nullptr, 0, s));
     if (c->r_atom_map) {   // shared reactant rows: sum the gradient over the copies first (gA2 is free until the dgrad below)
-      RR_CUDA(cudaMemsetAsync(W.gA2, 0, static_cast<size_t>(A_r) * hp * sizeof(float), s));
-      RR_TRY(scatter_add_rows(A, hp, W.dD, c->r_atom_map, W.gA2, s));
-      RR_TRY(relu_bwd(A_r, hp, W.gA2, W.enc[0].hid, -keep, 0, W.gA1, nullptr, 0, s));
+      RR_CUDA(cudaMemsetAsync(W.gA2, 0, static_cast<size_t>(A_r) * hpe * sizeof(float), s));
+      RR_TRY(scatter_add_rows(A, hpe, W.dD, c->r_atom_map, W.gA2, s));
+      RR_TRY(relu_bwd(A_r, hpe, W.gA2, W.enc[0].hid, -keep_e, 0, W.gA1, nullptr, 0, s));
     } else {
-      RR_TRY(relu_bwd(A_r, hp, W.dD, W.enc[0].hid, -keep, 0, W.gA1, nullptr, 0, s));
+      RR_TRY(relu_bwd(A_r, hpe, W.dD, W.enc[0].hid, -keep_e, 0, W.gA1, nullptr, 0, s));
     }
-    RR_TRY(linear_wgrad(A_J, hp, RR_FA_LD, W.gA1, hp, g->f_atoms, RR_FA_LD, G + L.enc_Wo_a, RR_FA_LD, G + L.enc_bo, s, W.det, W.det_bytes));
-    RR_TRY(linear_wgrad(A_J, hp, hp, W.gA1, hp, e.am, hp, G + L.enc_Wo_m, hp, nullptr, s, W.det, W.det_bytes));
-    RR_TRY(linear_dgrad(A_J, hp, hp, W.gA1, hp, P + L.enc_Wo_m, hp, P + L.enc_Wo_m_T, hp, W.gA2, hp, 0, W.img, s));
-    if (T >= 1) RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.m[T], keep, 0, W.dinp, 1, 0, s, W.det, W.det_bytes));
-    else RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 1, 1, s, W.det, W.det_bytes));
+    RR_TRY(linear_wgrad(A_J, hpe, RR_FA_LD, W.gA1, hpe, g->f_atoms, RR_FA_LD, G + L.enc_Wo_a, RR_FA_LD, G + L.enc_bo, s, W.det, W.det_bytes));
+    RR_TRY(linear_wgrad(A_J, hpe, hpe, W.gA1, hpe, e.am, hpe, G + L.enc_Wo_m, hpe, nullptr, s, W.det, W.det_bytes));
+    RR_TRY(linear_dgrad(A_J, hpe, hpe, W.gA1, hpe, P + L.enc_Wo_m, hpe, P + L.enc_Wo_m_T, hpe, W.gA2, hpe, 0, W.img, s));
+    if (T >= 1) RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hpe, e.m[T], keep_e, 0, W.dinp, 1, 0, s, W.det, W.det_bytes));
+    else RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hpe, e.inp, 1.f, 1, W.dinp, 1, 1, s, W.det, W.det_bytes));
     for (int t = T; t >= 1; --t) {
-      RR_TRY(linear_wgrad(B_J, hp, hp, W.gB1, hp, e.pre[t - 1], hp, G + L.enc_Wh, hp, G + L.enc_bh, s, W.det, W.det_bytes));
-      RR_TRY(linear_dgrad(B_J, hp, hp, W.gB1, hp, P + L.enc_Wh, hp, P + L.enc_Wh_T, hp, W.gB2, hp, 0, W.img, s));
-      if (t - 1 >= 1) RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.m[t - 1], keep, 0, W.dinp, 2, 0, s, W.det, W.det_bytes));
-      else RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hp, e.inp, 1.f, 1, W.dinp, 2, 1, s, W.det, W.det_bytes));
+      RR_TRY(linear_wgrad(B_J, hpe, hpe, W.gB1, hpe, e.pre[t - 1], hpe, G + L.enc_Wh, hpe, G + L.enc_bh, s, W.det, W.det_bytes));
+      RR_TRY(linear_dgrad(B_J, hpe, hpe, W.gB1, hpe, P + L.enc_Wh, hpe, P + L.enc_Wh_T, hpe, W.gB2, hpe, 0, W.img, s));
+      if (t - 1 >= 1) RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hpe, e.m[t - 1], keep_e, 0, W.dinp, 2, 0, s, W.det, W.det_bytes));
+      else RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hpe, e.inp, 1.f, 1, W.dinp, 2, 1, s, W.det, W.det_bytes));
     }
-    RR_TRY(linear_wgrad(B_J, hp, RR_FB_LD, W.dinp, hp, g->f_bonds, RR_FB_LD, G + L.enc_Wi, RR_FB_LD, G + L.enc_bi, s, W.det, W.det_bytes));
+    RR_TRY(linear_wgrad(B_J, hpe, RR_FB_LD, W.dinp, hpe, g->f_bonds, RR_FB_LD, G + L.enc_Wi, RR_FB_LD, G + L.enc_bi, s, W.det, W.det_bytes));
   }
 
-  PackTable Tb = make_table(*c, L, *grads, false);
+  PackTable Tb = make_table(*cx, L, *grads, false);
   k_pack<<<dim3(32, Tb.n), 256, 0, s>>>(Tb, G, 1, 0, 0, nullptr, nullptr);
   RR_LAUNCH_CHECK("k_pack(grads)");
   return RR_OK;

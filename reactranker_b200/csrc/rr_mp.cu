@@ -308,9 +308,9 @@ __global__ void k_readout_fwd(rr_graph g, const float* __restrict__ hid, int hp,
   }
 }
 
-// dz[a] = dvec[mol]/size * [vec != 0]*keep_scale * [hid[a] != 0]*keep_scale  (relu + both dropouts)
+// dz[a] = dvec[mol]/size * [vec != 0]*keep_vec * [hid[a] != 0]*keep_hid  (relu + both dropouts: the FFN's on vec, the diff encoder's on hid)
 __global__ void k_readout_bwd(rr_graph g, const float* __restrict__ dvec, int vp, const float* __restrict__ vec, const float* __restrict__ hid,
-                              float* __restrict__ dz, int hp, float inv_keep) {
+                              float* __restrict__ dz, int hp, float keep_vec, float keep_hid) {
   const int cpr = hp >> 2;
   const long long total = static_cast<long long>(g.n_mols) * cpr;
   for (long long t = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; t < total; t += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -321,15 +321,15 @@ __global__ void k_readout_bwd(rr_graph g, const float* __restrict__ dvec, int vp
     float4 d = f4_zero();
     if (c4 < vp) {
       d = ld_f4(dvec + static_cast<size_t>(i) * vp + c4);
-      if (inv_keep != 1.f) {  // the FFN's first dropout acted on vec
+      if (keep_vec != 1.f) {  // the FFN's first dropout acted on vec
         const float4 y = ld_f4(vec + static_cast<size_t>(i) * vp + c4);
-        d.x = y.x != 0.f ? d.x * inv_keep : 0.f;
-        d.y = y.y != 0.f ? d.y * inv_keep : 0.f;
-        d.z = y.z != 0.f ? d.z * inv_keep : 0.f;
-        d.w = y.w != 0.f ? d.w * inv_keep : 0.f;
+        d.x = y.x != 0.f ? d.x * keep_vec : 0.f;
+        d.y = y.y != 0.f ? d.y * keep_vec : 0.f;
+        d.z = y.z != 0.f ? d.z * keep_vec : 0.f;
+        d.w = y.w != 0.f ? d.w * keep_vec : 0.f;
       }
     }
-    const float s = inv_keep / static_cast<float>(size);
+    const float s = keep_hid / static_cast<float>(size);
     d = f4_scale(s, d);
     for (int a = start; a < start + size; ++a) {
       const float4 h = ld_f4(hid + static_cast<size_t>(a) * hp + c4);
@@ -589,7 +589,8 @@ int readout_fwd(const rr_graph* g, const float* hid, int hp, int hidden, const f
   return RR_OK;
 }
 
-int readout_bwd(const rr_graph* g, const float* dvec, int vp, const float* vec, const float* hid, float* dz, int hp, float p, cudaStream_t s) {
+int readout_bwd(const rr_graph* g, const float* dvec, int vp, const float* vec, const float* hid, float* dz, int hp, float p_vec, float p_hid,
+                cudaStream_t s) {
   ProfScope prof_scope(KC_READOUT, s);
   RR_REQUIRE(g && g->n_mols > 0 && g->mol_start && g->mol_size && g->pad_atoms, "graph has no molecule scope");
   RR_REQUIRE((hp & 3) == 0 && (vp & 3) == 0 && vp >= hp, "readout_bwd needs vp >= hp (vp %d hp %d)", vp, hp);
@@ -597,7 +598,8 @@ int readout_bwd(const rr_graph* g, const float* dvec, int vp, const float* vec, 
   const long long total = static_cast<long long>(g->n_mols) * (hp >> 2);
   int blocks = static_cast<int>((total + 255) / 256);
   if (blocks > num_sms() * 8) blocks = num_sms() * 8;
-  k_readout_bwd<<<blocks, 256, 0, s>>>(*g, dvec, vp, vec, hid, dz, hp, p > 0.f ? 1.f / (1.f - p) : 1.f);
+  k_readout_bwd<<<blocks, 256, 0, s>>>(*g, dvec, vp, vec, hid, dz, hp, p_vec > 0.f ? 1.f / (1.f - p_vec) : 1.f,
+                                       p_hid > 0.f ? 1.f / (1.f - p_hid) : 1.f);
   RR_LAUNCH_CHECK("k_readout_bwd");
   return RR_OK;
 }

@@ -65,7 +65,7 @@ def reactant_dedup_exact(model) -> bool:
     that rr_model_backward forms with atomics, so the deterministic backward refuses it."""
     if not getattr(model, "dedup_reactants", False):
         return False
-    if model.training and getattr(model, "_dropout", 0) > 0:
+    if model.training and model.any_dropout():
         return False
     return not _lib.deterministic_requested() or (not model.training and not torch.is_grad_enabled())
 
@@ -109,18 +109,18 @@ class _ReactionFn(torch.autograd.Function):
         cfg = model._cfg(training=model.training)
         amap = getattr(rg, "atom_map", None)
         if amap is not None:
-            if model.training and model._dropout > 0:
+            if model.training and model.any_dropout():
                 raise _lib.RRError("de-duplicated reactants are exact only without dropout (eval mode or dropout = 0)")
             cfg.r_atom_map = amap.data_ptr()
         w = model._param_struct(params)
-        ws_bytes = L.rr_model_workspace_bytes(ctypes.byref(cfg), ctypes.byref(rg.c), ctypes.byref(pg.c))
+        ws_bytes = L.rr_model_workspace_bytes_ex(ctypes.byref(cfg), ctypes.byref(rg.c), ctypes.byref(pg.c))
         if ws_bytes < 0:
             _lib.check(-1)
         dev = params[0].device
         ws = model._ws_pool.take(int(ws_bytes), dev)
         n = pg.n_mols
         scores = torch.empty((n,) if cfg.task_num == 1 else (n, cfg.task_num), dtype=torch.float32, device=dev)
-        _lib.check(L.rr_model_forward(ctypes.byref(cfg), ctypes.byref(w), ctypes.byref(rg.c), ctypes.byref(pg.c),
+        _lib.check(L.rr_model_forward_ex(ctypes.byref(cfg), ctypes.byref(w), ctypes.byref(rg.c), ctypes.byref(pg.c),
                                       _lib.ptr(addf), scores.data_ptr(), ws.data_ptr(), ws.numel(), _lib.stream_ptr()))
         if not any(ctx.needs_input_grad):        # inference: nothing will come back for the activations
             model._ws_pool.give(ws)
@@ -149,7 +149,7 @@ class _ReactionFn(torch.autograd.Function):
         gw = model._param_struct(grads)
         dscores = dscores.contiguous().float()
         _lib.set_deterministic(ctx.det)
-        _lib.check(L.rr_model_backward(ctypes.byref(ctx.cfg), ctypes.byref(w), ctypes.byref(ctx.rg.c), ctypes.byref(ctx.pg.c),
+        _lib.check(L.rr_model_backward_ex(ctypes.byref(ctx.cfg), ctypes.byref(w), ctypes.byref(ctx.rg.c), ctypes.byref(ctx.pg.c),
                                        dscores.data_ptr(), ctypes.byref(gw), ctx.ws.data_ptr(), ctx.ws.numel(), _lib.stream_ptr()))
         model._ws_pool.give(ctx.ws)
         ctx.ws = None
@@ -165,10 +165,6 @@ class ReactionModel(nn.Module):
                  ffn_hidden_size: int = 300, ffn_bias: bool = True, ffn_dropout=0.2, ffn_depth: int = 3, task_num: int = 2,
                  task_type: str = 'no_softplus', addtion_react_featrues: int = 0):
         super().__init__()
-        if not (mpnn_hidden_size == mpnn_diff_hidden_size == ffn_hidden_size):
-            raise NotImplementedError("build_model ties all hidden sizes (base_model.py:266-280); unequal sizes are not built")
-        if not (mpnn_dropout == mpnn_diff_dropout == ffn_dropout) or not (mpnn_bias == mpnn_diff_bias == ffn_bias):
-            raise NotImplementedError("build_model ties dropout and bias across sub-modules; mixed settings are not built")
         if task_type in _UNBUILT_HEADS:
             raise NotImplementedError(f"FFN head '{task_type}' is outside the five north-star task keys")
         self.encoder = MPN(bond_fdim=ATOM_FDIM + BOND_FDIM, atom_fdim=ATOM_FDIM, MPN_hidden_size=mpnn_hidden_size, MPN_bias=mpnn_bias,
@@ -177,8 +173,10 @@ class ReactionModel(nn.Module):
                                     MPNDiff_bias=mpnn_diff_bias, MPNDiff_depth=mpnn_diff_depth, MPNDiff_dropout=mpnn_diff_dropout)
         self.ffn = FFN(reacvec_fdim=mpnn_diff_hidden_size + addtion_react_featrues, ffn_hidden_size=ffn_hidden_size,
                        ffn_dropout=ffn_dropout, ffn_num_layers=ffn_depth, task_num=task_num, ffn_bias=ffn_bias, task_type=task_type)
-        self._hidden, self._depth, self._diff_depth, self._ffn_depth = mpnn_hidden_size, mpnn_depth, mpnn_diff_depth, ffn_depth
-        self._task_num, self._add, self._dropout = task_num, addtion_react_featrues, float(mpnn_dropout)
+        self._he, self._hd, self._hf = mpnn_hidden_size, mpnn_diff_hidden_size, ffn_hidden_size
+        self._pe, self._pd, self._pf = float(mpnn_dropout), float(mpnn_diff_dropout), float(ffn_dropout)
+        self._depth, self._diff_depth, self._ffn_depth = mpnn_depth, mpnn_diff_depth, ffn_depth
+        self._task_num, self._add = task_num, addtion_react_featrues
         self._head = _HEADS.get(task_type, _lib.HEAD_RAW)     # every other name returns the raw output (base_model.py:105-106)
         self.last_h2d_bytes = 0
         self.dedup_reactants = True      # encode repeated reactants once whenever that is exact (eval mode, dropout 0)
@@ -193,7 +191,7 @@ class ReactionModel(nn.Module):
                  ("enc_Wo", e.W_o.weight), ("enc_bo", e.W_o.bias),
                  ("dif_Wi", d.W_i.weight), ("dif_bi", d.W_i.bias),
                  ("dif_Wh", getattr(d, "W_h", None) and d.W_h.weight), ("dif_bh", getattr(d, "W_h", None) and d.W_h.bias),
-                 ("dif_Wo", d.W_o.weight), ("dif_bo", d.W_o.bias)]
+                 ("dif_Wo", getattr(d, "W_o", None) and d.W_o.weight), ("dif_bo", getattr(d, "W_o", None) and d.W_o.bias)]
         for i, lin in enumerate(self.ffn.linears()):
             slots += [(("ffn_W", i), lin.weight), (("ffn_b", i), lin.bias)]
         return [(k, v) for k, v in slots if v is not None]
@@ -207,12 +205,16 @@ class ReactionModel(nn.Module):
                 setattr(s, slot, t.data_ptr())
         return s
 
-    def _cfg(self, training: bool) -> _lib.RRModelCfg:
+    def any_dropout(self) -> bool:
+        return max(self._pe, self._pd, self._pf) > 0
+
+    def _cfg(self, training: bool) -> _lib.RRModelCfgEx:
         seed = 0
-        if training and self._dropout > 0:
+        if training and self.any_dropout():
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())        # follows torch.manual_seed
-        return _lib.RRModelCfg(self._hidden, self._depth, self._diff_depth, self._ffn_depth, self._task_num, self._add,
-                               self._head, int(training), self._dropout, seed)
+        base = _lib.RRModelCfg(self._he, self._depth, self._diff_depth, self._ffn_depth, self._task_num, self._add,
+                               self._head, int(training), self._pe, seed)
+        return _lib.RRModelCfgEx(base, self._hd, self._hf, self._pd, self._pf)
 
     def hot_parameters(self):
         """The trainable parameters in the order of the flat gradient buffer."""
@@ -222,7 +224,7 @@ class ReactionModel(nn.Module):
         """A forward activation kept in the workspace of the autograd node behind ``out`` (per-layer parity tests):
         see rr_model_buffer_offset for the names."""
         node = out.grad_fn
-        off = _lib.lib().rr_model_buffer_offset(ctypes.byref(node.cfg), ctypes.byref(node.rg.c), ctypes.byref(node.pg.c), name.encode())
+        off = _lib.lib().rr_model_buffer_offset_ex(ctypes.byref(node.cfg), ctypes.byref(node.rg.c), ctypes.byref(node.pg.c), name.encode())
         if off < 0:
             _lib.check(-1)
         return node.ws[off:off + rows * cols * 4].view(torch.float32).reshape(rows, cols)
