@@ -309,6 +309,22 @@ int rr_loss_max_group(void);
 int rr_rank_metrics(int N, int G, const float* scores, int score_ld, const double* targets, const int32_t* seg_off, int max_group,
                     double ratio, double* out, void* stream);
 
+/* Per-item ranking statistics of a prediction pass (reactranker_b200/predict.py) over T samples of the scores: T = 1 for one eval-mode
+   forward, T > 1 for MC dropout (one train-mode forward per sample).  No targets: one CTA per group, nothing but the table comes back.
+     scores  fp32, item i of sample t at scores[t * sample_stride + i * score_ld] (score_ld = task_num picks column 0 of [N, task] outputs)
+     seg_off [G + 1], max_group <= rr_loss_max_group() = 8192, T >= 1
+   out [N, RR_PREDICT_COLS] fp32, one row per item:
+     0 mean of the score over the samples | 1 its standard deviation, population form (ddof 0; 0 when T = 1) | 2 1-based rank of column 0
+     within the group | 3 mean over samples of the within-group softmax (ListNet / Plackett-Luce probability of ranking first) | 4 fraction
+     of samples in which the item ranks first | 5 mean over samples of the item's rank.
+   Ranks are the stable descending order of k_rank_metrics (rank(i) = 1 + #{j : x_j > x_i} + #{j < i : x_j == x_i}); column 2 ranks the
+   fp32 value of column 0, so it is the stable order of the returned means.  The softmax is shifted by the group maximum and every sum is
+   taken in double without atomics: a repeated call is bit-identical.  An empty group writes nothing; a group larger than max_group gets
+   NaN in all of its rows. */
+#define RR_PREDICT_COLS 6
+int rr_rank_predict(int N, int G, int T, const float* scores, int64_t sample_stride, int score_ld, const int32_t* seg_off, int max_group,
+                    float* out, void* stream);
+
 /* ---- whole model (models/base_model.py:150-171) ---------------------------------------- */
 /* bytes of workspace rr_model_forward/backward need for these sizes */
 int64_t rr_model_workspace_bytes(const rr_model_cfg* cfg, const rr_graph* r, const rr_graph* p);

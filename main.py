@@ -42,6 +42,13 @@ _MODEL_FOR_TASK = {
 }
 
 
+def make_model(task_type, hidden_size, depth, dropout):
+    """The ReactionModel main.py trains for ``task_type`` (predict.py rebuilds it to load a checkpoint)."""
+    task_num, model_task, last_layer = _MODEL_FOR_TASK.get(task_type, (1, None, 'with_softplus'))
+    return build_model(hidden_size=hidden_size, mpnn_depth=depth, mpnn_diff_depth=depth, ffn_depth=3, use_bias=True, dropout=dropout,
+                       task_num=task_num, ffn_last_layer=last_layer, task_type=model_task, add_features_dim=1)
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--path", default="runs/reactranker", help="save path (checkpoints, output.log)")
@@ -115,7 +122,6 @@ def main():
     split_strategy = a.split_strategy
     init_lr, max_lr, final_lr = a.init_lr, a.max_lr, a.final_lr
     save_metric = a.save_metric
-    add_features_dim = 1
     add_features_name = 'temp'
     logger.info('Task type is: {}, and target name is: {}'.format(task_type, target_name))
     logger.info('{} fold train with {} epochs every fold. The batch size is: {}'.format(k_fold, total_epochs, batch_size))
@@ -127,8 +133,8 @@ def main():
             os.makedirs(p, exist_ok=True)
     # evidential_ranking / gauss_regression need two outputs; main.py's default build (task_num=1, task_type commented out,
     # main.py:114-123) serves mle / listnet / regression
-    # The experimental keys need the head their loss reads (base_model.py:252-264 resolves task_num / task_type / ffn_last_layer to it).
-    task_num, model_task, last_layer = _MODEL_FOR_TASK.get(task_type, (1, None, 'with_softplus'))
+    # The experimental keys need the head their loss reads (base_model.py:252-264 resolves task_num / task_type / ffn_last_layer to it):
+    # make_model looks it up in _MODEL_FOR_TASK.
     for ii in range(k_fold):
         print('**********************************')
         print('**   This is the fold [{}/{}]   **'.format(ii + 1, k_fold))
@@ -148,8 +154,7 @@ def main():
         torch.manual_seed(seed)
         torch.cuda.manual_seed(seed)
         torch.cuda.manual_seed_all(seed)
-        model = build_model(hidden_size=a.hidden_size, mpnn_depth=a.depth, mpnn_diff_depth=a.depth, ffn_depth=3, use_bias=True, dropout=a.dropout,
-                            task_num=task_num, ffn_last_layer=last_layer, task_type=model_task, add_features_dim=add_features_dim)
+        model = make_model(task_type, a.hidden_size, a.depth, a.dropout)
         logger.info('Model Structure')
         logger.info(model)
         torch.cuda.set_device(gpu)

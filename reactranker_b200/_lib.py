@@ -56,7 +56,7 @@ EXPORTS = [
     "rr_version", "rr_last_error", "rr_device_check", "rr_padded",
     "rr_graph_assemble", "rr_batch_build", "rr_bond_message_fwd", "rr_bond_message_bwd", "rr_neighbor_sum_fwd", "rr_neighbor_sum_bwd",
     "rr_bond_message_bwd_act", "rr_neighbor_sum_bwd_act", "rr_readout_fwd", "rr_readout_bwd", "rr_linear_fwd", "rr_linear_dgrad", "rr_linear_dgrad_tc", "rr_linear_dgrad_tc_scratch_bytes", "rr_linear_wgrad", "rr_relu_bwd", "rr_sub",
-    "rr_loss_fwdbwd", "rr_loss_fwdbwd_ex", "rr_loss_max_group", "rr_rank_metrics",
+    "rr_loss_fwdbwd", "rr_loss_fwdbwd_ex", "rr_loss_max_group", "rr_rank_metrics", "rr_rank_predict",
     "rr_model_workspace_bytes", "rr_model_buffer_offset", "rr_model_forward", "rr_model_backward", "rr_model_workspace_bytes_ex",
     "rr_model_buffer_offset_ex", "rr_model_forward_ex", "rr_model_backward_ex", "rr_launch_count", "rr_launch_count_reset",
     "rr_profile_begin", "rr_profile_end", "rr_profile_classes", "rr_set_gemm_mode", "rr_get_gemm_mode", "rr_set_backward_bf16", "rr_get_backward_bf16",
@@ -152,6 +152,7 @@ def lib() -> ctypes.CDLL:
                 L.rr_loss_fwdbwd.argtypes = [i32, i32, i32, vp, vp, vp, f32, f32, vp, vp, vp]
                 L.rr_loss_fwdbwd_ex.argtypes = [i32, i32, i32, vp, vp, vp, i32, f32, f32, vp, vp, vp]
                 L.rr_rank_metrics.argtypes = [i32, i32, vp, i32, vp, vp, i32, ctypes.c_double, vp, vp]
+                L.rr_rank_predict.argtypes = [i32, i32, i32, vp, i64, i32, vp, i32, vp, vp]
                 L.rr_model_workspace_bytes.argtypes = [vp, vp, vp]
                 L.rr_model_buffer_offset.argtypes = [vp, vp, vp, ctypes.c_char_p]
                 L.rr_model_buffer_offset.restype = ctypes.c_int64

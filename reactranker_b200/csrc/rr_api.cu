@@ -146,6 +146,10 @@ int rr_rank_metrics(int N, int G, const float* scores, int score_ld, const doubl
                     double* out, void* stream) {
   return rr::rank_metrics(N, G, scores, score_ld, targets, seg_off, max_group, ratio, out, S(stream));
 }
+int rr_rank_predict(int N, int G, int T, const float* scores, int64_t sample_stride, int score_ld, const int32_t* seg_off, int max_group,
+                    float* out, void* stream) {
+  return rr::rank_predict(N, G, T, scores, sample_stride, score_ld, seg_off, max_group, out, S(stream));
+}
 
 int64_t rr_model_workspace_bytes_ex(const rr_model_cfg_ex* cfg, const rr_graph* r, const rr_graph* p) {
   if (!cfg || !r || !p) {

@@ -285,6 +285,7 @@ int scatter_add_rows(long long rows, int ld, const float* src, const int* map, f
 int loss_fwdbwd(int, int, int, const float*, const float*, const int*, float, float, float*, float*, cudaStream_t, int max_group = 0);
 int loss_max_group();
 int rank_metrics(int, int, const float*, int, const double*, const int*, int, double, double*, cudaStream_t);
+int rank_predict(int, int, int, const float*, long long, int, const int*, int, float*, cudaStream_t);
 int graph_assemble(const rr_mol_store*, int, const int*, const int*, const int*, const int*, const int*, const int*, int, const int*, const int*,
                    const int*, const rr_graph*, cudaStream_t);
 long long model_workspace_bytes(const rr_model_cfg_ex*, const rr_graph*, const rr_graph*);

@@ -743,4 +743,127 @@ int rank_metrics(int N, int G, const float* scores, int score_ld, const double* 
   return RR_OK;
 }
 
+// ---------------------------------------------------------------------------------------
+// Prediction: per-item ranking statistics over T score samples (MC dropout; T = 1 for one deterministic pass), one CTA per group.
+// Ranks use the rule of k_rank_metrics, 1-based:  rank(i) = 1 + #{j : x_j > x_i} + #{j < i : x_j == x_i}.
+// Sample t of the group is staged in shared memory (n floats: the comparisons and the max are exact on floats), the within-group
+// softmax is shifted by the group maximum and taken in double.  The group's n = 8192 items cannot keep five double accumulators each
+// on chip, so the items are taken in passes of kPredictItems * blockDim.x: in a pass every thread owns kPredictItems items and keeps
+// their accumulators in registers across the whole T loop; a later pass streams the T samples again.  Sums are in double, the reductions
+// are the fixed block_sum_d tree and nothing is atomic, so a repeated call is bit-identical.
+// ---------------------------------------------------------------------------------------
+constexpr int kPredictItems = 4;
+
+__global__ void __launch_bounds__(kLossThreads) k_rank_predict(int T, const float* __restrict__ scores, long long sample_stride, int score_ld,
+                                                               const int* __restrict__ seg, int max_group, float* __restrict__ out) {
+  extern __shared__ float pred_sm[];             // x | mean, n entries each
+  __shared__ double red[32];
+  const int o = seg[blockIdx.x], n = seg[blockIdx.x + 1] - o;
+  if (n <= 0) return;
+  float* rows = out + static_cast<size_t>(o) * RR_PREDICT_COLS;
+  if (n > max_group) {           // shared memory was sized for max_group: NaN rows, never an overrun
+    for (int i = threadIdx.x; i < n * RR_PREDICT_COLS; i += blockDim.x) rows[i] = CUDART_NAN_F;
+    return;
+  }
+  float* x = pred_sm;
+  float* mean = pred_sm + n;
+  const float* base = scores + static_cast<size_t>(o) * score_ld;
+  const double dt = static_cast<double>(T);
+  for (int p0 = 0; p0 < n; p0 += kPredictItems * blockDim.x) {
+    double sum[kPredictItems], dev[kPredictItems], dev2[kPredictItems], prob[kPredictItems], rsum[kPredictItems];
+    float x0[kPredictItems];
+    int top1[kPredictItems];
+#pragma unroll
+    for (int k = 0; k < kPredictItems; ++k) {
+      sum[k] = dev[k] = dev2[k] = prob[k] = rsum[k] = 0.0;
+      x0[k] = 0.f;
+      top1[k] = 0;
+    }
+    for (int t = 0; t < T; ++t) {
+      const float* st = base + static_cast<size_t>(t) * sample_stride;
+      float mx = -CUDART_INF_F;
+      __syncthreads();                           // the previous sample's x[] has been read by everyone
+      for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const float v = st[static_cast<size_t>(i) * score_ld];
+        x[i] = v;
+        mx = fmaxf(mx, v);
+      }
+      mx = block_max(mx, reinterpret_cast<float*>(red));     // synchronises: x[] is complete
+      const double dmx = static_cast<double>(mx);
+      double z = 0.0;
+      for (int i = threadIdx.x; i < n; i += blockDim.x) z += exp(static_cast<double>(x[i]) - dmx);
+      z = block_sum_d(z, red);
+      const double inv_z = 1.0 / z;
+      float xi[kPredictItems];
+      int cnt[kPredictItems];
+#pragma unroll
+      for (int k = 0; k < kPredictItems; ++k) {
+        const int i = p0 + k * blockDim.x + threadIdx.x;
+        xi[k] = i < n ? x[i] : 0.f;
+        cnt[k] = 1;
+      }
+      for (int j = 0; j < n; ++j) {
+        const float xj = x[j];
+#pragma unroll
+        for (int k = 0; k < kPredictItems; ++k) {
+          const int i = p0 + k * blockDim.x + threadIdx.x;
+          cnt[k] += (xj > xi[k]) || (xj == xi[k] && j < i);
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < kPredictItems; ++k) {
+        if (t == 0) x0[k] = xi[k];
+        const double v = static_cast<double>(xi[k]), d = v - static_cast<double>(x0[k]);
+        sum[k] += v;
+        dev[k] += d;
+        dev2[k] += d * d;
+        prob[k] += exp(v - dmx) * inv_z;
+        rsum[k] += static_cast<double>(cnt[k]);
+        top1[k] += cnt[k] == 1;
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < kPredictItems; ++k) {
+      const int i = p0 + k * blockDim.x + threadIdx.x;
+      if (i < n) {
+        const double var = fmax((dev2[k] - dev[k] * dev[k] / dt) / dt, 0.0);    // about the first sample: no cancellation
+        const float m = static_cast<float>(sum[k] / dt);
+        float* r = rows + static_cast<size_t>(i) * RR_PREDICT_COLS;
+        r[0] = m;
+        r[1] = static_cast<float>(sqrt(var));
+        r[3] = static_cast<float>(prob[k] / dt);
+        r[4] = static_cast<float>(static_cast<double>(top1[k]) / dt);
+        r[5] = static_cast<float>(rsum[k] / dt);
+        mean[i] = m;
+      }
+    }
+  }
+  __syncthreads();
+  // rank of the mean score: the fp32 value of column 0, so the rank is the stable order of the returned scores
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const float mi = mean[i];
+    int c = 1;
+    for (int j = 0; j < n; ++j) c += (mean[j] > mi) || (mean[j] == mi && j < i);
+    rows[static_cast<size_t>(i) * RR_PREDICT_COLS + 2] = static_cast<float>(c);
+  }
+}
+
+int rank_predict(int N, int G, int T, const float* scores, long long sample_stride, int score_ld, const int* seg_off, int max_group, float* out,
+                 cudaStream_t s) {
+  ProfScope prof_scope(KC_LOSS, s);
+  RR_REQUIRE(N > 0 && G > 0 && scores && seg_off && out, "rank_predict: NULL argument or empty input");
+  RR_REQUIRE(T >= 1, "rank_predict: T must be >= 1 (got %d)", T);
+  RR_REQUIRE(score_ld >= 1 && sample_stride >= 0, "rank_predict: score_ld must be >= 1 and sample_stride >= 0");
+  RR_REQUIRE(max_group >= 1 && max_group <= kMaxGroup, "rank_predict: largest group %d outside [1, %d]", max_group, kMaxGroup);
+  const size_t smem = 2 * sizeof(float) * static_cast<size_t>(max_group);
+  static PerDeviceOnce attr_set;
+  if (attr_set.need()) {
+    RR_CUDA(cudaFuncSetAttribute(k_rank_predict, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * sizeof(float) * kMaxGroup));
+    attr_set.mark();
+  }
+  k_rank_predict<<<G, kLossThreads, smem, s>>>(T, scores, sample_stride, score_ld, seg_off, max_group, out);
+  RR_LAUNCH_CHECK("rank_predict kernel");
+  return RR_OK;
+}
+
 }  // namespace rr

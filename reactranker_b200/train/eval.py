@@ -17,12 +17,10 @@ from .loss import segment_offsets
 GROUPS_PER_LAUNCH = 256
 
 
-def _forward_chunks(model, gpu, chunks, smiles2graph_dic):
+def _launch_graphs(chunks, smiles2graph_dic, dev, dedup):
     """chunks: list of (smiles [n,2], add_features | None); every chunk becomes ONE segment of the DeviceGraph (its own padding rows and
-    ``max_num_bonds``, exactly as if it had been the reference's whole BatchMolGraph).  Yields ``(lo, hi, preds)`` with the scores of
-    chunks[lo:hi] on the device, rows in chunk order."""
-    dev = torch.device("cuda", gpu) if isinstance(gpu, int) else torch.device(gpu)
-    dedup = reactant_dedup_exact(model)
+    ``max_num_bonds``, exactly as if it had been the reference's whole BatchMolGraph).  Yields ``(lo, hi, rg, pg, feats)`` per launch of up
+    to GROUPS_PER_LAUNCH chunks: the two device graphs of chunks[lo:hi], rows in chunk order, and their extra features (host, or None)."""
     fast = hasattr(smiles2graph_dic, "parsing_ids")
     for lo in range(0, len(chunks), GROUPS_PER_LAUNCH):
         part = chunks[lo:lo + GROUPS_PER_LAUNCH]
@@ -42,7 +40,15 @@ def _forward_chunks(model, gpu, chunks, smiles2graph_dic):
                 rg, pg = DeviceGraph.from_batches_dedup(r_b, p_b, dev)       # a group's candidates share one reactant graph
             else:
                 rg, pg = DeviceGraph.from_batches(r_b, dev), DeviceGraph.from_batches(p_b, dev)
-        yield lo, lo + len(part), model(rg, pg, gpu=gpu, add_features=feats)
+        yield lo, lo + len(part), rg, pg, feats
+
+
+def _forward_chunks(model, gpu, chunks, smiles2graph_dic):
+    """Yields ``(lo, hi, preds)`` with the scores of chunks[lo:hi] on the device, rows in chunk order: one forward per launch of
+    ``_launch_graphs``."""
+    dev = torch.device("cuda", gpu) if isinstance(gpu, int) else torch.device(gpu)
+    for lo, hi, rg, pg, feats in _launch_graphs(chunks, smiles2graph_dic, dev, reactant_dedup_exact(model)):
+        yield lo, hi, model(rg, pg, gpu=gpu, add_features=feats)
 
 
 def compute_NDCG(truth, pred):
