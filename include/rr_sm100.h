@@ -141,7 +141,8 @@ typedef struct {
 /* Parameters in the reference's state_dict layout (row-major [out, in], SURVEY.md §5); he / hd / hf: the encoder's, diff encoder's
  * and FFN's hidden size (all = hidden with rr_model_cfg).  NULL bias = use_bias False.  encoder.W_h is needed for depth > 1,
  * diff_encoder.W_h for diff_depth > 1, diff_encoder.W_o for diff_depth > 0.  The same struct with writable pointers receives the
- * gradients (overwritten, not accumulated). */
+ * gradients (overwritten, not accumulated).  In that role a NULL pointer means "not needed": the tensor's gradient is neither computed
+ * nor written (a frozen parameter).  A split weight is one tensor (encoder.W_o, diff_encoder.W_h, diff_encoder.W_o). */
 typedef struct {
   float* enc_Wi; float* enc_bi;   /* encoder.W_i   [he, 83]        mpn.py:50  */
   float* enc_Wh; float* enc_bh;   /* encoder.W_h   [he, he]        mpn.py:57  */
@@ -242,7 +243,8 @@ int rr_get_forward_bf16(void);
  * the weight gradient's slab count follows the SM count, so a part with a different SM count may round differently.
  * Scratch: rr_model_workspace_bytes includes it when the switch is on (rr_model_backward fails with RR_ERR_WORKSPACE, writing nothing,
  * if the workspace was sized without it); entry points without a workspace take it from the stream-ordered allocator (cudaMallocAsync /
- * cudaFreeAsync on `stream`) in this mode only.  rr_model_backward with rr_model_cfg.r_atom_map returns RR_ERR_UNSUPPORTED in this mode.
+ * cudaFreeAsync on `stream`) in this mode only.  rr_model_backward with rr_model_cfg.r_atom_map returns RR_ERR_UNSUPPORTED in this mode
+ * when an encoder gradient is requested (the sum over shared reactant rows lives in the encoder's backward only).
  * on must be 0 (default) or 1, else RR_ERR_INVALID.  Process-wide. */
 int rr_set_deterministic(int on);
 int rr_get_deterministic(void);
@@ -336,7 +338,12 @@ int64_t rr_model_buffer_offset(const rr_model_cfg* cfg, const rr_graph* r, const
  * matching rr_model_backward has run. */
 int rr_model_forward(const rr_model_cfg* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p,
                      const float* add_features, float* scores, void* ws, int64_t ws_bytes, void* stream);
-/* dscores has the shape of scores; grads receives d/d(parameter) in state_dict layout */
+/* dscores has the shape of scores; grads receives d/d(parameter) in state_dict layout.  Only the non-NULL gradients of grads are
+ * computed (see rr_params): layers in graph order are encoder W_i < W_h < W_o < diff encoder W_i < W_h < W_o < FFN 0 .. F-1, and the
+ * backward runs through a layer only while some tensor below it is requested; nothing below the lowest requested tensor is launched.
+ * A weight gradient is launched only when the weight is requested; a requested bias under a NULL weight gets its own column-sum
+ * kernel (bit-identical run to run in both modes).  All NULL: RR_OK without a launch.  With every pointer set the result and the
+ * launches are those of the full backward. */
 int rr_model_backward(const rr_model_cfg* cfg, const rr_params* w, const rr_graph* r, const rr_graph* p,
                       const float* dscores, rr_params* grads, void* ws, int64_t ws_bytes, void* stream);
 /* The same four with per-sub-module widths and dropouts.  The entry points above are these with diff_hidden = ffn_hidden = hidden and

@@ -6,6 +6,10 @@ command-line arguments.  ``--synthetic G,N`` trains on G synthetic reactant grou
     python main.py --data_path reactions.csv --path runs/exp1 --gpu 0 --task_type listnet --batch_size 4096 --total_epochs 30
     python main.py --synthetic 100,20 --path /tmp/rr --gpu 0 --task_type mle --batch_size 100 --total_epochs 2
 
+Fine-tuning (new): start from a pretrained checkpoint and keep sub-modules fixed; frozen layers cost no backward work,
+
+    python main.py --data_path small.csv --path runs/ft --pretrained runs/exp1/T1/0.pt --freeze encoder,diff_encoder --total_epochs 30
+
 Data-parallel over the GPUs of one box (new; the reference is single-device): launch the same command under torchrun,
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 main.py --data_path ... --batch_size 32768
@@ -24,6 +28,8 @@ import torch
 from reactranker.data.load_reactions import get_data, Parsing_features
 from reactranker.train.utils import build_optimizer, build_lr_scheduler
 from reactranker.models.base_model import build_model
+from reactranker_b200.models.base_model import freeze, parse_freeze
+from reactranker_b200.utils import load_pretrained
 from reactranker.train.train_listwise import train
 from reactranker.train.test_listwise import test
 
@@ -75,7 +81,41 @@ def parse():
     ap.add_argument("--dropout", type=float, default=0.1)
     ap.add_argument("--deterministic", action="store_true",
                     help="torch.use_deterministic_algorithms(True): bit-identical losses, gradients and weights from the same seed")
-    return ap.parse_args()
+    add_finetune_args(ap)
+    return check_finetune_args(ap, ap.parse_args())
+
+
+def add_finetune_args(ap):
+    """--pretrained / --freeze, shared with main_ranknet.py."""
+    ap.add_argument("--pretrained", default=None,
+                    help="checkpoint to start from: every state_dict tensor whose name and shape match is copied (utils.load_pretrained)")
+    ap.add_argument("--freeze", type=_freeze_arg, default=None, metavar="encoder[,diff_encoder][,ffn:N]",
+                    help="keep these pretrained sub-modules fixed (ffn:N = the first N FFN layers); needs --pretrained")
+
+
+def _freeze_arg(spec):
+    try:
+        return parse_freeze(spec)
+    except ValueError as e:
+        raise argparse.ArgumentTypeError(str(e))
+
+
+def check_finetune_args(ap, a):
+    if a.freeze is not None and a.pretrained is None:
+        ap.error("--freeze needs --pretrained: freezing randomly initialised weights is always a mistake")
+    return a
+
+
+def apply_finetune_args(a, model, logger):
+    """--pretrained, then --freeze, on a freshly built model (before .cuda()); returns whether anything is frozen."""
+    if a.pretrained is not None:
+        skipped = load_pretrained(model, a.pretrained)
+        logger.info('Loaded {} tensors from {}; not loaded: {}'.format(len(model.pretrained_names), a.pretrained, skipped))
+    if a.freeze is None:
+        return False
+    frozen = freeze(model, **a.freeze)
+    logger.info('Frozen tensors: {}'.format(frozen))
+    return True
 
 
 def main():
@@ -157,9 +197,10 @@ def main():
         model = make_model(task_type, a.hidden_size, a.depth, a.dropout)
         logger.info('Model Structure')
         logger.info(model)
+        frozen = apply_finetune_args(a, model, logger)
         torch.cuda.set_device(gpu)
         model = model.cuda(gpu)
-        optimizer = build_optimizer(model)
+        optimizer = build_optimizer(model, freeze=frozen)
         scheduler = build_lr_scheduler(optimizer, warmup_epochs=2, total_epochs=total_epochs, train_data_size=train_len, batch_size=batch_size,
                                        init_lr=init_lr, max_lr=max_lr, final_lr=final_lr)
         resume_path = os.path.join(a.path, str(ii) + '.state.pt') if a.resume else None

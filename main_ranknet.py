@@ -15,6 +15,7 @@ from reactranker.models.base_model import build_model
 from reactranker.train.run_train_pairwise import run_train
 from reactranker.train.test_ranknet import test
 from reactranker.train.utils import build_optimizer, build_lr_scheduler
+from main import add_finetune_args, apply_finetune_args, check_finetune_args
 
 
 def parse():
@@ -37,7 +38,8 @@ def parse():
     ap.add_argument("--resume", action="store_true", help="write <path>/<fold>.state.pt after every epoch and continue from it if present")
     ap.add_argument("--deterministic", action="store_true",
                     help="torch.use_deterministic_algorithms(True): bit-identical losses, gradients and weights from the same seed")
-    return ap.parse_args()
+    add_finetune_args(ap)
+    return check_finetune_args(ap, ap.parse_args())
 
 
 def main():
@@ -91,9 +93,10 @@ def main():
         torch.cuda.manual_seed_all(seed)
         model = build_model(hidden_size=300, mpnn_depth=3, mpnn_diff_depth=3, ffn_depth=3, use_bias=True, dropout=0.2, task_num=1,
                             ffn_last_layer='no_softplus', add_features_dim=add_features_dim)       # main_ranknet.py:113-121
+        frozen = apply_finetune_args(a, model, logger)
         torch.cuda.set_device(gpu)
         model = model.cuda(gpu)
-        optimizer = build_optimizer(model)
+        optimizer = build_optimizer(model, freeze=frozen)
         scheduler = build_lr_scheduler(optimizer, warmup_epochs=2, total_epochs=total_epochs, train_data_size=train_len, batch_size=batch_size,
                                        init_lr=init_lr, max_lr=max_lr, final_lr=final_lr)
         run_train(model, scheduler, train_data, val_data, path_checkpoints, optimizer, total_epochs, smiles2graph_dic, batch_size=batch_size,

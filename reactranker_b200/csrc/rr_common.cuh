@@ -317,6 +317,10 @@ int linear_dgrad_tc(int M, int n, int k, const float* dZ, int lddz, const float*
 int linear_wgrad(int, int, int, const float*, int, const float*, int, float*, int, float*, cudaStream_t, void* det = nullptr, long long det_bytes = 0);
 // deterministic mode: bytes of scratch linear_wgrad(M, n, k, ...) needs (row-slab partials of dW and of the bias gradient), any GEMM mode
 long long wgrad_det_bytes(int M, int n, int k);
+// dbias[n] += colsum(dZ[M, n]) over every row, for a bias whose weight is frozen: row slabs store partials, a second pass adds them in slab
+// order (no atomics, the same bits on every run in both modes).  Scratch: det when given (>= bias_grad_bytes(M, n)), else transient.
+int linear_bias_grad(int M, int n, const float* dZ, int lddz, float* dbias, cudaStream_t s, void* det = nullptr, long long det_bytes = 0);
+long long bias_grad_bytes(int M, int n);
 
 // fp32 SIMT launchers (rr_gemm_simt.cu)
 int simt_fwd(int M, int n, const float* X1, int ldx1, const float* W1, int k1, const float* X2, int ldx2, const float* W2, int k2, const float* bias,

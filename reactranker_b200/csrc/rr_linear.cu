@@ -16,6 +16,7 @@
 //     the caller's images or split on chip (rr_linear_fwd).  Of a TC dgrad and wgrad: 3 x bf16 when rr_set_backward_bf16(1) (the default),
 //     else 3 x TF32 (the wgrad's k_tc_wgrad2).  A shape the bf16 forward / dgrad refuses takes the TF32 kernel.
 //   - Deterministic mode changes none of these choices: the wgrad's row slabs store their partials and k_wgrad_slab_sum adds them in order.
+//   - A bias gradient without its weight's (rr_model_backward with the weight frozen) is linear_bias_grad, fp32 SIMT in every mode.
 #include "rr_common.cuh"
 
 namespace rr {
@@ -229,6 +230,66 @@ int linear_wgrad(int M, int n, int k, const float* dZ, int lddz, const float* X,
   if (blocks > num_sms() * 8) blocks = num_sms() * 8;
   k_wgrad_slab_sum<<<static_cast<int>(blocks), 256, 0, s>>>(n, k, splits, slab, slab + splits * static_cast<long long>(n) * k, dW, lddw, dbias);
   RR_LAUNCH_CHECK("k_wgrad_slab_sum");
+  return RR_OK;
+}
+
+// ---- bias gradient alone -------------------------------------------------------------------------
+// The column sum of dZ over all M rows, padding rows included, as the weight gradient's fused bias partial takes it; not the same bits.
+// Slab z of rows_per_slab rows: a (32 x 8) block sums 32 float4 columns over its rows, eight row lanes reduced in lane order, and stores the
+// partial to part[z * n ..]; k_bias_colsum_total adds the partials of each column in slab order.
+__global__ void __launch_bounds__(256) k_bias_colsum_slabs(int M, int n, int rows_per_slab, const float* __restrict__ dZ, int lddz,
+                                                           float* __restrict__ part) {
+  __shared__ float4 red[8][32];
+  const int c = (blockIdx.y * 32 + threadIdx.x) * 4;
+  const long long r0 = static_cast<long long>(blockIdx.x) * rows_per_slab;
+  const long long r1 = r0 + rows_per_slab < M ? r0 + rows_per_slab : M;
+  float4 acc = f4_zero();
+  if (c < n)
+    for (long long r = r0 + threadIdx.y; r < r1; r += 8) acc = f4_add(acc, ld_f4(dZ + r * lddz + c));
+  red[threadIdx.y][threadIdx.x] = acc;
+  __syncthreads();
+  if (threadIdx.y == 0 && c < n) {
+#pragma unroll
+    for (int y = 1; y < 8; ++y) acc = f4_add(acc, red[y][threadIdx.x]);
+    st_f4(part + static_cast<long long>(blockIdx.x) * n + c, acc);
+  }
+}
+__global__ void k_bias_colsum_total(int n, int slabs, const float* __restrict__ part, float* __restrict__ dbias) {
+  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < n; c += gridDim.x * blockDim.x) {
+    float acc = part[c];
+    for (int z = 1; z < slabs; ++z) acc += part[static_cast<long long>(z) * n + c];
+    dbias[c] += acc;
+  }
+}
+
+// slab height: at least 64 rows, at most 2 slabs per SM; a multiple of the 8 row lanes
+static int bias_grad_rows_per_slab(int M) {
+  const int per = (M + 2 * num_sms() - 1) / (2 * num_sms());
+  return ((per > 64 ? per : 64) + 7) / 8 * 8;
+}
+long long bias_grad_bytes(int M, int n) {
+  if (M <= 0 || n <= 0) return 0;
+  const int rows = bias_grad_rows_per_slab(M);
+  return static_cast<long long>((M + rows - 1) / rows) * n * static_cast<long long>(sizeof(float));
+}
+
+int linear_bias_grad(int M, int n, const float* dZ, int lddz, float* dbias, cudaStream_t s, void* det, long long det_bytes) {
+  RR_REQUIRE(M >= 0 && n > 0 && (n & 3) == 0, "linear_bias_grad: M %d n %d", M, n);
+  RR_TRY(check_mat("dZ", dZ, lddz));
+  RR_REQUIRE(dbias != nullptr, "linear_bias_grad: dbias is NULL");
+  if (M == 0) return RR_OK;
+  const int rows = bias_grad_rows_per_slab(M), slabs = (M + rows - 1) / rows;
+  DetScratch ds;
+  RR_TRY(det_scratch(&ds, det, det_bytes, bias_grad_bytes(M, n), s));
+  float* part = static_cast<float*>(ds.p);
+  {
+    ProfScope prof_scope(KC_GEMM_WGRAD, s);
+    k_bias_colsum_slabs<<<dim3(slabs, (n / 4 + 31) / 32), dim3(32, 8), 0, s>>>(M, n, rows, dZ, lddz, part);
+    RR_LAUNCH_CHECK("k_bias_colsum_slabs");
+  }
+  ProfScope prof_scope(KC_GEMM_WGRAD, s);
+  k_bias_colsum_total<<<(n + 255) / 256, 256, 0, s>>>(n, slabs, part, dbias);
+  RR_LAUNCH_CHECK("k_bias_colsum_total");
   return RR_OK;
 }
 

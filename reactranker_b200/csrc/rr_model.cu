@@ -376,6 +376,10 @@ static int carve(const rr_model_cfg_ex& cx, const rr_graph& r, const rr_graph& p
     at_least(wgrad_det_bytes(A_, hd, hd));                // diff encoder W_h, W_o (message parts)
     at_least(wgrad_det_bytes(A_, hd, RR_FB_LD));          // diff encoder W_h (bond features)
     for (int l = 0; l < c.ffn_depth; ++l) at_least(wgrad_det_bytes(N_, W->L.ffn_out[l], W->L.ffn_in[l]));
+    at_least(bias_grad_bytes(B_J_, he));                  // a bias that trains under a frozen weight (linear_bias_grad)
+    at_least(bias_grad_bytes(A_J_, he));
+    at_least(bias_grad_bytes(A_, hd));
+    at_least(bias_grad_bytes(N_, static_cast<int>(hpf) > RR_OUT_LD ? static_cast<int>(hpf) : RR_OUT_LD));
     at_least(pad_parts_bytes(A_J_, r.n_segments + p.n_segments, he));   // gathers over the joint graph
     at_least(pad_parts_bytes(A_, p.n_segments, hd));                    // and over the product graph
     W->det = take(static_cast<size_t>((need + 3) / 4));
@@ -579,13 +583,33 @@ int model_forward(const rr_model_cfg_ex* cx, const rr_params* w, const rr_graph*
   return RR_OK;
 }
 
+// Only the gradients the caller asks for are computed: a NULL pointer in `grads` means that tensor is neither computed nor written
+// (frozen).  Layers in graph order from the input up: encoder W_i < W_h < W_o < diff encoder W_i < W_h < W_o < FFN 0 .. F-1.  A layer's
+// weight gradient runs when its weight is requested (its bias fused in), its bias gradient alone (linear_bias_grad) when only the bias
+// is; the dgrad chain runs through a layer only while some layer below it trains.  With every pointer set this is the full backward,
+// launch for launch.
 int model_backward(const rr_model_cfg_ex* cx, const rr_params* w, const rr_graph* r, const rr_graph* p, const float* dscores, rr_params* grads,
                    void* ws, long long ws_bytes, cudaStream_t s) {
   Workspace W;
   RR_TRY(check_model_args(cx, w, r, p, ws, ws_bytes, &W));
   const rr_model_cfg* c = &cx->base;
   RR_REQUIRE(dscores && grads, "backward: NULL argument");
-  if (deterministic() && c->r_atom_map)
+  enum { E_I, E_H, E_O, D_I, D_H, D_O, F0 };
+  const rr_params& gp = *grads;
+  const int nlev = F0 + c->ffn_depth;
+  bool wreq[F0 + RR_MAX_FFN] = {gp.enc_Wi != nullptr, gp.enc_Wh != nullptr, gp.enc_Wo != nullptr, gp.dif_Wi != nullptr, gp.dif_Wh != nullptr,
+                                gp.dif_Wo != nullptr};
+  bool breq[F0 + RR_MAX_FFN] = {gp.enc_bi != nullptr, gp.enc_bh != nullptr, gp.enc_bo != nullptr, gp.dif_bi != nullptr, gp.dif_bh != nullptr,
+                                gp.dif_bo != nullptr};
+  for (int l = 0; l < c->ffn_depth; ++l) {
+    wreq[F0 + l] = gp.ffn_W[l] != nullptr;
+    breq[F0 + l] = gp.ffn_b[l] != nullptr;
+  }
+  bool below[F0 + RR_MAX_FFN + 1];   // below[lv]: some layer under lv trains
+  below[0] = false;
+  for (int lv = 0; lv < nlev; ++lv) below[lv + 1] = below[lv] || wreq[lv] || breq[lv];
+  if (!below[nlev]) return RR_OK;
+  if (deterministic() && c->r_atom_map && below[D_I])
     return fail(RR_ERR_UNSUPPORTED, "deterministic mode: the backward pass of de-duplicated reactants (r_atom_map) sums rows with atomics");
   const PackedLayout& L = W.L;
   const int hpe = L.hpe, hpd = L.hpd, hpf = L.hpf, vp = L.vp;
@@ -596,63 +620,80 @@ int model_backward(const rr_model_cfg_ex* cx, const rr_params* w, const rr_graph
   float* G = W.dpacked;
   RR_CUDA(cudaMemsetAsync(G, 0, L.grad_total * sizeof(float), s));
   const int N = p->n_mols, A = p->n_atoms;
+  // the bias gradient of layer lv when its weight is frozen (otherwise the weight gradient computes it, or it is not wanted)
+  auto bias_only = [&](int lv, int M, int n, const float* dZ, int lddz, size_t db) -> int {
+    return (!wreq[lv] && breq[lv]) ? linear_bias_grad(M, n, dZ, lddz, G + db, s, W.det, W.det_bytes) : RR_OK;
+  };
 
-  {
-    const int n = N * RR_OUT_LD;
-    k_head_bwd<<<(n + 255) / 256, 256, 0, s>>>(N, c->task_num, c->head, W.zout, dscores, W.dzout);
-    RR_LAUNCH_CHECK("k_head_bwd");
-  }
-  // FFN
-  {
-    const float* g = W.dzout;
-    int ldg = RR_OUT_LD;
-    float* scratch[2] = {W.gN1, W.gN2};
-    for (int l = c->ffn_depth - 1; l >= 0; --l) {
-      const float* x = (l == 0) ? W.vec : W.x[l - 1];
-      RR_TRY(linear_wgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, x, L.ffn_in[l], G + L.ffn_W[l], L.ffn_in[l], G + L.ffn_b[l], s, W.det, W.det_bytes));
-      if (l > 0) {
-        float* dx = scratch[l & 1];
-        RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], dx, hpf, 0, W.img, s));
-        RR_TRY(relu_bwd(N, hpf, dx, W.x[l - 1], keep_f, 0, dx, nullptr, 0, s));
-        g = dx;
-        ldg = hpf;
-      } else {
-        RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], W.dvec, vp, 0, W.img, s));
+  auto chain = [&]() -> int {
+    {
+      const int n = N * RR_OUT_LD;
+      k_head_bwd<<<(n + 255) / 256, 256, 0, s>>>(N, c->task_num, c->head, W.zout, dscores, W.dzout);
+      RR_LAUNCH_CHECK("k_head_bwd");
+    }
+    // FFN
+    {
+      const float* g = W.dzout;
+      int ldg = RR_OUT_LD;
+      float* scratch[2] = {W.gN1, W.gN2};
+      for (int l = c->ffn_depth - 1; l >= 0; --l) {
+        const float* x = (l == 0) ? W.vec : W.x[l - 1];
+        if (wreq[F0 + l])
+          RR_TRY(linear_wgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, x, L.ffn_in[l], G + L.ffn_W[l], L.ffn_in[l], G + L.ffn_b[l], s, W.det, W.det_bytes));
+        RR_TRY(bias_only(F0 + l, N, L.ffn_out[l], g, ldg, L.ffn_b[l]));
+        if (!below[F0 + l]) return RR_OK;
+        if (l > 0) {
+          float* dx = scratch[l & 1];
+          RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], dx, hpf, 0, W.img, s));
+          RR_TRY(relu_bwd(N, hpf, dx, W.x[l - 1], keep_f, 0, dx, nullptr, 0, s));
+          g = dx;
+          ldg = hpf;
+        } else {
+          RR_TRY(linear_dgrad(N, L.ffn_out[l], L.ffn_in[l], g, ldg, P + L.ffn_W[l], L.ffn_in[l], P + L.ffn_W_T[l], L.ffn_out[l], W.dvec, vp, 0, W.img, s));
+        }
       }
     }
-  }
-  // readout: the gradient of the diff encoder's last layer (W_o, or W_i at diff_depth 0) through hid2's ReLU / dropout mask
-  RR_TRY(readout_bwd(p, W.dvec, vp, W.vec, W.hid2, W.gA1, hpd, pf, pd, s));
-  const float* dWi = W.gA1;   // gradient of W_i's output
-  if (c->diff_depth > 0) {
-    RR_TRY(linear_wgrad(A, hpd, hpe, W.gA1, hpd, W.d, hpe, G + L.dif_Wo_d, hpe, G + L.dif_bo, s, W.det, W.det_bytes));
-    RR_TRY(linear_wgrad(A, hpd, hpd, W.gA1, hpd, W.am2, hpd, G + L.dif_Wo_m, hpd, nullptr, s, W.det, W.det_bytes));
-    RR_TRY(linear_dgrad(A, hpd, hpe, W.gA1, hpd, P + L.dif_Wo_d, hpe, P + L.dif_Wo_d_T, hpd, W.dD, hpe, 0, W.img, s));
-    RR_TRY(linear_dgrad(A, hpd, hpd, W.gA1, hpd, P + L.dif_Wo_m, hpd, P + L.dif_Wo_m_T, hpd, W.gA2, hpd, 0, W.img, s));
-    // Every gather backward is followed by exactly one ReLU (+ dropout) backward: the mask of the message it produced the gradient of.
-    // Both run as one kernel (rr_mp_pipe.cu): t_next >= 1 -> mask of m2^{t_next}, result kept (gA1) and summed into dI2;
-    // t_next == 0 -> mask [inp2 > 0] of m2^0 = relu(inp2), only the sum into dI2 is wanted.
-    auto diff_nbr_bwd = [&](int t_next) {
-      if (t_next >= 1)
-        return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA1, hpd, W.m2[t_next], keep_d, 0, W.dI2, t_next == Td ? 1 : 2, 0, s, W.det, W.det_bytes);
-      return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA3, hpd, W.inp2, 1.f, 1, W.dI2, Td == 0 ? 1 : 2, 1, s, W.det, W.det_bytes);
-    };
-    RR_TRY(diff_nbr_bwd(Td));
-    for (int t = Td; t >= 1; --t) {
-      RR_TRY(linear_wgrad(A, hpd, hpd, W.gA1, hpd, W.nm[t - 1], hpd, G + L.dif_Wh_m, hpd, G + L.dif_bh, s, W.det, W.det_bytes));
-      RR_TRY(linear_wgrad(A, hpd, RR_FB_LD, W.gA1, hpd, W.nf, RR_FB_LD, G + L.dif_Wh_f, RR_FB_LD, nullptr, s, W.det, W.det_bytes));
-      RR_TRY(linear_dgrad(A, hpd, hpd, W.gA1, hpd, P + L.dif_Wh_m, hpd, P + L.dif_Wh_m_T, hpd, W.gA2, hpd, 0, W.img, s));
-      RR_TRY(diff_nbr_bwd(t - 1));
+    // readout: the gradient of the diff encoder's last layer (W_o, or W_i at diff_depth 0) through hid2's ReLU / dropout mask
+    RR_TRY(readout_bwd(p, W.dvec, vp, W.vec, W.hid2, W.gA1, hpd, pf, pd, s));
+    const float* dWi = W.gA1;   // gradient of W_i's output
+    if (c->diff_depth > 0) {
+      if (wreq[D_O]) {
+        RR_TRY(linear_wgrad(A, hpd, hpe, W.gA1, hpd, W.d, hpe, G + L.dif_Wo_d, hpe, G + L.dif_bo, s, W.det, W.det_bytes));
+        RR_TRY(linear_wgrad(A, hpd, hpd, W.gA1, hpd, W.am2, hpd, G + L.dif_Wo_m, hpd, nullptr, s, W.det, W.det_bytes));
+      }
+      RR_TRY(bias_only(D_O, A, hpd, W.gA1, hpd, L.dif_bo));
+      if (!below[D_O]) return RR_OK;
+      if (below[D_I]) RR_TRY(linear_dgrad(A, hpd, hpe, W.gA1, hpd, P + L.dif_Wo_d, hpe, P + L.dif_Wo_d_T, hpd, W.dD, hpe, 0, W.img, s));  // only the encoder reads dD
+      RR_TRY(linear_dgrad(A, hpd, hpd, W.gA1, hpd, P + L.dif_Wo_m, hpd, P + L.dif_Wo_m_T, hpd, W.gA2, hpd, 0, W.img, s));
+      // Every gather backward is followed by exactly one ReLU (+ dropout) backward: the mask of the message it produced the gradient of.
+      // Both run as one kernel (rr_mp_pipe.cu): t_next >= 1 -> mask of m2^{t_next}, result kept (gA1) and summed into dI2;
+      // t_next == 0 -> mask [inp2 > 0] of m2^0 = relu(inp2), only the sum into dI2 is wanted.
+      auto diff_nbr_bwd = [&](int t_next) {
+        if (t_next >= 1)
+          return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA1, hpd, W.m2[t_next], keep_d, 0, W.dI2, t_next == Td ? 1 : 2, 0, s, W.det, W.det_bytes);
+        return neighbor_sum_bwd_act(p, 1, W.gA2, W.gA3, hpd, W.inp2, 1.f, 1, W.dI2, Td == 0 ? 1 : 2, 1, s, W.det, W.det_bytes);
+      };
+      RR_TRY(diff_nbr_bwd(Td));
+      for (int t = Td; t >= 1; --t) {
+        if (wreq[D_H]) {
+          RR_TRY(linear_wgrad(A, hpd, hpd, W.gA1, hpd, W.nm[t - 1], hpd, G + L.dif_Wh_m, hpd, G + L.dif_bh, s, W.det, W.det_bytes));
+          RR_TRY(linear_wgrad(A, hpd, RR_FB_LD, W.gA1, hpd, W.nf, RR_FB_LD, G + L.dif_Wh_f, RR_FB_LD, nullptr, s, W.det, W.det_bytes));
+        }
+        RR_TRY(bias_only(D_H, A, hpd, W.gA1, hpd, L.dif_bh));
+        if (t == 1 && !below[D_H]) return RR_OK;   // what follows feeds W_i and the encoder only
+        RR_TRY(linear_dgrad(A, hpd, hpd, W.gA1, hpd, P + L.dif_Wh_m, hpd, P + L.dif_Wh_m_T, hpd, W.gA2, hpd, 0, W.img, s));
+        RR_TRY(diff_nbr_bwd(t - 1));
+      }
+      dWi = W.dI2;
     }
-    dWi = W.dI2;
-  }
-  RR_TRY(linear_wgrad(A, hpd, hpe, dWi, hpd, W.d, hpe, G + L.dif_Wi, hpe, G + L.dif_bi, s, W.det, W.det_bytes));
-  // accumulates onto W_o's share of dD; at diff_depth 0 it is the only share
-  RR_TRY(linear_dgrad(A, hpd, hpe, dWi, hpd, P + L.dif_Wi, hpe, P + L.dif_Wi_T, hpd, W.dD, hpe, c->diff_depth > 0 ? 1 : 0, W.img, s));
+    if (wreq[D_I]) RR_TRY(linear_wgrad(A, hpd, hpe, dWi, hpd, W.d, hpe, G + L.dif_Wi, hpe, G + L.dif_bi, s, W.det, W.det_bytes));
+    RR_TRY(bias_only(D_I, A, hpd, dWi, hpd, L.dif_bi));
+    if (!below[D_I]) return RR_OK;
+    // accumulates onto W_o's share of dD; at diff_depth 0 it is the only share
+    RR_TRY(linear_dgrad(A, hpd, hpe, dWi, hpd, P + L.dif_Wi, hpe, P + L.dif_Wi_T, hpd, W.dD, hpe, c->diff_depth > 0 ? 1 : 0, W.img, s));
 
-  // shared encoder, once over [reactant rows | product rows]: d(hid_p) = +dD, d(hid_r) = -dD (base_model.py:168), each through the
-  // ReLU / dropout mask of its own rows; the weight gradients of both halves come out of one launch per layer (base_model.py:155-156)
-  {
+    // shared encoder, once over [reactant rows | product rows]: d(hid_p) = +dD, d(hid_r) = -dD (base_model.py:168), each through the
+    // ReLU / dropout mask of its own rows; the weight gradients of both halves come out of one launch per layer (base_model.py:155-156)
     // (the joint graph's tables, and its feature copy if one was needed, are in the workspace since the forward)
     const rr_graph* g = &W.J;
     EncBufs& e = W.j;
@@ -666,19 +707,27 @@ int model_backward(const rr_model_cfg_ex* cx, const rr_params* w, const rr_graph
     } else {
       RR_TRY(relu_bwd(A_r, hpe, W.dD, W.enc[0].hid, -keep_e, 0, W.gA1, nullptr, 0, s));
     }
-    RR_TRY(linear_wgrad(A_J, hpe, RR_FA_LD, W.gA1, hpe, g->f_atoms, RR_FA_LD, G + L.enc_Wo_a, RR_FA_LD, G + L.enc_bo, s, W.det, W.det_bytes));
-    RR_TRY(linear_wgrad(A_J, hpe, hpe, W.gA1, hpe, e.am, hpe, G + L.enc_Wo_m, hpe, nullptr, s, W.det, W.det_bytes));
+    if (wreq[E_O]) {
+      RR_TRY(linear_wgrad(A_J, hpe, RR_FA_LD, W.gA1, hpe, g->f_atoms, RR_FA_LD, G + L.enc_Wo_a, RR_FA_LD, G + L.enc_bo, s, W.det, W.det_bytes));
+      RR_TRY(linear_wgrad(A_J, hpe, hpe, W.gA1, hpe, e.am, hpe, G + L.enc_Wo_m, hpe, nullptr, s, W.det, W.det_bytes));
+    }
+    RR_TRY(bias_only(E_O, A_J, hpe, W.gA1, hpe, L.enc_bo));
+    if (!below[E_O]) return RR_OK;
     RR_TRY(linear_dgrad(A_J, hpe, hpe, W.gA1, hpe, P + L.enc_Wo_m, hpe, P + L.enc_Wo_m_T, hpe, W.gA2, hpe, 0, W.img, s));
     if (T >= 1) RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hpe, e.m[T], keep_e, 0, W.dinp, 1, 0, s, W.det, W.det_bytes));
     else RR_TRY(neighbor_sum_bwd_act(g, 0, W.gA2, W.gB1, hpe, e.inp, 1.f, 1, W.dinp, 1, 1, s, W.det, W.det_bytes));
     for (int t = T; t >= 1; --t) {
-      RR_TRY(linear_wgrad(B_J, hpe, hpe, W.gB1, hpe, e.pre[t - 1], hpe, G + L.enc_Wh, hpe, G + L.enc_bh, s, W.det, W.det_bytes));
+      if (wreq[E_H]) RR_TRY(linear_wgrad(B_J, hpe, hpe, W.gB1, hpe, e.pre[t - 1], hpe, G + L.enc_Wh, hpe, G + L.enc_bh, s, W.det, W.det_bytes));
+      RR_TRY(bias_only(E_H, B_J, hpe, W.gB1, hpe, L.enc_bh));
+      if (t == 1 && !below[E_H]) return RR_OK;   // what follows feeds W_i only
       RR_TRY(linear_dgrad(B_J, hpe, hpe, W.gB1, hpe, P + L.enc_Wh, hpe, P + L.enc_Wh_T, hpe, W.gB2, hpe, 0, W.img, s));
       if (t - 1 >= 1) RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hpe, e.m[t - 1], keep_e, 0, W.dinp, 2, 0, s, W.det, W.det_bytes));
       else RR_TRY(bond_message_bwd_act(g, W.gB2, W.gB1, hpe, e.inp, 1.f, 1, W.dinp, 2, 1, s, W.det, W.det_bytes));
     }
-    RR_TRY(linear_wgrad(B_J, hpe, RR_FB_LD, W.dinp, hpe, g->f_bonds, RR_FB_LD, G + L.enc_Wi, RR_FB_LD, G + L.enc_bi, s, W.det, W.det_bytes));
-  }
+    if (wreq[E_I]) RR_TRY(linear_wgrad(B_J, hpe, RR_FB_LD, W.dinp, hpe, g->f_bonds, RR_FB_LD, G + L.enc_Wi, RR_FB_LD, G + L.enc_bi, s, W.det, W.det_bytes));
+    return bias_only(E_I, B_J, hpe, W.dinp, hpe, L.enc_bi);
+  };
+  RR_TRY(chain());
 
   PackTable Tb = make_table(*cx, L, *grads, false);
   k_pack<<<dim3(32, Tb.n), 256, 0, s>>>(Tb, G, 1, 0, 0, nullptr, nullptr);

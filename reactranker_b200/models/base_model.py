@@ -14,6 +14,7 @@ import torch
 import torch.nn as nn
 
 from .. import _lib
+from ..parallel import flat_layout
 from ..features.featurization import ATOM_FDIM, BOND_FDIM, BatchMolGraph, DeviceGraph
 from .mpn import MPN, MPNDiff
 
@@ -137,15 +138,16 @@ class _ReactionFn(torch.autograd.Function):
         w = model._param_struct(params)
         # All gradients are written into ONE flat buffer (state_dict layout, parameter order of _named_slots, each tensor 16-byte aligned)
         # and handed to autograd as views of it: p.grad then aliases the buffer, and the data-parallel gradient exchange is a single
-        # all-reduce of `model._grad_flat` in place -- no flatten / unflatten copies (parallel.GradSync).
-        offs, total = [], 0
-        for p in params:
-            offs.append(total)
-            total += (p.numel() + 3) // 4 * 4
+        # all-reduce of `model._grad_flat` in place -- no flatten / unflatten copies (parallel.GradSync).  Only the tensors autograd asks
+        # for are in it: a frozen one gets a NULL pointer, which rr_model_backward neither computes nor writes.
+        needs = ctx.needs_input_grad[4:]
+        hot = [p for p, n in zip(params, needs) if n]
+        offs, total = flat_layout(hot)
         flat = torch.empty(total, dtype=torch.float32, device=params[0].device)
-        if total != sum(p.numel() for p in params):
+        if total != sum(p.numel() for p in hot):
             flat.zero_()                                     # alignment gaps take part in the all-reduce
-        grads = [flat[o:o + p.numel()].view(p.shape) for o, p in zip(offs, params)]
+        views = iter([flat[o:o + p.numel()].view(p.shape) for o, p in zip(offs, hot)])
+        grads = [next(views) if n else None for n in needs]
         gw = model._param_struct(grads)
         dscores = dscores.contiguous().float()
         _lib.set_deterministic(ctx.det)
@@ -197,8 +199,11 @@ class ReactionModel(nn.Module):
         return [(k, v) for k, v in slots if v is not None]
 
     def _param_struct(self, tensors) -> _lib.RRParams:
+        """The C struct of one tensor per slot of _named_slots; None leaves the slot NULL."""
         s = _lib.RRParams()
         for (slot, _), t in zip(self._named_slots(), tensors):
+            if t is None:
+                continue
             if isinstance(slot, tuple):
                 getattr(s, slot[0])[slot[1]] = t.data_ptr()
             else:
@@ -218,7 +223,7 @@ class ReactionModel(nn.Module):
 
     def hot_parameters(self):
         """The trainable parameters in the order of the flat gradient buffer."""
-        return [p for _, p in self._named_slots()]
+        return [p for _, p in self._named_slots() if p.requires_grad]
 
     def saved_activation(self, out: torch.Tensor, name: str, rows: int, cols: int) -> torch.Tensor:
         """A forward activation kept in the workspace of the autograd node behind ``out`` (per-layer parity tests):
@@ -286,3 +291,44 @@ def build_model(hidden_size: int = 300, mpnn_depth: int = 3, mpnn_diff_depth: in
                          mpnn_diff_dropout=dropout, ffn_hidden_size=hidden_size, ffn_bias=use_bias, ffn_dropout=dropout,
                          ffn_depth=ffn_depth, task_num=task_num, task_type=task_type,
                          addtion_react_featrues=0 if bimolecule else add_features_dim)
+
+
+_FREEZE_MODULES = ("encoder", "diff_encoder")
+
+
+def parse_freeze(spec: str) -> dict:
+    """``freeze()``'s keyword arguments from the command-line form ``encoder[,diff_encoder][,ffn:N]`` (any order); ValueError on anything
+    else, so that argparse reports it."""
+    kw = dict(encoder=False, diff_encoder=False, ffn_layers=0)
+    for tok in (t.strip() for t in spec.split(",")):
+        if tok in _FREEZE_MODULES:
+            kw[tok] = True
+        elif tok.startswith("ffn:") and tok[4:].isdigit() and int(tok[4:]) > 0:
+            kw["ffn_layers"] = int(tok[4:])
+        else:
+            raise ValueError(f"unknown module {tok!r} in --freeze {spec!r}: expected encoder, diff_encoder or ffn:N (N >= 1)")
+    return kw
+
+
+def freeze(model: ReactionModel, encoder: bool = False, diff_encoder: bool = False, ffn_layers: int = 0) -> List[str]:
+    """Fine-tuning: ``requires_grad = False`` on the encoder, the diff encoder and / or the first ``ffn_layers`` Linear layers of
+    ``ffn.ffn`` (chemprop's frozen MPN / frozen FFN layers).  Their gradients are then neither computed nor written by the backward pass,
+    and everything below the lowest trainable layer is skipped (rr_model_backward).  Setting ``requires_grad_(False)`` on single tensors
+    by hand works the same way.  Every frozen tensor must have been loaded by ``load_pretrained`` (freezing random weights is always a
+    mistake): raises ``ValueError`` otherwise.  Returns the frozen ``state_dict`` names."""
+    linears = model.ffn.linears()
+    if not 0 <= ffn_layers <= len(linears):
+        raise ValueError(f"ffn_layers = {ffn_layers}: the FFN has {len(linears)} Linear layers")
+    mods = [m for m, on in (("encoder", encoder), ("diff_encoder", diff_encoder)) if on]
+    names = dict(model.named_parameters())
+    frozen = [n for n in names if n.split(".")[0] in mods and "cached_zero" not in n]
+    ffn_ids = {id(p) for lin in linears[:ffn_layers] for p in lin.parameters()}
+    frozen += [n for n, p in names.items() if id(p) in ffn_ids]
+    loaded = getattr(model, "pretrained_names", set())
+    missing = [n for n in frozen if n not in loaded]
+    if missing:
+        raise ValueError(f"freeze: {len(missing)} tensors to freeze were not loaded from a pretrained checkpoint (load_pretrained): "
+                         f"{missing}")
+    for n in frozen:
+        names[n].requires_grad_(False)
+    return frozen

@@ -48,29 +48,49 @@ def shard_rows(scope: Sequence[int], lo: int, hi: int) -> Tuple[int, int]:
     return int(off[lo]), int(off[hi])
 
 
+def flat_layout(tensors) -> Tuple[List[int], int]:
+    """(element offset of each tensor, total elements) of the flat gradient buffer: the tensors in the given order, each starting on a
+    16-byte boundary.  ``ReactionModel``'s backward lays its buffer out over the trainable tensors with this, and ``GradSync`` its
+    staging bucket, so that the in-place and the staged all-reduce have the same element count."""
+    offsets, total = [], 0
+    for t in tensors:
+        offsets.append(total)
+        total += (t.numel() + 3) // 4 * 4
+    return offsets, total
+
+
 class GradSync:
     """SUM all-reduce of all gradients as ONE collective per step.
 
     Fast path: ``ReactionModel`` writes the gradients of a backward pass into one flat buffer and gives autograd views of it, so
     ``p.grad`` aliases ``model._grad_flat``; the buffer is all-reduced in place (3.16 MB at h = 300, 12.1 MB at h = 600) and nothing
     is copied.  Whenever that aliasing does not hold (gradients accumulated over several backward passes into older tensors, a
-    hook that replaced ``p.grad``, parameters outside the model) the gradients go through a flat staging bucket instead."""
+    hook that replaced ``p.grad``, parameters outside the model) the gradients go through a flat staging bucket instead.
+
+    Only the tensors of ``params`` that have ``requires_grad`` take part, decided at every call: frozen tensors are neither exchanged nor
+    given a gradient, and the collective carries the trainable bytes only.  Freezing or unfreezing tensors after this object was built
+    is therefore exact; the first step after such a change may take the staging path."""
 
     def __init__(self, params, group=None, model=None):
-        self.params = [p for p in params if p.requires_grad]
+        self.candidates = list(params)
         self.group = group
         self.model = model
-        # ONE layout for both paths (every tensor starts on a 16-byte boundary, as ReactionModel's backward lays its flat buffer out):
-        # a rank whose shard is empty has no backward pass and goes through the staging bucket while its peers all-reduce their
-        # aliased buffers in place -- the collective must have the same element count on every rank
-        self.offsets, total = [], 0
-        for p in self.params:
-            self.offsets.append(total)
-            total += (p.numel() + 3) // 4 * 4
-        self.numel = total
         self.flat = None
         self.fast_path_steps = 0
         self.copy_path_steps = 0
+        self.params = None
+        self._refresh()
+
+    def _refresh(self):
+        # ONE layout for both paths (flat_layout, as ReactionModel's backward lays its flat buffer out): a rank whose shard is empty has no
+        # backward pass and goes through the staging bucket while its peers all-reduce their aliased buffers in place -- the collective
+        # must have the same element count on every rank
+        params = [p for p in self.candidates if p.requires_grad]
+        if self.params is not None and len(params) == len(self.params) and all(a is b for a, b in zip(params, self.params)):
+            return
+        self.params = params
+        self.offsets, self.numel = flat_layout(params)
+        self.flat = None
 
     def _aliased(self):
         m = self.model
@@ -90,6 +110,7 @@ class GradSync:
     def __call__(self):
         if not dist.is_available() or not dist.is_initialized() or dist.get_world_size(self.group) == 1:
             return
+        self._refresh()
         flat = self._aliased()
         if flat is not None:
             dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=self.group)
@@ -100,6 +121,8 @@ class GradSync:
             if p.grad is None:                     # a rank whose shard is empty still takes part in the collective
                 p.grad = torch.zeros_like(p)
         grads = [p.grad for p in self.params]
+        if not grads:
+            return
         if self.flat is None or self.flat.device != grads[0].device:
             self.flat = torch.zeros(self.numel, dtype=grads[0].dtype, device=grads[0].device)      # the alignment gaps stay zero
         views = [self.flat[o:o + g.numel()].view_as(g) for o, g in zip(self.offsets, grads)]

@@ -55,8 +55,7 @@ class TrainStep:
         self.sync = None
         if self.world > 1:
             parallel.broadcast_parameters(model, 0, group)             # every rank starts from rank 0's weights
-            params = model.hot_parameters() if hasattr(model, "hot_parameters") else [p for p in model.parameters() if p.requires_grad]
-            self.sync = parallel.GradSync(params, group, model)
+            self.sync = parallel.GradSync(model.parameters(), group, model)     # the trainable ones, decided at every step
 
     # ---- host side ---------------------------------------------------------------------------
     def prepare(self, batch, smiles2graph_dic, pinned: bool = True, device_graphs: bool = False) -> PreparedBatch:

@@ -38,7 +38,7 @@ def _dp_shard(model, window, smiles2graph_dic):
         return window, None
     sync = getattr(model, "_dp_sync", None)
     if sync is None:
-        sync = model._dp_sync = parallel.GradSync(model.hot_parameters(), None, model)
+        sync = model._dp_sync = parallel.GradSync(model.parameters(), None, model)
     atoms = [smiles2graph_dic.parsing_smiles(w[1]).n_atoms - 1 for w in window]
     lo, hi = parallel.shard_groups(atoms, world)[rank]
     return window[lo:hi], sync

@@ -94,6 +94,30 @@ def load_checkpoint(path, allow_unsafe_pickle=None):
         return torch.load(path, map_location=loc, weights_only=False)
 
 
+def load_pretrained(model, path):
+    """Start fine-tuning from a pretrained checkpoint: copies every ``state_dict`` tensor of ``path`` whose name and shape match the
+    model's (read through ``load_checkpoint``, same ``weights_only`` policy) and records the copied names in ``model.pretrained_names``,
+    which ``freeze`` checks.  A different ``task_num`` or ``add_features_dim`` changes the shape of the last or the first FFN layer only,
+    so e.g. a model pretrained with 'mle' fine-tunes as 'evidential_ranking' with those layers left as initialised.  Returns the
+    ``(name, reason)`` pairs that were not copied."""
+    state = load_checkpoint(path)
+    src = state["state_dict"] if isinstance(state, dict) and "state_dict" in state else state
+    own = model.state_dict()
+    skipped, loaded = [], set()
+    with torch.no_grad():
+        for name, t in own.items():
+            if name not in src:
+                skipped.append((name, "not in the checkpoint"))
+            elif tuple(src[name].shape) != tuple(t.shape):
+                skipped.append((name, f"shape {tuple(src[name].shape)} in the checkpoint, {tuple(t.shape)} in the model"))
+            else:
+                t.copy_(src[name])
+                loaded.add(name)
+    skipped += [(name, "not in the model") for name in src if name not in own]
+    model.pretrained_names = getattr(model, "pretrained_names", set()) | loaded
+    return skipped
+
+
 def index_select_ND(source: torch.Tensor, index: torch.Tensor) -> torch.Tensor:
     """``source[index]`` with the reference's shape contract (utils.py:176-193): [R, h], [A, W] -> [A, W, h].
     The hot path never materialises this tensor (the gather kernels sum on the fly); kept for API parity."""
