@@ -285,13 +285,15 @@ typedef enum {
   RR_LOSS_RANKNET_ACC = 10,/* RankNet 'accelerate_grad' train_pairwise.py:123-137: same cost, dscore = the row sums only (half of autograd's) */
   RR_LOSS_LOGNORM = 11,   /* Lognorm           loss.py:165-184 (scores [N,2] = m, v, both positive; norm = N) */
   RR_LOSS_DIRICHLET_UQ = 12,/* Dirichlet_uq    loss.py:440-474 (1-D positive concentrations; `sigma` = annealing coefficient; norm = groups) */
-  RR_LOSS_NIG = 13        /* evidential_loss_new loss.py:402-437 as called at train_listwise.py:229-260: scores [N,4] = mu, v, alpha, beta
+  RR_LOSS_NIG = 13,       /* evidential_loss_new loss.py:402-437 as called at train_listwise.py:229-260: scores [N,4] = mu, v, alpha, beta
                              against EVERY target of the batch (the [N,1] x [N] broadcast); norm = N*N; `sigma` = lam; no seg_off */
+  RR_LOSS_LAMBDARANK = 14,/* LambdaRank: RankNet over each group's pairs t_i > t_j (each once), weighted by |dNDCG| of swapping them; norm = groups */
+  RR_LOSS_LAMBDARANK_TOP = 15 /* the same with the NDCG cut at K = max(1, round_half_even(n / 4)), the validation's NDCG@25% */
 } rr_loss_kind;
-/* norm: the divisor the reference applies (G, N or the window's ordered-pair count); sigma: RankNet */
+/* norm: the divisor the reference applies (G, N or the window's ordered-pair count); sigma: RankNet, LambdaRank */
 int rr_loss_fwdbwd(int kind, int N, int G, const float* scores, const float* targets, const int32_t* seg_off,
                    float norm, float sigma, float* loss, float* dscore, void* stream);
-/* The same with the size of the largest group given (the caller has `scope` on the host): ListMLE and RankNet keep a group in shared
+/* The same with the size of the largest group given (the caller has `scope` on the host): ListMLE, RankNet and LambdaRank keep a group in shared
  * memory and size it for max_group, up to rr_loss_max_group() = 8192 candidates.  rr_loss_fwdbwd assumes groups of at most 2048; a
  * group larger than the capacity yields NaN in loss and dscore, never a shared-memory overrun. */
 int rr_loss_fwdbwd_ex(int kind, int N, int G, const float* scores, const float* targets, const int32_t* seg_off, int max_group,

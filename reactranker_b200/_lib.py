@@ -24,6 +24,7 @@ RR_OUT_LD = 16
 FA_LD, FB_LD = 64, 88
 HEAD_RAW, HEAD_EVIDENTIAL_RANKING, HEAD_GAUSS_SOFTPLUS, HEAD_SOFTPLUS, HEAD_LOGNORM, HEAD_SOFTPLUS_P1, HEAD_NIG = range(7)
 LOSS_LISTMLE, LOSS_LISTNET, LOSS_EVIDENTIAL, LOSS_RANKNET, LOSS_GAUSS, LOSS_MSE, LOSS_EXPMSE, LOSS_LISTMLE_DIS, LOSS_LISTNET_DIS, LOSS_LISTNET_UQ, LOSS_RANKNET_ACC, LOSS_LOGNORM, LOSS_DIRICHLET_UQ, LOSS_NIG = range(14)
+LOSS_LAMBDARANK, LOSS_LAMBDARANK_TOP = 14, 15
 
 c_f32p = ctypes.c_void_p   # device pointers travel as plain integers
 

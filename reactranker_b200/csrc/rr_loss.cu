@@ -68,6 +68,29 @@ __device__ void block_scan(float* buf, float* tmp, int n) {
   __syncthreads();
 }
 
+// bitonic sort of (key, id)[0..P), P a power of two, descending by key with ties by ascending id; pad with key -inf and ids >= the
+// group size, and the padding sorts last.  Synchronises before and after.
+__device__ __forceinline__ void block_sort_desc(float* key, int* id, int P) {
+  for (int k = 2; k <= P; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      __syncthreads();
+      for (int i = threadIdx.x; i < P; i += blockDim.x) {
+        const int l = i ^ j;
+        if (l > i) {
+          const bool desc = (i & k) == 0;
+          const float ki = key[i], kl = key[l];
+          const int ii = id[i], il = id[l];
+          const bool i_first = (ki > kl) || (ki == kl && ii < il);  // i should precede l in descending order
+          if (desc ? !i_first : i_first) {
+            key[i] = kl; key[l] = ki;
+            id[i] = il; id[l] = ii;
+          }
+        }
+      }
+    }
+  __syncthreads();
+}
+
 // A block's share of the loss: added into loss[0] with an atomic, or (DET, deterministic mode) stored to loss[block], the partials that
 // k_sum_parts then adds in block order.  (A macro, not a function: the default kernels then compile exactly as they did before DET existed.)
 #define RR_PUT_LOSS(loss, v)                                          \
@@ -104,25 +127,8 @@ __global__ void __launch_bounds__(kLossThreads) k_listmle(const float* __restric
     key[i] = i < n ? targets[o + i] : -CUDART_INF_F;
     id[i] = i;
   }
-  // bitonic sort, descending by target (ties by index; torch.argsort leaves them unspecified)
-  for (int k = 2; k <= P; k <<= 1)
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      __syncthreads();
-      for (int i = threadIdx.x; i < P; i += blockDim.x) {
-        const int l = i ^ j;
-        if (l > i) {
-          const bool desc = (i & k) == 0;
-          const float ki = key[i], kl = key[l];
-          const int ii = id[i], il = id[l];
-          const bool i_first = (ki > kl) || (ki == kl && ii < il);  // i should precede l in descending order
-          if (desc ? !i_first : i_first) {
-            key[i] = kl; key[l] = ki;
-            id[i] = il; id[l] = ii;
-          }
-        }
-      }
-    }
-  __syncthreads();
+  // descending by target (ties by index; torch.argsort leaves them unspecified)
+  block_sort_desc(key, id, P);
   // x = scores sorted; reuse key[] for x
   float mx = -CUDART_INF_F;
   float vsum = 0.f;
@@ -477,6 +483,87 @@ __global__ void __launch_bounds__(kLossThreads) k_ranknet(const float* __restric
 }
 
 // ---------------------------------------------------------------------------------------
+// LambdaRank (Burges et al.): RankNet with each pair weighted by |dNDCG@K|, the change of the validation's NDCG (eval.py:460-472: gain
+// exp(t), discount 1 / log2(1 + rank)) if the two items swapped places.  Per group, with G_i = exp(t_i - max t) (the shift cancels in every
+// NDCG ratio), r_i the 1-based descending rank of s_i with ties by index (the rule of k_rank_metrics) and D(r) = 1 / log2(1 + r) for
+// r <= K, else 0:
+//   w_ij = |G_i - G_j| |D(r_i) - D(r_j)| / IDCG_K,    L = (1 / norm) sum_{t_i > t_j} w_ij softplus(-sigma (s_i - s_j))
+// (each unordered pair once).  w is constant in s, so dL/ds is RankNet's pair gradient times w.  K = n, or with TOP the K of the
+// validation's NDCG@25 %: max(1, round_half_even(n / 4)).  A group without an ordered pair adds 0 and gets a zero gradient.
+// ---------------------------------------------------------------------------------------
+template <bool TOP, bool DET>
+__global__ void __launch_bounds__(kLossThreads) k_lambdarank(const float* __restrict__ scores, const float* __restrict__ targets,
+                                                             const int* __restrict__ seg, float inv_norm, float sigma,
+                                                             float* __restrict__ loss, float* __restrict__ dscore, int cap) {
+  extern __shared__ float loss_dyn[];            // ss | gs | key | id, `cap` entries each (cap = a power of two >= the largest group)
+  float* ss = loss_dyn;
+  float* gs = loss_dyn + cap;
+  float* key = loss_dyn + 2 * cap;               // the sorts' keys, then D(r_i) by item
+  int* id = reinterpret_cast<int*>(loss_dyn + 3 * cap);
+  float* ts = loss_dyn + 3 * cap;                // id[]'s space, after the sorts: the targets
+  __shared__ float red[32];
+  const int o = seg[blockIdx.x], n = seg[blockIdx.x + 1] - o;
+  if (n <= 0) return;
+  if (n > cap) {   // as in k_listmle: NaN, never a shared-memory overrun
+    for (int i = threadIdx.x; i < n; i += blockDim.x) dscore[o + i] = CUDART_NAN_F;
+    if (threadIdx.x == 0) RR_PUT_LOSS(loss, CUDART_NAN_F);
+    return;
+  }
+  int P = 1;
+  while (P < n) P <<= 1;
+  const int K = TOP ? max(1, __float2int_rn(0.25f * static_cast<float>(n))) : n;    // n / 4 is exact in fp32; _rn rounds half to even
+  float mt = -CUDART_INF_F;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    ss[i] = scores[o + i];
+    mt = fmaxf(mt, targets[o + i]);
+  }
+  mt = block_max(mt, red);
+  for (int i = threadIdx.x; i < P; i += blockDim.x) {
+    const float g = i < n ? expf(targets[o + i] - mt) : -CUDART_INF_F;
+    if (i < n) gs[i] = g;
+    key[i] = g;
+    id[i] = i;
+  }
+  // IDCG_K from the gains in descending order
+  block_sort_desc(key, id, P);
+  float idcg = 0.f;
+  for (int k = threadIdx.x; k < K; k += blockDim.x) idcg += key[k] / log2f(2.f + static_cast<float>(k));
+  idcg = block_sum(idcg, red);                   // >= 1: the largest gain is exp(0) at rank 1
+  // D(r_i): sort the scores (ties by index: the stable rank) and scatter each position's discount to its item
+  for (int i = threadIdx.x; i < P; i += blockDim.x) {
+    key[i] = i < n ? ss[i] : -CUDART_INF_F;
+    id[i] = i;
+  }
+  block_sort_desc(key, id, P);
+  for (int k = threadIdx.x; k < n; k += blockDim.x) key[id[k]] = k < K ? 1.f / log2f(2.f + static_cast<float>(k)) : 0.f;
+  __syncthreads();
+  for (int i = threadIdx.x; i < n; i += blockDim.x) ts[i] = targets[o + i];
+  __syncthreads();
+  // The pair costs span many orders of magnitude (discounts of neighbouring deep ranks differ by ~1e-6): a thread's fp32 running sum of
+  // ~n^2 / 512 of them would drop those below its half ulp and come out 3e-5 low at n = 8192, so it is kept in double.  The per-item
+  // gradient sums n terms and stays in fp32.
+  double part = 0.0;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    const float si = ss[i], ti = ts[i], gi = gs[i], di = key[i];
+    float g = 0.f;
+    for (int j = 0; j < n; ++j) {
+      const float d = sigma * (si - ss[j]);
+      const float tj = ts[j];
+      const float w = fabsf(gi - gs[j]) * fabsf(di - key[j]);
+      if (ti > tj) {          // i should rank above j: C = w log(1 + exp(-sigma (s_i - s_j)))
+        part += static_cast<double>(w * softplus_f(-d));
+        g -= w * sigmoid_f(-d);
+      } else if (ti < tj) {   // j should rank above i: the same pair seen from its lower item, gradient only
+        g += w * sigmoid_f(d);
+      }
+    }
+    dscore[o + i] = sigma * g * inv_norm / idcg;
+  }
+  const float total = block_sum(static_cast<float>(part), red);
+  if (threadIdx.x == 0) RR_PUT_LOSS(loss, total * inv_norm / idcg);
+}
+
+// ---------------------------------------------------------------------------------------
 // pointwise: GaussDisLoss (loss.py:144-162), nn.MSELoss (train_listwise.py:166-167), the 'regression_exploss' key (276-281)
 // ---------------------------------------------------------------------------------------
 template <bool DET>
@@ -539,7 +626,7 @@ static int loss_launch(int kind, int N, int G, const float* scores, const float*
   RR_REQUIRE(N > 0 && scores && targets && loss && dscore, "loss: NULL argument or N <= 0");
   RR_REQUIRE(norm > 0.f, "loss: norm must be positive (got %g)", norm);
   RR_REQUIRE(max_group <= kMaxGroup, "loss: groups of up to %d candidates are supported (max_group %d)", kMaxGroup, max_group);
-  // capacity of the per-group shared arrays of ListMLE / RankNet: the next power of two >= max_group (the bitonic sort pads to it);
+  // capacity of the per-group shared arrays of ListMLE / RankNet / LambdaRank: the next power of two >= max_group (the bitonic sort pads to it);
   // without a hint (max_group <= 0) kDefaultGroupCap.  A group larger than the capacity yields NaN, never an overrun.
   int cap = kDefaultGroupCap;
   if (max_group > 0) {
@@ -579,6 +666,8 @@ static int loss_launch(int kind, int N, int G, const float* scores, const float*
     case RR_LOSS_LISTNET_UQ:
     case RR_LOSS_RANKNET_ACC:
     case RR_LOSS_DIRICHLET_UQ:
+    case RR_LOSS_LAMBDARANK:
+    case RR_LOSS_LAMBDARANK_TOP:
       RR_REQUIRE(G > 0 && seg_off, "loss: segmented kinds need seg_off and G > 0");
       {
         static PerDeviceOnce attr_set;           // up to 128 KB of dynamic shared memory for groups of up to kMaxGroup candidates
@@ -586,6 +675,8 @@ static int loss_launch(int kind, int N, int G, const float* scores, const float*
           RR_CUDA(cudaFuncSetAttribute(k_listmle<false, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
           RR_CUDA(cudaFuncSetAttribute(k_listmle<true, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
           RR_CUDA(cudaFuncSetAttribute(k_ranknet<DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * kMaxGroup * static_cast<int>(sizeof(float))));
+          RR_CUDA(cudaFuncSetAttribute(k_lambdarank<false, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
+          RR_CUDA(cudaFuncSetAttribute(k_lambdarank<true, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * kMaxGroup * static_cast<int>(sizeof(float))));
           attr_set.mark();
         }
       }
@@ -596,6 +687,8 @@ static int loss_launch(int kind, int N, int G, const float* scores, const float*
       else if (kind == RR_LOSS_EVIDENTIAL) k_evidential<DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, out, dscore);
       else if (kind == RR_LOSS_DIRICHLET_UQ) k_dirichlet_uq<DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, sigma, out, dscore);
       else if (kind == RR_LOSS_LISTNET_UQ) k_listnet_uq<DET><<<G, kLossThreads, 0, s>>>(scores, targets, seg_off, inv, sigma, out, dscore);
+      else if (kind == RR_LOSS_LAMBDARANK) k_lambdarank<false, DET><<<G, kLossThreads, 4 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, sigma, out, dscore, cap);
+      else if (kind == RR_LOSS_LAMBDARANK_TOP) k_lambdarank<true, DET><<<G, kLossThreads, 4 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, sigma, out, dscore, cap);
       else k_ranknet<DET><<<G, kLossThreads, 2 * cap * sizeof(float), s>>>(scores, targets, seg_off, inv, sigma, kind == RR_LOSS_RANKNET_ACC ? 1.f : 2.f, out, dscore, cap);
       break;
     case RR_LOSS_NIG: {            // norm = N * N (the reference's mean over the broadcast matrix); `sigma` carries lam

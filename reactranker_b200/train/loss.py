@@ -11,7 +11,8 @@ like the reference, the others a 0-d tensor.
 Every task key the reference can run is dispatched by ``train()`` (train_listwise.batch_loss): the five north-star keys, the composite
 keys that are sums of their terms, the distribution-valued ``MLEDisLoss`` / ``Listnet_For_Gauss``, ``Listnet_with_uq``, ``Dirichlet_uq``,
 ``Lognorm`` and the NIG ``evidential_loss_new``.  Only the two losses no task key constructs (``Listnetlognorm``,
-``Listnet_For_evidential``) raise.
+``Listnet_For_evidential``) raise.  ``LambdaRankLoss`` (keys ``lambdarank`` / ``lambdarank_top``) is this project's own, not the
+reference's: it trains for the validation's NDCG.
 """
 from __future__ import annotations
 
@@ -148,6 +149,22 @@ class MLEloss(_DPNorm):
 
     def forward(self, score, scope, targets_train, gpu: int):
         return _segmented(_lib.LOSS_LISTMLE, score, scope, targets_train, gpu, norm=self._norm(len(scope)), out_shape=(1,), check_max=True)
+
+
+class LambdaRankLoss(_DPNorm):
+    """LambdaRank (Burges et al.), this project's own key: RankNet over each group's pairs ``t_i > t_j`` (each once), every pair weighted
+    by ``|dNDCG@K|``, the change of the validation's NDCG (gain ``exp(t)``, discount ``1 / log2(1 + rank)``) if the two items swapped
+    places at the current scores; the sum over groups divided by the number of groups.  ``top=False``: ``K = n``; ``top=True``: the
+    ``K = max(1, round(n / 4))`` of NDCG@25%.  The weights are constants of the scores, so the gradient is RankNet's pair gradient times
+    the weight.  Returns shape [1]."""
+
+    def __init__(self, sigma: float = 1.0, top: bool = False, global_norm=None):
+        super().__init__(global_norm)
+        self.sigma, self.top = float(sigma), bool(top)
+
+    def forward(self, score, scope, targets, gpu: int):
+        kind = _lib.LOSS_LAMBDARANK_TOP if self.top else _lib.LOSS_LAMBDARANK
+        return _segmented(kind, score, scope, targets, gpu, norm=self._norm(len(scope)), out_shape=(1,), sigma=self.sigma, check_max=True)
 
 
 class ListnetLoss(_DPNorm):

@@ -3,7 +3,7 @@ dispatch, optimiser stepping and per-epoch checkpointing (train/train_listwise.p
 
 Differences, all on purpose:
 * every task key the reference can run is dispatched (``batch_loss``); only ``mle_dirichlet``, which cannot run in the reference
-  either, raises ``NotImplementedError``;
+  either, raises ``NotImplementedError``; ``lambdarank`` / ``lambdarank_top`` are keys of this project alone;
 * launched under ``torchrun`` (WORLD_SIZE > 1) the same call trains data-parallel: every rank plans the same global batches and takes
   its shard of whole reactant groups (train/step.py, parallel.py); rank 0 validates, checkpoints and prints;
 * the reference copies ``encoder.W_i.weight`` to the host EVERY step to look for NaNs (train_listwise.py:190-195); here the
@@ -29,8 +29,8 @@ from ..data.load_reactions import DataProcessor
 from ..utils import load_train_state, save_checkpoint, save_train_state
 from .eval import calculate_mse, ranking_metrics
 from .step import TrainStep
-from .loss import (Dirichlet_uq, ExpMSELoss, GaussDisLoss, Listnet_For_Gauss, Listnet_with_uq, ListnetLoss, Lognorm, MLEDisLoss, MLEloss,
-                   MSELoss, evidential_loss_new, evidential_ranking)
+from .loss import (Dirichlet_uq, ExpMSELoss, GaussDisLoss, LambdaRankLoss, Listnet_For_Gauss, Listnet_with_uq, ListnetLoss, Lognorm, MLEDisLoss,
+                   MLEloss, MSELoss, evidential_loss_new, evidential_ranking)
 
 try:  # only used as the default value of ``writer`` in the reference signature
     from torch.utils.tensorboard import SummaryWriter
@@ -43,7 +43,9 @@ BUILT_TASKS = ("mle", "listnet", "evidential_ranking", "gauss_regression",
                # distribution-valued ListMLE / ListNet (loss.py:102-141, 233-272) + the Gaussian NLL (196-203, 211-215)
                "mledis_gaussian", "listnetdis_gauss", "listnet_uq",
                # the remaining experimental keys (215-219, 229-260, 269-270)
-               "listnetdis_lognorm", "dirichlet_uq", "evidential", "mle_evidential", "mledis_evidential", "listnet_evidential")
+               "listnetdis_lognorm", "dirichlet_uq", "evidential", "mle_evidential", "mledis_evidential", "listnet_evidential",
+               # this project's own: LambdaRank, trained for the validation's NDCG@all / NDCG@25% (loss.LambdaRankLoss)
+               "lambdarank", "lambdarank_top")
 # 'mle_dirichlet' cannot run in the reference either: no branch of train_listwise.py:128-167 constructs ``dirichlet_loss`` for it and the
 # call at 267-268 passes four arguments to a seven-argument forward.
 UNBUILT_TASKS = ("mle_dirichlet",)
@@ -91,6 +93,8 @@ def batch_loss(task_type, output, scope, targets, gpu, max_coeff=0.0001, epoch=0
         variance = betas / (lambdas * (alphas - 1))
         rank = MLEDisLoss() if task_type == 'mledis_evidential' else Listnet_For_Gauss()
         return rank(mu, variance, scope, targets, gpu) + evidential_loss_new(mu, lambdas, alphas, betas, targets, gpu, lam=0.1)
+    if task_type in ('lambdarank', 'lambdarank_top'):    # not keys of the reference, whose fall-through below they would otherwise take
+        return LambdaRankLoss(top=task_type == 'lambdarank_top')(output, scope, targets, gpu)
     return MSELoss()(output, targets)
 
 
